@@ -4,6 +4,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W                           # N ranks, frame-sharded, no collective
     python bench.py --impl reference --steps K --warmup W                # the reference algorithm on the host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR              # + what the last timed step returned, as DIR/*.npy
 
 A step = one pass of the hot path over one batch of 8 synthetic KITTI-shaped frames per GPU (BASELINE.json
 configs[1]): P = 120 000 points, FPN maps (256,104,336)/(256,52,168)/(256,26,84), grid 352x400x10, T = 35.
@@ -31,6 +32,45 @@ METRIC = 'frames/sec voxelize+fuse+VFE+scatter'
 WORKLOAD = ('configs[1]: batch-8 synthetic KITTI-shaped frames per GPU (P=120000 pts/frame, FPN maps '
             '256x{104x336,52x168,26x84} fp32, grid 352x400x10, T=35): voxelize + project + 4-corner gather + '
             '8-layer fusion/VFE stack (fp32) + dense (128,10,352,400) grid')
+# --dump-outputs budget (< 64 MB): 16 MB of uniformly sampled grid values (98 % of the cells are empty: this catches writes
+# outside the voxels) + up to 8 frames x 8192 voxel rows x (128 features + 4 coordinates) = 36 MB from the occupied cells
+DUMP_GRID_SAMPLES = 1 << 22
+DUMP_VOXEL_ROWS = 8192
+
+
+def grid_sample_index(numel: int) -> np.ndarray:
+    """Flat indices into the (B,128,nz,nx,ny) grid whose values --dump-outputs writes (sorted, drawn with replacement). They
+    depend on the seed and the grid size only, so two builds of the project are compared at the same elements."""
+    return np.sort(np.random.default_rng(0).integers(0, numel, min(DUMP_GRID_SAMPLES, numel), dtype=np.int64))
+
+
+def voxel_sample_rows(f: int, n: int) -> np.ndarray:
+    """Rows of frame f's (n,128) voxel features that --dump-outputs writes: all of them up to DUMP_VOXEL_ROWS, else a sorted
+    sample drawn from a seed that depends on f only (builds with equal voxel counts are compared at the same voxels)."""
+    if n <= DUMP_VOXEL_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(f).choice(n, DUMP_VOXEL_ROWS, replace=False))
+
+
+def dump_outputs(out_dir: str, path, grid, counts):
+    """Writes what one step of the timed path returned, for output-for-output comparison of two builds:
+    counts.npy         (B,4) float64, the int32 per-frame counts (voxels, kept rows, invalid points, max points in one voxel)
+    grid_sample.npy    (n,) float32, the grid at the flat indices of grid_sample_index(grid.numel())
+    voxel_features.npy (m,128) float32, rows voxel_sample_rows(f, N_f) of path.voxel_features(f), frame after frame
+    voxel_index.npy    (m,4) float64, their [frame, ix, iy, iz]"""
+    import torch
+    idx = torch.from_numpy(grid_sample_index(grid.numel())).to(grid.device)
+    feats, coords = [], []
+    for f in range(counts.shape[0]):
+        vfeat, vidx = path.voxel_features(f)
+        rows = torch.from_numpy(voxel_sample_rows(f, vfeat.shape[0])).to(vfeat.device)
+        feats.append(vfeat[rows].cpu())
+        coords.append(vidx[rows].cpu())
+    arrays = dict(counts=counts.cpu().numpy().astype(np.float64), grid_sample=grid.reshape(-1)[idx].cpu().numpy(),
+                  voxel_features=torch.cat(feats).numpy(), voxel_index=torch.cat(coords).numpy().astype(np.float64))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def static_config(world: int, dense: bool = False):
@@ -226,12 +266,9 @@ def run_reference(args):
     from oracle import pointpath_oracle as O
     O.build_c_oracle() if not os.path.exists(os.path.join(ROOT, 'oracle', '_build', 'libvoxel_oracle.so')) else None
     threads = os.cpu_count() or 1
-    budget = 240.0
-    t_first, _ = cpu_reference_frame(0, threads)            # warm-up step 1 (also sizes the run)
-    steps = max(1, min(args.steps, int(budget / max(t_first, 1e-3)) - 1))
-    warm = max(0, min(args.warmup - 1, int((budget - steps * t_first) / max(t_first, 1e-3)) - 1))
-    for w in range(warm):
-        cpu_reference_frame(1 + w, threads)
+    steps = args.steps
+    for w in range(args.warmup):
+        cpu_reference_frame(w, threads)
     times, stages_acc = [], {}
     for s in range(steps):
         t, st = cpu_reference_frame(100 + s, threads)
@@ -241,9 +278,8 @@ def run_reference(args):
     total = sum(times)
     fps = steps / total
     sample = (f'each step = ONE full-size frame (1 of the 8 frames of the batch, P={POINTS}) through the numpy/torch-CPU port of '
-              f'the reference path (oracle/pointpath_oracle.py), {threads} torch threads; {steps} of {args.steps} requested steps '
-              f'(time-bounded to ~{int(budget)} s)')
-    line = dict(impl='reference', metric=METRIC, value=fps, unit='frames/s', n_gpus=args.gpus, steps=steps, warmup=warm + 1,
+              f'the reference path (oracle/pointpath_oracle.py), {threads} torch threads')
+    line = dict(impl='reference', metric=METRIC, value=fps, unit='frames/s', n_gpus=args.gpus, steps=steps, warmup=args.warmup,
                 ms_per_step=1e3 * total / steps, higher_is_better=True, scaling='weak', vs_baseline=None, dtype='f32',
                 data='synthetic', config=static_config(int(os.environ.get('WORLD_SIZE', str(args.gpus)))),
                 cpu_baseline=dict(value=fps, unit='frames/s', cores=threads, kind='port', sample=sample,
@@ -336,7 +372,7 @@ def run_ours(args):
         sampler.begin()
     e0.record()
     for _ in range(args.steps):
-        step()
+        out = step()
     e1.record()
     barrier()
     if sampler:
@@ -344,6 +380,8 @@ def run_ours(args):
     ms_total = e0.elapsed_time(e1)
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:     # before the passes below overwrite the outputs of the last timed step
+        dump_outputs(args.dump_outputs, path, *out)
     # per-stage pass (outside the timed region): CUDA events around every stage on the stream it runs on, with the map
     # branch serialised behind the point branch (fusion mode 2) so that a stage's time is its own and not the time it
     # spent sharing the SMs with the other branch; `value` above is the default, overlapped schedule
@@ -639,7 +677,14 @@ def main():
     ap.add_argument('--host-chunk', type=int, default=2, help='frames per sub-batch of the host-buffer (e2e) leg')
     ap.add_argument('--dtype', default='f32', choices=['f32', 'bf16'],
                     help="'bf16' = reduced-precision mode of the layer stack (tolerance stated separately: tests/test_gpu_parity.py); not the headline line")
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one returned as DIR/*.npy: the counts, and fixed, seeded '
+                         'samples of the grid and of the voxel features (see dump_outputs); forward and dense workloads of --impl ours')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and (args.impl != 'ours' or args.workload == 'train'):
+        ap.error('--dump-outputs applies to the forward and dense workloads of --impl ours')
     refuse_debug_env()
     if args.impl == 'reference':
         run_reference(args)

@@ -22,6 +22,11 @@ def sha(*arrays):
     return h.hexdigest()
 
 
+def rel_err(a, ref):
+    a, ref = torch.as_tensor(a).double(), torch.as_tensor(ref).double()
+    return float((a - ref).abs().max() / ref.abs().max())
+
+
 def small_maps(seed, shapes=((13, 42), (7, 21), (4, 11))):
     rng = np.random.default_rng(seed)
     return [rng.standard_normal((1, 256, h, w), dtype=np.float32) for (h, w) in shapes]
@@ -61,9 +66,17 @@ def test_path_oracle_matches_reference_golden(golden_dir, tag):
     im768 = r['im768'].reshape(-1, 768)
     assert np.array_equal(im768[g['im768_rows']].numpy(), g['im768_sample'])
     np.testing.assert_allclose(im768.double().sum(0).numpy(), g['im768_colsum'], rtol=1e-12)
-    # same torch build, same ops: expect bit-equality; tolerate accumulation-order noise only
-    np.testing.assert_allclose(r['im16'].numpy(), g['im16'], rtol=1e-5, atol=1e-5)
-    np.testing.assert_allclose(r['vfeat'].numpy(), g['vfeat'], rtol=1e-5, atol=1e-5)
+    # Tolerate accumulation-order noise only. The fp32 evaluation is bit-equal to the golden on the CPU that wrote it, but the
+    # BLAS picks its kernels (and so its summation order) by CPU, and the batch-statistic BatchNorms amplify that: on another
+    # x86 host the fp32 im16 / vfeat differ from the golden by up to 1.0e-4 / 4.6e-4 of max (fp32 vs fp64 there: 0.5-1.3e-4).
+    # The fp64 evaluation is the same on every CPU. Both fp32 evaluations, the reference's and this CPU's, must lie within the
+    # 5e-4 that bounds fp32 against fp32 in tests/test_gpu_parity.py (the golden: 1.1-3.5e-4; a 1 % change of any one bias: > 6e-4)
+    with torch.no_grad():
+        r64 = O.forward_frame(g['pcd4'], synth.kitti_calib(), maps, sd, G, synth.KITTI_IMSIZE_HW, dtype=torch.float64)
+    for k in ('im16', 'vfeat'):
+        assert rel_err(g[k], r64[k]) < 5e-4 and rel_err(r[k], r64[k]) < 5e-4, (k, rel_err(g[k], r64[k]), rel_err(r[k], r64[k]))
+    if np.array_equal(r['im16'].numpy(), g['im16']):     # this CPU sums like the one that wrote the golden: exact from here on
+        assert np.array_equal(r['vfeat'].numpy(), g['vfeat'])
     grid = r['grid'].numpy()
     assert tuple(grid.shape) == tuple(g['grid_shape'])
     assert int((grid != 0).sum()) == int(g['grid_nonzero'])
