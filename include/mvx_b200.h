@@ -261,6 +261,19 @@ int mvx_cml_conv1_workspace_bytes(const mvx_pointpath_args_t *args, size_t *byte
 int mvx_cml_conv1_sparse(const mvx_pointpath_args_t *args, const float *conv_w, const float *conv_b, double eps, float *out,
                          void *ws, size_t ws_bytes);
 
+/* Training through the hand-off: the backward of mvx_cml_conv1_sparse, i.e. of CRB3d (voxelnet/Pipe.py:31-43, Blocks.py
+ * CRB3d: relu, Conv3d(128, 64, 3, (2,1,1), (1,1,1)), BatchNorm3d with batch statistics) with respect to conv_w, conv_b and
+ * the voxel features the layer read. Call after mvx_cml_conv1_sparse with the SAME args, conv_w, conv_b, eps and the same
+ * untouched ws (read only here); the path workspace of that forward must still hold its voxel features.
+ * d_out (B, 64, (nz+1)/2, nx, ny) fp32 = dLoss/d out. d_w (64,128,3,3,3) and d_b (64) receive the gradients summed over the
+ * frames (accumulate != 0: added to their contents). d_vfeat (B, cap, 128) receives dLoss/d voxel features for rows
+ * 0 .. N_f-1 of every frame (other rows untouched), the input of mvx_pointpath_backward; NULL skips that product.
+ * bws: mvx_cml_conv1_backward_workspace_bytes() of scratch. */
+int mvx_cml_conv1_backward_workspace_bytes(const mvx_pointpath_args_t *args, size_t *bytes);
+int mvx_cml_conv1_sparse_backward(const mvx_pointpath_args_t *args, const float *conv_w, const float *conv_b, double eps,
+                                  const float *d_out, float *d_vfeat, float *d_w, float *d_b, int32_t accumulate,
+                                  const void *ws, size_t ws_bytes, void *bws, size_t bws_bytes);
+
 /* ------------------------------------------------------------------------------------------------
  * Label side of the same native extension (SURVEY.md §8f rank 3).
  *

@@ -25,14 +25,14 @@ constexpr int kCinTrue[MVX_NUM_LAYERS] = {768, 768, 128, 128, 16, 23, 32, 128};
 
 struct RowSet {            // which rows of a frame a kernel walks
     const int *counts;     // [B][4]
-    int mode;              // 1: K_f + 1 rows (frame pad row last), 2: K_f + N_f rows (one pad row per voxel)
+    int mode;              // 1: K_f + 1 rows (frame pad row last), 2: K_f + N_f rows (one pad row per voxel), 3: N_f rows (one per voxel)
     int rowcap;            // frame stride in rows
     const float *row_w;    // [B][rowcap] BatchNorm multiplicity
     int T;
 };
 __device__ __forceinline__ int rows_of(const RowSet &rs, int f) {
     const int N = rs.counts[f * 4 + 0], K = rs.counts[f * 4 + 1];
-    return rs.mode == 1 ? K + 1 : K + N;
+    return rs.mode == 1 ? K + 1 : (rs.mode == 3 ? N : K + N);
 }
 
 struct BnArgs {
@@ -564,6 +564,16 @@ int launch_dw_auto(const DwArgs &a, int B, cudaStream_t st) {
     set_error("dw_gemm: unsupported layer shape %d x %d", a.Cout, a.Cin);
     return MVX_EINVAL;
 }
+
+}  // namespace
+
+int launch_dw_voxel_rows(const float *D, int Cout, const float *X, int Cin, const int *counts, int rowcap, const int *dmax, float *dW, int B,
+                         cudaStream_t st) {
+    const DwArgs dw{D, X, Cin, Cin, Cin, Cout, nullptr, 0.0, dW, 0, RowSet{counts, 3, rowcap, nullptr, 1}, dmax, nullptr};
+    return launch_dw_auto(dw, B, st);
+}
+
+namespace {
 
 // ---- W (Cout, CinPad) row-major from the stored W^T (CinPad, Cout) -------------------------------------------
 __global__ void __launch_bounds__(256) transpose_w_kernel(const float *__restrict__ wt, float *__restrict__ w, int Cin, int Cout) {

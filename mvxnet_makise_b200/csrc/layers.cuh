@@ -108,6 +108,12 @@ void set_tc_persistent(int on);  // 0 = one 256 x BN tile per CTA (default), 1 =
 int gemm_mode();
 int launch_layer_auto(const LayerArgs &a, int F, float *wpack, cudaStream_t st);
 
+// dW (Cout, Cin) += sum over the frames and their N_f voxel rows r of D[f][r]^T X[f][r] (backward.cu): rows of weight 1, X used
+// as stored (no BatchNorm on load, |x| = O(1)); D [B][rowcap][Cout], X [B][rowcap][Cin]; dmax [B][Cout] bounds |D| per column
+// (float bits) for the power-of-two scales of the tensor-core kernel
+int launch_dw_voxel_rows(const float *D, int Cout, const float *X, int Cin, const int *counts, int rowcap, const int *dmax, float *dW, int B,
+                         cudaStream_t st);
+
 // number of rows BN statistics are taken over for frame f: N_f * T (fused path) or rows_fixed (dense API)
 struct NormSrc {
     const double *stats;   // [F][C][2]

@@ -1361,7 +1361,8 @@ bool tc_persistent_enabled() { return g_tc_persistent != 0; }
 void set_tc_persistent(int on) { g_tc_persistent = on; }
 
 bool tc_layer_eligible(const LayerArgs &a) {
-    return a.Cin % kBK == 0 && a.Cin <= 768 && a.Cout % 128 == 0 && a.ldx % 4 == 0 &&
+    // the 768 bound sizes the shared BatchNorm tables of the input: a plain product without them may be deeper
+    return a.Cin % kBK == 0 && (a.Cin <= 768 || (a.plain && !a.in_stats)) && a.Cout % 128 == 0 && a.ldx % 4 == 0 &&
            (a.Y == nullptr || a.ldy % 4 == 0);
 }
 

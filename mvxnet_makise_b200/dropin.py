@@ -96,6 +96,68 @@ def hot_path(path: PointPath, voxels, idx, maps, params: Sequence[torch.Tensor])
     return grid
 
 
+class SparseConv1Function(torch.autograd.Function):
+    """y1 = backbone.cml.conv1(hot_path(voxels, idx, fpn maps; 16 parameters)) without the dense grid: the sparse hand-off
+    (`PointPath.cml_conv1`) reads the voxel features directly. Differentiable with respect to the 16 hot-path parameters and
+    the conv1 weight / bias. `train` says whether a hot parameter wants a gradient: without one the path forward runs in
+    inference mode and the backward skips d_vfeat and the path backward (fine-tuning of the CML alone)."""
+
+    @staticmethod
+    def forward(ctx, path: PointPath, eps: float, train: bool, voxels, idx, maps, *params):
+        hot, weight, bias = params[:-2], params[-2], params[-1]
+        _push_parameters(path, hot)
+        path.forward_voxels(voxels, idx, maps, want_grid=False, train=train)
+        y1 = path.cml_conv1(weight, bias, eps)
+        ctx.path, ctx.eps, ctx.train = path, eps, train
+        ctx.call_id = path._train_call = getattr(path, '_train_call', 0) + 1
+        ctx.save_for_backward(weight, bias)
+        return y1
+
+    @staticmethod
+    def backward(ctx, d_y1):
+        path = ctx.path
+        if path._train_call != ctx.call_id:
+            raise RuntimeError('the hot path ran another training forward before this backward: its saved activations are gone '
+                               '(one forward/backward at a time per accelerated model)')
+        weight, bias = ctx.saved_tensors
+        d_vfeat, d_w, d_b = path.cml_conv1_backward(d_y1.contiguous(), weight, bias, ctx.eps, want_d_vfeat=ctx.train)
+        grads = [None] * (2 * len(_HOT))
+        if ctx.train:
+            flat = torch.empty(sum(int(np.prod(s)) for _, _, s in PointPath.grad_layout()), dtype=torch.float32, device=path.device)
+            path.backward(d_vfeat=d_vfeat, grad_flat=flat, accumulate=False)
+            grads = [flat[o:o + int(np.prod(shape))].view(*shape) for _, o, shape in PointPath.grad_layout()]
+        return (None, None, None, None, None, None, *grads, d_w, d_b)
+
+
+def sparse_conv1(path: PointPath, voxels, idx, maps, params: Sequence[torch.Tensor], weight, bias, eps: float) -> torch.Tensor:
+    """`backbone.cml.conv1` of the grid `hot_path` would return, (B, 64, (nz+1)//2, nx, ny), computed without that grid. Records an
+    autograd node when gradients are enabled and any of the 18 tensors wants one."""
+    maps = [m.detach().to(torch.float32).contiguous() for m in maps]
+    train = any(p.requires_grad for p in params)
+    if torch.is_grad_enabled() and (train or weight.requires_grad or bias.requires_grad):
+        return SparseConv1Function.apply(path, eps, train, voxels, idx, maps, *params, weight, bias)
+    _push_parameters(path, params)
+    path.forward_voxels(voxels, idx, maps, want_grid=False, train=False)
+    return path.cml_conv1(weight, bias, eps)
+
+
+def _stock_conv1_eps(cml) -> float:
+    """`cml.conv1` must be the stock CRB3d(128, 64, 3, (2,1,1), (1,1,1)) (voxelnet/Pipe.py:31-43, Blocks.py CRB3d): Conv3d with
+    bias, ReLU, BatchNorm3d(affine=False, track_running_stats=False). Returns that BatchNorm's eps; raises otherwise."""
+    block = cml.conv1
+    conv = getattr(block, 'conv', None)
+    bns = [m for m in block.modules() if isinstance(m, torch.nn.modules.batchnorm._BatchNorm)]
+    ok = (isinstance(conv, torch.nn.Conv3d) and conv.in_channels == 128 and conv.out_channels == 64 and conv.kernel_size == (3, 3, 3)
+          and conv.stride == (2, 1, 1) and conv.padding == (1, 1, 1) and conv.dilation == (1, 1, 1) and conv.groups == 1
+          and conv.bias is not None and conv.padding_mode == 'zeros'
+          and len(bns) == 1 and isinstance(bns[0], torch.nn.BatchNorm3d) and not bns[0].affine and not bns[0].track_running_stats
+          and sum(1 for m in block.modules() if isinstance(m, torch.nn.Conv3d)) == 1)
+    if not ok:
+        raise ValueError('sparse_cml_conv1=True needs the stock backbone.cml.conv1: CRB3d(128, 64, 3, (2,1,1), (1,1,1)) = Conv3d with '
+                         'bias, ReLU, BatchNorm3d(affine=False, track_running_stats=False)')
+    return float(bns[0].eps)
+
+
 def _forward(self, voxels, imgs, idx, calibs, imsize):
     """`MVXNet.forward(voxels, imgs, idx, calibs, imsize)` (MVXNet.py:21-27): same arguments, same (score, reg) result.
     `calibs` is accepted and unused, as in the reference's featureMaping (the projection already sits in voxels[..., 7:9])."""
@@ -106,8 +168,14 @@ def _forward(self, voxels, imgs, idx, calibs, imsize):
         self._mvx_imsize[id(imsize)] = hw
     path.imsize_hw = hw
     feats = self.head.extractor(imgs)                # FPN levels '0','1','2' (Pipe.py:17-21), frozen
-    grid = hot_path(path, voxels, idx.to(torch.int64), feats, hot_parameters(self))
     nx, ny = path.grid.shape[0], path.grid.shape[1]
+    if self._mvx_sparse_conv1:                       # CML.forward (voxelnet/Pipe.py:31-43) with conv1 taken from the voxel features
+        cml = self.backbone.cml
+        y1 = sparse_conv1(path, voxels, idx.to(torch.int64), feats, hot_parameters(self), cml.conv1.conv.weight, cml.conv1.conv.bias,
+                          self._mvx_conv1_eps)
+        outs = [self.backbone.rpn(cml.conv3(cml.conv2(y1[b:b + 1])).reshape((1, -1, nx, ny))) for b in range(y1.shape[0])]
+        return outs[0] if len(outs) == 1 else outs
+    grid = hot_path(path, voxels, idx.to(torch.int64), feats, hot_parameters(self))
     outs = []
     for b in range(grid.shape[0]):                   # CML / RPN are batch-1 in the reference (VoxelNet.py:35-37)
         x = self.backbone.cml(grid[b:b + 1])
@@ -115,16 +183,24 @@ def _forward(self, voxels, imgs, idx, calibs, imsize):
     return outs[0] if len(outs) == 1 else outs
 
 
-def accelerate(model, grid: synth.GridSpec = synth.KITTI_GRID, imsize_hw: Sequence[int] = synth.KITTI_IMSIZE_HW, eps: float = 1e-6):
+def accelerate(model, grid: synth.GridSpec = synth.KITTI_GRID, imsize_hw: Sequence[int] = synth.KITTI_IMSIZE_HW, eps: float = 1e-6,
+               sparse_cml_conv1: bool = False):
     """Swap the hot path of a reference `MVXNet` instance (already on its CUDA device) for the fused sm_100a path, in place.
-    `grid` / `eps` mirror config.yml (velorange, voxelshape, samplenum; eps 1e-6 with half: False). Returns the model."""
+    `grid` / `eps` mirror config.yml (velorange, voxelshape, samplenum; eps 1e-6 with half: False). Returns the model.
+
+    sparse_cml_conv1=True also computes `backbone.cml.conv1` sparsely from the voxel features, forward and backward, so the
+    dense (B,128,nz,nx,ny) grid is never written; conv2 / conv3 and the RPN remain the model's own modules. Opt-in because a
+    caller can tell the difference: `backbone.cml` and `cml.conv1` are not called as modules (their hooks do not fire) and
+    no grid tensor exists. conv1 must be the stock block (ValueError otherwise)."""
     params = hot_parameters(model)                   # raises AttributeError if this is not the reference's module tree
+    conv1_eps = _stock_conv1_eps(model.backbone.cml) if sparse_cml_conv1 else None
     dev = params[0].device
     if dev.type != 'cuda':
         raise RuntimeError('accelerate() needs the model on a CUDA device; mvxnet_makise_b200 has no CPU fallback')
     sd = {name + suffix: _get(model, name + suffix).detach() for name in _HOT for suffix in ('.weight', '.bias')}
     model._mvx_path = PointPath(sd, grid, imsize_hw, eps, device=dev)
     model._mvx_imsize = {}
+    model._mvx_sparse_conv1, model._mvx_conv1_eps = bool(sparse_cml_conv1), conv1_eps
     model.forward = types.MethodType(_forward, model)
     return model
 

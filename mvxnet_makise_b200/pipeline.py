@@ -194,6 +194,7 @@ class PointPath:
         a.counts = self.counts.data_ptr()
         a.workspace, a.workspace_bytes = self._ws.data_ptr(), self._ws.numel()
         a.stream = torch.cuda.current_stream().cuda_stream
+        self._fwd_call = getattr(self, '_fwd_call', 0) + 1
         if train:
             check(lib.mvx_pointpath_forward_train(ctypes.byref(a)), 'pointpath_forward_train')
             self._train_args = (a, off, points, calib32, maps, point_calib, calib64, calib_f64)      # kept alive for backward()
@@ -258,6 +259,7 @@ class PointPath:
         a.workspace, a.workspace_bytes = self._ws.data_ptr(), self._ws.numel()
         a.stream = torch.cuda.current_stream().cuda_stream
         keep = (a, voff_c, vcat, icat, maps)
+        self._fwd_call = getattr(self, '_fwd_call', 0) + 1
         if train:
             check(lib.mvx_pointpath_forward_train(ctypes.byref(a)), 'pointpath_forward_train')
             self._train_args = keep
@@ -291,7 +293,60 @@ class PointPath:
         a.stream = torch.cuda.current_stream().cuda_stream
         check(lib.mvx_cml_conv1_sparse(ctypes.byref(a), ptr(w), ptr(b), float(self.eps if eps is None else eps), ptr(out),
                                        ptr(self._cml_ws), self._cml_ws.numel()), 'cml_conv1_sparse')
+        self._cml_call = self._fwd_call      # the saved state in _cml_ws belongs to this forward
         return out
+
+    def cml_conv1_backward(self, d_out: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, eps: float | None = None,
+                           want_d_vfeat: bool = True, grads=None):
+        """Backward of the last `cml_conv1` (same weight, bias, eps): d_out = dLoss/d its output (B,64,(nz+1)//2,nx,ny).
+        Returns (d_vfeat, d_w, d_b): d_vfeat (B, cap, 128) = dLoss/d voxel features for `backward(d_vfeat=...)` (rows past
+        each frame's voxel count are zero), or None with want_d_vfeat=False; d_w (64,128,3,3,3) and d_b (64) summed over the
+        frames. grads=(d_w, d_b): add into these tensors instead of returning new ones."""
+        if getattr(self, '_cml_call', None) is None or self._cml_call != getattr(self, '_fwd_call', None) or self._subs_active:
+            raise RuntimeError('cml_conv1_backward() needs the cml_conv1() of the latest forward on this PointPath')
+        a = self._last_args[0]
+        w = weight.detach().to(self.device, torch.float32).contiguous()
+        b = bias.detach().to(self.device, torch.float32).contiguous()
+        nz, nx, ny = self.grid.shape[2], self.grid.shape[0], self.grid.shape[1]
+        assert tuple(d_out.shape) == (self.B, 64, (nz + 2 - 3) // 2 + 1, nx, ny) and d_out.dtype == torch.float32 and d_out.is_cuda
+        d_out = d_out.contiguous()
+        nbytes = ctypes.c_size_t()
+        check(lib.mvx_cml_conv1_backward_workspace_bytes(ctypes.byref(a), ctypes.byref(nbytes)), 'cml_conv1_backward_workspace_bytes')
+        if getattr(self, '_cml_bws', None) is None or self._cml_bws.numel() < nbytes.value:
+            self._cml_bws = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+        if grads is None:
+            d_w = torch.empty((64, 128, 3, 3, 3), dtype=torch.float32, device=self.device)
+            d_b = torch.empty(64, dtype=torch.float32, device=self.device)
+        else:
+            d_w, d_b = grads
+            assert d_w.is_contiguous() and d_w.dtype == torch.float32 and tuple(d_w.shape) == (64, 128, 3, 3, 3)
+            assert d_b.is_contiguous() and d_b.dtype == torch.float32 and tuple(d_b.shape) == (64,)
+        d_vfeat = torch.zeros((self.B, self.cap, 128), dtype=torch.float32, device=self.device) if want_d_vfeat else None
+        a.stream = torch.cuda.current_stream().cuda_stream
+        check(lib.mvx_cml_conv1_sparse_backward(ctypes.byref(a), ptr(w), ptr(b), float(self.eps if eps is None else eps), ptr(d_out),
+                                                ptr(d_vfeat), ptr(d_w), ptr(d_b), int(grads is not None),
+                                                ptr(self._cml_ws), self._cml_ws.numel(), ptr(self._cml_bws), self._cml_bws.numel()),
+              'cml_conv1_sparse_backward')
+        return d_vfeat, d_w, d_b
+
+    def cml_saved(self):
+        """Read-only views of what the last `cml_conv1` saved for its backward (tests / diagnostics): act_count (B,) active
+        output positions per frame, act_idx (B, Go) compact row of each position (-1: background), Yact (B, Go, 64) relu(conv)
+        of the active rows (rows >= act_count unused). Mirrors the workspace layout of sparse_conv.cu (sc_layout)."""
+        nz, nx, ny = self.grid.shape[2], self.grid.shape[0], self.grid.shape[1]
+        B, go = self.B, ((nz + 2 - 3) // 2 + 1) * nx * ny
+        sizes = [('wt', 128 * 1792 * 4), ('wpack', 2 * 128 * 1792 * 4), ('P', B * self.cap * 1792 * 4), ('act_count', B * 4),
+                 ('act_idx', B * go * 4), ('yact', B * go * 64 * 4), ('stats', B * 64 * 2 * 8)]
+        off, o = {}, 0
+        for name, n in sizes:
+            off[name] = o
+            o += (n + 255) // 256 * 256
+        nbytes = ctypes.c_size_t()
+        check(lib.mvx_cml_conv1_workspace_bytes(ctypes.byref(self._last_args[0]), ctypes.byref(nbytes)), 'cml_conv1_workspace_bytes')
+        assert o == nbytes.value, 'cml_saved() is out of step with sc_layout'
+        view = lambda name, dtype, shape: self._cml_ws[off[name]:off[name] + int(np.prod(shape)) * 4].view(dtype).view(*shape)
+        return dict(act_count=view('act_count', torch.int32, (B,)), act_idx=view('act_idx', torch.int32, (B, go)),
+                    Yact=view('yact', torch.float32, (B, go, 64)))
 
     # ---- training mode -------------------------------------------------------------------------------------
     def forward_train(self, points, offsets, calib32, maps, want_grid: bool = True, cap: int | None = None,
