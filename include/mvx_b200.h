@@ -248,6 +248,16 @@ int64_t mvx_grad_floats(void);
 int mvx_pointpath_backward(const mvx_pointpath_args_t *args, const float *d_vfeat, const float *d_grid, float *grad_flat,
                            int32_t accumulate, void *backward_ws, size_t backward_ws_bytes);
 
+/* Gradient into the FPN maps (the adjoint of featureMaping's 4-corner gather, modules/imhead/Pipe.py:62-75), for callers
+ * that train the image backbone. Call after mvx_pointpath_backward with the SAME args and backward workspace (it reads
+ * fcn1's dpre that this left there, and the projections of the training forward). d_maps[l]: (B, 256, map_h[l], map_w[l])
+ * fp32 contiguous, OVERWRITTEN with dLoss/d map l; corners on the zero pad row / column of Pipe.py:47-48, pad slots and
+ * origin points contribute nothing. Deterministic: no floating-point atomics, two calls give bit-identical results.
+ * ws: mvx_pointpath_backward_maps_workspace_bytes() of scratch. */
+int mvx_pointpath_backward_maps_workspace_bytes(const mvx_pointpath_args_t *args, size_t *bytes);
+int mvx_pointpath_backward_maps(const mvx_pointpath_args_t *args, const void *backward_ws, size_t backward_ws_bytes,
+                                float *const d_maps[MVX_NUM_LEVELS], void *ws, size_t ws_bytes);
+
 /* ------------------------------------------------------------------------------------------------
  * After the path (SURVEY.md §8f rank 2) — sparse hand-off to the first middle-layer convolution.
  * Replaces `CML.conv1` = CRB3d(128, 64, 3, (2,1,1), (1,1,1)) (modules/voxelnet/Pipe.py:31-43; Blocks.py CRB3d:

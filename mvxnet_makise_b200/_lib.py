@@ -30,7 +30,7 @@ EXPORTS = [
     'mvx_set_gemm_mode', 'mvx_layer_workspace_bytes', 'mvx_fcn_forward', 'mvx_vfe_forward', 'mvx_fcn_max_forward', 'mvx_set_grid_mode', 'mvx_scatter_dense',
     'mvx_pointpath_workspace_bytes', 'mvx_pointpath_layout', 'mvx_pointpath_layout_name', 'mvx_pointpath_forward',
     'mvx_set_fusion_mode', 'mvx_set_fold_mode', 'mvx_pointpath_train_workspace_bytes', 'mvx_pointpath_forward_train', 'mvx_grad_floats',
-    'mvx_pointpath_backward', 'mvx_cml_conv1_workspace_bytes', 'mvx_cml_conv1_sparse',
+    'mvx_pointpath_backward', 'mvx_pointpath_backward_maps_workspace_bytes', 'mvx_pointpath_backward_maps', 'mvx_cml_conv1_workspace_bytes', 'mvx_cml_conv1_sparse',
     'mvx_cml_conv1_backward_workspace_bytes', 'mvx_cml_conv1_sparse_backward',
     'mvx_bbox_pairwise', 'mvx_classify_anchors_workspace_bytes', 'mvx_classify_anchors',
     'mvx_timing_enable', 'mvx_timing_read', 'mvx_timing_segment_name',
@@ -112,6 +112,8 @@ def _load():
     lib.mvx_cml_conv1_backward_workspace_bytes.argtypes = [POINTER(PointPathArgs), POINTER(c_size_t)]
     lib.mvx_cml_conv1_sparse_backward.argtypes = [POINTER(PointPathArgs), vp, vp, c_double, vp, vp, vp, vp, i32, vp, c_size_t, vp, c_size_t]
     lib.mvx_pointpath_backward.argtypes = [POINTER(PointPathArgs), vp, vp, vp, i32, vp, c_size_t]
+    lib.mvx_pointpath_backward_maps_workspace_bytes.argtypes = [POINTER(PointPathArgs), POINTER(c_size_t)]
+    lib.mvx_pointpath_backward_maps.argtypes = [POINTER(PointPathArgs), vp, c_size_t, POINTER(vp), vp, c_size_t]
     lib.mvx_bbox_pairwise.argtypes = [vp, i64, vp, i64, i32, vp, vp]
     lib.mvx_classify_anchors_workspace_bytes.argtypes = [i64, i64, i64, i32, POINTER(c_size_t)]
     lib.mvx_classify_anchors.argtypes = [vp, i64, vp, i64, i64, i32, vp, vp, c_float, c_float, vp, vp, vp, i64, vp, vp, c_size_t, vp]

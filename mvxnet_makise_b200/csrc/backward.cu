@@ -709,6 +709,20 @@ void make_blayout(const mvx_pointpath_args_t *a, const Layout &L, BLayout &BL) {
 
 }  // namespace
 
+void backward_ws_layout(const mvx_pointpath_args_t *a, const Layout &L, size_t *total, size_t *dpre1_off) {
+    BLayout BL;
+    make_blayout(a, L, BL);
+    *total = BL.total;
+    *dpre1_off = BL.off[BR_G1];
+}
+
+int launch_transpose_w(const float *wt, float *w, int Cin, int Cout, cudaStream_t st) {
+    const int n = Cin * Cout;
+    transpose_w_kernel<<<(n + 255) / 256, 256, 0, st>>>(wt, w, Cin, Cout);
+    MVX_LAUNCH_CHECK();
+    return MVX_OK;
+}
+
 size_t grad_floats() {
     size_t n = 0;
     for (int l = 0; l < MVX_NUM_LAYERS; ++l) n += (size_t)kCout[l] * kCinTrue[l] + kCout[l];
@@ -750,7 +764,7 @@ int pointpath_backward(const mvx_pointpath_args_t *a, const float *d_vfeat, cons
     MVX_CUDA_CHECK(cudaMemsetAsync(dmax, 0, (size_t)MVX_NUM_LAYERS * B * 768 * 4, st));
     auto dmax_of = [&](int l) { return dmax + (size_t)l * B * 768; };   // [B][Cout_l] inside
     float *wT = BF(BR_WT);
-    for (int l = 1; l < MVX_NUM_LAYERS; ++l) {   // fcn1 needs no dx (the FPN maps are inputs of the path)
+    for (int l = 1; l < MVX_NUM_LAYERS; ++l) {   // fcn1 needs no dx here: the map gradient is pixel-first (map_backward.cu)
         const int n = kCin[l] * kCout[l];
         transpose_w_kernel<<<(n + 255) / 256, 256, 0, st>>>(a->wt[l], wT + BL.wt_off[l], kCin[l], kCout[l]);
         MVX_LAUNCH_CHECK();

@@ -303,19 +303,6 @@ constexpr int kCombCout = 768;
 constexpr int kCombWarps = 6;        // one warp per 128 output columns (one float4 per lane)
 constexpr int kCombRows = 256;       // sorted rows per CTA
 
-struct CellRef {
-    int i0, i1;
-    float wa, wb;
-};
-__device__ __forceinline__ CellRef cell_of(float prow, float pcol, float rs_h, float rs_w, float eps) {
-    // index math and (inverted) weights of Pipe.py:62-75, same fp32 order as gather_row_warp
-    const float q0 = __fsub_rn(__fdiv_rn(prow, rs_h), eps);
-    const float q1 = __fsub_rn(__fdiv_rn(pcol, rs_w), eps);
-    CellRef c;
-    c.i0 = (int)q0, c.i1 = (int)q1;
-    c.wa = __fsub_rn(q0, (float)c.i0), c.wb = __fsub_rn(q1, (float)c.i1);
-    return c;
-}
 __device__ __forceinline__ int combine_key(const CombineArgs &a, int f, int r, int K) {
     const size_t ro = (size_t)f * a.capA + r;
     const float4 xyz = __ldg(reinterpret_cast<const float4 *>(a.vox8 + ro * 8));
@@ -442,12 +429,9 @@ __global__ void __launch_bounds__(kCombWarps * 32, MVX_COMB_MINB) combine_rows_k
         for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
             const CellRef c = cell_of(pr.x, pr.y, a.rs_h[l], a.rs_w[l], a.eps);
             const int H = a.h[l], W = a.w[l];
-            const bool r0 = c.i0 >= 0 && c.i0 < H, r1 = c.i0 + 1 >= 0 && c.i0 + 1 < H;
-            const bool c0 = c.i1 >= 0 && c.i1 < W, c1 = c.i1 + 1 >= 0 && c.i1 + 1 < W;
-            const float wa_ = __fsub_rn(1.0f, c.wa), wb_ = __fsub_rn(1.0f, c.wb);
+            const float4 cw = corner_weights(c, H, W);
             CombRec rec;
-            rec.w[0] = (r0 && c0) ? c.wa * c.wb : 0.f, rec.w[1] = (r1 && c0) ? wa_ * c.wb : 0.f;
-            rec.w[2] = (r0 && c1) ? c.wa * wb_ : 0.f, rec.w[3] = (r1 && c1) ? wa_ * wb_ : 0.f;
+            rec.w[0] = cw.x, rec.w[1] = cw.y, rec.w[2] = cw.z, rec.w[3] = cw.w;
             const int y0 = min(max(c.i0, 0), H - 1), y1 = min(max(c.i0 + 1, 0), H - 1);
             const int x0 = min(max(c.i1, 0), W - 1), x1 = min(max(c.i1 + 1, 0), W - 1);
             rec.cell = x0 | (y0 << 12) | ((x1 - x0) << 24) | ((y1 - y0) << 25);
@@ -622,13 +606,9 @@ __global__ void __launch_bounds__(kCombWarps * 32, MVX_COMB_MINB) combine_runs_k
         for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
             const CellRef c = cell_of(pr.x, pr.y, a.rs_h[l], a.rs_w[l], a.eps);
             const int H = a.h[l], W = a.w[l];
-            const bool r0 = c.i0 >= 0 && c.i0 < H, r1 = c.i0 + 1 >= 0 && c.i0 + 1 < H;
-            const bool c0 = c.i1 >= 0 && c.i1 < W, c1 = c.i1 + 1 >= 0 && c.i1 + 1 < W;
-            const float wa_ = __fsub_rn(1.0f, c.wa), wb_ = __fsub_rn(1.0f, c.wb);
             const int y0 = min(max(c.i0, 0), H - 1), y1 = min(max(c.i0 + 1, 0), H - 1);
             const int x0 = min(max(c.i1, 0), W - 1), x1 = min(max(c.i1 + 1, 0), W - 1);
-            s_recw[i][l] = make_float4((r0 && c0) ? c.wa * c.wb : 0.f, (r1 && c0) ? wa_ * c.wb : 0.f, (r0 && c1) ? c.wa * wb_ : 0.f,
-                                       (r1 && c1) ? wa_ * wb_ : 0.f);
+            s_recw[i][l] = corner_weights(c, H, W);
             s_cell[i][l] = none ? -1 : (x0 | (y0 << 12) | ((x1 - x0) << 24) | ((y1 - y0) << 25));
         }
     }

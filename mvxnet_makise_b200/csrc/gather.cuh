@@ -12,6 +12,31 @@ struct MapSet {
     int C;
 };
 
+// The 2x2 corner block a projected point samples at one FPN level: top-left corner (i0, i1) and the fractional parts.
+// Index math and (inverted) weights of Pipe.py:62-75 in the fp32 order of gather_row_warp; the forward's combine and the
+// map backward's pixel CSR both take their corners from here, so the adjoint picks exactly the forward's pixels.
+struct CellRef {
+    int i0, i1;
+    float wa, wb;
+};
+__device__ __forceinline__ CellRef cell_of(float prow, float pcol, float rs_h, float rs_w, float eps) {
+    const float q0 = __fsub_rn(__fdiv_rn(prow, rs_h), eps);
+    const float q1 = __fsub_rn(__fdiv_rn(pcol, rs_w), eps);
+    CellRef c;
+    c.i0 = (int)q0, c.i1 = (int)q1;   // .long(): truncation toward zero
+    c.wa = __fsub_rn(q0, (float)c.i0), c.wb = __fsub_rn(q1, (float)c.i1);
+    return c;
+}
+// weights of the corners (i0,i1), (i0+1,i1), (i0,i1+1), (i0+1,i1+1); 0 where the corner lies outside the H x W map (row H /
+// column W are the zero pad of Pipe.py:47-48)
+__device__ __forceinline__ float4 corner_weights(const CellRef &c, int H, int W) {
+    const bool r0 = c.i0 >= 0 && c.i0 < H, r1 = c.i0 + 1 >= 0 && c.i0 + 1 < H;
+    const bool c0 = c.i1 >= 0 && c.i1 < W, c1 = c.i1 + 1 >= 0 && c.i1 + 1 < W;
+    const float wa_ = __fsub_rn(1.0f, c.wa), wb_ = __fsub_rn(1.0f, c.wb);
+    return make_float4((r0 && c0) ? c.wa * c.wb : 0.f, (r1 && c0) ? wa_ * c.wb : 0.f, (r0 && c1) ? c.wa * wb_ : 0.f,
+                       (r1 && c1) ? wa_ * wb_ : 0.f);
+}
+
 // NCHW (B,C,H,W) -> NHWC (B,H,W,C)
 // rowmax (optional): [B][HW] max |x| over the C channels of every pixel (float; zeroed and filled here)
 // chmax (optional): [B][chmax_stride] ints (float bits, zeroed by the caller): max |x| of every channel over the frame's pixels

@@ -50,6 +50,8 @@ struct LayerArgs {
     int y_bf16;              // 1 (bf16 mode): Y holds bf16 elements (ldy in elements)
     int x_bf16;              // 1 (bf16 mode, tc3 kernel): X holds bf16 elements (ldx in elements)
     int plain;               // 1: Y = norm_in(X) W^T only (no bias, no ReLU, no statistics, no max) - the per-pixel half of fcn1
+    int y_nchw;              // 1 (plain 3xTF32 one-tile kernel only): Y is channel-major [F][Cout][rowcap], e.g. (B, C, H, W)
+                             // maps with rows_fixed = rowcap = H * W pixel rows per frame
 };
 // Work-skipping switches (no epilogue, no producers ...) exist for timing experiments only: a release build compiles them
 // out (the expression is the literal 0), so no environment variable can remove work from a timed region.

@@ -31,4 +31,9 @@ struct Layout {
 int make_layout(const mvx_pointpath_args_t *a, Layout &L);
 int pointpath_forward(const mvx_pointpath_args_t *a, bool train);
 
+// backward workspace of mvx_pointpath_backward (backward.cu): its size, and where fcn1's dpre [B][capA][768] stays after it
+void backward_ws_layout(const mvx_pointpath_args_t *a, const Layout &L, size_t *total, size_t *dpre1_off);
+// W (Cout, Cin) row-major from W^T (Cin, Cout)
+int launch_transpose_w(const float *wt, float *w, int Cin, int Cout, cudaStream_t st);
+
 }  // namespace mvx

@@ -531,7 +531,13 @@ __global__ void __launch_bounds__(tc_producer_warps(F16, TWO) * 32 + 64, TWO ? 2
             if (tid < 256) {
                 const int rbase = TWO ? hp * 128 : 0;    // first CTA-tile row of the staging tile
                 // coalesced raw stores first (one warp per row, 32 lanes x 16 bytes = 128 columns): they drain while the sums run
-                if (a.Y) {
+                if (a.Y && a.y_nchw) {   // channel-major: a warp stores one column, its lanes consecutive rows (128-byte runs)
+                    const long long nr = min((long long)TR, n_rows - row0 - rbase);
+                    for (int c = warp; c < kEpiCols; c += 8) {
+                        float *ycol = a.Y + ((size_t)f * a.Cout + n0 + pass * kEpiCols + c) * a.rowcap + row0 + rbase;
+                        for (int r = lane; r < nr; r += 32) ycol[r] = ytile[(size_t)r * kEpiLd + c];
+                    }
+                } else if (a.Y) {
                     for (int r = warp; r < TR; r += 8) {
                         if (row0 + rbase + r >= n_rows) break;
                         const float4 o = *reinterpret_cast<const float4 *>(ytile + (size_t)r * kEpiLd + lane * 4);
@@ -1395,6 +1401,11 @@ int launch_layer_tc(const LayerArgs &a_in, int F, float *wpack, cudaStream_t st)
     MVX_REQUIRE(tc_layer_eligible(a) && wpack, MVX_EINVAL, "layer not eligible for the tensor-core kernel");
     const long long max_rows = a.counts ? a.rowcap : a.rows_fixed;
     if (max_rows <= 0) return MVX_OK;
+    if (a.y_nchw) {
+        MVX_REQUIRE(a.plain && !a.f16_ok && !a.y_bf16 && !a.a_pack && !a.counts && a.rows_fixed == a.rowcap && a.Y, MVX_EINVAL,
+                    "channel-major output: plain 3xTF32 product over rows_fixed == rowcap rows per frame");
+        return a.Cout % 256 == 0 ? launch_tc<256, false>(a, F, wpack, st) : launch_tc<128, false>(a, F, wpack, st);
+    }
     if (a.vmax == nullptr && !a.plain && !a.X2 && a.rows_mode != 3 && tc_persistent_enabled())  // persistent kernel: 256 x 128 tiles, double-buffered accumulators
         return launch_tc_persist<128>(a, F, wpack, st);
     MVX_REQUIRE(!a.X2 || (a.f16_ok && (g_tc_bf16 || tc_f16_enabled()) && a.Cin % 32 == 0 && a.x2_cols % 32 == 0 && a.counts),

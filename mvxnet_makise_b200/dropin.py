@@ -11,8 +11,9 @@ underneath them runs on the sm_100a kernels.
 What `accelerate` replaces is the body of `MVXNet.forward` (MVXNet.py:21-27) between the image backbone and the CML:
 `featureMaping` -> `ImageFeatureFusion` -> concat -> `SVFE` -> `FCN` -> max over T -> `reindex` become one call of the fused
 path on the dense-voxel entry (`PointPath.forward_voxels`), wrapped in a `torch.autograd.Function` whose backward is the CUDA
-backward of the eight layers (`mvx_pointpath_backward`). `head.extractor` (frozen torchvision backbone), `backbone.cml` and
-`backbone.rpn` stay the reference's own modules. The model's `nn.Parameter`s remain the single source of truth: they are read
+backward of the eight layers (`mvx_pointpath_backward`) and, when the FPN maps want a gradient, of the 4-corner gather
+(`mvx_pointpath_backward_maps`). `head.extractor` (the torchvision backbone: frozen by Head.py:9-11, trained like any module
+after `model.head.extractor.requires_grad_(True)`), `backbone.cml` and `backbone.rpn` stay the reference's own modules. The model's `nn.Parameter`s remain the single source of truth: they are read
 on every forward (an optimiser step is picked up through the tensors' version counters) and receive `.grad` like any other
 parameter, so `model.parameters()`, `AdamW`, `state_dict()` / `load_state_dict()` and checkpoints are unaffected.
 """
@@ -59,17 +60,20 @@ def _push_parameters(path: PointPath, params: Sequence[torch.Tensor]):
 
 
 class HotPathFunction(torch.autograd.Function):
-    """grid = hot_path(voxels, idx, fpn maps; 16 parameters). Differentiable with respect to the parameters only: the image
-    backbone is frozen (Head.py:9-11) and the voxel tensor is data."""
+    """grid = hot_path(voxels, idx, fpn maps 0..2; 16 parameters). Differentiable with respect to the parameters and the three
+    FPN maps (the image backbone trains when `head.extractor` is unfrozen); the voxel tensor is data. Map gradients are
+    computed only where `needs_input_grad` asks for them, in each map's own dtype."""
 
     @staticmethod
-    def forward(ctx, path: PointPath, voxels, idx, maps, *params):
+    def forward(ctx, path: PointPath, voxels, idx, m0, m1, m2, *params):
         _push_parameters(path, params)
+        maps = [m.detach().to(torch.float32).contiguous() for m in (m0, m1, m2)]
         nz, nx, ny = path.grid.shape[2], path.grid.shape[0], path.grid.shape[1]
         B = len(voxels) if isinstance(voxels, (list, tuple)) else 1
         grid = torch.empty((B, 128, nz, nx, ny), dtype=torch.float32, device=path.device)   # a fresh tensor: the CML saves it for ITS backward
         path.forward_voxels(voxels, idx, maps, want_grid=True, train=True, grid_out=grid)
         ctx.path = path
+        ctx.map_dtypes = [m.dtype for m in (m0, m1, m2)]
         ctx.call_id = path._train_call = getattr(path, '_train_call', 0) + 1
         return grid
 
@@ -79,36 +83,61 @@ class HotPathFunction(torch.autograd.Function):
         if path._train_call != ctx.call_id:
             raise RuntimeError('the hot path ran another training forward before this backward: its saved activations are gone '
                                '(one forward/backward at a time per accelerated model)')
+        d_maps = _map_grad_buffers(path, ctx.needs_input_grad[3:6])
         flat = torch.empty(sum(int(np.prod(s)) for _, _, s in PointPath.grad_layout()), dtype=torch.float32, device=path.device)
-        path.backward(d_grid=d_grid.contiguous(), grad_flat=flat, accumulate=False)
-        grads = [flat[o:o + int(np.prod(shape))].view(*shape) for _, o, shape in PointPath.grad_layout()]
-        return (None, None, None, None, *grads)
+        path.backward(d_grid=d_grid.contiguous(), grad_flat=flat, accumulate=False, d_maps=d_maps)
+        grads = [None] * (2 * len(_HOT))
+        if any(ctx.needs_input_grad[6:]):
+            grads = [flat[o:o + int(np.prod(shape))].view(*shape) for _, o, shape in PointPath.grad_layout()]
+        return (None, None, None, *_map_grads(d_maps, ctx.needs_input_grad[3:6], ctx.map_dtypes), *grads)
+
+
+def _map_grad_buffers(path: PointPath, wanted):
+    """fp32 buffers for dLoss/d FPN maps when any map wants a gradient, else None (the map backward does not run)"""
+    if not any(wanted):
+        return None
+    return [torch.empty(m.shape, dtype=torch.float32, device=path.device) for m in path._train_args[4]]
+
+
+def _map_grads(d_maps, wanted, dtypes):
+    if d_maps is None:
+        return [None] * 3
+    return [d.to(dt) if w else None for d, w, dt in zip(d_maps, wanted, dtypes)]
+
+
+def _wants_grad(params, maps) -> bool:
+    return any(p.requires_grad for p in params) or any(m.requires_grad for m in maps)
 
 
 def hot_path(path: PointPath, voxels, idx, maps, params: Sequence[torch.Tensor]) -> torch.Tensor:
     """The dense grid (B,128,nz,nx,ny) for the reference's (voxels, idx) arguments. Records an autograd node when gradients are
-    enabled and a parameter wants one; otherwise takes the inference route (pixel-first fcn1, no saved activations)."""
+    enabled and a parameter or an FPN map wants one; otherwise takes the inference route (pixel-first fcn1, no saved
+    activations)."""
+    maps = list(maps)
+    if torch.is_grad_enabled() and _wants_grad(params, maps):
+        return HotPathFunction.apply(path, voxels, idx, *maps, *params)
     maps = [m.detach().to(torch.float32).contiguous() for m in maps]
-    if torch.is_grad_enabled() and any(p.requires_grad for p in params):
-        return HotPathFunction.apply(path, voxels, idx, maps, *params)
     _push_parameters(path, params)
     grid, _ = path.forward_voxels(voxels, idx, maps, want_grid=True, train=False)
     return grid
 
 
 class SparseConv1Function(torch.autograd.Function):
-    """y1 = backbone.cml.conv1(hot_path(voxels, idx, fpn maps; 16 parameters)) without the dense grid: the sparse hand-off
-    (`PointPath.cml_conv1`) reads the voxel features directly. Differentiable with respect to the 16 hot-path parameters and
-    the conv1 weight / bias. `train` says whether a hot parameter wants a gradient: without one the path forward runs in
-    inference mode and the backward skips d_vfeat and the path backward (fine-tuning of the CML alone)."""
+    """y1 = backbone.cml.conv1(hot_path(voxels, idx, fpn maps 0..2; 16 parameters)) without the dense grid: the sparse hand-off
+    (`PointPath.cml_conv1`) reads the voxel features directly. Differentiable with respect to the 16 hot-path parameters, the
+    three FPN maps and the conv1 weight / bias. `train` says whether a hot parameter or a map wants a gradient: without one
+    the path forward runs in inference mode and the backward skips d_vfeat and the path backward (fine-tuning of the CML
+    alone)."""
 
     @staticmethod
-    def forward(ctx, path: PointPath, eps: float, train: bool, voxels, idx, maps, *params):
+    def forward(ctx, path: PointPath, eps: float, train: bool, voxels, idx, m0, m1, m2, *params):
         hot, weight, bias = params[:-2], params[-2], params[-1]
         _push_parameters(path, hot)
+        maps = [m.detach().to(torch.float32).contiguous() for m in (m0, m1, m2)]
         path.forward_voxels(voxels, idx, maps, want_grid=False, train=train)
         y1 = path.cml_conv1(weight, bias, eps)
         ctx.path, ctx.eps, ctx.train = path, eps, train
+        ctx.map_dtypes = [m.dtype for m in (m0, m1, m2)]
         ctx.call_id = path._train_call = getattr(path, '_train_call', 0) + 1
         ctx.save_for_backward(weight, bias)
         return y1
@@ -122,20 +151,25 @@ class SparseConv1Function(torch.autograd.Function):
         weight, bias = ctx.saved_tensors
         d_vfeat, d_w, d_b = path.cml_conv1_backward(d_y1.contiguous(), weight, bias, ctx.eps, want_d_vfeat=ctx.train)
         grads = [None] * (2 * len(_HOT))
+        map_grads = [None] * 3
         if ctx.train:
+            d_maps = _map_grad_buffers(path, ctx.needs_input_grad[5:8])
             flat = torch.empty(sum(int(np.prod(s)) for _, _, s in PointPath.grad_layout()), dtype=torch.float32, device=path.device)
-            path.backward(d_vfeat=d_vfeat, grad_flat=flat, accumulate=False)
-            grads = [flat[o:o + int(np.prod(shape))].view(*shape) for _, o, shape in PointPath.grad_layout()]
-        return (None, None, None, None, None, None, *grads, d_w, d_b)
+            path.backward(d_vfeat=d_vfeat, grad_flat=flat, accumulate=False, d_maps=d_maps)
+            if any(ctx.needs_input_grad[8:8 + 2 * len(_HOT)]):
+                grads = [flat[o:o + int(np.prod(shape))].view(*shape) for _, o, shape in PointPath.grad_layout()]
+            map_grads = _map_grads(d_maps, ctx.needs_input_grad[5:8], ctx.map_dtypes)
+        return (None, None, None, None, None, *map_grads, *grads, d_w, d_b)
 
 
 def sparse_conv1(path: PointPath, voxels, idx, maps, params: Sequence[torch.Tensor], weight, bias, eps: float) -> torch.Tensor:
     """`backbone.cml.conv1` of the grid `hot_path` would return, (B, 64, (nz+1)//2, nx, ny), computed without that grid. Records an
-    autograd node when gradients are enabled and any of the 18 tensors wants one."""
-    maps = [m.detach().to(torch.float32).contiguous() for m in maps]
-    train = any(p.requires_grad for p in params)
+    autograd node when gradients are enabled and any of the 18 tensors or an FPN map wants one."""
+    maps = list(maps)
+    train = _wants_grad(params, maps)
     if torch.is_grad_enabled() and (train or weight.requires_grad or bias.requires_grad):
-        return SparseConv1Function.apply(path, eps, train, voxels, idx, maps, *params, weight, bias)
+        return SparseConv1Function.apply(path, eps, train, voxels, idx, *maps, *params, weight, bias)
+    maps = [m.detach().to(torch.float32).contiguous() for m in maps]
     _push_parameters(path, params)
     path.forward_voxels(voxels, idx, maps, want_grid=False, train=False)
     return path.cml_conv1(weight, bias, eps)
@@ -167,7 +201,7 @@ def _forward(self, voxels, imgs, idx, calibs, imsize):
         hw = (float(imsize[0]), float(imsize[1]))
         self._mvx_imsize[id(imsize)] = hw
     path.imsize_hw = hw
-    feats = self.head.extractor(imgs)                # FPN levels '0','1','2' (Pipe.py:17-21), frozen
+    feats = self.head.extractor(imgs)                # FPN levels '0','1','2' (Pipe.py:17-21); trains when unfrozen
     nx, ny = path.grid.shape[0], path.grid.shape[1]
     if self._mvx_sparse_conv1:                       # CML.forward (voxelnet/Pipe.py:31-43) with conv1 taken from the voxel features
         cml = self.backbone.cml

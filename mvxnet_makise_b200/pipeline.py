@@ -367,10 +367,14 @@ class PointPath:
         return out
 
     def backward(self, d_vfeat: torch.Tensor | None = None, d_grid: torch.Tensor | None = None,
-                 grad_flat: torch.Tensor | None = None, accumulate: bool = False) -> torch.Tensor:
+                 grad_flat: torch.Tensor | None = None, accumulate: bool = False,
+                 d_maps: Sequence[torch.Tensor] | None = None) -> torch.Tensor:
         """Gradients of the 8 hot-path layers for the last forward_train call, summed over its frames, as ONE flat fp32
         bucket (the message of the NCCL all-reduce; `grad_layout()` names its slices). Give dLoss/d voxel features
-        (B, cap, 128) or dLoss/d dense grid (B,128,nz,nx,ny)."""
+        (B, cap, 128) or dLoss/d dense grid (B,128,nz,nx,ny).
+        d_maps: three contiguous fp32 CUDA tensors shaped like the forward's FPN maps (B,256,H_l,W_l): they are overwritten
+        with dLoss/d maps (the gradient an unfrozen image backbone receives; mvx_pointpath_backward_maps). None: no map
+        gradient, and nothing beyond the parameter backward runs."""
         if getattr(self, '_train_args', None) is None:
             raise RuntimeError('backward() needs a preceding forward_train() on this PointPath')
         a = self._train_args[0]
@@ -385,7 +389,25 @@ class PointPath:
         a.stream = torch.cuda.current_stream().cuda_stream
         check(lib.mvx_pointpath_backward(ctypes.byref(a), ptr(d_vfeat), ptr(d_grid), grad_flat.data_ptr(), int(bool(accumulate)),
                                          self._bws.data_ptr(), self._bws.numel()), 'pointpath_backward')
+        if d_maps is not None:
+            maps = self._train_args[4]
+            assert len(d_maps) == len(maps) == _lib.NUM_LEVELS
+            for t, m in zip(d_maps, maps):
+                assert t.is_cuda and t.is_contiguous() and t.dtype == torch.float32 and t.shape == m.shape, (tuple(t.shape), tuple(m.shape))
+            nbytes = ctypes.c_size_t()
+            check(lib.mvx_pointpath_backward_maps_workspace_bytes(ctypes.byref(a), ctypes.byref(nbytes)), 'pointpath_backward_maps_workspace_bytes')
+            if getattr(self, '_map_bws', None) is None or self._map_bws.numel() < nbytes.value:
+                self._map_bws = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+            out = (ctypes.c_void_p * _lib.NUM_LEVELS)(*[t.data_ptr() for t in d_maps])
+            check(lib.mvx_pointpath_backward_maps(ctypes.byref(a), self._bws.data_ptr(), self._bws.numel(), out, self._map_bws.data_ptr(),
+                                                  self._map_bws.numel()), 'pointpath_backward_maps')
         return grad_flat
+
+    def backward_saved(self):
+        """Read-only view of what the last `backward` left for the map gradient (tests / diagnostics): dpre1 (B, capA, 768),
+        dLoss/d fcn1's pre-activation of every compact row. Mirrors make_blayout of backward.cu (its first region)."""
+        capA = self.cap + 128
+        return dict(dpre1=self._bws[:self.B * capA * 768 * 4].view(torch.float32).view(self.B, capA, 768))
 
     def grads(self, grad_flat: torch.Tensor) -> Dict[str, torch.Tensor]:
         """Named views into a flat gradient bucket (reference state-dict names)."""
