@@ -134,7 +134,7 @@ int mvx_feature_mapping(float *voxels, int64_t R, const float *const *maps, cons
  * group of T rows: y (R, 2*Cout) = [pointwise | max] (modules/voxelnet/Pipe.py:12-18).
  * mvx_fcn_max_forward returns only the per-voxel max (R/T, Cout) (VoxelNet.py:28-32).
  * ------------------------------------------------------------------------------------------------ */
-int mvx_set_gemm_mode(int32_t mode); /* 0 = SIMT fp32 everywhere, 1 = tensor cores, one 256xBN tile per CTA (default), 2 = tensor cores, persistent 256x128 variant, (3 was the CTA-pair kernel: removed, rejected with MVX_EINVAL), 4 = tensor cores with 3xTF32 operands everywhere (mode 1 uses fp16 hi/lo operands, "3xFP16", for the layers of the fused path whose inputs are BatchNorm-ed or row-scaled), 5 = like 1 and the dense layer entry points below also use fp16 operands (caller promises inputs of O(1) magnitude), 6 = bf16 mode: one bf16 product per K-step instead of the three-product split for those layers (reduced precision; tolerance in tests/test_gpu_parity.py::test_bf16_mode_tolerance), 7 = like 1 with conv1 / fcn2 of the fused path in the persistent 3xFP16 kernel (TMEM accumulator ping-pong, epilogue overlapped with the next tile; experimental, measured slower), 8 = 1 (default since round 2: conv1 / fcn2 / the last FCN of the fused path run in the persistent TMA-fed kernel with the A operand in tensor memory, csrc/tc3_layer.cu), 9 = like 1 but those layers in the one-tile kernel of csrc/tc_layer.cu (the round-1 default, kept for A/B timing), 10 = like 1 with the VFE inputs materialised by prep kernels as in training (inspection of X6 / X7, A/B timing), 12 = like 1 with the one-tile two-CTAs-per-SM kernel for the per-pixel GEMM of fcn1 instead of the persistent one (A/B timing) */
+int mvx_set_gemm_mode(int32_t mode); /* 0 = SIMT fp32 everywhere, 1 = tensor cores (default): fp16 hi/lo operands ("3xFP16") for the layers of the fused path whose inputs are BatchNorm-ed or row-scaled, 3xTF32 for the dense layer entry points below; conv1 / fcn2 / the last FCN of the fused path run in the persistent TMA-fed kernel with the A operand in tensor memory (csrc/tc3_layer.cu), 5 = like 1 with those layers in the one-tile kernel of csrc/tc_layer.cu, and the dense layer entry points also use fp16 operands (caller promises inputs of O(1) magnitude), 6 = bf16 mode: one bf16 product per K-step instead of the three-product split for the 3xFP16 layers (reduced precision; tolerance in tests/test_gpu_parity.py::test_bf16_mode_tolerance), 9 = like 1 but conv1 / fcn2 / the last FCN in the one-tile kernel of csrc/tc_layer.cu (kept for A/B timing), 10 = like 1 with the VFE inputs materialised by prep kernels as in training (inspection of X6 / X7, A/B timing), 12 = like 1 with the one-tile two-CTAs-per-SM kernel for the per-pixel GEMM of fcn1 instead of the persistent one (A/B timing). Every other value, among them the removed modes 2, 3, 4, 7 and 8, is rejected with MVX_EINVAL. */
 int mvx_layer_workspace_bytes(int32_t Cin, int32_t Cout, size_t *bytes);
 int mvx_fcn_forward(const float *x, int64_t R, int32_t Cin, const float *wt, const float *bias, int32_t Cout,
                     double eps, float *y, void *stats_ws, void *stream);
@@ -148,7 +148,6 @@ int mvx_fcn_max_forward(const float *x, int64_t R, int32_t T, int32_t Cin, const
  * (`reindex`): out (1,C,nz,nx,ny) fp32 fully written (zeros + features) in ONE streaming pass.
  * idx (N,4) int64 [batch, ix, iy, iz] (train.py:119,126).  map_ws: (G + G/32 + 1) int32 of scratch, G = nz*nx*ny.
  * ------------------------------------------------------------------------------------------------ */
-int mvx_set_grid_mode(int32_t mode); /* 2 = plane-sequential stores + occupancy bits (default), 0 = cell-major st.global.cs, 1 = cp.async.bulk stores, 3 = (fused path, experimental, measured slower) the zeros go out early on a side stream and only the sectors that hold a voxel are written at the end */
 int mvx_scatter_dense(const float *feat, const int64_t *idx, int64_t N, int32_t C, int32_t nx, int32_t ny,
                       int32_t nz, float *out, int32_t *map_ws, void *stream);
 
@@ -222,11 +221,9 @@ int mvx_pointpath_forward(const mvx_pointpath_args_t *args);
  *   2           pixel-first like 1 but without running the map branch (channels-last copy + pixel GEMMs) on a side stream
  *               concurrently with the point branch (voxelization, row build, row sort) - for per-stage profiling. */
 int mvx_set_fusion_mode(int32_t mode);
-/* Pixel-first inference only. 1: the combine kernel writes fcn1's raw rows directly as conv1's pre-packed tensor-core operand
- * (fp16 hi/lo images, per-row power-of-two scale from an a-priori bound) and conv1 (Pipe.py:96) runs with fcn1's BatchNorm
- * folded into per-frame weights: W' = W diag(rstd), b' = b - W'' mean, W'' = W' as its fp16 hi + lo images represent it;
- * 0: conv1 reads the fp32 rows and normalises them while loading (default);
- * 2: like 0, with the first version of the combine kernel (row-by-row walk; kept for A/B measurements). */
+/* Pixel-first inference only. 0: the run-structured combine kernel (default);
+ * 2: the first version of the combine kernel (row-by-row walk; kept for A/B measurements). Any other value is rejected with
+ * MVX_EINVAL (1, conv1 with fcn1's BatchNorm folded into per-frame weights, was removed). */
 int mvx_set_fold_mode(int32_t mode);
 
 /* ------------------------------------------------------------------------------------------------

@@ -27,7 +27,7 @@ EXPORTS = [
     'mvx_voxelize_workspace_bytes', 'mvx_voxelize', 'mvx_group_emit7', 'mvx_group_emit9',
     'mvx_crop_workspace_bytes', 'mvx_crop_points', 'mvx_crop_points_f64',
     'mvx_lidar2img', 'mvx_lidar2img_f64', 'mvx_dense_voxel_counts', 'mvx_maps_nhwc_bytes', 'mvx_feature_mapping',
-    'mvx_set_gemm_mode', 'mvx_layer_workspace_bytes', 'mvx_fcn_forward', 'mvx_vfe_forward', 'mvx_fcn_max_forward', 'mvx_set_grid_mode', 'mvx_scatter_dense',
+    'mvx_set_gemm_mode', 'mvx_layer_workspace_bytes', 'mvx_fcn_forward', 'mvx_vfe_forward', 'mvx_fcn_max_forward', 'mvx_scatter_dense',
     'mvx_pointpath_workspace_bytes', 'mvx_pointpath_layout', 'mvx_pointpath_layout_name', 'mvx_pointpath_forward',
     'mvx_set_fusion_mode', 'mvx_set_fold_mode', 'mvx_pointpath_train_workspace_bytes', 'mvx_pointpath_forward_train', 'mvx_grad_floats',
     'mvx_pointpath_backward', 'mvx_pointpath_backward_maps_workspace_bytes', 'mvx_pointpath_backward_maps', 'mvx_cml_conv1_workspace_bytes', 'mvx_cml_conv1_sparse',
@@ -95,7 +95,6 @@ def _load():
     lib.mvx_fcn_forward.argtypes = [vp, i64, i32, vp, vp, i32, c_double, vp, vp, vp]
     lib.mvx_vfe_forward.argtypes = [vp, i64, i32, i32, vp, vp, i32, c_double, vp, vp, vp, vp]
     lib.mvx_fcn_max_forward.argtypes = [vp, i64, i32, i32, vp, vp, i32, c_double, vp, vp, vp, vp]
-    lib.mvx_set_grid_mode.argtypes = [i32]
     lib.mvx_scatter_dense.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp, vp, vp]
     lib.mvx_pointpath_workspace_bytes.argtypes = [POINTER(PointPathArgs), POINTER(c_size_t)]
     lib.mvx_pointpath_layout.argtypes = [POINTER(PointPathArgs), POINTER(i64)]
@@ -158,18 +157,18 @@ c_float = c_float  # re-export for callers building timing buffers
 
 
 def set_gemm_mode(mode: int):
-    """0 = exact-fp32 SIMT layers everywhere, 1 = tcgen05 3xTF32 layers, one tile per CTA (default),
-    2 = tcgen05 3xTF32 layers, persistent variant with overlapped register epilogue (experimental), (3 = CTA-pair kernel: removed)
-    (experimental), 4 = 3xTF32 operands everywhere (mode 1 uses fp16 hi/lo operands for BatchNorm-ed / row-scaled inputs),
-    5 = like 1 and the dense layer API also uses fp16 operands (inputs must be O(1)), 6 = bf16 mode (single-pass bf16
-    operands for the layers mode 1 runs in 3xFP16; reduced precision), 7 = persistent 3xFP16 register-producer kernel (experimental),
-    8 = 1 (conv1 / fcn2 / last FCN in the TMA-fed A-from-TMEM persistent kernel, tc3_layer.cu: the default), 9 = like 1 with the
-    one-tile kernel of round 1 for those layers (A/B timing), 10 = like 1 with the VFE inputs materialised by prep_vfe1 / prep_vfe2
-    as in training, 12 = like 1 with the one-tile kernel for the per-pixel GEMM of fcn1 instead of the persistent one (A/B timing)."""
+    """0 = exact-fp32 SIMT layers everywhere, 1 = tcgen05 layers (default): 3xFP16 operands for the fused path's BatchNorm-ed /
+    row-scaled inputs, 3xTF32 for the dense layer API, conv1 / fcn2 / last FCN in the TMA-fed A-from-TMEM persistent kernel
+    (tc3_layer.cu), 5 = like 1 with the one-tile kernel for those layers, and the dense layer API also uses fp16 operands (inputs
+    must be O(1)), 6 = bf16 mode (single-pass bf16 operands for the layers mode 1 runs in 3xFP16; reduced precision), 9 = like 1
+    with the one-tile kernel of tc_layer.cu for conv1 / fcn2 / last FCN (A/B timing), 10 = like 1 with the VFE inputs materialised
+    by prep_vfe1 / prep_vfe2 as in training, 12 = like 1 with the one-tile kernel for the per-pixel GEMM of fcn1 instead of the
+    persistent one (A/B timing). Any other number raises: 2, 3, 4, 7 and 8 selected variants that have been removed."""
     check(lib.mvx_set_gemm_mode(int(mode)), 'set_gemm_mode')
 
 
 def set_fold_mode(mode: int):
+    """0 = the run-structured combine kernel (default), 2 = its first, row-by-row version (A/B runs)."""
     check(lib.mvx_set_fold_mode(int(mode)), 'set_fold_mode')
 
 

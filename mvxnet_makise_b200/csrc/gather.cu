@@ -356,32 +356,6 @@ __global__ void __launch_bounds__(256) combine_scatter_kernel(CombineArgs a) {
     a.perm[(size_t)f * a.capA + pos] = r;
 }
 
-__device__ __forceinline__ float pow2_scale_f(float mx) {   // 2^-e with mx = m * 2^e, m in [0.5, 1): mx * scale < 1
-    if (!(mx > 0.f) || !isfinite(mx)) return 1.f;
-    int e;
-    frexpf(mx, &e);
-    e = max(-100, min(100, e));
-    return exp2f((float)-e);
-}
-
-// wbound[l] = max over outputs o of sum_c |W1^T[256 l + c][o]| (l = 0, 1, 2), wbound[3] = max |bias|; values >= 0, so the
-// float bits order like ints (atomicMax on a zeroed buffer)
-__global__ void __launch_bounds__(128) fcn1_bounds_kernel(const float *__restrict__ w1t, const float *__restrict__ bias, int *__restrict__ wbound) {
-    const int l = blockIdx.y, o = blockIdx.x * 128 + threadIdx.x;
-    float s = 0.f;
-    for (int c = 0; c < 256; ++c) s += fabsf(__ldg(w1t + (size_t)(l * 256 + c) * kCombCout + o));
-    float b = l == 0 ? fabsf(__ldg(bias + o)) : 0.f;
-#pragma unroll
-    for (int d = 16; d >= 1; d >>= 1) {
-        s = fmaxf(s, __shfl_xor_sync(0xffffffffu, s, d));
-        b = fmaxf(b, __shfl_xor_sync(0xffffffffu, b, d));
-    }
-    if ((threadIdx.x & 31) == 0) {
-        atomicMax(wbound + l, __float_as_int(s));
-        if (l == 0) atomicMax(wbound + 3, __float_as_int(b));
-    }
-}
-
 // per-row, per-level sampling record, computed once per row by one thread (the six column warps only read it)
 struct CombRec {
     int cell;        // x0 | y0 << 12 | dx << 24 | dy << 25 : clamped corner coordinates; also the cache tag
@@ -402,11 +376,10 @@ __device__ __forceinline__ uint2 f4_to_bf16x4(float4 v) {
 }
 
 // ZB / YB: Z is read / Y1 is written as bf16 (the reduced-precision mode; the arithmetic in between stays fp32)
-template <bool PACK, bool ZB = false, bool YB = false>
+template <bool ZB = false, bool YB = false>
 __global__ void __launch_bounds__(kCombWarps * 32, MVX_COMB_MINB) combine_rows_kernel(CombineArgs a) {
     __shared__ int s_row[kCombRows];                     // compact row; ~row for rows without corners
     __shared__ float s_w[kCombRows];                     // BatchNorm multiplicity
-    __shared__ float s_sc[PACK ? kCombRows : 1];         // PACK: power-of-two scale of the row
     __shared__ float4 s_recw[kCombRows][MVX_NUM_LEVELS];   // corner weights: one 16-byte broadcast load per row and level
     __shared__ int s_cell[kCombRows][MVX_NUM_LEVELS];      // packed corner coordinates (the cache tag)
     const int f = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -424,7 +397,6 @@ __global__ void __launch_bounds__(kCombWarps * 32, MVX_COMB_MINB) combine_rows_k
         s_row[i] = none ? ~r : r;
         s_w[i] = __ldg(a.row_w + ro);
         const float2 pr = __ldg(reinterpret_cast<const float2 *>(a.proj) + ro);
-        float bound = PACK ? __ldg(a.wbound + 3) : 0.f;   // max |bias|
 #pragma unroll
         for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
             const CellRef c = cell_of(pr.x, pr.y, a.rs_h[l], a.rs_w[l], a.eps);
@@ -437,16 +409,6 @@ __global__ void __launch_bounds__(kCombWarps * 32, MVX_COMB_MINB) combine_rows_k
             rec.cell = x0 | (y0 << 12) | ((x1 - x0) << 24) | ((y1 - y0) << 25);
             s_recw[i][l] = make_float4(rec.w[0], rec.w[1], rec.w[2], rec.w[3]);
             s_cell[i][l] = rec.cell;
-            if constexpr (PACK) {   // |Z_l| at the four corners <= L1max_l * (bound of max |F| of that pixel); the weights sum to 1
-                const float *pb = a.pix_bound[l] + (size_t)f * H * W;
-                const float m = fmaxf(fmaxf(__ldg(pb + y0 * W + x0), __ldg(pb + y1 * W + x0)), fmaxf(__ldg(pb + y0 * W + x1), __ldg(pb + y1 * W + x1)));
-                bound = fmaf(__ldg(a.wbound + l), m, bound);
-            }
-        }
-        if constexpr (PACK) {
-            const float sc = pow2_scale_f(none ? __ldg(a.wbound + 3) : bound);
-            s_sc[i] = sc;
-            a.y1_rowinv[ro] = 1.f / sc;
         }
     }
     __syncthreads();
@@ -500,18 +462,7 @@ __global__ void __launch_bounds__(kCombWarps * 32, MVX_COMB_MINB) combine_rows_k
         }
         float4 y;
         y.x = fmaxf(acc.x, 0.f), y.y = fmaxf(acc.y, 0.f), y.z = fmaxf(acc.z, 0.f), y.w = fmaxf(acc.w, 0.f);
-        if constexpr (PACK) {
-            // this lane's 4 columns are 8 bytes of hi and 8 bytes of lo inside one 16-byte unit of the row's 64-byte chunk row
-            const float sc = s_sc[i];
-            uint2 hi, lo;
-            pk_split(y.x * sc, y.y * sc, hi.x, lo.x);
-            pk_split(y.z * sc, y.w * sc, hi.y, lo.y);
-            const uint32_t t = (uint32_t)r >> 8, rr = (uint32_t)r & 255u, kc = (uint32_t)col0 >> 5, c16 = ((uint32_t)col0 & 31u) >> 3;
-            unsigned char *dst = a.y1pack + (((size_t)f * a.pack_tiles + t) * (kCombCout / 32) + kc) * 32768 + rr * 64u +
-                                 ((c16 ^ ((rr >> 1) & 3u)) << 4) + (((uint32_t)col0 >> 2) & 1u) * 8u;
-            *reinterpret_cast<uint2 *>(dst) = hi;
-            *reinterpret_cast<uint2 *>(dst + 16384) = lo;
-        } else if constexpr (YB) {
+        if constexpr (YB) {
             // the statistics below are those of the values conv1 will actually read: the bf16-rounded ones
             const uint2 yb = f4_to_bf16x4(y);
             *reinterpret_cast<uint2 *>(reinterpret_cast<__nv_bfloat16 *>(a.Y1) + ((size_t)f * a.capA + r) * kCombCout + col0) = yb;
@@ -793,13 +744,6 @@ int launch_combine_sort(const CombineArgs &a, int B, cudaStream_t st) {
     return MVX_OK;
 }
 
-int launch_fcn1_bounds(const float *w1t, const float *bias, float *wbound, cudaStream_t st) {
-    MVX_CUDA_CHECK(cudaMemsetAsync(wbound, 0, 4 * sizeof(float), st));
-    fcn1_bounds_kernel<<<dim3(kCombCout / 128, MVX_NUM_LEVELS), 128, 0, st>>>(w1t, bias, reinterpret_cast<int *>(wbound));
-    MVX_LAUNCH_CHECK();
-    return MVX_OK;
-}
-
 static int g_comb_v1 = 0;     // 1: the first combine kernel (row-by-row walk) instead of the run-structured one - kept for A/B runs
 void set_combine_v1(int on) { g_comb_v1 = on; }
 
@@ -819,16 +763,13 @@ static int launch_combine_runs_t(const CombineArgs &a, dim3 grid, cudaStream_t s
 int launch_combine_rows(const CombineArgs &a, int B, cudaStream_t st) {
     dim3 grid((a.capA + kCombRows - 1) / kCombRows, B);
     MVX_REQUIRE(a.capA <= 0xFFFFFF, MVX_EINVAL, "combine: more than 2^24 rows per frame");
-    if (a.y1pack) {
-        MVX_REQUIRE(a.y1_rowinv && a.wbound && a.pack_tiles * 256 >= a.capA, MVX_EINVAL, "combine: bad packed-output arguments");
-        combine_rows_kernel<true><<<grid, kCombWarps * 32, 0, st>>>(a);
-    } else if (a.z_bf16 || a.y1_bf16) {
+    if (a.z_bf16 || a.y1_bf16) {
         MVX_REQUIRE(a.z_bf16 && a.y1_bf16, MVX_EINVAL, "combine: the bf16 mode stores both Z and Y1 as bf16");
         if (!g_comb_v1) return launch_combine_runs_t<true, true>(a, grid, st);
-        combine_rows_kernel<false, true, true><<<grid, kCombWarps * 32, 0, st>>>(a);
+        combine_rows_kernel<true, true><<<grid, kCombWarps * 32, 0, st>>>(a);
     } else {
         if (!g_comb_v1) return launch_combine_runs_t<false, false>(a, grid, st);
-        combine_rows_kernel<false><<<grid, kCombWarps * 32, 0, st>>>(a);
+        combine_rows_kernel<><<<grid, kCombWarps * 32, 0, st>>>(a);
     }
     MVX_LAUNCH_CHECK();
     return MVX_OK;

@@ -91,19 +91,9 @@ struct CombineArgs {
     int *bin_start;         // [B][nbins + 2] scratch
     int *perm;              // [B][capA] sorted position -> compact row
     int nbins;
-    // optional: instead of the fp32 Y1, write the rows as the pre-packed fp16 hi/lo A operand of conv1 (per frame:
-    // pack_tiles 256-row tiles x 24 chunks of 32 channels x [hi 16 KB | lo 16 KB], SWIZZLE_64B), each row scaled by a power of two
-    // 2^-e >= its bound |b|max + sum_l L1max_l * max corner |F| (so |y * scale| <= 1); y1_rowinv[f][r] = 1 / scale
-    unsigned char *y1pack;
-    float *y1_rowinv;       // [B][capA]
-    int pack_tiles;
-    const float *pix_bound[MVX_NUM_LEVELS];   // [B][HW_l]: power-of-two upper bound of max |F| of every pixel (the pixel GEMM's inverse row scale)
-    const float *wbound;    // device [4]: max_o sum_c |W1[o][256 l + c]| for l = 0, 1, 2 and max |bias|
     // bf16 mode (mvx_set_gemm_mode(6)): Z and / or Y1 hold bf16 elements (same indexing in elements, half the bytes)
     int z_bf16, y1_bf16;
 };
-// wbound (device [4], see above) from W1^T (768, 768) and the bias
-int launch_fcn1_bounds(const float *w1t, const float *bias, float *wbound, cudaStream_t st);
 // scratch sizes (ints per frame) for the level-0 extents of the call
 inline int combine_bins(int h0, int w0) { return ((h0 + 3) / 4) * ((w0 + 3) / 4) * 16; }
 int launch_combine_sort(const CombineArgs &a, int B, cudaStream_t st);   // counting sort of the rows (needs vox8 / proj only)

@@ -600,15 +600,24 @@ static int dense_layer(const float *x, int64_t R, int32_t T, int32_t Cin, const 
 
 }  // namespace mvx
 
+// 0 = the exact-fp32 SIMT kernel everywhere
+// 1 = tensor cores where eligible (default): 3xFP16 for the fused path's BatchNorm-ed layers, 3xTF32 for the dense layer API;
+//     conv1 / fcn2 / last FCN through the TMA-fed A-from-TMEM persistent kernel (tc3_layer.cu)
+// 5 = like 1 with tc_layer.cu's one-tile kernel for those layers, and the dense layer API (mvx_fcn_forward ...) also uses fp16
+//     operands: the caller promises inputs of O(1) magnitude (tests)
+// 6 = bf16 mode: single-pass bf16 operands for the same layers mode 1 runs in 3xFP16
+// 9 = like 1 with the one-tile kernel of tc_layer.cu for conv1 / fcn2 / last FCN
+// 10 = like 1 with prep_vfe1 / prep_vfe2 materialising the VFE inputs also in inference (the earlier default, kept for A/B timing and
+//      for inspecting X6 / X7)
+// 12 = like 1 with the one-tile two-CTAs-per-SM kernel (tc_layer.cu) for the pixel GEMM instead of the persistent one (A/B timing)
+// 2, 3, 4, 7, 8 and 11 selected variants that have been removed (DESIGN.md §5) and are rejected; the modes above keep their numbers.
 extern "C" int mvx_set_gemm_mode(int32_t mode) {
-    if (mode < 0 || mode > 12 || mode == 3 || mode == 11) return MVX_EINVAL;   // 12 = like 1 with the one-tile two-CTAs-per-SM kernel (tc_layer.cu) for the pixel GEMM instead of the persistent one (A/B timing)   // 10 = like 1 with prep_vfe1 / prep_vfe2 materialising the VFE inputs also in inference (the earlier default, kept for A/B timing and for inspecting X6 / X7)   // 1 and 8: conv1 / fcn2 / last FCN through the TMA-fed A-from-TMEM persistent kernel (tc3_layer.cu); 9 = like 1 with the one-tile kernel of tc_layer.cu for those layers   // 3 (CTA-pair kernel) was removed: measured slower, never default   // 7 = like 1, conv1 / fcn2 through the persistent 3xFP16 kernel (experimental, measured slower)   // 6 = bf16 mode: single-pass bf16 operands for the same layers mode 1 runs in 3xFP16
-    mvx::set_tc_bf16(mode == 6);   // 4 = tensor cores, 3xTF32 everywhere (no fp16 operands)
-    mvx::set_tc_f16(mode != 4);                    // 5 = like 1, and the dense layer API (mvx_fcn_forward ...) also uses fp16
-    mvx::g_dense_f16 = mode == 5;                  //     operands: the caller promises inputs of O(1) magnitude (tests)   // 2 = tensor cores, persistent 256x128 variant (measured slower: SS-mode
-    mvx::g_gemm_mode = mode == 0 ? 0 : 1;          //     MMAs at N=128 saturate shared-memory bandwidth); kept for experiments
-    mvx::set_tc_persistent(mode == 2);
-    mvx::set_tc_persist16(mode == 7);
-    mvx::set_tc3(mode == 1 || mode == 8 || mode == 6 || mode == 10 || mode == 12);
+    constexpr unsigned kModes = 1u << 0 | 1u << 1 | 1u << 5 | 1u << 6 | 1u << 9 | 1u << 10 | 1u << 12;
+    MVX_REQUIRE(mode >= 0 && mode <= 12 && (kModes >> mode & 1u), MVX_EINVAL, "gemm mode must be 0, 1, 5, 6, 9, 10 or 12");
+    mvx::set_tc_bf16(mode == 6);
+    mvx::g_dense_f16 = mode == 5;
+    mvx::g_gemm_mode = mode == 0 ? 0 : 1;
+    mvx::set_tc3(mode == 1 || mode == 6 || mode == 10 || mode == 12);
     mvx::set_pixel_persistent(mode != 12);
     mvx::set_vfe_fused(mode != 10);
     return MVX_OK;

@@ -30,15 +30,12 @@ struct LayerArgs {
     int f16_ok;              // 1: the tensor-core kernel may use fp16 operands (3xFP16): inputs are BatchNorm-ed (in_stats, or
                              // stored normalised) or row_max is given; 0 keeps 3xTF32 (arbitrary input range)
     const float *row_max;    // [F][rowcap] max|x| of each input row for the fp16 row scaling, or NULL (scale 1)
-    // pre-packed A (rows_mode 0 only): the producing kernel already wrote the fp16 hi/lo shared-memory images of every
-    // (256-row tile, 32-k chunk) [hi 16 KB | lo 16 KB]; the layer kernel then has no register producers at all, the A tiles
-    // arrive by bulk copy like the weights. a_rowinv[r] = 1 / (power-of-two scale the packer applied to row r).
+    // pre-packed A (rows_mode 0, one frame): the producing kernel already wrote the fp16 hi/lo shared-memory images of every
+    // (256-row tile, 32-k chunk) [hi 16 KB | lo 16 KB], tile t and chunk kc at (t * nk + kc) * 32 KB; the layer kernel then has no
+    // register producers at all, the A tiles arrive by bulk copy like the weights. a_rowinv[r] = 1 / (power-of-two scale the packer
+    // applied to row r).
     const void *a_pack;
     const float *a_rowinv;   // NULL: no per-row scale
-    int a_frame_tiles;       // 256-row tiles per frame inside a_pack (frame f, tile t, chunk kc at ((f * a_frame_tiles + t) * nk + kc) * 32 KB)
-    // per-frame pre-packed weights (BatchNorm of the producer folded into them by the caller): wpack holds F consecutive
-    // [blob | colinv] sets packed by the caller, `bias` is [F][Cout]; the kernel then does no weight packing itself
-    int w_per_frame;
     // fused concat (16-bit tensor-core producer only): input columns [Cin - x2_cols, Cin) of row r come from
     // X2[f][v(r)][0:x2_cols] (float bits, e.g. the per-voxel max of the producer layer) instead of X, with
     // v(r) = r >= K_f ? r - K_f : cat_row_vox[f][r]; both parts are normalised with the same in_stats (in_C channels)
@@ -83,13 +80,6 @@ void set_vfe_fused(int on);
 bool tc_layer_eligible(const LayerArgs &a);
 size_t tc_wpack_bytes(int Cin, int Cout);
 int launch_layer_tc(const LayerArgs &a, int F, float *wpack, cudaStream_t st);
-// Per-frame weight sets for a layer whose A operand arrives pre-packed and UN-normalised (LayerArgs::w_per_frame): the
-// BatchNorm of the producer is folded in, W'[o][c] = W[o][c] * rstd_c, bias'[o] = b[o] - sum_c W''[o][c] * mean_c, where W'' is
-// W' exactly as its fp16 hi + lo images represent it (so the weight rounding multiplies (y - mean), not y). Output: B
-// consecutive [blob Cin*Cout*4 bytes | colinv Cout floats] sets for 128-column tiles, and bias_sets [B][Cout].
-size_t tc_fold_set_bytes(int Cin, int Cout);
-int launch_fold_pack_weights(const float *Wt, const float *bias, const double *in_stats, const int *counts, int T, double eps,
-                             int Cin, int Cout, int B, void *blob_sets, float *bias_sets, cudaStream_t st);
 // TMA-fed persistent kernel with the A operand in tensor memory (tc3_layer.cu): BatchNorm-ed 128-column layers of the fused path
 bool tc3_layer_eligible(const LayerArgs &a);
 int launch_layer_tc3(const LayerArgs &a, int F, float *wpack, cudaStream_t st);
@@ -99,13 +89,8 @@ int launch_pixel_gemm_persistent(const LayerArgs &a, float *wpack, cudaStream_t 
 void set_pixel_persistent(int on);
 bool pixel_persistent_enabled();
 void set_tc3(int on);
-bool tc_persistent_enabled();
-bool tc_f16_enabled();
 bool tc_bf16_enabled();
 void set_tc_bf16(int on);  // 1: single-pass bf16 operands where LayerArgs::f16_ok (reduced precision, tolerance stated in the tests)
-void set_tc_f16(int on);   // 1 (default): 3xFP16 where LayerArgs::f16_ok, 0: 3xTF32 everywhere
-void set_tc_persist16(int on);   // 1: conv1 / fcn2 of the fused path through the persistent 3xFP16 kernel (TMEM double buffering; experimental)
-void set_tc_persistent(int on);  // 0 = one 256 x BN tile per CTA (default), 1 = persistent 256 x 128 kernel with overlapped epilogue
 // dispatch by mvx_set_gemm_mode(): 0 = SIMT everywhere, 1 = tensor cores where eligible (default)
 int gemm_mode();
 int launch_layer_auto(const LayerArgs &a, int F, float *wpack, cudaStream_t st);

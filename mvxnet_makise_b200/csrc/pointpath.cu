@@ -12,7 +12,6 @@
 #include "voxelize.cuh"
 #include "pointpath.cuh"
 
-#include <cstdlib>
 #include <vector>
 
 namespace mvx {
@@ -20,17 +19,13 @@ namespace mvx {
 const char *kRegionNames[R_COUNT] = {
     "vox_ws", "vox_coord", "vox_cnt", "vox_row0", "row_point", "row_vox", "cell2vid", "nhwc0", "nhwc1", "nhwc2",
     "vox8", "proj", "rowA_w", "A1", "Y1", "Y2", "Y3", "Y4", "Y5", "X6", "Y6", "X7", "Y7", "rowB_w", "rowB_v", "X8",
-    "vfeat", "stats", "vmax6", "vmax7", "vmax8", "wpack", "occ", "vfeat_t", "Z", "bin_count", "bin_start", "perm", "rowmax", "chmax", "A1max", "wfold", "bfold", "wbound", "Y8"};
+    "vfeat", "stats", "vmax6", "vmax7", "vmax8", "wpack", "occ", "vfeat_t", "Z", "bin_count", "bin_start", "perm", "rowmax", "chmax", "A1max", "Y8"};
 
 // 1 (default): pixel-first fcn1 - one tensor-core GEMM per FPN level over the map pixels, then a 12-corner combine per
 // point row (gather.cuh CombineArgs); 0: materialise the gathered (K,768) matrix A1 and run fcn1 over the point rows
 // (the layout the training-mode backward needs: dW1 = dpre1^T A1).
 static int g_fusion_mode = 1;
 int fusion_mode() { return g_fusion_mode; }
-static int g_apack = 1;     // MVX_APACK=0: channels-last fp32 copy + register producers for the pixel GEMM (A/B comparison)
-static int g_split_fill = 1;   // where the zero pass of the split grid fill (mvx_set_grid_mode(3)) starts: 1 after voxelization, 2 after the combine kernel, 3 after conv1
-static int g_fold = 0;         // mvx_set_fold_mode(1): fcn1_combine writes the rows as conv1's pre-packed fp16 A operand, conv1 runs with fcn1's BatchNorm folded into per-frame weights
-static int g_zero_ctas = 1;    // persistent CTAs per SM of the zero pass
 static int g_overlap = 1;   // 1: run the map branch of the pixel-first path on a side stream (mvx_set_fusion_mode(2) = pixel-first, serial)
 
 int make_layout(const mvx_pointpath_args_t *a, Layout &L) {
@@ -95,9 +90,6 @@ int make_layout(const mvx_pointpath_args_t *a, Layout &L) {
         take(R_ROWMAX, B * px * 4);
         take(R_CHMAX, B * 768 * 4);
         take(R_A1MAX, B * capA * 4);
-        take(R_WFOLD, B * tc_fold_set_bytes(768, 128));   // per-frame conv1 weights with fcn1's BatchNorm folded in (fold mode)
-        take(R_BFOLD, B * 128 * 4);
-        take(R_WBOUND, 4 * 4);
     }
     L.total = o;
     take(R_Y8, B * capB * 128 * 4);   // last region: only present in a training workspace
@@ -153,7 +145,6 @@ struct Stamp {
 struct SideStream {
     cudaStream_t stream = nullptr;
     cudaEvent_t fork = nullptr, join = nullptr;
-    cudaEvent_t occ = nullptr, zero = nullptr;   // split grid fill: occupancy bits ready (caller's stream) / zero pass done (side stream)
     int device = -1;
 };
 static int side_stream(SideStream **out) {
@@ -166,8 +157,6 @@ static int side_stream(SideStream **out) {
         MVX_CUDA_CHECK(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
         MVX_CUDA_CHECK(cudaEventCreateWithFlags(&s.fork, cudaEventDisableTiming));
         MVX_CUDA_CHECK(cudaEventCreateWithFlags(&s.join, cudaEventDisableTiming));
-        MVX_CUDA_CHECK(cudaEventCreateWithFlags(&s.occ, cudaEventDisableTiming));
-        MVX_CUDA_CHECK(cudaEventCreateWithFlags(&s.zero, cudaEventDisableTiming));
         s.device = dev;
     }
     *out = &s;
@@ -209,16 +198,6 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     auto F32 = [&](Region r) { return reinterpret_cast<float *>(ws + L.off[r]); };
     auto I32 = [&](Region r) { return reinterpret_cast<int *>(ws + L.off[r]); };
 
-#ifdef MVX_DEVTOOLS   // A/B switches for experiments; a release build reads no environment variable
-    static const bool env_read = [] {
-        if (const char *e = getenv("MVX_APACK")) g_apack = atoi(e);
-        if (const char *e = getenv("MVX_SPLIT_FILL")) g_split_fill = atoi(e);
-        if (const char *e = getenv("MVX_ZERO_CTAS")) g_zero_ctas = atoi(e);
-        if (const char *e = getenv("MVX_FOLD")) g_fold = atoi(e);
-        return true;
-    }();
-    (void)env_read;
-#endif
     const Stamp stamp(st);
     if (train) MVX_CUDA_CHECK(cudaMemsetAsync(I32(R_CHMAX), 0, (size_t)B * 768 * 4, st));
     // training keeps the gathered matrix A1 (dW1 = dpre1^T A1), so it always runs row-first
@@ -243,8 +222,7 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     // bf16 mode too: its per-pixel GEMM keeps the 3xFP16 products of the pre-packed operands (the persistent kernel is bound by its
     // loads and stores, not by the MMAs) and only writes Z as bf16; without the persistent kernel (gemm mode 12) the bf16 mode keeps its
     // channels-last copy + one-product kernel
-    const bool apack = pixel_first && tc_f16_enabled() && g_apack && (!tc_bf16_enabled() || pixel_persistent_enabled());
-    const bool fold = apack && g_fold;
+    const bool apack = pixel_first && (!tc_bf16_enabled() || pixel_persistent_enabled());
     // bf16 mode (mvx_set_gemm_mode(6)): the two largest intermediates - the per-pixel products Z and the raw fcn1 rows Y1 - are
     // stored as bf16 (half the bytes written and read back); every sum in between stays fp32
     const bool bf16_mem = pixel_first && tc_bf16_enabled();
@@ -326,23 +304,6 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     if (rc) return rc;
     }
 
-    // split grid fill: the zeros of the dense grid need only the occupancy bits. They go out on the side stream, behind the
-    // pixel GEMM, and stream to HBM under the combine / tensor-core layer kernels; the occupied sectors follow at the end
-    const bool split_fill = side && grid_split_fill() && a->grid_out && L.G % 32 == 0;
-    auto zero_pass = [&]() -> int {   // enqueued on the side stream once the caller's stream has reached this point
-        MVX_CUDA_CHECK(cudaEventRecord(side->occ, st));
-        MVX_CUDA_CHECK(cudaStreamWaitEvent(ms, side->occ, 0));
-        int r = launch_grid_zero_sectors(reinterpret_cast<unsigned *>(ws + L.off[R_OCC]), a->grid_out, B, L.G, 128, g_zero_ctas, ms);
-        if (r) return r;
-        MVX_CUDA_CHECK(cudaEventRecord(side->zero, ms));
-        return MVX_OK;
-    };
-    if (split_fill) {
-        MVX_REQUIRE((reinterpret_cast<uintptr_t>(a->grid_out) & 31) == 0, MVX_EINVAL, "grid_out must be 32-byte aligned");
-        rc = launch_occ_from_map(vo.cell2vid, reinterpret_cast<unsigned *>(ws + L.off[R_OCC]), B, L.G, st);
-        if (rc) return rc;
-        if (g_split_fill == 1) { rc = zero_pass(); if (rc) return rc; }
-    }
     stamp.mark(S_CLEAR);
     MVX_CUDA_CHECK(cudaMemsetAsync(stats, 0, (size_t)MVX_NUM_LAYERS * B * kStatStride * 8, st));
     zero_vmax_kernel<<<dim3(kSMs, B), 256, 0, st>>>(a->counts, cap, I32(R_VMAX6), I32(R_VMAX7), I32(R_VMAX8));
@@ -361,17 +322,6 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
         ca.bin_count = I32(R_BINCNT), ca.bin_start = I32(R_BINSTART), ca.perm = I32(R_PERM);
         ca.nbins = combine_bins(a->map_h[0], a->map_w[0]);
         ca.z_bf16 = ca.y1_bf16 = bf16_mem;
-        if (fold) {   // rows leave the combine kernel as conv1's pre-packed A operand (the idle A1 / Y1 regions hold it)
-            ca.y1pack = reinterpret_cast<unsigned char *>(ws + L.off[R_A1]), ca.y1_rowinv = F32(R_A1MAX), ca.pack_tiles = (int)ceil_div(L.capA, 256);
-            ca.wbound = F32(R_WBOUND);
-            size_t boff = 0;
-            for (int lv = 0; lv < MVX_NUM_LEVELS; ++lv) {
-                ca.pix_bound[lv] = F32(R_ROWMAX) + boff;
-                boff += (size_t)B * a->map_h[lv] * a->map_w[lv];
-            }
-            rc = launch_fcn1_bounds(a->wt[0], a->bias[0], F32(R_WBOUND), st);
-            if (rc) return rc;
-        }
         rc = launch_combine_sort(ca, B, st);      // needs only the projections: still part of the point branch
         if (rc) return rc;
     }
@@ -391,7 +341,6 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
         if (l == 0 && pixel_first) {
             rc = launch_combine_rows(ca, B, st);
             if (rc) return rc;
-            if (split_fill && g_split_fill == 2) { rc = zero_pass(); if (rc) return rc; }
             continue;
         }
         LayerArgs la{};
@@ -404,20 +353,8 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
         la.f16_ok = 1;       // BatchNorm-ed inputs; fcn1 row-first reads raw gathered features: per-row power-of-two scaling
         if (l == 0) la.row_max = F32(R_A1MAX);
         if (l == 1) la.x_bf16 = bf16_mem;   // conv1 reads the bf16 Y1 of the combine kernel
-        if (l == 1 && fold) {   // conv1 on the packed rows: fcn1's BatchNorm lives in per-frame weights and biases
-            rc = launch_fold_pack_weights(a->wt[1], a->bias[1], stat_of(0), a->counts, T, a->bn_eps, 768, 128, B, ws + L.off[R_WFOLD],
-                                          F32(R_BFOLD), st);
-            if (rc) return rc;
-            la.X = nullptr, la.in_stats = nullptr;
-            la.a_pack = ws + L.off[R_A1], la.a_rowinv = F32(R_A1MAX), la.a_frame_tiles = (int)ceil_div(L.capA, 256);
-            la.w_per_frame = 1, la.bias = F32(R_BFOLD);
-            rc = launch_layer_auto(la, B, reinterpret_cast<float *>(ws + L.off[R_WFOLD]), st);
-            if (rc) return rc;
-            continue;
-        }
         rc = launch_layer_auto(la, B, F32(R_WPACK), st);
         if (rc) return rc;
-        if (split_fill && g_split_fill == 3 && l == 1) { rc = zero_pass(); if (rc) return rc; }
     }
     VfePrepArgs vp{};
     vp.B = B, vp.cap = cap, vp.capA = L.capA, vp.capB = L.capB, vp.T = T;
@@ -426,7 +363,7 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     vp.Y6 = F32(R_Y6), vp.vmax6 = I32(R_VMAX6), vp.X7 = F32(R_X7), vp.rowB_w = F32(R_ROWB_W), vp.rowB_v = I32(R_ROWB_V);
     vp.Y7 = F32(R_Y7), vp.vmax7 = I32(R_VMAX7), vp.X8 = F32(R_X8);
     vp.vmax8 = I32(R_VMAX8), vp.vfeat = F32(R_VFEAT);
-    vp.vfeat_t = (grid_mode() == 2 && L.G % 32 == 0 && a->grid_out && !split_fill) ? F32(R_VFEAT_T) : nullptr;
+    vp.vfeat_t = (L.G % 32 == 0 && a->grid_out) ? F32(R_VFEAT_T) : nullptr;
     vp.n5 = NormSrc{stat_of(4), a->counts, 0, T, a->bn_eps};
     vp.n6 = NormSrc{stat_of(5), a->counts, 0, T, a->bn_eps};
     vp.n7 = NormSrc{stat_of(6), a->counts, 0, T, a->bn_eps};
@@ -481,7 +418,7 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     stamp.mark(S_PREP3);
     // inference: the concat [norm7(Y7) | norm7(max7)] that prep_fcn materialises as X8 is built by the FCN's own
     // A-producer instead (16-bit tensor-core kernel); training keeps X8 (dW8 = dpre8^T X8)
-    const bool fuse_cat = !train && gemm_mode() == 1 && tc_f16_enabled();
+    const bool fuse_cat = !train && gemm_mode() == 1;
     if (!fuse_cat) {
         rc = launch_prep_fcn(vp, st);
         if (rc) return rc;
@@ -509,10 +446,7 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     // ---- stage 4 ----------------------------------------------------------------------------------------
     if (a->grid_out) {
         MVX_REQUIRE((reinterpret_cast<uintptr_t>(a->grid_out) & 15) == 0, MVX_EINVAL, "grid_out must be 16-byte aligned");
-        if (split_fill) {
-            MVX_CUDA_CHECK(cudaStreamWaitEvent(st, side->zero, 0));
-            rc = launch_grid_patch_sectors(a->counts, vo.vox_coord, vo.cell2vid, F32(R_VFEAT), cap, a->grid_out, B, L.G, 128, st);
-        } else if (vp.vfeat_t) {
+        if (vp.vfeat_t) {
             unsigned *occ = reinterpret_cast<unsigned *>(ws + L.off[R_OCC]);
             rc = launch_occ_from_map(vo.cell2vid, occ, B, L.G, st);
             if (rc) return rc;
@@ -589,8 +523,8 @@ extern "C" const char *mvx_pointpath_layout_name(int32_t region) {
 extern "C" int mvx_pointpath_forward(const mvx_pointpath_args_t *args) { return mvx::pointpath_forward(args, false); }
 
 extern "C" int mvx_set_fold_mode(int32_t mode) {
-    if (mode < 0 || mode > 2) return MVX_EINVAL;
-    mvx::g_fold = mode == 1;
+    // 1 (conv1 with fcn1's BatchNorm folded into per-frame weights) was removed: measured slower
+    MVX_REQUIRE(mode == 0 || mode == 2, MVX_EINVAL, "fold mode must be 0 or 2");
     mvx::set_combine_v1(mode == 2);
     return MVX_OK;
 }

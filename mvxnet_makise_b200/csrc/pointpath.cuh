@@ -8,7 +8,7 @@ namespace mvx {
 enum Region {
     R_VOXWS = 0, R_VOX_COORD, R_VOX_CNT, R_VOX_ROW0, R_ROW_POINT, R_ROW_VOX, R_CELL2VID, R_NHWC0, R_NHWC1, R_NHWC2,
     R_VOX8, R_PROJ, R_ROWA_W, R_A1, R_Y1, R_Y2, R_Y3, R_Y4, R_Y5, R_X6, R_Y6, R_X7, R_Y7, R_ROWB_W, R_ROWB_V, R_X8,
-    R_VFEAT, R_STATS, R_VMAX6, R_VMAX7, R_VMAX8, R_WPACK, R_OCC, R_VFEAT_T, R_Z, R_BINCNT, R_BINSTART, R_PERM, R_ROWMAX, R_CHMAX, R_A1MAX, R_WFOLD, R_BFOLD, R_WBOUND, R_Y8, R_COUNT
+    R_VFEAT, R_STATS, R_VMAX6, R_VMAX7, R_VMAX8, R_WPACK, R_OCC, R_VFEAT_T, R_Z, R_BINCNT, R_BINSTART, R_PERM, R_ROWMAX, R_CHMAX, R_A1MAX, R_Y8, R_COUNT
 };
 static_assert(R_COUNT <= MVX_WS_REGIONS, "too many regions");
 

@@ -49,7 +49,7 @@ __global__ void __launch_bounds__(256) grid_fill_kernel(const int *__restrict__ 
     }
 }
 
-// ---- plane-sequential variant (default) -----------------------------------------------------------------
+// ---- plane-sequential variant (every grid whose cell count is a multiple of 32) ----------------------------
 // HBM only reaches its write peak (7.5 TB/s measured for a plain fill) when the CTAs of a wave write one long
 // contiguous region. So the launch order walks ONE channel plane at a time: blockIdx.x = 32 KB run of cells,
 // blockIdx.y = channel, blockIdx.z = frame. Per run a CTA reads 1 KB of occupancy bits (not the 32 KB int map);
@@ -83,69 +83,6 @@ __global__ void __launch_bounds__(256) grid_fill_planes_kernel(const unsigned *_
     }
 }
 
-// ---- split fill: zeros early, occupied sectors late ---------------------------------------------------------------------
-// 98.5 % of the grid is zeros whose positions are known right after voxelization, long before the features exist. The
-// zero pass writes every EMPTY 32-byte sector (8 cells of one channel plane) and can therefore run on a side stream under the
-// tensor-/latency-bound layer kernels; the patch pass at the end of the chain writes only the sectors that hold a voxel
-// (about 12 % of the bytes), whole sectors, so neither pass ever needs a read-modify-write.
-//
-// Zero pass: ONE persistent CTA per SM (256 threads, <= 32 registers: it fits next to a 576-thread tensor-core CTA in
-// the register file instead of displacing it), walking the (frame, plane, run) items plane-sequentially like the fused fill.
-__global__ void __launch_bounds__(256) grid_zero_sectors_kernel(const unsigned *__restrict__ occ, float *__restrict__ out, long long G,
-                                                                int C, int B) {
-    const int tid = threadIdx.x;
-    const int runs = (int)((G + kRunCells - 1) / kRunCells);
-    const long long items = (long long)runs * C * B;
-    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (long long it = blockIdx.x; it < items; it += gridDim.x) {
-        const int run = (int)(it % runs);
-        const long long pc = it / runs;          // f * C + c
-        const int f = (int)(pc / C);
-        const long long cell0 = (long long)run * kRunCells;
-        const unsigned *bits = occ + (size_t)f * (G / 32) + cell0 / 32;
-        float *o = out + (size_t)pc * G + cell0;
-        const int nrun = (int)min((long long)kRunCells, G - cell0);
-#pragma unroll
-        for (int i = 0; i < kRunCells / 1024; ++i) {
-            const int cell = i * 1024 + tid * 4;
-            if (cell < nrun) {
-                const unsigned sector = (__ldg(bits + (cell >> 5)) >> (cell & 24)) & 0xFFu;   // the 8 cells of this 32-byte sector
-                if (sector == 0) st_cs_f4(reinterpret_cast<float4 *>(o + cell), z);
-            }
-        }
-    }
-}
-
-// Patch pass: one warp per voxel. The voxel whose cell is the first occupied one of its sector writes the sector for all C
-// channels (lane = channel: the feature rows are read coalesced, every store is one full 32-byte sector).
-__global__ void __launch_bounds__(256) grid_patch_sectors_kernel(const int *__restrict__ counts, const int *__restrict__ vox_coord,
-                                                                 const int *__restrict__ cell2vid, const float *__restrict__ feat,
-                                                                 int vcap, float *__restrict__ out, long long G, int C) {
-    const int f = blockIdx.y, lane = threadIdx.x & 31;
-    const int v = blockIdx.x * 8 + (threadIdx.x >> 5);
-    if (v >= counts[f * 4 + 0]) return;
-    const int cell = vox_coord[((size_t)f * vcap + v) * 4 + 3];
-    if (cell < 0) return;
-    const int sb = cell & ~7;
-    const int4 m0 = __ldg(reinterpret_cast<const int4 *>(cell2vid + (size_t)f * G + sb));
-    const int4 m1 = __ldg(reinterpret_cast<const int4 *>(cell2vid + (size_t)f * G + sb + 4));
-    const int vid[8] = {m0.x, m0.y, m0.z, m0.w, m1.x, m1.y, m1.z, m1.w};
-    int first = 0;
-#pragma unroll
-    for (int j = 7; j >= 0; --j)
-        if (vid[j] >= 0) first = j;
-    if (first != (cell & 7)) return;   // another voxel of this sector writes it
-    const float *ff = feat + (size_t)f * vcap * C;
-    for (int c = lane; c < C; c += 32) {
-        float q[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) q[j] = vid[j] >= 0 ? __ldg(ff + (size_t)vid[j] * C + c) : 0.f;
-        float *o = out + ((size_t)f * C + c) * G + sb;
-        st_cs_f4(reinterpret_cast<float4 *>(o), make_float4(q[0], q[1], q[2], q[3]));
-        st_cs_f4(reinterpret_cast<float4 *>(o + 4), make_float4(q[4], q[5], q[6], q[7]));
-    }
-}
-
 __global__ void __launch_bounds__(256) occ_from_map_kernel(const int *__restrict__ cell2vid, unsigned *__restrict__ occ, long long G) {
     const int f = blockIdx.y;
     const long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // one thread per 32 cells
@@ -160,68 +97,6 @@ __global__ void __launch_bounds__(256) occ_from_map_kernel(const int *__restrict
     occ[(size_t)f * (G / 32) + w] = bits;
 }
 
-// ---- bulk-store variant (TMA engine) -------------------------------------------------------------------
-// A CTA owns kTileCells consecutive cells of one frame and a group of channels. Two shared-memory images of the tile
-// are zeroed once; for every channel the (few) occupied cells are patched with feat[vid][c] and the whole 32 KB run
-// of that channel plane leaves through ONE cp.async.bulk shared->global store (SASS UBLKCP). The occupied positions
-// are the same for every channel, so the images never need re-zeroing. 98.5 % of the grid is written without
-// a single per-thread store instruction.
-constexpr int kTileCells = 8192;            // 32 KB per channel plane per store
-constexpr int kCellsPerThread = kTileCells / 256;
-
-__device__ __forceinline__ void bulk_s2g(void *dst, uint32_t src_smem, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src_smem), "r"(bytes) : "memory");
-}
-
-__global__ void __launch_bounds__(256) grid_fill_bulk_kernel(const int *__restrict__ cell2vid, const float *__restrict__ feat,
-                                                             float *__restrict__ out, long long G, int C, int vcap, int cgroups) {
-    extern __shared__ __align__(128) float tile[];  // [2][kTileCells]
-    const int f = blockIdx.z, cg = blockIdx.y, cper = C / cgroups, tid = threadIdx.x;
-    const long long cell0 = (long long)blockIdx.x * kTileCells;
-    const int ncell = (int)min((long long)kTileCells, G - cell0);
-    const int *map = cell2vid + (size_t)f * G + cell0;
-    const float *ff = feat + (size_t)f * vcap * C + (size_t)cg * cper;
-    float *o = out + ((size_t)f * C + (size_t)cg * cper) * G + cell0;
-
-    // this thread's 32 consecutive cells: occupancy mask (vids are re-read from L1/L2 when the mask is non-zero)
-    unsigned mask = 0;
-    const int base = tid * kCellsPerThread;
-#pragma unroll
-    for (int q = 0; q < kCellsPerThread / 4; ++q) {
-        const int cidx = base + q * 4;
-        if (cidx < ncell) {  // ncell is a multiple of 4
-            const int4 v = __ldg(reinterpret_cast<const int4 *>(map + cidx));
-            mask |= (v.x >= 0 ? 1u : 0u) << (q * 4) | (v.y >= 0 ? 2u : 0u) << (q * 4) | (v.z >= 0 ? 4u : 0u) << (q * 4) |
-                    (v.w >= 0 ? 8u : 0u) << (q * 4);
-        }
-    }
-    const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int i = tid; i < 2 * kTileCells / 4; i += 256) reinterpret_cast<float4 *>(tile)[i] = z4;
-    __syncthreads();
-    const uint32_t tile_s = (uint32_t)__cvta_generic_to_shared(tile);
-    for (int c = 0; c < cper; ++c) {
-        float *img = tile + (c & 1) * kTileCells;
-        if (c >= 2) {  // the store issued two channels ago must have finished READING this image
-            if (tid == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-            __syncthreads();
-        }
-        unsigned m = mask;
-        while (m) {
-            const int j = __ffs(m) - 1;
-            m &= m - 1;
-            const int vid = __ldg(map + base + j);
-            img[base + j] = __ldg(ff + (size_t)vid * C + c);
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncthreads();
-        if (tid == 0) {
-            bulk_s2g(o + (size_t)c * G, tile_s + (c & 1) * kTileCells * 4, (uint32_t)ncell * 4u);
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-        }
-    }
-    if (tid == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-}
-
 __global__ void __launch_bounds__(256) map_from_idx_kernel(const long long *__restrict__ idx, long long N, int nx, int ny,
                                                            int nz, int *__restrict__ map) {
     const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -233,8 +108,6 @@ __global__ void __launch_bounds__(256) map_from_idx_kernel(const long long *__re
 }
 
 }  // namespace
-
-static int g_grid_mode = 2;  // 2 = plane-sequential + occupancy bits (default), 0 = cell-major streaming, 1 = bulk stores
 
 int launch_occ_from_map(const int *cell2vid, unsigned *occ, int B, long long G, cudaStream_t st) {
     dim3 grid((unsigned)ceil_div(G / 32, 256), B);
@@ -252,53 +125,15 @@ int launch_grid_fill_planes(const unsigned *occ, const int *cell2vid, const floa
     return MVX_OK;
 }
 
-int launch_grid_zero_sectors(const unsigned *occ, float *out, int B, long long G, int C, int ctas_per_sm, cudaStream_t st) {
-    MVX_REQUIRE(G % 32 == 0 && ctas_per_sm >= 1, MVX_EINVAL, "split grid fill needs a cell count divisible by 32");
-    grid_zero_sectors_kernel<<<kSMs * ctas_per_sm, 256, 0, st>>>(occ, out, G, C, B);
-    MVX_LAUNCH_CHECK();
-    return MVX_OK;
-}
-
-int launch_grid_patch_sectors(const int *counts, const int *vox_coord, const int *cell2vid, const float *feat, int vcap, float *out,
-                              int B, long long G, int C, cudaStream_t st) {
-    dim3 grid((unsigned)ceil_div(vcap, 8), B);
-    grid_patch_sectors_kernel<<<grid, 256, 0, st>>>(counts, vox_coord, cell2vid, feat, vcap, out, G, C);
-    MVX_LAUNCH_CHECK();
-    return MVX_OK;
-}
-
-int grid_mode() { return g_grid_mode == 3 ? 2 : g_grid_mode; }   // mode 3 = mode 2 kernels, split in time by the fused path
-bool grid_split_fill() { return g_grid_mode == 3; }
-
 int launch_grid_fill(const int *cell2vid, const float *feat, float *out, int B, long long G, int C, int vcap, cudaStream_t st) {
     const int cgroups = (C % 4 == 0) ? 4 : 1;
-    if (g_grid_mode == 1 && G % 4 == 0) {
-        static bool attr_set = false;
-        const int smem = 2 * kTileCells * (int)sizeof(float);
-        if (!attr_set) {
-            MVX_CUDA_CHECK(cudaFuncSetAttribute(grid_fill_bulk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            attr_set = true;
-        }
-        dim3 grid((unsigned)ceil_div(G, kTileCells), cgroups, B);
-        grid_fill_bulk_kernel<<<grid, 256, smem, st>>>(cell2vid, feat, out, G, C, vcap, cgroups);
-        MVX_LAUNCH_CHECK();
-        return MVX_OK;
-    }
     dim3 grid((unsigned)ceil_div(G, kCellsPerBlock), cgroups, B);
     grid_fill_kernel<<<grid, 256, 0, st>>>(cell2vid, feat, out, G, C, vcap, cgroups);
     MVX_LAUNCH_CHECK();
     return MVX_OK;
 }
 
-void set_grid_mode(int m) { g_grid_mode = m; }
-
 }  // namespace mvx
-
-extern "C" int mvx_set_grid_mode(int32_t mode) {
-    if (mode < 0 || mode > 3) return MVX_EINVAL;
-    mvx::set_grid_mode(mode);
-    return MVX_OK;
-}
 
 extern "C" int mvx_scatter_dense(const float *feat, const int64_t *idx, int64_t N, int32_t C, int32_t nx, int32_t ny,
                                  int32_t nz, float *out, int32_t *map_ws, void *stream) {
@@ -314,7 +149,7 @@ extern "C" int mvx_scatter_dense(const float *feat, const int64_t *idx, int64_t 
                                                                                ny, nz, map_ws);
         MVX_LAUNCH_CHECK();
     }
-    if (mvx::grid_mode() == 2 && G % 32 == 0) {  // map_ws holds G map entries followed by G/32 occupancy words
+    if (G % 32 == 0) {  // map_ws holds G map entries followed by G/32 occupancy words
         unsigned *occ = reinterpret_cast<unsigned *>(map_ws + G);
         int rc = mvx::launch_occ_from_map(map_ws, occ, 1, G, st);
         if (rc) return rc;

@@ -9,12 +9,4 @@ int launch_occ_from_map(const int *cell2vid, unsigned *occ, int B, long long G, 
 // plane-sequential fill: feat element (v, c) of frame f at feat[f*feat_frame_stride + v*feat_vs + c*feat_cs]
 int launch_grid_fill_planes(const unsigned *occ, const int *cell2vid, const float *feat, long long feat_frame_stride, int feat_vs,
                             int feat_cs, float *out, int B, long long G, int C, cudaStream_t st);
-// split fill (fused path, overlapped): every empty 32-byte sector is zeroed from the occupancy bits alone (side stream, right after
-// voxelization); the sectors that hold a voxel are written whole once the features exist. feat (B, vcap, C) voxel-major.
-int launch_grid_zero_sectors(const unsigned *occ, float *out, int B, long long G, int C, int ctas_per_sm, cudaStream_t st);
-int launch_grid_patch_sectors(const int *counts, const int *vox_coord, const int *cell2vid, const float *feat, int vcap, float *out,
-                              int B, long long G, int C, cudaStream_t st);
-int grid_mode();
-bool grid_split_fill();   // mvx_set_grid_mode(3): early zero pass + late patch of the occupied sectors (fused path, experimental)
-void set_grid_mode(int m);  // 2 = plane-sequential (default), 0 = cell-major streaming stores, 1 = bulk-store (TMA) kernel
 }  // namespace mvx

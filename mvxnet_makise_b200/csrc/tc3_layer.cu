@@ -825,7 +825,7 @@ int launch_tc3_t(const T3Args &g, const CUtensorMap &tmX, const CUtensorMap &tmY
 }  // namespace
 
 bool tc3_layer_eligible(const LayerArgs &a) {
-    if (!(a.f16_ok && a.in_stats && a.counts && !a.row_max && !a.plain && !a.a_pack && !a.w_per_frame)) return false;
+    if (!(a.f16_ok && a.in_stats && a.counts && !a.row_max && !a.plain && !a.a_pack)) return false;
     if (a.Cout != T3_BN || a.Cin % (2 * T3_KB) != 0 || (a.Cin != 128 && a.Cin % (3 * T3_KB) != 0) || a.Cin > 768 || (a.rows_mode != 1 && a.rows_mode != 2)) return false;
     if (a.rowcap % T3_TM != 0 || a.ldx % 4 != 0 || (a.Y && a.ldy % 4 != 0)) return false;
     if (a.vmax && !a.row_v) return false;
@@ -881,7 +881,7 @@ bool pixel_persistent_enabled() { return g_pixel_persistent != 0; }
 
 bool pixel_gemm_persistent_eligible(const LayerArgs &a) {
     return g_pixel_persistent && a.plain && a.a_pack && a.Y && !a.counts && a.rows_fixed > 0 && a.Cin % PG_KB == 0 && a.Cout % PG_BN == 0 &&
-           a.Cout <= 768 && a.ldy % 8 == 0 && !a.w_per_frame;
+           a.Cout <= 768 && a.ldy % 8 == 0;
 }
 
 int launch_pixel_gemm_persistent(const LayerArgs &a, float *wpack, cudaStream_t st) {

@@ -29,7 +29,6 @@ namespace {
 
 constexpr int kTM = 256;        // rows per CTA
 constexpr int kStages = 3;
-constexpr int kProducerThreads = 256;
 constexpr int kEpiCols = 128;   // columns per epilogue pass
 constexpr int kEpiLd = kEpiCols + 4;
 
@@ -111,63 +110,6 @@ __global__ void __launch_bounds__(256) pack_weights_f16_kernel(const float *__re
     }
 }
 
-// Folded-BatchNorm weight sets (see layers.cuh): one CTA per (output column, frame), 128-column tile images.
-__global__ void __launch_bounds__(256) fold_pack_weights_kernel(const float *__restrict__ Wt, const float *__restrict__ bias,
-                                                                const double *__restrict__ in_stats, const int *__restrict__ counts,
-                                                                int T, double eps, int Cin, int Cout, uint8_t *__restrict__ sets,
-                                                                float *__restrict__ bias_sets) {
-    __shared__ float s_max[256];
-    __shared__ double s_sum[256];
-    const int n = blockIdx.x, f = blockIdx.y, tid = threadIdx.x;
-    const double R = (double)counts[f * 4 + 0] * (double)T;
-    const size_t set_bytes = (size_t)Cin * Cout * 4 + (size_t)Cout * 4;
-    uint8_t *out = sets + (size_t)f * set_bytes;
-    float mx = 0.f;
-    for (int k = tid; k < Cin; k += 256) {
-        const double *st = in_stats + ((size_t)f * Cin + k) * 2;
-        const double m = st[0] / R;
-        double var = st[1] / R - m * m;
-        var = var < 0.0 ? 0.0 : var;
-        const float rstd = (float)(1.0 / sqrt(var + eps));
-        mx = fmaxf(mx, fabsf(Wt[(size_t)k * Cout + n] * rstd));
-    }
-    s_max[tid] = mx;
-    __syncthreads();
-    for (int s = 128; s > 0; s >>= 1) {
-        if (tid < s) s_max[tid] = fmaxf(s_max[tid], s_max[tid + s]);
-        __syncthreads();
-    }
-    const float sc = pow2_scale(s_max[0]);
-    const double inv = 1.0 / (double)sc;
-    double acc = 0.0;
-    for (int k = tid; k < Cin; k += 256) {
-        const double *st = in_stats + ((size_t)f * Cin + k) * 2;
-        const double m = st[0] / R;
-        double var = st[1] / R - m * m;
-        var = var < 0.0 ? 0.0 : var;
-        const float rstd = (float)(1.0 / sqrt(var + eps));
-        const float v = Wt[(size_t)k * Cout + n] * rstd * sc;
-        const __half h = __float2half_rn(v);
-        const __half l = __float2half_rn(v - __half2float(h));
-        acc += ((double)__half2float(h) + (double)__half2float(l)) * inv * m;
-        const int kc = k >> 5, kl = k & 31;
-        const size_t blob = (size_t)kc * (2 * 128 * 64);   // bytes; one 128-column tile (Cout == 128)
-        const uint32_t off = sw64_offset(n, kl >> 3) + (kl & 7) * 2;
-        *reinterpret_cast<__half *>(out + blob + off) = h;
-        *reinterpret_cast<__half *>(out + blob + 128 * 64 + off) = l;
-    }
-    s_sum[tid] = acc;
-    __syncthreads();
-    for (int s = 128; s > 0; s >>= 1) {
-        if (tid < s) s_sum[tid] += s_sum[tid + s];
-        __syncthreads();
-    }
-    if (tid == 0) {
-        reinterpret_cast<float *>(out + (size_t)Cin * Cout * 4)[n] = 1.f / sc;
-        bias_sets[(size_t)f * Cout + n] = (float)((double)bias[n] - s_sum[0]);
-    }
-}
-
 // BF1: single-pass bf16 operands (no lo parts, one MMA per K-step, no scaling: bf16 has the fp32 exponent range) - the
 // reduced-precision mode whose tolerance is stated separately (tests/test_gpu_parity.py::test_bf16_mode_tolerance).
 // TWO: two CTAs per SM (BN = 128, 16-bit operands): 2 pipeline stages, the epilogue staged one 128-row half at a time (96 KB of
@@ -230,12 +172,10 @@ __global__ void __launch_bounds__(tc_producer_warps(F16, TWO) * 32 + 64, TWO ? 2
             s_rstd[c] = (float)(1.0 / sqrt(var + a.eps));
         }
     }
-    for (int c = tid; c < BN; c += NT) s_bias[c] = a.plain ? 0.f : a.bias[(a.w_per_frame ? (size_t)f * a.Cout : 0) + n0 + c];
+    for (int c = tid; c < BN; c += NT) s_bias[c] = a.plain ? 0.f : a.bias[n0 + c];
     if constexpr (F16) {
-        // [blob: Cin*Cout*4 bytes | colinv: Cout floats], one such set per frame when the weights are per frame
-        const size_t wset = (size_t)a.Cin * a.Cout * 4 + (size_t)a.Cout * 4;
-        const uint8_t *wbase = reinterpret_cast<const uint8_t *>(wpack) + (a.w_per_frame ? (size_t)f * wset : 0);
-        const float *colinv = reinterpret_cast<const float *>(wbase + (size_t)a.Cin * a.Cout * 4);
+        // [blob: Cin*Cout*4 bytes | colinv: Cout floats]
+        const float *colinv = reinterpret_cast<const float *>(reinterpret_cast<const uint8_t *>(wpack) + (size_t)a.Cin * a.Cout * 4);
         for (int c = tid; c < BN; c += NT) s_colinv[c] = colinv[n0 + c];
         for (int r = tid; r < kTM; r += NT) {
             const long long rr = row0 + r;
@@ -430,14 +370,13 @@ __global__ void __launch_bounds__(tc_producer_warps(F16, TWO) * 32 + 64, TWO ? 2
         // ================= B producer: one bulk copy per stage ===================================================
         if (lane == 0) {
             const float *src = wpack + (size_t)ctile * nk * (2 * BN * kBK);
-            if (F16 && a.w_per_frame) src += (size_t)f * (((size_t)a.Cin * a.Cout * 4 + (size_t)a.Cout * 4) / 4);
             for (int kc = 0; kc < nk; ++kc) {
                 const int s = kc % STAGES;
                 const uint32_t ph = (kc / STAGES) & 1;
                 mbar_wait(empty_bar(s), ph ^ 1);
                 if constexpr (APK) {
                     mbar_arrive_expect_tx(full_bar(s), 2 * S::kAHalf + 2 * S::kBHalf);
-                    const uint8_t *asrc = static_cast<const uint8_t *>(a.a_pack) + (((size_t)f * a.a_frame_tiles + blockIdx.y) * nk + kc) * (2 * S::kAHalf);
+                    const uint8_t *asrc = static_cast<const uint8_t *>(a.a_pack) + ((size_t)blockIdx.y * nk + kc) * (2 * S::kAHalf);
                     bulk_g2s(sbase + s * S::kStage, asrc, 2 * S::kAHalf, full_bar(s));
                 } else {
                     mbar_arrive_expect_tx(full_bar(s), 2 * S::kBHalf);
@@ -641,9 +580,7 @@ int launch_tc(const LayerArgs &a, int F, float *wpack, cudaStream_t st) {
         attr_set = true;
     }
     const int total = a.Cin * a.Cout;
-    if (a.w_per_frame) {
-        // the caller packed one [blob | colinv] set per frame (folded BatchNorm): nothing to do here
-    } else if (F16) {   // [fp16 hi|lo images: Cin*Cout*4 bytes][inverse column scales: Cout floats]
+    if (F16) {   // [fp16 hi|lo images: Cin*Cout*4 bytes][inverse column scales: Cout floats]
         uint8_t *blob = reinterpret_cast<uint8_t *>(wpack);
         pack_weights_f16_kernel<BN, BF1><<<a.Cout, 256, 0, st>>>(a.Wt, a.Cin, a.Cout, blob, reinterpret_cast<float *>(blob + (size_t)total * 4));
     } else {
@@ -657,681 +594,6 @@ int launch_tc(const LayerArgs &a, int F, float *wpack, cudaStream_t st) {
     return MVX_OK;
 }
 
-
-// =====================================================================================================================
-// Persistent variant (layers without a per-voxel max: fcn1, conv1, fcn2). One CTA per SM walks the (frame, row tile,
-// column tile) list; the epilogue has its own four warps and works from registers (no shared staging tile), so while
-// tile i drains from TMEM the producers already fill the stages of tile i+1 and the tensor pipe only idles for the
-// TMEM drain itself:
-//   warps 0-7  A producers      warp 8  B bulk-copy producer      warp 9  MMA issuer (+ TMEM alloc)
-//   warps 10-13 epilogue: tcgen05.ld -> bias/ReLU -> direct 16-byte row stores; column sums by a 31-shuffle butterfly
-//               transpose-reduction per 32x32 block (fp32 inside a warp's 32 rows, fp64 across warps/tiles/CTAs).
-// =====================================================================================================================
-constexpr int kPThreads = 14 * 32;
-constexpr int kPStages = 4;    // 48 KB per stage at BN = 128
-constexpr int kAccBufs = 2;    // TMEM accumulator ping-pong: 2 x (2 halves x BN columns) = 512 columns
-
-template <int BN>
-struct PSmem {
-    static constexpr int kAHalf = kTM * kBK * 4;
-    static constexpr int kBHalf = BN * kBK * 4;
-    static constexpr int kStage = 2 * kAHalf + 2 * kBHalf;
-    static constexpr int kTiles = kPStages * kStage;
-    static constexpr int kMean = kTiles;
-    static constexpr int kRstd = kMean + 768 * 4;
-    static constexpr int kPart = kRstd + 768 * 4;              // [4 warps][BN][2] fp64 column partials
-    static constexpr int kBars = kPart + 4 * BN * 2 * 8;       // full[4], empty[4], accum_full[2], tmem_empty[2]
-    static constexpr int kTmemPtr = kBars + 8 * (2 * kPStages + 2 * kAccBufs);
-    static constexpr int kTotal = kTmemPtr + 16 + 1024;
-};
-
-template <int BN>
-__global__ void __launch_bounds__(kPThreads, 1) tc_layer_persist_kernel(LayerArgs a, const float *__restrict__ wpack, int F,
-                                                                         int row_tiles, int col_tiles) {
-    using S = PSmem<BN>;
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t *smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    const uint32_t sbase = smem_u32(smem);
-    float *s_mean = reinterpret_cast<float *>(smem + S::kMean);
-    float *s_rstd = reinterpret_cast<float *>(smem + S::kRstd);
-    double *s_part = reinterpret_cast<double *>(smem + S::kPart);
-    const uint32_t bars = sbase + S::kBars;
-    auto full_bar = [&](int s) { return bars + 8u * s; };
-    auto empty_bar = [&](int s) { return bars + 8u * (kPStages + s); };
-    auto accum_bar = [&](int b) { return bars + 8u * (2 * kPStages + b); };
-    auto tmem_empty_bar = [&](int b) { return bars + 8u * (2 * kPStages + kAccBufs + b); };
-    volatile uint32_t *tmem_ptr = reinterpret_cast<volatile uint32_t *>(smem + S::kTmemPtr);
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int nk = a.Cin / kBK;
-    const int total = F * row_tiles * col_tiles;
-
-    // tile decode shared by every role: identical decisions => identical pipeline phase bookkeeping
-    auto decode = [&](int t, int &f, int &ct, long long &row0, long long &n_rows) -> bool {
-        ct = t % col_tiles;
-        const int rt = (t / col_tiles) % row_tiles;
-        f = t / (col_tiles * row_tiles);
-        n_rows = a.rows_fixed;
-        if (a.counts) {
-            const int N = a.counts[f * 4 + 0], K = a.counts[f * 4 + 1];
-            n_rows = a.rows_mode == 1 ? K + 1 : (a.rows_mode == 2 ? K + N : a.rows_fixed);
-        }
-        row0 = (long long)rt * kTM;
-        return row0 < n_rows;
-    };
-
-    if (tid == 0) {
-        for (int s = 0; s < kPStages; ++s) {
-            mbar_init(full_bar(s), kProducerThreads + 1);
-            mbar_init(empty_bar(s), 1);
-        }
-        for (int b = 0; b < kAccBufs; ++b) {
-            mbar_init(accum_bar(b), 1);
-            mbar_init(tmem_empty_bar(b), 4);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 9) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(sbase + S::kTmemPtr), "r"(kAccBufs * 2 * BN)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr;
-
-    if (warp < 8) {
-        // ================= A producers ===========================================================================
-        const int c = tid & 3, rsub = tid >> 2;
-        const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        int g = 0, cur_f = -1;  // global chunk counter of this CTA (ring position), frame whose BN coefficients are loaded
-        for (int t = blockIdx.x; t < total; t += gridDim.x) {
-            int f, ct;
-            long long row0, n_rows;
-            if (!decode(t, f, ct, row0, n_rows)) continue;
-            if (a.in_stats && f != cur_f) {  // BatchNorm coefficients of the producer layer for this frame
-                named_bar_sync(1, kProducerThreads);
-                const double Rstat = a.counts ? (double)a.counts[f * 4 + 0] * (double)a.T : (double)a.rows_fixed;
-                for (int cc = tid; cc < a.Cin; cc += kProducerThreads) {
-                    const double *st = a.in_stats + ((size_t)f * a.Cin + cc) * 2;
-                    const double m = st[0] / Rstat;
-                    double var = st[1] / Rstat - m * m;
-                    var = var < 0.0 ? 0.0 : var;
-                    s_mean[cc] = (float)m;
-                    s_rstd[cc] = (float)(1.0 / sqrt(var + a.eps));
-                }
-                named_bar_sync(1, kProducerThreads);
-            }
-            cur_f = f;
-            const float *Xf = a.X + ((size_t)f * a.rowcap + row0) * a.ldx + c * 4;
-            bool valid[4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) valid[i] = row0 + rsub + 64 * i < n_rows;
-            auto load_chunk = [&](float4 (&buf)[4], int kc) {
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    buf[i] = valid[i] ? __ldg(reinterpret_cast<const float4 *>(Xf + (size_t)(rsub + 64 * i) * a.ldx + kc * kBK)) : z4;
-            };
-            auto produce = [&](float4 (&buf)[4], int kc) {
-                float4 cur[4];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) cur[i] = buf[i];
-                if (a.in_stats) {
-                    const int k = kc * kBK + c * 4;
-                    const float m0 = s_mean[k], m1 = s_mean[k + 1], m2 = s_mean[k + 2], m3 = s_mean[k + 3];
-                    const float r0 = s_rstd[k], r1 = s_rstd[k + 1], r2 = s_rstd[k + 2], r3 = s_rstd[k + 3];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        if (valid[i]) {
-                            cur[i].x = (cur[i].x - m0) * r0;
-                            cur[i].y = (cur[i].y - m1) * r1;
-                            cur[i].z = (cur[i].z - m2) * r2;
-                            cur[i].w = (cur[i].w - m3) * r3;
-                        }
-                    }
-                }
-                if (kc + 2 < nk) load_chunk(buf, kc + 2);
-                const int s = g % kPStages;
-                const uint32_t ph = (g / kPStages) & 1;
-                ++g;
-                if (lane == 0) mbar_wait(empty_bar(s), ph ^ 1);
-                __syncwarp();
-                uint8_t *stage = smem + (size_t)s * S::kStage;
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    float4 hi, lo;
-                    split_tf32(cur[i].x, hi.x, lo.x);
-                    split_tf32(cur[i].y, hi.y, lo.y);
-                    split_tf32(cur[i].z, hi.z, lo.z);
-                    split_tf32(cur[i].w, hi.w, lo.w);
-                    const uint32_t off = sw64_offset(rsub + 64 * i, c);
-                    *reinterpret_cast<float4 *>(stage + off) = hi;
-                    *reinterpret_cast<float4 *>(stage + S::kAHalf + off) = lo;
-                }
-                if (!(MVX_DBG(a) & 1)) fence_async_smem();
-                mbar_arrive(full_bar(s));
-            };
-            float4 buf0[4], buf1[4];
-            load_chunk(buf0, 0);
-            if (nk > 1) load_chunk(buf1, 1);
-            for (int kc = 0; kc < nk; kc += 2) {
-                produce(buf0, kc);
-                if (kc + 1 < nk) produce(buf1, kc + 1);
-            }
-        }
-    } else if (warp == 8) {
-        // ================= B producer ============================================================================
-        if (lane == 0) {
-            int g = 0;
-            for (int t = blockIdx.x; t < total; t += gridDim.x) {
-                int f, ct;
-                long long row0, n_rows;
-                if (!decode(t, f, ct, row0, n_rows)) continue;
-                const float *src = wpack + (size_t)ct * nk * (2 * BN * kBK);
-                for (int kc = 0; kc < nk; ++kc, ++g) {
-                    const int s = g % kPStages;
-                    const uint32_t ph = (g / kPStages) & 1;
-                    mbar_wait(empty_bar(s), ph ^ 1);
-                    mbar_arrive_expect_tx(full_bar(s), 2 * S::kBHalf);
-                    bulk_g2s(sbase + s * S::kStage + 2 * S::kAHalf, src + (size_t)kc * (2 * BN * kBK), 2 * S::kBHalf, full_bar(s));
-                }
-            }
-        }
-    } else if (warp == 9) {
-        // ================= MMA issuer ============================================================================
-        if (lane == 0) {
-            constexpr uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(BN >> 3) << 17) | ((128u >> 4) << 24);
-            int g = 0, it = 0;
-            for (int t = blockIdx.x; t < total; t += gridDim.x) {
-                int f, ct;
-                long long row0, n_rows;
-                if (!decode(t, f, ct, row0, n_rows)) continue;
-                const int ab = it & 1;                              // accumulator buffer of this tile
-                mbar_wait(tmem_empty_bar(ab), ((it >> 1) & 1) ^ 1);  // the epilogue drained this buffer two tiles ago
-                tc_fence_after();
-                for (int kc = 0; kc < nk; ++kc, ++g) {
-                    const int s = g % kPStages;
-                    const uint32_t ph = (g / kPStages) & 1;
-                    mbar_wait(full_bar(s), ph);
-                    tc_fence_after();
-                    const uint32_t sA = sbase + s * S::kStage, sB = sA + 2 * S::kAHalf;
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        const uint32_t d = tmem_base + ab * (2 * BN) + h * BN;
-                        const uint32_t aoff = h * (128 * 64);
-#pragma unroll
-                        for (int ks = 0; ks < 2; ++ks) {
-                            const uint64_t a_hi = make_desc(sA + aoff + ks * 32), a_lo = make_desc(sA + S::kAHalf + aoff + ks * 32);
-                            const uint64_t b_hi = make_desc(sB + ks * 32), b_lo = make_desc(sB + S::kBHalf + ks * 32);
-                            mma_tf32(d, a_lo, b_hi, idesc, (kc | ks) != 0);
-                            mma_tf32(d, a_hi, b_lo, idesc, 1);
-                            mma_tf32(d, a_hi, b_hi, idesc, 1);
-                        }
-                    }
-                    mma_commit(empty_bar(s));
-                }
-                mma_commit(accum_bar(ab));
-                ++it;
-            }
-        }
-    } else {
-        // ================= epilogue warps (10..13): TMEM lane quarter q = warp % 4 ================================
-        const int q = warp & 3, ew = warp - 10, et = tid - 10 * 32;  // et: 0..127
-        int it = 0;
-        for (int t = blockIdx.x; t < total; t += gridDim.x) {
-            int f, ct;
-            long long row0, n_rows;
-            if (!decode(t, f, ct, row0, n_rows)) continue;
-            const int n0 = ct * BN;
-            double acc_s[BN / 32], acc_ss[BN / 32];
-#pragma unroll
-            for (int cb = 0; cb < BN / 32; ++cb) acc_s[cb] = 0.0, acc_ss[cb] = 0.0;
-            // zero the fp64 partials of the "heavy" rows (BN multiplicity != 1) before anybody adds to them
-            named_bar_sync(2, 128);  // previous tile's partial reads are done
-            for (int i = et; i < 4 * BN * 2; i += 128) s_part[i] = 0.0;
-            named_bar_sync(2, 128);
-            const int ab = it & 1;
-            mbar_wait(accum_bar(ab), (it >> 1) & 1);
-            tc_fence_after();
-#pragma unroll 1
-            for (int h = 0; h < 2; ++h) {
-                const long long r = row0 + h * 128 + q * 32 + lane;
-                const bool valid = r < n_rows;
-                const float w = valid ? (a.row_w ? a.row_w[(size_t)f * a.rowcap + r] : 1.f) : 0.f;
-                const float m = w == 1.f ? 1.f : 0.f;         // ordinary rows go through the fp32 butterfly
-                const bool heavy = w != 0.f && w != 1.f;      // the weighted pad row: exact fp64 side path
-                float *yrow = a.Y ? a.Y + ((size_t)f * a.rowcap + r) * a.ldy + n0 : nullptr;
-#pragma unroll 1
-                for (int cb = 0; cb < BN / 32; ++cb) {
-                    float v[32], p2[32];
-                    tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + ab * (2 * BN) + h * BN + cb * 32, v);
-#pragma unroll
-                    for (int j = 0; j < 32; j += 4) {
-                        const float4 b4 = __ldg(reinterpret_cast<const float4 *>(a.bias + n0 + cb * 32 + j));
-                        v[j] = fmaxf(v[j] + b4.x, 0.f);
-                        v[j + 1] = fmaxf(v[j + 1] + b4.y, 0.f);
-                        v[j + 2] = fmaxf(v[j + 2] + b4.z, 0.f);
-                        v[j + 3] = fmaxf(v[j + 3] + b4.w, 0.f);
-                    }
-                    if (yrow && valid) {
-#pragma unroll
-                        for (int j = 0; j < 32; j += 4)
-                            *reinterpret_cast<float4 *>(yrow + cb * 32 + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-                    }
-                    if (heavy) {
-                        for (int j = 0; j < 32; ++j) {
-                            const double y = (double)v[j], wy = (double)w * y;
-                            atomicAdd(&s_part[((size_t)ew * BN + cb * 32 + j) * 2], wy);
-                            atomicAdd(&s_part[((size_t)ew * BN + cb * 32 + j) * 2 + 1], wy * y);
-                        }
-                    }
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) {
-                        v[j] *= m;
-                        p2[j] = v[j] * v[j];
-                    }
-                    acc_s[cb] += (double)butterfly_colsum(v, lane);
-                    acc_ss[cb] += (double)butterfly_colsum(p2, lane);
-                }
-            }
-            // accumulators are drained: the MMA warp may start the next tile
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(tmem_empty_bar(ab));
-            // combine the four warps' column partials and publish one fp64 atomicAdd per column and quantity
-#pragma unroll
-            for (int cb = 0; cb < BN / 32; ++cb) {
-                atomicAdd(&s_part[((size_t)ew * BN + cb * 32 + lane) * 2], acc_s[cb]);
-                atomicAdd(&s_part[((size_t)ew * BN + cb * 32 + lane) * 2 + 1], acc_ss[cb]);
-            }
-            named_bar_sync(2, 128);
-            for (int i = et; i < BN * 2; i += 128) {
-                const double s4 = s_part[i] + s_part[BN * 2 + i] + s_part[2 * BN * 2 + i] + s_part[3 * BN * 2 + i];
-                atomicAdd(a.out_stats + ((size_t)f * a.Cout + n0) * 2 + i, s4);
-            }
-            ++it;
-        }
-    }
-    __syncwarp();  // warps 8/9: lanes 1-31 wait here for their looping lane 0, so every warp reaches the barrier converged
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 9) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kAccBufs * 2 * BN) : "memory");
-    }
-}
-
-template <int BN>
-int launch_tc_persist(const LayerArgs &a, int F, float *wpack, cudaStream_t st) {
-    using S = PSmem<BN>;
-    static bool attr_set = false;
-    if (!attr_set) {
-        MVX_CUDA_CHECK(cudaFuncSetAttribute(tc_layer_persist_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
-        attr_set = true;
-    }
-    const int total = a.Cin * a.Cout;
-    pack_weights_kernel<BN><<<(total + 255) / 256, 256, 0, st>>>(a.Wt, a.Cin, a.Cout, wpack);
-    MVX_LAUNCH_CHECK();
-    const long long max_rows = a.counts ? a.rowcap : a.rows_fixed;
-    const int row_tiles = (int)ceil_div(max_rows, kTM), col_tiles = a.Cout / BN;
-    const long long slots = (long long)F * row_tiles * col_tiles;
-    const int grid = (int)(slots < kSMs ? slots : kSMs);
-    tc_layer_persist_kernel<BN><<<grid, kPThreads, S::kTotal, st>>>(a, wpack, F, row_tiles, col_tiles);
-    MVX_LAUNCH_CHECK();
-    return MVX_OK;
-}
-
-
-// =====================================================================================================================
-// Persistent 3xFP16 variant (conv1, fcn2: BatchNorm-ed inputs, no per-voxel max, 128 output columns). Same roles and
-// barrier protocol as the TF32 persistent kernel above, with the operand format of the one-tile 16-bit kernel:
-//   warps 0-15  A producers (fp32 rows -> BatchNorm of the producer layer -> fp16 hi/lo, 32 k = one 64-byte swizzle row per stage)
-//   warp 16     B bulk-copy producer      warp 17  MMA issuer (kind::f16, 3 products per K-step) + TMEM alloc
-//   warps 18-25 epilogue: tcgen05.ld -> scale, bias, ReLU -> 32 x 32 transposition tile -> full-line stores and column sums (two warps per TMEM lane quarter): tcgen05.ld -> column scale, bias, ReLU -> 16-byte row stores; butterfly column sums
-// The switch timings of the one-tile kernel (DESIGN.md §5) show its producer, MMA and epilogue phases running one after the
-// other; here the accumulators ping-pong between two TMEM buffers, so tile i drains while tile i+1 is produced and multiplied.
-// =====================================================================================================================
-constexpr int kP16ProducerWarps = 16, kP16ProducerThreads = kP16ProducerWarps * 32;
-constexpr int kP16EpiWarps = 8;            // one per TMEM lane quarter (8: two per quarter, each pair splits the 128 columns)
-constexpr int kP16Threads = (kP16ProducerWarps + 2 + kP16EpiWarps) * 32;   // 832
-constexpr int kP16Stages = 3;   // 3 x 48 KB: leaves room for the 8 transposition tiles
-constexpr int kP16RS = kP16ProducerThreads / 4, kP16RPT = kTM / kP16RS;   // row stride between a producer thread's rows, rows per thread
-
-struct P16Smem {
-    static constexpr int BN = 128;
-    static constexpr int kAHalf = kTM * 64;        // 256 rows x 64 bytes (32 fp16)
-    static constexpr int kBHalf = BN * 64;
-    static constexpr int kStage = 2 * kAHalf + 2 * kBHalf;   // 48 KB
-    static constexpr int kTiles = kP16Stages * kStage;
-    static constexpr int kMean = kTiles;
-    static constexpr int kRstd = kMean + 768 * 4;
-    static constexpr int kPart = kRstd + 768 * 4;              // [epilogue warps][BN][2] fp64 column partials
-    static constexpr int kBars = kPart + kP16EpiWarps * BN * 2 * 8;       // full[4], empty[4], accum_full[2], tmem_empty[2]
-    static constexpr int kTmemPtr = kBars + 8 * (2 * kP16Stages + 2 * kAccBufs);
-    static constexpr int kEpi = kTmemPtr + 16;                 // per epilogue warp: a 32 x 33 float transposition tile
-    static constexpr int kEpiWarpBytes = 32 * 33 * 4;
-    static constexpr int kTotal = kEpi + kP16EpiWarps * kEpiWarpBytes + 1024;
-};
-static_assert(P16Smem::kTotal <= 232448, "persistent 16-bit kernel: shared memory");
-
-__global__ void __launch_bounds__(kP16Threads, 1) tc_layer_persist16_kernel(LayerArgs a, const float *__restrict__ wpack, int F,
-                                                                            int row_tiles) {
-    using S = P16Smem;
-    constexpr int BN = 128, KB = 32;
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t *smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    const uint32_t sbase = smem_u32(smem);
-    float *s_mean = reinterpret_cast<float *>(smem + S::kMean);
-    float *s_rstd = reinterpret_cast<float *>(smem + S::kRstd);
-    double *s_part = reinterpret_cast<double *>(smem + S::kPart);
-    const uint32_t bars = sbase + S::kBars;
-    auto full_bar = [&](int s) { return bars + 8u * s; };
-    auto empty_bar = [&](int s) { return bars + 8u * (kP16Stages + s); };
-    auto accum_bar = [&](int b) { return bars + 8u * (2 * kP16Stages + b); };
-    auto tmem_empty_bar = [&](int b) { return bars + 8u * (2 * kP16Stages + kAccBufs + b); };
-    volatile uint32_t *tmem_ptr = reinterpret_cast<volatile uint32_t *>(smem + S::kTmemPtr);
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int nk = a.Cin / KB;
-    const int total = F * row_tiles;
-    constexpr int W_B = kP16ProducerWarps, W_MMA = kP16ProducerWarps + 1, W_EPI = kP16ProducerWarps + 2;
-
-    // tile decode shared by every role: identical decisions => identical pipeline phase bookkeeping
-    auto decode = [&](int t, int &f, long long &row0, long long &n_rows) -> bool {
-        const int rt = t % row_tiles;
-        f = t / row_tiles;
-        n_rows = a.rows_fixed;
-        if (a.counts) {
-            const int N = a.counts[f * 4 + 0], K = a.counts[f * 4 + 1];
-            n_rows = a.rows_mode == 1 ? K + 1 : (a.rows_mode == 2 ? K + N : a.rows_fixed);
-        }
-        row0 = (long long)rt * kTM;
-        return row0 < n_rows;
-    };
-
-    if (tid == 0) {
-        for (int s = 0; s < kP16Stages; ++s) {
-            mbar_init(full_bar(s), kP16ProducerThreads + 1);
-            mbar_init(empty_bar(s), 1);
-        }
-        for (int b = 0; b < kAccBufs; ++b) {
-            mbar_init(accum_bar(b), 1);
-            mbar_init(tmem_empty_bar(b), kP16EpiWarps);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == W_MMA) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(sbase + S::kTmemPtr), "r"(kAccBufs * 2 * BN)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr;
-
-    if (warp < kP16ProducerWarps) {
-        // ================= A producers: a thread owns 8 k (one 16-byte unit of fp16) of 2 rows per stage =============
-        constexpr int RS = kP16RS, RPT = kP16RPT;
-        const int c = tid & 3, rsub = tid >> 2;   // rows rsub + RS * i
-        const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        int g = 0, cur_f = -1;
-        for (int t = blockIdx.x; t < total; t += gridDim.x) {
-            int f;
-            long long row0, n_rows;
-            if (!decode(t, f, row0, n_rows)) continue;
-            if (f != cur_f) {  // BatchNorm coefficients of the producer layer for this frame
-                named_bar_sync(1, kP16ProducerThreads);
-                const double Rstat = a.counts ? (double)a.counts[f * 4 + 0] * (double)a.T : (double)a.rows_fixed;
-                for (int cc = tid; cc < a.Cin; cc += kP16ProducerThreads) {
-                    const double *st = a.in_stats + ((size_t)f * a.Cin + cc) * 2;
-                    const double m = st[0] / Rstat;
-                    double var = st[1] / Rstat - m * m;
-                    var = var < 0.0 ? 0.0 : var;
-                    s_mean[cc] = (float)m;
-                    s_rstd[cc] = (float)(1.0 / sqrt(var + a.eps));
-                }
-                named_bar_sync(1, kP16ProducerThreads);
-            }
-            cur_f = f;
-            const float *Xf = a.X + ((size_t)f * a.rowcap + row0) * a.ldx + c * 8;
-            bool valid[RPT];
-#pragma unroll
-            for (int i = 0; i < RPT; ++i) valid[i] = row0 + rsub + RS * i < n_rows;
-            auto load_chunk = [&](float4 (&buf)[2 * RPT], int kc) {
-#pragma unroll
-                for (int i = 0; i < RPT; ++i) {
-                    const float4 *p = reinterpret_cast<const float4 *>(Xf + (size_t)(rsub + RS * i) * a.ldx + kc * KB);
-                    buf[2 * i] = valid[i] ? __ldg(p) : z4;
-                    buf[2 * i + 1] = valid[i] ? __ldg(p + 1) : z4;
-                }
-            };
-            auto produce = [&](float4 (&buf)[2 * RPT], int kc) {
-                float4 cur[2 * RPT];
-#pragma unroll
-                for (int i = 0; i < 2 * RPT; ++i) cur[i] = buf[i];
-                const int k = kc * KB + c * 8;
-                const float4 m0 = *reinterpret_cast<const float4 *>(s_mean + k), m1 = *reinterpret_cast<const float4 *>(s_mean + k + 4);
-                const float4 r0 = *reinterpret_cast<const float4 *>(s_rstd + k), r1 = *reinterpret_cast<const float4 *>(s_rstd + k + 4);
-#pragma unroll
-                for (int i = 0; i < RPT; ++i) {
-                    if (valid[i]) {
-                        cur[2 * i].x = (cur[2 * i].x - m0.x) * r0.x, cur[2 * i].y = (cur[2 * i].y - m0.y) * r0.y;
-                        cur[2 * i].z = (cur[2 * i].z - m0.z) * r0.z, cur[2 * i].w = (cur[2 * i].w - m0.w) * r0.w;
-                        cur[2 * i + 1].x = (cur[2 * i + 1].x - m1.x) * r1.x, cur[2 * i + 1].y = (cur[2 * i + 1].y - m1.y) * r1.y;
-                        cur[2 * i + 1].z = (cur[2 * i + 1].z - m1.z) * r1.z, cur[2 * i + 1].w = (cur[2 * i + 1].w - m1.w) * r1.w;
-                    }
-                }
-                if (kc + 2 < nk) load_chunk(buf, kc + 2);
-                const int s = g % kP16Stages;
-                const uint32_t ph = (g / kP16Stages) & 1;
-                ++g;
-                if (lane == 0) mbar_wait(empty_bar(s), ph ^ 1);
-                __syncwarp();
-                uint8_t *stage = smem + (size_t)s * S::kStage;
-#pragma unroll
-                for (int i = 0; i < RPT; ++i) {
-                    const uint32_t off = sw64_offset(rsub + RS * i, c);
-                    uint4 hi, lo;
-                    split_f16_pair(cur[2 * i].x, cur[2 * i].y, hi.x, lo.x);
-                    split_f16_pair(cur[2 * i].z, cur[2 * i].w, hi.y, lo.y);
-                    split_f16_pair(cur[2 * i + 1].x, cur[2 * i + 1].y, hi.z, lo.z);
-                    split_f16_pair(cur[2 * i + 1].z, cur[2 * i + 1].w, hi.w, lo.w);
-                    *reinterpret_cast<uint4 *>(stage + off) = hi;
-                    *reinterpret_cast<uint4 *>(stage + S::kAHalf + off) = lo;
-                }
-                fence_async_smem();
-                mbar_arrive(full_bar(s));
-            };
-            float4 buf0[2 * RPT], buf1[2 * RPT];
-            load_chunk(buf0, 0);
-            if (nk > 1) load_chunk(buf1, 1);
-            for (int kc = 0; kc < nk; kc += 2) {
-                produce(buf0, kc);
-                if (kc + 1 < nk) produce(buf1, kc + 1);
-            }
-        }
-    } else if (warp == W_B) {
-        // ================= B producer ============================================================================
-        if (lane == 0) {
-            int g = 0;
-            for (int t = blockIdx.x; t < total; t += gridDim.x) {
-                int f;
-                long long row0, n_rows;
-                if (!decode(t, f, row0, n_rows)) continue;
-                for (int kc = 0; kc < nk; ++kc, ++g) {
-                    const int s = g % kP16Stages;
-                    const uint32_t ph = (g / kP16Stages) & 1;
-                    mbar_wait(empty_bar(s), ph ^ 1);
-                    mbar_arrive_expect_tx(full_bar(s), 2 * S::kBHalf);
-                    bulk_g2s(sbase + s * S::kStage + 2 * S::kAHalf, reinterpret_cast<const uint8_t *>(wpack) + (size_t)kc * (2 * S::kBHalf),
-                             2 * S::kBHalf, full_bar(s));
-                }
-            }
-        }
-    } else if (warp == W_MMA) {
-        // ================= MMA issuer ============================================================================
-        if (lane == 0) {
-            constexpr uint32_t idesc = (1u << 4) | (0u << 7) | (0u << 10) | ((uint32_t)(BN >> 3) << 17) | ((128u >> 4) << 24);   // kind::f16, fp16 x fp16 -> fp32
-            int g = 0, it = 0;
-            for (int t = blockIdx.x; t < total; t += gridDim.x) {
-                int f;
-                long long row0, n_rows;
-                if (!decode(t, f, row0, n_rows)) continue;
-                const int ab = it & 1;                              // accumulator buffer of this tile
-                mbar_wait(tmem_empty_bar(ab), ((it >> 1) & 1) ^ 1);  // the epilogue drained this buffer two tiles ago
-                tc_fence_after();
-                for (int kc = 0; kc < nk; ++kc, ++g) {
-                    const int s = g % kP16Stages;
-                    const uint32_t ph = (g / kP16Stages) & 1;
-                    mbar_wait(full_bar(s), ph);
-                    tc_fence_after();
-                    const uint32_t sA = sbase + s * S::kStage, sB = sA + 2 * S::kAHalf;
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        const uint32_t d = tmem_base + ab * (2 * BN) + h * BN;
-                        const uint32_t aoff = h * (128 * 64);
-#pragma unroll
-                        for (int ks = 0; ks < 2; ++ks) {
-                            const uint64_t a_hi = make_desc(sA + aoff + ks * 32), a_lo = make_desc(sA + S::kAHalf + aoff + ks * 32);
-                            const uint64_t b_hi = make_desc(sB + ks * 32), b_lo = make_desc(sB + S::kBHalf + ks * 32);
-                            mma_f16(d, a_lo, b_hi, idesc, (kc | ks) != 0);
-                            mma_f16(d, a_hi, b_lo, idesc, 1);
-                            mma_f16(d, a_hi, b_hi, idesc, 1);
-                        }
-                    }
-                    mma_commit(empty_bar(s));
-                }
-                mma_commit(accum_bar(ab));
-                ++it;
-            }
-        }
-    } else {
-        // ================= epilogue warps: TMEM lane quarter q = warp % 4 =========================================
-        const int q = warp & 3, ew = warp - W_EPI, et = tid - W_EPI * 32;  // et: 0 .. 32 * kP16EpiWarps - 1
-        constexpr int NCB = (BN / 32) / (kP16EpiWarps / 4), ET = kP16EpiWarps * 32;   // 32-column blocks per warp
-        const int cb0 = (ew >> 2) * NCB;   // with 8 epilogue warps, warps ew and ew + 4 share a lane quarter and split the columns
-        const float *colinv = reinterpret_cast<const float *>(reinterpret_cast<const uint8_t *>(wpack) + (size_t)a.Cin * a.Cout * 4);
-        float *etile = reinterpret_cast<float *>(smem + S::kEpi + (size_t)ew * S::kEpiWarpBytes);
-        int it = 0;
-        for (int t = blockIdx.x; t < total; t += gridDim.x) {
-            int f;
-            long long row0, n_rows;
-            if (!decode(t, f, row0, n_rows)) continue;
-            double acc_s[NCB], acc_ss[NCB];
-#pragma unroll
-            for (int cb = 0; cb < NCB; ++cb) acc_s[cb] = 0.0, acc_ss[cb] = 0.0;
-            named_bar_sync(2, ET);  // previous tile's partial reads are done
-            for (int i = et; i < kP16EpiWarps * BN * 2; i += ET) s_part[i] = 0.0;
-            named_bar_sync(2, ET);
-            const int ab = it & 1;
-            mbar_wait(accum_bar(ab), (it >> 1) & 1);
-            tc_fence_after();
-#pragma unroll 1
-            for (int h = 0; h < ((MVX_DBG(a) & 2) ? 0 : 2); ++h) {   // dbg 2: no epilogue work (timing experiments)
-                const long long r = row0 + h * 128 + q * 32 + lane;
-                const bool valid = r < n_rows;
-                const float w = valid ? (a.row_w ? a.row_w[(size_t)f * a.rowcap + r] : 1.f) : 0.f;
-                const float m = w == 1.f ? 1.f : 0.f;         // ordinary rows go through the fp32 butterfly
-                const bool heavy = w != 0.f && w != 1.f;      // the weighted pad row: exact fp64 side path
-#pragma unroll 1
-                for (int cbl = 0; cbl < NCB; ++cbl) {
-                    const int cb = cb0 + cbl;
-                    float v[32];
-                    tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + ab * (2 * BN) + h * BN + cb * 32, v);
-#pragma unroll
-                    for (int j = 0; j < 32; j += 4) {
-                        const float4 b4 = __ldg(reinterpret_cast<const float4 *>(a.bias + cb * 32 + j));
-                        const float4 c4 = __ldg(reinterpret_cast<const float4 *>(colinv + cb * 32 + j));   // undo the column scales (exact)
-                        v[j] = fmaxf(v[j] * c4.x + b4.x, 0.f);
-                        v[j + 1] = fmaxf(v[j + 1] * c4.y + b4.y, 0.f);
-                        v[j + 2] = fmaxf(v[j + 2] * c4.z + b4.z, 0.f);
-                        v[j + 3] = fmaxf(v[j + 3] * c4.w + b4.w, 0.f);
-                    }
-                    if (heavy) {
-                        for (int j = 0; j < 32; ++j) {
-                            const double y = (double)v[j], wy = (double)w * y;
-                            atomicAdd(&s_part[((size_t)ew * BN + cb * 32 + j) * 2], wy);
-                            atomicAdd(&s_part[((size_t)ew * BN + cb * 32 + j) * 2 + 1], wy * y);
-                        }
-                    }
-                    // transpose the 32 x 32 block through this warp's tile: lane = row before, lane = column after. Row stores
-                    // become full 128-byte lines (8 lanes per row, 4 rows per instruction) and the column sums a plain loop.
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) etile[lane * 33 + j] = v[j];
-                    __syncwarp();
-                    if (a.Y && !(MVX_DBG(a) & 16)) {   // dbg 16: no row stores
-                        const int c4 = (lane & 7) * 4;
-#pragma unroll
-                        for (int it8 = 0; it8 < 8; ++it8) {
-                            const int rr = it8 * 4 + (lane >> 3);
-                            const long long rg = row0 + h * 128 + q * 32 + rr;
-                            if (rg < n_rows) {
-                                const float *src = etile + rr * 33 + c4;
-                                *reinterpret_cast<float4 *>(a.Y + ((size_t)f * a.rowcap + rg) * a.ldy + cb * 32 + c4) =
-                                    make_float4(src[0], src[1], src[2], src[3]);
-                            }
-                        }
-                    }
-                    if (!(MVX_DBG(a) & 32)) {   // dbg 32: no column sums
-                        float ps = 0.f, pss = 0.f;
-#pragma unroll
-                        for (int rr = 0; rr < 32; ++rr) {
-                            const float y = etile[rr * 33 + lane];
-                            const float my = y * __shfl_sync(0xffffffffu, m, rr);   // ordinary rows only (multiplicity 1)
-                            ps += my;
-                            pss = fmaf(my, y, pss);
-                        }
-                        acc_s[cbl] += (double)ps;
-                        acc_ss[cbl] += (double)pss;
-                    }
-                    __syncwarp();
-                }
-            }
-            // accumulators are drained: the MMA warp may start the next tile
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(tmem_empty_bar(ab));
-#pragma unroll
-            for (int cbl = 0; cbl < NCB; ++cbl) {
-                atomicAdd(&s_part[((size_t)ew * BN + (cb0 + cbl) * 32 + lane) * 2], acc_s[cbl]);
-                atomicAdd(&s_part[((size_t)ew * BN + (cb0 + cbl) * 32 + lane) * 2 + 1], acc_ss[cbl]);
-            }
-            named_bar_sync(2, ET);
-            for (int i = et; i < BN * 2; i += ET) {
-                double s8 = 0.0;
-#pragma unroll
-                for (int w8 = 0; w8 < kP16EpiWarps; ++w8) s8 += s_part[w8 * BN * 2 + i];
-                atomicAdd(a.out_stats + (size_t)f * a.Cout * 2 + i, s8);
-            }
-            ++it;
-        }
-    }
-    __syncwarp();  // single-lane role warps: lanes 1-31 wait here for their looping lane 0
-    tc_fence_before();
-    __syncthreads();
-    if (warp == W_MMA) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kAccBufs * 2 * BN) : "memory");
-    }
-}
-
-int launch_tc_persist16(const LayerArgs &a, int F, float *wpack, cudaStream_t st) {
-    using S = P16Smem;
-    static bool attr_set = false;
-    if (!attr_set) {
-        MVX_CUDA_CHECK(cudaFuncSetAttribute(tc_layer_persist16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
-        attr_set = true;
-    }
-    const int total = a.Cin * a.Cout;
-    uint8_t *blob = reinterpret_cast<uint8_t *>(wpack);
-    pack_weights_f16_kernel<128, false><<<a.Cout, 256, 0, st>>>(a.Wt, a.Cin, a.Cout, blob, reinterpret_cast<float *>(blob + (size_t)total * 4));
-    MVX_LAUNCH_CHECK();
-    const long long max_rows = a.counts ? a.rowcap : a.rows_fixed;
-    const int row_tiles = (int)ceil_div(max_rows, kTM);
-    const long long slots = (long long)F * row_tiles;
-    const int grid = (int)(slots < kSMs ? slots : kSMs);
-    tc_layer_persist16_kernel<<<grid, kP16Threads, S::kTotal, st>>>(a, wpack, F, row_tiles);
-    MVX_LAUNCH_CHECK();
-    return MVX_OK;
-}
 
 }  // namespace
 
@@ -1347,41 +609,14 @@ int pack_weights_f16_128(const float *Wt, int Cin, int Cout, void *wpack, cudaSt
 static int g_tc3 = 1;           // conv1 / fcn2 / last FCN through the TMA-fed, A-from-TMEM persistent kernel (tc3_layer.cu): default since r4
                                 // (conv1 0.79 -> 0.68 ms, fcn2 0.32 -> 0.21, FCN 0.47 -> 0.39); mvx_set_gemm_mode(9) = mode 1 with the one-tile kernel
 void set_tc3(int on) { g_tc3 = on; }
-static int g_tc_two = 0;        // MVX_TC_TWO=1: 128-column 16-bit layers run as two CTAs per SM (measured slower for conv1/fcn2: 0.99 vs 0.86 ms, 0.42 vs 0.35 ms;
-                                // 1-deep prefetch and a 2-stage ring cost more than the overlapped epilogue gains) - experimental
-static int g_apk_two = 1;       // pre-packed-A layers (the pixel GEMM) run as two CTAs per SM: 0.593 -> 0.552 ms (MVX_APK_TWO=0: one 256-column CTA)
-static int g_persist16 = 0;     // mvx_set_gemm_mode(7) / MVX_PERSIST16=1: conv1 / fcn2 through the persistent 3xFP16 kernel. Correct (parity tests pass) but
-                                // measured SLOWER than the one-tile kernel (conv1 0.77 ms, fcn2 0.32): 16 producer + 4 epilogue warps, 4 stages: 0.94 / 0.49;
-                                // 16 + 8 warps, 3 stages (this configuration): 1.12 / 0.38; without the epilogue work: 0.78 / 0.15 and 1.02 / 0.18 (DESIGN.md §5)
-static int g_tc_two_wide = 0;   // 1: also split 256-column tiles (the pixel GEMM) into 128-column two-CTA tiles (MVX_TC_TWO=2)
 static int g_tc_bf16 = 0;
 void set_tc_bf16(int on) { g_tc_bf16 = on; }
 bool tc_bf16_enabled() { return g_tc_bf16 != 0; }
-static int g_tc_f16 = 1;
-bool tc_f16_enabled() { return g_tc_f16 != 0; }
-void set_tc_f16(int on) { g_tc_f16 = on; }
-
-void set_tc_persist16(int on) { g_persist16 = on; }
-static int g_tc_persistent = 0;
-bool tc_persistent_enabled() { return g_tc_persistent != 0; }
-void set_tc_persistent(int on) { g_tc_persistent = on; }
 
 bool tc_layer_eligible(const LayerArgs &a) {
     // the 768 bound sizes the shared BatchNorm tables of the input: a plain product without them may be deeper
     return a.Cin % kBK == 0 && (a.Cin <= 768 || (a.plain && !a.in_stats)) && a.Cout % 128 == 0 && a.ldx % 4 == 0 &&
            (a.Y == nullptr || a.ldy % 4 == 0);
-}
-
-size_t tc_fold_set_bytes(int Cin, int Cout) { return (size_t)Cin * Cout * 4 + (size_t)Cout * 4; }
-
-int launch_fold_pack_weights(const float *Wt, const float *bias, const double *in_stats, const int *counts, int T, double eps,
-                             int Cin, int Cout, int B, void *blob_sets, float *bias_sets, cudaStream_t st) {
-    MVX_REQUIRE(Cout == 128 && Cin % 32 == 0 && Wt && bias && in_stats && counts && blob_sets && bias_sets, MVX_EINVAL,
-                "folded weight sets: 128 output columns, Cin a multiple of 32");
-    fold_pack_weights_kernel<<<dim3(Cout, B), 256, 0, st>>>(Wt, bias, in_stats, counts, T, eps, Cin, Cout,
-                                                            static_cast<uint8_t *>(blob_sets), bias_sets);
-    MVX_LAUNCH_CHECK();
-    return MVX_OK;
 }
 
 size_t tc_wpack_bytes(int Cin, int Cout) { return (size_t)2 * Cin * Cout * sizeof(float); }
@@ -1390,13 +625,6 @@ int launch_layer_tc(const LayerArgs &a_in, int F, float *wpack, cudaStream_t st)
     LayerArgs a = a_in;
 #ifdef MVX_DEVTOOLS
     if (const char *e = getenv("MVX_DBG")) a.dbg = atoi(e);
-    static const bool env_read = [] {
-        if (const char *e = getenv("MVX_TC_TWO")) g_tc_two = atoi(e) != 0, g_tc_two_wide = atoi(e) == 2;
-        if (const char *e = getenv("MVX_APK_TWO")) g_apk_two = atoi(e) != 0;
-        if (const char *e = getenv("MVX_PERSIST16")) g_persist16 = atoi(e) != 0;
-        return true;
-    }();
-    (void)env_read;
 #endif
     MVX_REQUIRE(tc_layer_eligible(a) && wpack, MVX_EINVAL, "layer not eligible for the tensor-core kernel");
     const long long max_rows = a.counts ? a.rowcap : a.rows_fixed;
@@ -1406,33 +634,24 @@ int launch_layer_tc(const LayerArgs &a_in, int F, float *wpack, cudaStream_t st)
                     "channel-major output: plain 3xTF32 product over rows_fixed == rowcap rows per frame");
         return a.Cout % 256 == 0 ? launch_tc<256, false>(a, F, wpack, st) : launch_tc<128, false>(a, F, wpack, st);
     }
-    if (a.vmax == nullptr && !a.plain && !a.X2 && a.rows_mode != 3 && tc_persistent_enabled())  // persistent kernel: 256 x 128 tiles, double-buffered accumulators
-        return launch_tc_persist<128>(a, F, wpack, st);
-    MVX_REQUIRE(!a.X2 || (a.f16_ok && (g_tc_bf16 || tc_f16_enabled()) && a.Cin % 32 == 0 && a.x2_cols % 32 == 0 && a.counts),
-                MVX_EINVAL, "fused concat input needs the 16-bit tensor-core producer");
+    MVX_REQUIRE(!a.X2 || (a.f16_ok && a.Cin % 32 == 0 && a.x2_cols % 32 == 0 && a.counts), MVX_EINVAL,
+                "fused concat input needs the 16-bit tensor-core producer");
     if (g_tc3 && g_tc_bf16 && tc3_layer_eligible(a)) return launch_layer_tc3(a, F, wpack, st);   // bf16 mode of the TMA-fed kernel
     if (a.f16_ok && g_tc_bf16 && a.Cin % 32 == 0) {          // reduced precision: one bf16 product per K-step
-        if (a.Cout % 256 == 0 && !g_tc_two_wide) return launch_tc<256, true, true>(a, F, wpack, st);
-        if (g_tc_two) return launch_tc<128, true, true, true>(a, F, wpack, st);
+        if (a.Cout % 256 == 0) return launch_tc<256, true, true>(a, F, wpack, st);
         return launch_tc<128, true, true>(a, F, wpack, st);
     }
     if (a.a_pack) {   // A pre-packed by the producing kernel: pure bulk-copy + MMA pipeline
-        MVX_REQUIRE(a.Cin % 32 == 0 && !a.in_stats && !a.X2 && (a.Cout % 256 == 0 || a.Cout == 128), MVX_EINVAL,
+        MVX_REQUIRE(a.Cin % 32 == 0 && !a.in_stats && !a.X2 && a.rows_mode == 0 && F == 1, MVX_EINVAL,
                     "pre-packed A: unsupported layer configuration");
-        MVX_REQUIRE((a.rows_mode == 0 && F == 1) || a.a_frame_tiles > 0, MVX_EINVAL, "pre-packed A: per-frame tile count missing");
-        if (a.Cout == 128) return launch_tc<128, true, false, false, true>(a, F, wpack, st);
         // no register producers here, so the two-CTAs-per-SM form (128-column tiles, 2 stages, half-at-a-time epilogue) costs
-        // no duplicated operand conversion: one CTA's epilogue overlaps the other's bulk copies and MMAs
-        if (g_apk_two) return launch_tc<128, true, false, true, true>(a, F, wpack, st);
-        return launch_tc<256, true, false, false, true>(a, F, wpack, st);
+        // no duplicated operand conversion: one CTA's epilogue overlaps the other's bulk copies and MMAs (0.552 ms for the pixel
+        // GEMM against 0.593 ms with one 256-column CTA per SM)
+        return launch_tc<128, true, false, true, true>(a, F, wpack, st);
     }
-    if (g_tc3 && tc_f16_enabled() && tc3_layer_eligible(a)) return launch_layer_tc3(a, F, wpack, st);
-    if (g_persist16 && a.f16_ok && tc_f16_enabled() && a.Cin % 32 == 0 && a.Cout == 128 && !a.vmax && !a.X2 && !a.plain && a.in_stats &&
-        !a.row_max && a.rows_mode != 3 && !a.in_C)
-        return launch_tc_persist16(a, F, wpack, st);   // conv1, fcn2: persistent kernel, epilogue overlapped with the next tile
-    if (a.f16_ok && tc_f16_enabled() && a.Cin % 32 == 0) {   // 3xFP16: half the tensor cycles and operand bytes of 3xTF32
-        if (a.Cout % 256 == 0 && !g_tc_two_wide) return launch_tc<256, true>(a, F, wpack, st);
-        if (g_tc_two) return launch_tc<128, true, false, true>(a, F, wpack, st);   // two CTAs per SM: epilogue of one overlaps the main loop of the other
+    if (g_tc3 && tc3_layer_eligible(a)) return launch_layer_tc3(a, F, wpack, st);
+    if (a.f16_ok && a.Cin % 32 == 0) {   // 3xFP16: half the tensor cycles and operand bytes of 3xTF32
+        if (a.Cout % 256 == 0) return launch_tc<256, true>(a, F, wpack, st);
         return launch_tc<128, true>(a, F, wpack, st);
     }
     if (a.Cout % 256 == 0) return launch_tc<256, false>(a, F, wpack, st);

@@ -63,6 +63,23 @@ def test_argument_validation_without_gpu():
         _lib.check(-3, 'demo')
 
 
+def test_mode_switches_accept_only_the_modes_that_exist():
+    from mvxnet_makise_b200 import _lib
+    einval = -1
+    try:
+        for m in (2, 3, 4, 7, 8, 11):
+            assert _lib.lib.mvx_set_gemm_mode(m) == einval, m
+            assert b'gemm mode must be' in _lib.lib.mvx_last_error()
+        for m in (0, 1, 5, 6, 9, 10, 12):
+            assert _lib.lib.mvx_set_gemm_mode(m) == 0, m
+        assert _lib.lib.mvx_set_fold_mode(1) == einval
+        assert b'fold mode must be' in _lib.lib.mvx_last_error()
+        assert _lib.lib.mvx_set_fold_mode(2) == 0
+    finally:
+        assert _lib.lib.mvx_set_gemm_mode(1) == 0
+        assert _lib.lib.mvx_set_fold_mode(0) == 0
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason='CPU-only behaviour')
 def test_no_cpu_fallback():
     from mvxnet_makise_b200 import voxelize, modules, pipeline, synth

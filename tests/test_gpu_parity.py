@@ -272,7 +272,7 @@ def test_layer_modules_match_oracle(mvx):
 
 
 @pytest.mark.parametrize('R,cin,cout', [(1000, 768, 768), (5003, 768, 128), (777, 128, 128), (256, 768, 768)])
-def test_tensor_core_layer_is_fp32_accurate(mvx, R, cin, cout):
+def test_tensor_core_layer_modes_are_fp32_accurate(mvx, R, cin, cout):
     """tcgen05 3xTF32 layer vs the exact-fp32 SIMT layer and vs an fp64 evaluation (ragged row counts)."""
     from mvxnet_makise_b200 import _lib
     torch.manual_seed(R)
@@ -283,8 +283,6 @@ def test_tensor_core_layer_is_fp32_accurate(mvx, R, cin, cout):
         with torch.no_grad():
             _lib.set_gemm_mode(0)
             y_simt = fcn(x)
-            _lib.set_gemm_mode(2)      # persistent variant, overlapped register epilogue
-            y_tc2 = fcn(x)
             _lib.set_gemm_mode(5)      # fp16 hi/lo operands (3xFP16), the default of the fused path's BatchNorm-ed layers
             y_f16 = fcn(x)
             _lib.set_gemm_mode(1)      # one 256 x BN tile per CTA (default), 3xTF32 for the dense API
@@ -293,7 +291,7 @@ def test_tensor_core_layer_is_fp32_accurate(mvx, R, cin, cout):
         _lib.set_gemm_mode(1)
     y = torch.relu(x.double().reshape(-1, cin) @ fcn.fc.weight.double().t() + fcn.fc.bias.double())
     ref = (y - y.mean(0)) / torch.sqrt(y.var(0, unbiased=False) + 1e-6)
-    assert rel_err(y_tc, y_simt) < 2e-5 and rel_err(y_tc2, y_simt) < 2e-5 and rel_err(y_f16, y_simt) < 2e-5
+    assert rel_err(y_tc, y_simt) < 2e-5 and rel_err(y_f16, y_simt) < 2e-5
     assert rel_err(y_f16.reshape(-1, cout), ref) < 2e-5
     assert rel_err(y_tc.reshape(-1, cout), ref) < 2e-5 and rel_err(y_simt.reshape(-1, cout), ref) < 2e-5
 
@@ -311,6 +309,21 @@ def test_reindex_exact(mvx):
     assert got.shape == ref.shape and torch.equal(got.cpu(), ref)
     empty = mvx.M.reindex(torch.zeros(0, 128).cuda(), torch.zeros(0, 4, dtype=torch.int64).cuda(), G.voxelshape)
     assert float(empty.abs().max()) == 0.0
+
+
+def test_reindex_exact_when_cells_are_not_a_multiple_of_32(mvx):
+    """36 cells: a multiple of 4 but not of 32, so the cell-major fill runs instead of the plane-sequential one."""
+    shape = (6, 2, 3)
+    rng = np.random.default_rng(2)
+    for N, C in ((20, 128), (36, 5)):
+        cells = rng.choice(36, N, replace=False)
+        iz, rem = np.divmod(cells, 12)
+        ix, iy = np.divmod(rem, 2)
+        idx = torch.from_numpy(np.stack([np.zeros(N, np.int64), ix, iy, iz], 1))
+        x = torch.randn(N, C)
+        ref = O.reindex(x, idx, shape)
+        got = mvx.M.reindex(x.cuda(), idx.cuda(), shape)
+        assert got.shape == ref.shape and torch.equal(got.cpu(), ref), (N, C)
 
 
 # ------------------------------------------------------------------------------------------- fused path
@@ -392,11 +405,10 @@ def test_fused_path_matches_reference_golden(mvx, golden_dir, tag, fusion_mode):
     assert rel_err(gcpu, ref64['grid'][0]) < TOL
 
 
-def test_split_grid_fill_equals_single_fill(mvx):
-    """mvx_set_grid_mode(3): zeros written early on the side stream + occupied 32-byte sectors patched at the end must give
-    exactly the grid of the single plane-sequential fill (voxels sharing a sector, sectors at frame / plane borders, an
-    empty frame)."""
-    from mvxnet_makise_b200 import _lib
+def test_grid_fill_rewrites_every_cell(mvx):
+    """The plane-sequential fill of the fused path writes every cell of the grid, zeros included: a second run into a
+    NaN-filled grid gives the grid of the first run (voxels sharing a sector, sectors at frame / plane borders, an empty
+    frame)."""
     sd = synth.make_weights(6)
     maps = [torch.from_numpy(np.concatenate([small_maps(70 + f)[l] for f in range(3)], axis=0)) for l in range(3)]
     frames = [synth.make_points(71, 6000), np.zeros((0, 4), np.float32), synth.make_points(73, 2500)]
@@ -404,13 +416,9 @@ def test_split_grid_fill_equals_single_fill(mvx):
     path = mvx.P.PointPath(sd, G)
     ref, counts = path(frames, [calib] * 3, maps)
     ref, counts = ref.clone(), counts.clone()
-    try:
-        _lib.check(_lib.lib.mvx_set_grid_mode(3))
-        path.grid_out.fill_(float('nan'))      # every byte must be rewritten by one of the two passes
-        out, counts3 = path(frames, [calib] * 3, maps)
-        torch.cuda.synchronize()
-    finally:
-        _lib.check(_lib.lib.mvx_set_grid_mode(2))
+    path.grid_out.fill_(float('nan'))      # every byte must be rewritten
+    out, counts3 = path(frames, [calib] * 3, maps)
+    torch.cuda.synchronize()
     assert torch.equal(counts, counts3)
     assert not torch.isnan(out).any() and int((out[1] != 0).sum()) == 0
     occ = (out[0] != 0).any(0)
@@ -485,12 +493,10 @@ def test_fp16_operands_survive_extreme_feature_ranges(mvx, scale, fusion_mode):
 
 
 @pytest.mark.parametrize('case', ['path_a', 'path_b', 'shifted', 'large', 'tiny'])
-def test_fold_mode_conv1_with_folded_batchnorm(mvx, golden_dir, case):
-    """mvx_set_fold_mode(1): fcn1's rows leave the combine kernel as conv1's pre-packed fp16 operand and fcn1's BatchNorm is
-    folded into per-frame conv1 weights. Same bar as the default path (voxel features within 1e-4 of the fp64 oracle), incl.
-    features with a large common offset (|mean| >> sigma in every channel: the cancellation case of a folded mean) and
-    features far outside fp16's range."""
-    from mvxnet_makise_b200 import _lib
+def test_default_path_on_offset_and_extreme_features(mvx, golden_dir, case):
+    """The default path meets the fp32 bar (voxel features within 1e-4 of the fp64 oracle) and places the voxels of the
+    oracle's grid, also for features with a large common offset (|mean| >> sigma in every channel) and features far outside
+    fp16's range."""
     g = np.load(os.path.join(golden_dir, ('path_b' if case == 'path_b' else 'path_a') + '.npz'))
     maps = small_maps(int(g['map_seed']))
     if case == 'shifted':
@@ -502,61 +508,23 @@ def test_fold_mode_conv1_with_folded_batchnorm(mvx, golden_dir, case):
     sd = synth.make_weights(int(g['weight_seed']))
     calib = synth.kitti_calib()
     path = mvx.P.PointPath(sd, G)
-    res = {}
-    try:
-        for fold in (0, 1):
-            _lib.set_fold_mode(fold)
-            grid, counts = path([g['pcd4']], [calib], [torch.from_numpy(m) for m in maps])
-            torch.cuda.synchronize()
-            vf, idx = path.voxel_features(0)
-            res[fold] = (vf.clone(), idx.clone(), grid[0].clone())
-    finally:
-        _lib.set_fold_mode(0)
+    grid, counts = path([g['pcd4']], [calib], [torch.from_numpy(m) for m in maps])
+    torch.cuda.synchronize()
+    vf, idx = path.voxel_features(0)
     with torch.no_grad():
         ref64 = O.forward_frame(g['pcd4'], calib, maps, sd, G, synth.KITTI_IMSIZE_HW, dtype=torch.float64)
         ref32 = O.forward_frame(g['pcd4'], calib, maps, sd, G, synth.KITTI_IMSIZE_HW)
     noise = rel_err(ref32['vfeat'], ref64['vfeat'])
-    e0, e1 = rel_err(res[0][0], ref64['vfeat']), rel_err(res[1][0], ref64['vfeat'])
-    print(f'{case}: voxel features vs fp64: unfolded {e0:.2e}, folded {e1:.2e} (fp32 reference {noise:.2e})')
-    assert torch.equal(res[0][1], res[1][1]) and torch.isfinite(res[1][0]).all()
-    assert same_occupancy(res[1][2], ref64['grid'][0])
-    # Measured on B200: path_a 4.7e-5 (unfolded 1.8e-5), path_b 2.2e-5 (1.2e-5), shifted 1.9e-4 (2.0e-5). The folded mean cancels
-    # against W'y whose fp16 hi/lo representation error scales with |y|, not |y - mean|: with a common feature offset the
-    # 1e-4 bar is missed, which (with a slower packed store in the combine kernel) is why this mode is NOT the default.
-    bar = {'shifted': 5 * TOL, 'tiny': TOL + 2 * noise}.get(case, TOL)
-    assert e1 < bar, (e1, e0, noise)
-    assert e0 < (TOL if case != 'tiny' else TOL + 2 * noise), (e0, noise)   # the default (unfolded) path meets the bar on every case
+    e0 = rel_err(vf, ref64['vfeat'])
+    print(f'{case}: voxel features vs fp64: {e0:.2e} (fp32 reference {noise:.2e})')
+    assert np.array_equal(idx.cpu().numpy()[:, 1:], ref64['idx'].numpy()[:, 1:])
+    assert torch.isfinite(vf).all()
+    assert same_occupancy(grid[0], ref64['grid'][0])
+    assert e0 < (TOL if case != 'tiny' else TOL + 2 * noise), (e0, noise)
 
 
-def test_persistent_fp16_layer_kernel(mvx, golden_dir):
-    """mvx_set_gemm_mode(7): conv1 and fcn2 through the persistent 3xFP16 kernel (two TMEM accumulator buffers, dedicated
-    epilogue warps). Experimental (slower than the one-tile kernel), but it must meet the same bar."""
-    from mvxnet_makise_b200 import _lib
-    g = np.load(os.path.join(golden_dir, 'path_b.npz'))
-    maps = small_maps(int(g['map_seed']))
-    sd = synth.make_weights(int(g['weight_seed']))
-    calib = synth.kitti_calib()
-    path = mvx.P.PointPath(sd, G)
-    try:
-        _lib.set_gemm_mode(7)
-        frames = [g['pcd4'], synth.make_points(77, 900), np.zeros((0, 4), np.float32)]   # several tiles per CTA, a small and an empty frame
-        fm = [torch.from_numpy(np.concatenate([m, small_maps(5)[l], small_maps(6)[l]], axis=0)) for l, m in enumerate(maps)]
-        grid, counts = path(frames, [calib] * 3, fm)
-        torch.cuda.synchronize()
-        vf, idx = path.voxel_features(0)
-        vf1, _ = path.voxel_features(1)
-    finally:
-        _lib.set_gemm_mode(1)
-    with torch.no_grad():
-        ref64 = O.forward_frame(g['pcd4'], calib, maps, sd, G, synth.KITTI_IMSIZE_HW, dtype=torch.float64, want_grid=False)
-        ref64b = O.forward_frame(frames[1], calib, [m[1:2].numpy() for m in fm], sd, G, synth.KITTI_IMSIZE_HW, dtype=torch.float64,
-                                 want_grid=False)
-    assert rel_err(vf, ref64['vfeat']) < TOL and rel_err(vf1, ref64b['vfeat']) < TOL
-    assert int(counts[2, 0]) == 0
-
-
-def test_tma_fed_tmem_operand_layer_kernel(mvx, golden_dir):
-    """Default mode (1 = 8): conv1, fcn2 and the last FCN through the persistent TMA-fed kernel (tc3_layer.cu): raw fp32 tiles
+def test_tma_fed_tmem_operand_layer_kernel_matches_one_tile_kernel(mvx, golden_dir):
+    """Default mode 1: conv1, fcn2 and the last FCN through the persistent TMA-fed kernel (tc3_layer.cu): raw fp32 tiles
     by tensor copy, converter warps, A operand in tensor memory, double-buffered accumulators, tensor-store epilogue. Same
     3xFP16 arithmetic as the one-tile kernel: raw activations and BatchNorm sums agree with it to fp32 accumulation-order
     level, the voxel features meet the fp32 bar against the fp64 oracle; ragged batch with an empty frame, multi-tile frames."""
@@ -576,7 +544,7 @@ def test_tma_fed_tmem_operand_layer_kernel(mvx, golden_dir):
     st0 = base.region('stats', torch.float64, (8, 4 * 768 * 2)).clone()     # [layer][frame stride = 2 * Cout of the layer]
     vf0 = [base.voxel_features(f)[0].clone() for f in range(4)]
     try:
-        _lib.set_gemm_mode(8)
+        _lib.set_gemm_mode(1)
         path = mvx.P.PointPath(sd, G)
         _, counts = path(frames, [calib] * 4, fm, want_grid=False)
         torch.cuda.synchronize()
