@@ -124,6 +124,16 @@ int mvx_feature_mapping(float *voxels, int64_t R, const float *const *maps, cons
                         const int32_t *map_w, int32_t C, float imsize_h, float imsize_w, float eps, float *out,
                         void *nhwc_ws, size_t nhwc_ws_bytes, void *stream);
 
+/* Backward of mvx_feature_mapping (Pipe.py:62-75, the 4-corner sample) with respect to the three maps of the frame.
+ * voxels (R,9) as the forward left them (pad slots zeroed, projection (row, col) in columns 7-8), d_out (R, 3*C) = dLoss/d out;
+ * d_maps[l]: (C, map_h[l], map_w[l]) fp32 NCHW, OVERWRITTEN. Pad slots and corners on the zero pad row / column of Pipe.py:47-48
+ * contribute nothing. Deterministic: per-pixel sums in a fixed order, no floating-point atomics (two calls give bit-identical
+ * results). No gradient flows to voxels / the projection (data in the reference too). ws: the _workspace_bytes() of scratch. */
+int mvx_feature_mapping_backward_workspace_bytes(int64_t R, const int32_t *map_h, const int32_t *map_w, size_t *bytes);
+int mvx_feature_mapping_backward(const float *voxels, int64_t R, const float *d_out, const int32_t *map_h, const int32_t *map_w,
+                                 int32_t C, float imsize_h, float imsize_w, float eps, float *const *d_maps, void *ws, size_t ws_bytes,
+                                 void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Stage 3 — one layer primitive.  Replaces modules/layers/Blocks.py:5-18 (FCN) and :31-40 (CRB2d, k=1):
  * y = BatchNorm(relu(x W^T + b)), batch statistics over all R rows, biased variance, no affine.
@@ -143,6 +153,36 @@ int mvx_vfe_forward(const float *x, int64_t R, int32_t T, int32_t Cin, const flo
 int mvx_fcn_max_forward(const float *x, int64_t R, int32_t T, int32_t Cin, const float *wt, const float *bias,
                         int32_t Cout, double eps, float *y_max, void *stats_ws, void *vmax_ws, void *stream);
 
+/* Training through the dense layer entries (the backward of FCN / CRB2d, Blocks.py:5-18, 31-40; VFE, voxelnet/Pipe.py:5-18; the last
+ * FCN + max over T, VoxelNet.py:27-32; what autograd computes through the reference modules).
+ *   mvx_*_forward_train: the arguments and outputs of the forward entries above, bit-identical, plus y_raw (R, Cout) = the raw
+ *     post-ReLU output relu(x W^T + b); stats_ws then holds the layer's fp64 sums for the backward.
+ *   mvx_*_backward: x, wt, y_raw, stats_ws, eps of that training forward; dy = dLoss/d output in the forward's output layout:
+ *     (R, Cout) for FCN, (R, 2*Cout) = [pointwise | max tiled over T] for VFE, (R/T, Cout) for the last FCN's max. The max half goes
+ *     per voxel and column to the first row (slot order) attaining the maximum of y_raw. BatchNorm backward in fp64 over all R
+ *     rows. dx (R, Cin) = dLoss/d x (NULL skips that product); dW (Cout, Cin) and db (Cout) receive the parameter gradients
+ *     (accumulate != 0: added to their contents; the sums use fp32 atomics). Cin is the padded width of the forward (a multiple of 16,
+ *     <= 768): dW and dx have zero-input columns there. Every layer shape of the path is accepted (Cin/Cout 768/768, 768/128,
+ *     128/128, 128/16, 16/16, 32/16, 32/64). ws: mvx_*_backward_workspace_bytes() of scratch. */
+int mvx_fcn_forward_train(const float *x, int64_t R, int32_t Cin, const float *wt, const float *bias, int32_t Cout,
+                          double eps, float *y, float *y_raw, void *stats_ws, void *stream);
+int mvx_vfe_forward_train(const float *x, int64_t R, int32_t T, int32_t Cin, const float *wt, const float *bias,
+                          int32_t Cout, double eps, float *y, float *y_raw, void *stats_ws, void *vmax_ws, void *stream);
+int mvx_fcn_max_forward_train(const float *x, int64_t R, int32_t T, int32_t Cin, const float *wt, const float *bias,
+                              int32_t Cout, double eps, float *y_max, float *y_raw, void *stats_ws, void *vmax_ws, void *stream);
+int mvx_fcn_backward_workspace_bytes(int64_t R, int32_t Cin, int32_t Cout, size_t *bytes);
+int mvx_vfe_backward_workspace_bytes(int64_t R, int32_t T, int32_t Cin, int32_t Cout, size_t *bytes);
+int mvx_fcn_max_backward_workspace_bytes(int64_t R, int32_t T, int32_t Cin, int32_t Cout, size_t *bytes);
+int mvx_fcn_backward(const float *x, int64_t R, int32_t Cin, const float *wt, int32_t Cout, const float *y_raw, const void *stats_ws,
+                     double eps, const float *dy, float *dx, float *dW, float *db, int32_t accumulate, void *ws, size_t ws_bytes,
+                     void *stream);
+int mvx_vfe_backward(const float *x, int64_t R, int32_t T, int32_t Cin, const float *wt, int32_t Cout, const float *y_raw,
+                     const void *stats_ws, double eps, const float *dy, float *dx, float *dW, float *db, int32_t accumulate, void *ws,
+                     size_t ws_bytes, void *stream);
+int mvx_fcn_max_backward(const float *x, int64_t R, int32_t T, int32_t Cin, const float *wt, int32_t Cout, const float *y_raw,
+                         const void *stats_ws, double eps, const float *dy, float *dx, float *dW, float *db, int32_t accumulate,
+                         void *ws, size_t ws_bytes, void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Stage 4 — scatter into the dense middle-layer grid.  Replaces modules/voxelnet/VoxelNet.py:16-22
  * (`reindex`): out (1,C,nz,nx,ny) fp32 fully written (zeros + features) in ONE streaming pass.
@@ -150,6 +190,10 @@ int mvx_fcn_max_forward(const float *x, int64_t R, int32_t T, int32_t Cin, const
  * ------------------------------------------------------------------------------------------------ */
 int mvx_scatter_dense(const float *feat, const int64_t *idx, int64_t N, int32_t C, int32_t nx, int32_t ny,
                       int32_t nz, float *out, int32_t *map_ws, void *stream);
+/* Backward of `reindex` for the values (torch's index_put_ backward): d_feat (N,C)[n][c] = d_grid (1,C,nz,nx,ny)[0][c][iz][ix][iy], a
+ * gather, so voxels sharing a cell each receive that cell's gradient; rows whose cell lies outside the grid receive 0. */
+int mvx_scatter_dense_backward(const float *d_grid, const int64_t *idx, int64_t N, int32_t C, int32_t nx, int32_t ny, int32_t nz,
+                               float *d_feat, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
  * The fused batched path: stages 1-4 for B frames in one stream-ordered sequence with no host sync

@@ -28,6 +28,9 @@ EXPORTS = [
     'mvx_crop_workspace_bytes', 'mvx_crop_points', 'mvx_crop_points_f64',
     'mvx_lidar2img', 'mvx_lidar2img_f64', 'mvx_dense_voxel_counts', 'mvx_maps_nhwc_bytes', 'mvx_feature_mapping',
     'mvx_set_gemm_mode', 'mvx_layer_workspace_bytes', 'mvx_fcn_forward', 'mvx_vfe_forward', 'mvx_fcn_max_forward', 'mvx_scatter_dense',
+    'mvx_feature_mapping_backward_workspace_bytes', 'mvx_feature_mapping_backward', 'mvx_fcn_forward_train', 'mvx_vfe_forward_train',
+    'mvx_fcn_max_forward_train', 'mvx_fcn_backward_workspace_bytes', 'mvx_vfe_backward_workspace_bytes',
+    'mvx_fcn_max_backward_workspace_bytes', 'mvx_fcn_backward', 'mvx_vfe_backward', 'mvx_fcn_max_backward', 'mvx_scatter_dense_backward',
     'mvx_pointpath_workspace_bytes', 'mvx_pointpath_layout', 'mvx_pointpath_layout_name', 'mvx_pointpath_forward',
     'mvx_set_fusion_mode', 'mvx_set_fold_mode', 'mvx_pointpath_train_workspace_bytes', 'mvx_pointpath_forward_train', 'mvx_grad_floats',
     'mvx_pointpath_backward', 'mvx_pointpath_backward_maps_workspace_bytes', 'mvx_pointpath_backward_maps', 'mvx_cml_conv1_workspace_bytes', 'mvx_cml_conv1_sparse',
@@ -96,6 +99,19 @@ def _load():
     lib.mvx_vfe_forward.argtypes = [vp, i64, i32, i32, vp, vp, i32, c_double, vp, vp, vp, vp]
     lib.mvx_fcn_max_forward.argtypes = [vp, i64, i32, i32, vp, vp, i32, c_double, vp, vp, vp, vp]
     lib.mvx_scatter_dense.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp, vp, vp]
+    lib.mvx_feature_mapping_backward_workspace_bytes.argtypes = [i64, POINTER(i32), POINTER(i32), POINTER(c_size_t)]
+    lib.mvx_feature_mapping_backward.argtypes = [vp, i64, vp, POINTER(i32), POINTER(i32), i32, c_float, c_float, c_float, POINTER(vp),
+                                                 vp, c_size_t, vp]
+    lib.mvx_fcn_forward_train.argtypes = [vp, i64, i32, vp, vp, i32, c_double, vp, vp, vp, vp]
+    lib.mvx_vfe_forward_train.argtypes = [vp, i64, i32, i32, vp, vp, i32, c_double, vp, vp, vp, vp, vp]
+    lib.mvx_fcn_max_forward_train.argtypes = [vp, i64, i32, i32, vp, vp, i32, c_double, vp, vp, vp, vp, vp]
+    lib.mvx_fcn_backward_workspace_bytes.argtypes = [i64, i32, i32, POINTER(c_size_t)]
+    lib.mvx_vfe_backward_workspace_bytes.argtypes = [i64, i32, i32, i32, POINTER(c_size_t)]
+    lib.mvx_fcn_max_backward_workspace_bytes.argtypes = [i64, i32, i32, i32, POINTER(c_size_t)]
+    lib.mvx_fcn_backward.argtypes = [vp, i64, i32, vp, i32, vp, vp, c_double, vp, vp, vp, vp, i32, vp, c_size_t, vp]
+    lib.mvx_vfe_backward.argtypes = [vp, i64, i32, i32, vp, i32, vp, vp, c_double, vp, vp, vp, vp, i32, vp, c_size_t, vp]
+    lib.mvx_fcn_max_backward.argtypes = [vp, i64, i32, i32, vp, i32, vp, vp, c_double, vp, vp, vp, vp, i32, vp, c_size_t, vp]
+    lib.mvx_scatter_dense_backward.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp, vp]
     lib.mvx_pointpath_workspace_bytes.argtypes = [POINTER(PointPathArgs), POINTER(c_size_t)]
     lib.mvx_pointpath_layout.argtypes = [POINTER(PointPathArgs), POINTER(i64)]
     lib.mvx_pointpath_layout_name.argtypes = [i32]

@@ -568,9 +568,23 @@ int launch_dw_auto(const DwArgs &a, int B, cudaStream_t st) {
 }  // namespace
 
 int launch_dw_voxel_rows(const float *D, int Cout, const float *X, int Cin, const int *counts, int rowcap, const int *dmax, float *dW, int B,
-                         cudaStream_t st) {
-    const DwArgs dw{D, X, Cin, Cin, Cin, Cout, nullptr, 0.0, dW, 0, RowSet{counts, 3, rowcap, nullptr, 1}, dmax, nullptr};
+                         cudaStream_t st, const int *xmax) {
+    const DwArgs dw{D, X, Cin, Cin, Cin, Cout, nullptr, 0.0, dW, 0, RowSet{counts, 3, rowcap, nullptr, 1}, dmax, xmax};
     return launch_dw_auto(dw, B, st);
+}
+
+int launch_bn_back_voxel_rows(float *G, const float *Y, int C, const double *stats, double *bstats, float *dbias, double eps, const int *counts,
+                              int rowcap, const float *row_w, int *dmax, cudaStream_t st) {
+    MVX_REQUIRE(C == 768 || (C % 4 == 0 && C <= 512 && 256 % (C / 4) == 0), MVX_EINVAL,
+                "BatchNorm backward: C must be 768 or a multiple of 4 whose quarter divides 256");
+    const BnArgs bn{G, Y, C, stats, bstats, dbias, eps, RowSet{counts, 3, rowcap, row_w, 1}, dmax};
+    const int threads = C == 768 ? 192 : 256;
+    const dim3 grid((unsigned)ceil_div(rowcap, kBnRows), 1);
+    bn_back_reduce_kernel<<<grid, threads, 0, st>>>(bn);
+    MVX_LAUNCH_CHECK();
+    bn_back_apply_kernel<<<grid, threads, 0, st>>>(bn);
+    MVX_LAUNCH_CHECK();
+    return MVX_OK;
 }
 
 namespace {

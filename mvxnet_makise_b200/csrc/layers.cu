@@ -665,3 +665,46 @@ extern "C" int mvx_fcn_max_forward(const float *x, int64_t R, int32_t T, int32_t
     MVX_LAUNCH_CHECK();
     return MVX_OK;
 }
+
+// ---- training forward of the dense module API: the same launches plus the raw post-ReLU output y_raw (R, Cout) that the
+// backward (module_backward.cu) needs; stats_ws keeps the fp64 sums of the layer for it. The outputs are bit-identical to the
+// forward-only entries above: the same layer kernel, the same normalisation, and one extra copy (the last FCN: one extra store).
+extern "C" int mvx_fcn_forward_train(const float *x, int64_t R, int32_t Cin, const float *wt, const float *bias, int32_t Cout,
+                                     double eps, float *y, float *y_raw, void *stats_ws, void *stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MVX_REQUIRE(y && y_raw, MVX_EINVAL, "null output");
+    int rc = mvx::dense_layer(x, R, 1, Cin, wt, bias, Cout, eps, y, Cout, stats_ws, nullptr, st);
+    if (rc) return rc;
+    MVX_CUDA_CHECK(cudaMemcpyAsync(y_raw, y, (size_t)R * Cout * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    mvx::NormSrc n{static_cast<const double *>(stats_ws), nullptr, R, 1, eps};
+    mvx::normalize_rows_kernel<<<mvx::kSMs * 8, 256, 0, st>>>(y, R, Cout, Cout, n, nullptr, 1);
+    MVX_LAUNCH_CHECK();
+    return MVX_OK;
+}
+
+extern "C" int mvx_vfe_forward_train(const float *x, int64_t R, int32_t T, int32_t Cin, const float *wt, const float *bias,
+                                     int32_t Cout, double eps, float *y, float *y_raw, void *stats_ws, void *vmax_ws, void *stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MVX_REQUIRE(y && y_raw && vmax_ws && T > 0 && R % T == 0, MVX_EINVAL, "bad vfe argument");
+    int rc = mvx::dense_layer(x, R, T, Cin, wt, bias, Cout, eps, y, 2 * Cout, stats_ws, static_cast<int *>(vmax_ws), st);
+    if (rc) return rc;
+    MVX_CUDA_CHECK(cudaMemcpy2DAsync(y_raw, (size_t)Cout * sizeof(float), y, (size_t)2 * Cout * sizeof(float), (size_t)Cout * sizeof(float),
+                                     (size_t)R, cudaMemcpyDeviceToDevice, st));
+    mvx::NormSrc n{static_cast<const double *>(stats_ws), nullptr, R, 1, eps};
+    mvx::normalize_rows_kernel<<<mvx::kSMs * 8, 256, 0, st>>>(y, R, Cout, 2 * Cout, n, static_cast<const int *>(vmax_ws), T);
+    MVX_LAUNCH_CHECK();
+    return MVX_OK;
+}
+
+extern "C" int mvx_fcn_max_forward_train(const float *x, int64_t R, int32_t T, int32_t Cin, const float *wt, const float *bias,
+                                         int32_t Cout, double eps, float *y_max, float *y_raw, void *stats_ws, void *vmax_ws, void *stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MVX_REQUIRE(y_max && y_raw && vmax_ws && T > 0 && R % T == 0, MVX_EINVAL, "bad fcn_max argument");
+    int rc = mvx::dense_layer(x, R, T, Cin, wt, bias, Cout, eps, y_raw, Cout, stats_ws, static_cast<int *>(vmax_ws), st);
+    if (rc) return rc;
+    mvx::NormSrc n{static_cast<const double *>(stats_ws), nullptr, R, 1, eps};
+    mvx::normalize_vmax_kernel<<<dim3(mvx::kSMs * 2, 1), 256, 0, st>>>(static_cast<const int *>(vmax_ws), y_max, Cout, 0,
+                                                                      R / T, n);
+    MVX_LAUNCH_CHECK();
+    return MVX_OK;
+}

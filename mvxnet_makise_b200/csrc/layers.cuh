@@ -97,9 +97,15 @@ int launch_layer_auto(const LayerArgs &a, int F, float *wpack, cudaStream_t st);
 
 // dW (Cout, Cin) += sum over the frames and their N_f voxel rows r of D[f][r]^T X[f][r] (backward.cu): rows of weight 1, X used
 // as stored (no BatchNorm on load, |x| = O(1)); D [B][rowcap][Cout], X [B][rowcap][Cin]; dmax [B][Cout] bounds |D| per column
-// (float bits) for the power-of-two scales of the tensor-core kernel
+// (float bits) for the power-of-two scales of the tensor-core kernel; xmax [B][Cin] bounds |X| per column the same way, or NULL
+// (scale 1)
 int launch_dw_voxel_rows(const float *D, int Cout, const float *X, int Cin, const int *counts, int rowcap, const int *dmax, float *dW, int B,
-                         cudaStream_t st);
+                         cudaStream_t st, const int *xmax = nullptr);
+// batch-statistic BatchNorm + ReLU backward of ONE frame of N_f = counts[0] rows of multiplicity row_w (backward.cu, T = 1): G (rowcap,
+// C) holds dz on entry and dpre on exit; dbias (C) += column sums of dpre (fp32 atomics); bstats (C, 2) must be zeroed; dmax (C) as in
+// launch_dw_voxel_rows (zeroed by the caller) or NULL. C: 768 or a multiple of 4 up to 512 with C / 4 dividing 256.
+int launch_bn_back_voxel_rows(float *G, const float *Y, int C, const double *stats, double *bstats, float *dbias, double eps, const int *counts,
+                              int rowcap, const float *row_w, int *dmax, cudaStream_t st);
 
 // number of rows BN statistics are taken over for frame f: N_f * T (fused path) or rows_fixed (dense API)
 struct NormSrc {

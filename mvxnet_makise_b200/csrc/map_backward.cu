@@ -53,23 +53,43 @@ __device__ __forceinline__ int mb_cell_key(int ys, int xs, int w) {   // ys = i0
 
 // cell of compact row r at this level, or -1: the frame's pad row, an origin point (the forward zeroes its features,
 // Pipe.py:53-59,80), or a cell with no corner inside the map
+__device__ __forceinline__ int mb_cell_of(const MbLevel &L, float prow, float pcol, float eps, CellRef *cr) {
+    const CellRef c = cell_of(prow, pcol, L.rs_h, L.rs_w, eps);
+    if (c.i0 < -1 || c.i0 >= L.h || c.i1 < -1 || c.i1 >= L.w) return -1;
+    if (cr) *cr = c;
+    return mb_cell_key(c.i0 + 1, c.i1 + 1, L.w);
+}
 __device__ __forceinline__ int mb_row_key(const MbRows &a, const MbLevel &L, int f, int r, CellRef *cr) {
     if (r >= a.counts[f * 4 + 1]) return -1;
     const size_t ro = (size_t)f * a.capA + r;
     const float4 xyz = __ldg(reinterpret_cast<const float4 *>(a.vox8 + ro * 8));
     if (xyz.x == 0.f && xyz.y == 0.f && xyz.z == 0.f) return -1;
     const float2 pr = __ldg(reinterpret_cast<const float2 *>(a.proj) + ro);
-    const CellRef c = cell_of(pr.x, pr.y, L.rs_h, L.rs_w, a.eps);
-    if (c.i0 < -1 || c.i0 >= L.h || c.i1 < -1 || c.i1 >= L.w) return -1;
-    if (cr) *cr = c;
-    return mb_cell_key(c.i0 + 1, c.i1 + 1, L.w);
+    return mb_cell_of(L, pr.x, pr.y, a.eps, cr);
 }
 
-__global__ void __launch_bounds__(256) mb_hist_kernel(MbRows a, MbLevel L) {
+// the same rows read straight from a dense (R, 9) voxel tensor after featureMaping's forward (one frame, f = 0): every slot is a
+// row, pad slots (x == y == z == 0) sample nothing, the projection (row, col) is in columns 7 and 8
+struct MbDenseRows {
+    const float *vox9;
+    int capA;              // R: the row count and the stride of the CSR arrays
+    float eps;
+};
+__device__ __forceinline__ int mb_row_key(const MbDenseRows &a, const MbLevel &L, int f, int r, CellRef *cr) {
+    if (r >= a.capA) return -1;
+    const float *s = a.vox9 + (size_t)r * 9;
+    if (s[0] == 0.f && s[1] == 0.f && s[2] == 0.f) return -1;
+    return mb_cell_of(L, s[7], s[8], a.eps, cr);
+}
+
+template <class Rows>
+__device__ __forceinline__ void mb_hist(const Rows &a, const MbLevel &L) {
     const int f = blockIdx.y, r = blockIdx.x * blockDim.x + threadIdx.x;
     const int key = mb_row_key(a, L, f, r, nullptr);
     if (key >= 0) atomicAdd(L.bin_count + (size_t)f * L.nbins + key, 1);
 }
+__global__ void __launch_bounds__(256) mb_hist_kernel(MbRows a, MbLevel L) { mb_hist(a, L); }
+__global__ void __launch_bounds__(256) mbd_hist_kernel(MbDenseRows a, MbLevel L) { mb_hist(a, L); }
 
 __global__ void __launch_bounds__(1024) mb_scan_kernel(MbLevel L) {   // one CTA per frame, four bins per thread and round
     const int f = blockIdx.x, nb = L.nbins;
@@ -95,16 +115,20 @@ __global__ void __launch_bounds__(1024) mb_scan_kernel(MbLevel L) {   // one CTA
     if (threadIdx.x == 0) start[nb] = carry;
 }
 
-__global__ void __launch_bounds__(256) mb_scatter_kernel(MbRows a, MbLevel L) {
+template <class Rows>
+__device__ __forceinline__ void mb_scatter(const Rows &a, const MbLevel &L) {
     const int f = blockIdx.y, r = blockIdx.x * blockDim.x + threadIdx.x;
     const int key = mb_row_key(a, L, f, r, nullptr);
     if (key < 0) return;
     const int pos = L.bin_start[(size_t)f * (L.nbins + 1) + key] + atomicAdd(L.bin_count + (size_t)f * L.nbins + key, 1);
     L.tmp[(size_t)f * a.capA + pos] = r;
 }
+__global__ void __launch_bounds__(256) mb_scatter_kernel(MbRows a, MbLevel L) { mb_scatter(a, L); }
+__global__ void __launch_bounds__(256) mbd_scatter_kernel(MbDenseRows a, MbLevel L) { mb_scatter(a, L); }
 
 // the scatter's order inside a cell depends on which atomic came first: place every row at its rank among the cell's rows
-__global__ void __launch_bounds__(256) mb_rank_kernel(MbRows a, MbLevel L) {
+template <class Rows>
+__device__ __forceinline__ void mb_rank(const Rows &a, const MbLevel &L) {
     const int f = blockIdx.y, r = blockIdx.x * blockDim.x + threadIdx.x;
     CellRef c;
     const int key = mb_row_key(a, L, f, r, &c);
@@ -118,6 +142,8 @@ __global__ void __launch_bounds__(256) mb_rank_kernel(MbRows a, MbLevel L) {
     L.row[o] = r;
     L.wgt[o] = corner_weights(c, L.h, L.w);
 }
+__global__ void __launch_bounds__(256) mb_rank_kernel(MbRows a, MbLevel L) { mb_rank(a, L); }
+__global__ void __launch_bounds__(256) mbd_rank_kernel(MbDenseRows a, MbLevel L) { mb_rank(a, L); }
 
 __global__ void __launch_bounds__(kMbGroup * kMbGroups) mb_dz_kernel(MbRows a, MbLevel L, const float *__restrict__ dpre1) {
     const int f = blockIdx.y, grp = threadIdx.x / kMbGroup, col0 = (threadIdx.x % kMbGroup) * 4;
@@ -145,6 +171,41 @@ __global__ void __launch_bounds__(kMbGroup * kMbGroups) mb_dz_kernel(MbRows a, M
         }
         *reinterpret_cast<float4 *>(L.dz + ((size_t)f * L.h * L.w + (size_t)y * L.w + x) * kMbCols + col0) = acc;
     }
+}
+
+// featureMaping's adjoint (dense rows, one frame): d_map[c][p] = sum over the (row r, corner) that sample pixel p of
+// wgt * d_out[r][col0 + c], channel-major. A CTA owns 32 consecutive pixels x 32 channels, a warp four of the pixels with one
+// channel per lane (coalesced reads of the d_out rows); the sums run in the CSR order of mb_dz_kernel, then go through a shared
+// tile to the (C, H, W) map
+constexpr int kFmPix = 32;
+__global__ void __launch_bounds__(256) mbd_dz_kernel(MbDenseRows a, MbLevel L, const float *__restrict__ d_out, int ld, int col0, int C,
+                                                     float *__restrict__ d_map) {
+    __shared__ float tile[32][kFmPix + 1];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int hw = L.h * L.w, p0 = blockIdx.x * kFmPix, c0 = blockIdx.y * 32, c = c0 + lane;
+    const int *start = L.bin_start, *rows = L.row;
+    for (int i = 0; i < kFmPix / 8; ++i) {
+        const int pl = warp * (kFmPix / 8) + i, p = p0 + pl;
+        float acc = 0.f;
+        if (p < hw && c < C) {
+            const int y = p / L.w, x = p - y * L.w;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {   // pixel (y, x) is corner q = 00, 10, 01, 11 of the cell with top-left (y - dy, x - dx)
+                const int dy = q & 1, dx = q >> 1;
+                const int key = mb_cell_key(y - dy + 1, x - dx + 1, L.w);
+                const int e1 = start[key + 1];
+                for (int e = start[key]; e < e1; ++e) {
+                    const float4 w4 = L.wgt[e];
+                    const float w = q == 0 ? w4.x : (q == 1 ? w4.y : (q == 2 ? w4.z : w4.w));
+                    acc = fmaf(w, __ldg(d_out + (size_t)rows[e] * ld + col0 + c), acc);
+                }
+            }
+        }
+        tile[lane][pl] = acc;
+    }
+    __syncthreads();
+    for (int cc = warp; cc < 32; cc += 8)
+        if (c0 + cc < C && p0 + lane < hw) d_map[(size_t)(c0 + cc) * hw + p0 + lane] = tile[cc][lane];
 }
 
 struct MbLayout {
@@ -257,4 +318,87 @@ extern "C" int mvx_pointpath_backward_maps_workspace_bytes(const mvx_pointpath_a
 extern "C" int mvx_pointpath_backward_maps(const mvx_pointpath_args_t *args, const void *backward_ws, size_t backward_ws_bytes,
                                            float *const d_maps[MVX_NUM_LEVELS], void *ws, size_t ws_bytes) {
     return mvx::pointpath_backward_maps(args, backward_ws, backward_ws_bytes, d_maps, ws, ws_bytes);
+}
+
+namespace mvx {
+namespace {
+
+struct FmLayout {
+    size_t cnt[MVX_NUM_LEVELS], start[MVX_NUM_LEVELS], tmp[MVX_NUM_LEVELS], row[MVX_NUM_LEVELS], wgt[MVX_NUM_LEVELS], total;
+};
+
+int fm_layout(long long R, const int32_t *map_h, const int32_t *map_w, FmLayout &M) {
+    MVX_REQUIRE(map_h && map_w, MVX_EINVAL, "null map extents");
+    MVX_REQUIRE(R >= 0 && R <= 0x7FFFFFFF, MVX_EINVAL, "feature mapping backward: R must be in [0, 2^31)");
+    size_t o = 0;
+    auto take = [&](size_t &slot, size_t bytes) {
+        slot = o;
+        o += (bytes + 255) / 256 * 256;
+    };
+    for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
+        MVX_REQUIRE(map_h[l] > 0 && map_w[l] > 0, MVX_EINVAL, "bad map extent");
+        const size_t nb = mb_bins(map_h[l], map_w[l]);
+        take(M.cnt[l], nb * 4);
+        take(M.start[l], (nb + 1) * 4);
+        take(M.tmp[l], (size_t)R * 4);
+        take(M.row[l], (size_t)R * 4);
+        take(M.wgt[l], (size_t)R * 16);
+    }
+    M.total = o;
+    return MVX_OK;
+}
+
+}  // namespace
+}  // namespace mvx
+
+extern "C" int mvx_feature_mapping_backward_workspace_bytes(int64_t R, const int32_t *map_h, const int32_t *map_w, size_t *bytes) {
+    MVX_REQUIRE(bytes, MVX_EINVAL, "null pointer");
+    mvx::FmLayout M;
+    const int rc = mvx::fm_layout(R, map_h, map_w, M);
+    if (rc) return rc;
+    *bytes = M.total;
+    return MVX_OK;
+}
+
+extern "C" int mvx_feature_mapping_backward(const float *voxels, int64_t R, const float *d_out, const int32_t *map_h, const int32_t *map_w,
+                                            int32_t C, float imsize_h, float imsize_w, float eps, float *const *d_maps, void *ws_v,
+                                            size_t ws_bytes, void *stream) {
+    mvx::FmLayout M;
+    int rc = mvx::fm_layout(R, map_h, map_w, M);
+    if (rc) return rc;
+    MVX_REQUIRE(d_maps && ws_v && (R == 0 || (voxels && d_out)), MVX_EINVAL, "null pointer");
+    for (int l = 0; l < MVX_NUM_LEVELS; ++l) MVX_REQUIRE(d_maps[l], MVX_EINVAL, "null map gradient");
+    MVX_REQUIRE(C > 0 && C % 4 == 0, MVX_EINVAL, "C must be a multiple of 4");
+    MVX_REQUIRE(ws_bytes >= M.total, MVX_ESPACE, "feature mapping backward workspace too small");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    char *ws = static_cast<char *>(ws_v);
+    const mvx::MbDenseRows rows{voxels, (int)R, eps};
+    const dim3 rgrid((unsigned)mvx::ceil_div(R, 256), 1);
+    for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
+        mvx::MbLevel v{};
+        v.h = map_h[l], v.w = map_w[l];
+        v.rs_h = imsize_h / (float)v.h, v.rs_w = imsize_w / (float)v.w;   // as mvx_feature_mapping's MapSet
+        v.nbins = mvx::mb_bins(v.h, v.w);
+        v.bin_count = reinterpret_cast<int *>(ws + M.cnt[l]), v.bin_start = reinterpret_cast<int *>(ws + M.start[l]);
+        v.tmp = reinterpret_cast<int *>(ws + M.tmp[l]), v.row = reinterpret_cast<int *>(ws + M.row[l]);
+        v.wgt = reinterpret_cast<float4 *>(ws + M.wgt[l]), v.dz = nullptr;
+        MVX_CUDA_CHECK(cudaMemsetAsync(v.bin_count, 0, (size_t)v.nbins * 4, st));
+        if (R > 0) {
+            mvx::mbd_hist_kernel<<<rgrid, 256, 0, st>>>(rows, v);
+            MVX_LAUNCH_CHECK();
+        }
+        mvx::mb_scan_kernel<<<1, 1024, 0, st>>>(v);
+        MVX_LAUNCH_CHECK();
+        if (R > 0) {
+            mvx::mbd_scatter_kernel<<<rgrid, 256, 0, st>>>(rows, v);
+            MVX_LAUNCH_CHECK();
+            mvx::mbd_rank_kernel<<<rgrid, 256, 0, st>>>(rows, v);
+            MVX_LAUNCH_CHECK();
+        }
+        const long long hw = (long long)v.h * v.w;
+        mvx::mbd_dz_kernel<<<dim3((unsigned)mvx::ceil_div(hw, mvx::kFmPix), (unsigned)mvx::ceil_div(C, 32)), 256, 0, st>>>(
+            rows, v, d_out, 3 * C, l * C, C, d_maps[l]);
+        MVX_LAUNCH_CHECK();
+    }
+    return MVX_OK;
 }
