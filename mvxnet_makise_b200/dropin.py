@@ -23,10 +23,10 @@ import sys
 import types
 from typing import List, Sequence
 
-import numpy as np
 import torch
 
 from . import synth
+from .modules import _records
 from .pipeline import PointPath
 
 _HOT = [name for name, *_ in synth.HOT_LAYERS]
@@ -46,17 +46,34 @@ def hot_parameters(model) -> List[torch.nn.Parameter]:
     return out
 
 
-def _push_parameters(path: PointPath, params: Sequence[torch.Tensor]):
-    """parameters -> the W^T (Cin_pad, Cout) / bias tensors the kernels read; skipped while the version counters stand still"""
+def _path_inputs(path: PointPath, params: Sequence[torch.Tensor], maps) -> List[torch.Tensor]:
+    """Pushes the parameters into the path's W^T / bias tensors (skipped while their version counters stand still) and
+    returns the maps as the fp32 contiguous tensors the path reads."""
     versions = tuple((p.data_ptr(), p._version) for p in params)
-    if getattr(path, '_param_versions', None) == versions:
-        return
-    with torch.no_grad():
-        for l, (_, cin, cout, _) in enumerate(synth.HOT_LAYERS):
-            w, b = params[2 * l], params[2 * l + 1]
-            path.wt[l][:cin].copy_(w.reshape(cout, cin).t())
-            path.bias[l].copy_(b)
-    path._param_versions = versions
+    if path._param_versions != versions:
+        with torch.no_grad():
+            path.load_parameters(params)
+        path._param_versions = versions
+    return [m.detach().to(torch.float32).contiguous() for m in maps]
+
+
+def _check_record(ctx):
+    if ctx.path._record is not ctx.record:
+        raise RuntimeError('the hot path ran another forward before this backward: its saved activations are gone '
+                           '(one forward/backward at a time per accelerated model)')
+
+
+def _path_backward(ctx, wanted_maps, wanted_params, d_vfeat=None, d_grid=None):
+    """The path backward of a node: (16 parameter gradients, 3 map gradients in the maps' own dtypes), None where not wanted"""
+    path = ctx.path
+    d_maps = None
+    if any(wanted_maps):       # the map backward runs only when a map wants a gradient
+        d_maps = [torch.empty(m.shape, dtype=torch.float32, device=path.device) for m in ctx.record.maps]
+    flat = path.backward(d_vfeat=d_vfeat, d_grid=d_grid, d_maps=d_maps)
+    grads = list(path.grads(flat).values()) if any(wanted_params) else [None] * (2 * len(_HOT))
+    if d_maps is None:
+        return grads, [None] * 3
+    return grads, [d.to(dt) if w else None for d, w, dt in zip(d_maps, wanted_maps, ctx.map_dtypes)]
 
 
 class HotPathFunction(torch.autograd.Function):
@@ -66,47 +83,20 @@ class HotPathFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, path: PointPath, voxels, idx, m0, m1, m2, *params):
-        _push_parameters(path, params)
-        maps = [m.detach().to(torch.float32).contiguous() for m in (m0, m1, m2)]
+        maps = _path_inputs(path, params, (m0, m1, m2))
         nz, nx, ny = path.grid.shape[2], path.grid.shape[0], path.grid.shape[1]
         B = len(voxels) if isinstance(voxels, (list, tuple)) else 1
         grid = torch.empty((B, 128, nz, nx, ny), dtype=torch.float32, device=path.device)   # a fresh tensor: the CML saves it for ITS backward
         path.forward_voxels(voxels, idx, maps, want_grid=True, train=True, grid_out=grid)
-        ctx.path = path
+        ctx.path, ctx.record = path, path._record
         ctx.map_dtypes = [m.dtype for m in (m0, m1, m2)]
-        ctx.call_id = path._train_call = getattr(path, '_train_call', 0) + 1
         return grid
 
     @staticmethod
     def backward(ctx, d_grid):
-        path = ctx.path
-        if path._train_call != ctx.call_id:
-            raise RuntimeError('the hot path ran another training forward before this backward: its saved activations are gone '
-                               '(one forward/backward at a time per accelerated model)')
-        d_maps = _map_grad_buffers(path, ctx.needs_input_grad[3:6])
-        flat = torch.empty(sum(int(np.prod(s)) for _, _, s in PointPath.grad_layout()), dtype=torch.float32, device=path.device)
-        path.backward(d_grid=d_grid.contiguous(), grad_flat=flat, accumulate=False, d_maps=d_maps)
-        grads = [None] * (2 * len(_HOT))
-        if any(ctx.needs_input_grad[6:]):
-            grads = [flat[o:o + int(np.prod(shape))].view(*shape) for _, o, shape in PointPath.grad_layout()]
-        return (None, None, None, *_map_grads(d_maps, ctx.needs_input_grad[3:6], ctx.map_dtypes), *grads)
-
-
-def _map_grad_buffers(path: PointPath, wanted):
-    """fp32 buffers for dLoss/d FPN maps when any map wants a gradient, else None (the map backward does not run)"""
-    if not any(wanted):
-        return None
-    return [torch.empty(m.shape, dtype=torch.float32, device=path.device) for m in path._train_args[4]]
-
-
-def _map_grads(d_maps, wanted, dtypes):
-    if d_maps is None:
-        return [None] * 3
-    return [d.to(dt) if w else None for d, w, dt in zip(d_maps, wanted, dtypes)]
-
-
-def _wants_grad(params, maps) -> bool:
-    return any(p.requires_grad for p in params) or any(m.requires_grad for m in maps)
+        _check_record(ctx)
+        grads, map_grads = _path_backward(ctx, ctx.needs_input_grad[3:6], ctx.needs_input_grad[6:], d_grid=d_grid.contiguous())
+        return (None, None, None, *map_grads, *grads)
 
 
 def hot_path(path: PointPath, voxels, idx, maps, params: Sequence[torch.Tensor]) -> torch.Tensor:
@@ -114,11 +104,9 @@ def hot_path(path: PointPath, voxels, idx, maps, params: Sequence[torch.Tensor])
     enabled and a parameter or an FPN map wants one; otherwise takes the inference route (pixel-first fcn1, no saved
     activations)."""
     maps = list(maps)
-    if torch.is_grad_enabled() and _wants_grad(params, maps):
+    if _records(*params, *maps):
         return HotPathFunction.apply(path, voxels, idx, *maps, *params)
-    maps = [m.detach().to(torch.float32).contiguous() for m in maps]
-    _push_parameters(path, params)
-    grid, _ = path.forward_voxels(voxels, idx, maps, want_grid=True, train=False)
+    grid, _ = path.forward_voxels(voxels, idx, _path_inputs(path, params, maps), want_grid=True, train=False)
     return grid
 
 
@@ -132,33 +120,21 @@ class SparseConv1Function(torch.autograd.Function):
     @staticmethod
     def forward(ctx, path: PointPath, eps: float, train: bool, voxels, idx, m0, m1, m2, *params):
         hot, weight, bias = params[:-2], params[-2], params[-1]
-        _push_parameters(path, hot)
-        maps = [m.detach().to(torch.float32).contiguous() for m in (m0, m1, m2)]
-        path.forward_voxels(voxels, idx, maps, want_grid=False, train=train)
+        path.forward_voxels(voxels, idx, _path_inputs(path, hot, (m0, m1, m2)), want_grid=False, train=train)
         y1 = path.cml_conv1(weight, bias, eps)
-        ctx.path, ctx.eps, ctx.train = path, eps, train
+        ctx.path, ctx.record, ctx.eps, ctx.train = path, path._record, eps, train
         ctx.map_dtypes = [m.dtype for m in (m0, m1, m2)]
-        ctx.call_id = path._train_call = getattr(path, '_train_call', 0) + 1
         ctx.save_for_backward(weight, bias)
         return y1
 
     @staticmethod
     def backward(ctx, d_y1):
-        path = ctx.path
-        if path._train_call != ctx.call_id:
-            raise RuntimeError('the hot path ran another training forward before this backward: its saved activations are gone '
-                               '(one forward/backward at a time per accelerated model)')
+        _check_record(ctx)
         weight, bias = ctx.saved_tensors
-        d_vfeat, d_w, d_b = path.cml_conv1_backward(d_y1.contiguous(), weight, bias, ctx.eps, want_d_vfeat=ctx.train)
-        grads = [None] * (2 * len(_HOT))
-        map_grads = [None] * 3
+        d_vfeat, d_w, d_b = ctx.path.cml_conv1_backward(d_y1.contiguous(), weight, bias, ctx.eps, want_d_vfeat=ctx.train)
+        grads, map_grads = [None] * (2 * len(_HOT)), [None] * 3
         if ctx.train:
-            d_maps = _map_grad_buffers(path, ctx.needs_input_grad[5:8])
-            flat = torch.empty(sum(int(np.prod(s)) for _, _, s in PointPath.grad_layout()), dtype=torch.float32, device=path.device)
-            path.backward(d_vfeat=d_vfeat, grad_flat=flat, accumulate=False, d_maps=d_maps)
-            if any(ctx.needs_input_grad[8:8 + 2 * len(_HOT)]):
-                grads = [flat[o:o + int(np.prod(shape))].view(*shape) for _, o, shape in PointPath.grad_layout()]
-            map_grads = _map_grads(d_maps, ctx.needs_input_grad[5:8], ctx.map_dtypes)
+            grads, map_grads = _path_backward(ctx, ctx.needs_input_grad[5:8], ctx.needs_input_grad[8:8 + 2 * len(_HOT)], d_vfeat=d_vfeat)
         return (None, None, None, None, None, *map_grads, *grads, d_w, d_b)
 
 
@@ -166,12 +142,10 @@ def sparse_conv1(path: PointPath, voxels, idx, maps, params: Sequence[torch.Tens
     """`backbone.cml.conv1` of the grid `hot_path` would return, (B, 64, (nz+1)//2, nx, ny), computed without that grid. Records an
     autograd node when gradients are enabled and any of the 18 tensors or an FPN map wants one."""
     maps = list(maps)
-    train = _wants_grad(params, maps)
-    if torch.is_grad_enabled() and (train or weight.requires_grad or bias.requires_grad):
+    train = _records(*params, *maps)
+    if train or _records(weight, bias):
         return SparseConv1Function.apply(path, eps, train, voxels, idx, *maps, *params, weight, bias)
-    maps = [m.detach().to(torch.float32).contiguous() for m in maps]
-    _push_parameters(path, params)
-    path.forward_voxels(voxels, idx, maps, want_grid=False, train=False)
+    path.forward_voxels(voxels, idx, _path_inputs(path, params, maps), want_grid=False, train=False)
     return path.cml_conv1(weight, bias, eps)
 
 

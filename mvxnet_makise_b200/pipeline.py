@@ -18,9 +18,32 @@ import torch
 
 from . import _lib, synth
 from ._lib import lib, check, ptr, stream_ptr
-from .modules import _wt, pack_calib, pack_calib64, calib_is_f64
+from .modules import pack_calib, pack_calib64, calib_is_f64
 
 LAYER_NAMES = [name for name, *_ in synth.HOT_LAYERS]
+
+
+class _Forward:
+    """The record of one forward: everything a later call on its results (backward, cml_conv1, voxel_features, the drop-in's
+    autograd nodes) reads. Every forward makes a new one, so a stale holder can tell by identity."""
+
+    def __init__(self, args=None, keep=(), maps=None, train=False, subs=None):
+        self.args = args            # the PointPathArgs of the launch (workspace pointers, B, cap)
+        self.keep = keep            # host arrays and tensors the pointers in `args` refer to, kept alive with it
+        self.maps = maps            # the fp32 FPN maps it read (the shapes of dLoss/d maps)
+        self.train = train          # forward_train: the workspace holds the activations backward() needs
+        self.subs = subs            # None: results live in this path; else the _Sub list of forward_host / forward_device_split
+        self.cml_done = False       # cml_conv1 ran on it: the CML workspace holds what cml_conv1_backward reads
+
+
+class _Sub:
+    """Frames [f0, f1) of a batch run by forward_host / forward_device_split on their own PointPath context `path`."""
+
+    def __init__(self, path, f0: int, f1: int, stream=None):
+        self.path, self.f0, self.f1, self.stream = path, f0, f1, stream
+        # forward_host only: device input buffers, the event that marks them copied, this call's offsets and point count
+        self.in_points = self.in_calib = self.in_maps = self.ev = self.offsets = None
+        self.n_points = 0
 
 
 class _HostSlot:
@@ -48,17 +71,22 @@ class PointPath:
     def __init__(self, state_dict: Dict[str, torch.Tensor], grid: synth.GridSpec = synth.KITTI_GRID,
                  imsize_hw: Sequence[int] = synth.KITTI_IMSIZE_HW, eps: float = 1e-6, device='cuda'):
         _lib.require_cuda()
-        self.device = torch.device(device)
-        self.grid_spec = grid
-        self.grid = _lib.make_grid(grid.velorange, grid.voxelsize, grid.voxelshape, grid.T)
-        self.imsize_hw = (float(imsize_hw[0]), float(imsize_hw[1]))
-        self.eps = float(eps)
+        dev = torch.device(device)
+        # the parameter format the kernels read: W^T (Cin_pad16, Cout) with zero pad rows, and the bias, per layer; allocated
+        # once and only ever written in place (load_parameters), so sub-batch contexts and earlier launches see every update
+        wt = [torch.zeros((cin + (-cin) % 16, cout), dtype=torch.float32, device=dev) for _, cin, cout, _ in synth.HOT_LAYERS]
+        bias = [torch.empty(cout, dtype=torch.float32, device=dev) for _, _, cout, _ in synth.HOT_LAYERS]
+        self._init(dev, grid, (float(imsize_hw[0]), float(imsize_hw[1])), float(eps), wt, bias)
         self.load_state_dict(state_dict)
-        self._ws = None
-        self._ws_key = None
-        self._args = None
-        self._subs = None          # sub-batch contexts of the pipelined host entry (forward_host)
-        self._sub_chunk = 0
+
+    def _init(self, device, grid_spec: synth.GridSpec, imsize_hw, eps: float, wt, bias):
+        """Declares every attribute; `__init__` and `_sub_context` call it."""
+        self.device = device
+        self.grid_spec = grid_spec
+        self.grid = _lib.make_grid(grid_spec.velorange, grid_spec.voxelsize, grid_spec.voxelshape, grid_spec.T)
+        self.imsize_hw = imsize_hw
+        self.eps = eps
+        self.wt, self.bias = wt, bias
         self.host_chunk = 1        # frames per sub-batch of forward_host: H2D of chunk j+1 overlaps compute of chunk j
         self.host_streams = 2      # sub-batches alternate between this many compute streams (their kernels may overlap)
         self.host_taper = True     # split the last sub-batch in two: less compute left after the last copy has landed
@@ -70,20 +98,51 @@ class PointPath:
         self.shuffle = None
         self.shuffle_generator = None
         self.last_perm = None
+        self.B = self.cap = 0
+        self.grid_out = self.counts = None
+        self.layout = {}           # workspace region name -> byte offset (region())
+        self._ws = self._bws = None                # forward workspace; backward scratch of a training forward
+        self._ws_key = None
+        self._cml_ws = self._cml_bws = self._map_bws = None   # grown on demand (_scratch)
+        self._record = None        # _Forward of the last forward
+        self._param_versions = None                # (data_ptr, _version) of the parameters dropin last copied in
+        self._split, self._split_key = [], None    # forward_device_split's sub-batch contexts
+        self._slots, self._in_key = [], None       # forward_host's buffer sets
+        self._copy_stream, self._compute_streams, self._host_calls = None, [], 0
+        self._h2d_bytes = self._d2h_bytes = 0
+
+    def _sub_context(self, f0: int, f1: int, stream=None) -> _Sub:
+        """A context for frames [f0, f1) with its own workspace and outputs, sharing the grid, eps, shuffle settings and
+        parameter tensors."""
+        c = PointPath.__new__(PointPath)
+        c._init(self.device, self.grid_spec, self.imsize_hw, self.eps, self.wt, self.bias)
+        c.shuffle, c.shuffle_generator = self.shuffle, self.shuffle_generator
+        return _Sub(c, f0, f1, stream)
 
     def load_state_dict(self, sd):
-        self.wt, self.bias = [], []
-        for name in LAYER_NAMES:
-            w = torch.as_tensor(np.asarray(sd[name + '.weight']) if not isinstance(sd[name + '.weight'], torch.Tensor)
-                                else sd[name + '.weight'])
-            b = torch.as_tensor(np.asarray(sd[name + '.bias']) if not isinstance(sd[name + '.bias'], torch.Tensor)
-                                else sd[name + '.bias'])
-            self.wt.append(_wt(w.to(self.device)))
-            self.bias.append(b.detach().to(self.device, torch.float32).contiguous())
+        self.load_parameters([torch.as_tensor(np.asarray(v)) if not isinstance(v, torch.Tensor) else v.detach()
+                              for v in (sd[name + suffix] for name in LAYER_NAMES for suffix in ('.weight', '.bias'))])
+
+    def load_parameters(self, params: Sequence[torch.Tensor]):
+        """Copies the 16 tensors of the eight layers, checkpoint order (weight, bias per layer), into the W^T / bias tensors
+        the kernels read, in place: one copy per tensor. Call under torch.no_grad() when a tensor requires grad."""
+        for l, (_, cin, cout, _) in enumerate(synth.HOT_LAYERS):
+            self.wt[l][:cin].copy_(params[2 * l].reshape(cout, cin).t())
+            self.bias[l].copy_(params[2 * l + 1])
+
+    def _scratch(self, buf, bytes_fn):
+        """`buf`, or a new uint8 device buffer when it is missing or smaller than `bytes_fn` (a *_workspace_bytes entry of
+        the library) asks for on the last forward's arguments."""
+        nbytes = ctypes.c_size_t()
+        check(bytes_fn(ctypes.byref(self._record.args), ctypes.byref(nbytes)), bytes_fn.__name__)
+        if buf is None or buf.numel() < nbytes.value:
+            buf = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+        return buf
 
     # ------------------------------------------------------------------------------------------------
     def _prepare(self, B: int, cap: int, map_hw, own_outputs: bool = True, train: bool = False):
         key = (B, cap, tuple(map_hw), own_outputs, train)
+        self.cap, self.B = cap, B
         if self._ws_key == key:
             return
         a = _lib.PointPathArgs()
@@ -110,13 +169,12 @@ class PointPath:
             self._bws = torch.empty(bwd_b.value, dtype=torch.uint8, device=self.device)
         self._ws = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
         self._ws_key = key
-        self.cap, self.B = cap, B
         if own_outputs:
             self._alloc_outputs(B)
 
     def _alloc_outputs(self, B: int):
         nz, nx, ny = self.grid.shape[2], self.grid.shape[0], self.grid.shape[1]
-        if getattr(self, 'grid_out', None) is None or self.grid_out.shape[0] != B:
+        if self.grid_out is None or self.grid_out.shape[0] != B:
             self.grid_out = torch.empty((B, 128, nz, nx, ny), dtype=torch.float32, device=self.device)
             self.counts = torch.empty((B, 4), dtype=torch.int32, device=self.device)
 
@@ -143,12 +201,12 @@ class PointPath:
         (None: `self.shuffle`, which defaults to training mode only)."""
         B = len(offsets) - 1
         if shuffle is None:
-            shuffle = getattr(self, 'shuffle', None)
+            shuffle = self.shuffle
         if shuffle is None:
             shuffle = train
         self.last_perm = None
         if shuffle and points.shape[0] > 0:
-            gen = getattr(self, 'shuffle_generator', None)
+            gen = self.shuffle_generator
             perm = torch.cat([torch.randperm(int(offsets[f + 1]) - int(offsets[f]), device=points.device, generator=gen) + int(offsets[f])
                               for f in range(B)])
             points = points.index_select(0, perm)
@@ -162,10 +220,7 @@ class PointPath:
         if counts is not None:
             assert counts.is_contiguous() and counts.shape == (B, 4) and (grid_out is None or grid_out.is_contiguous())
             self.grid_out, self.counts = grid_out, counts
-        self._subs_active = False
         a = _lib.PointPathArgs()
-        a.grid = self.grid
-        a.B, a.cap = B, cap
         if points.shape[0] == 0:     # all-empty batch: the kernels read no point, but the ABI wants a valid pointer
             points = torch.zeros((1, max(4, points.shape[1])), dtype=torch.float32, device=self.device)
         a.points, a.point_stride = points.data_ptr(), points.shape[1]
@@ -180,8 +235,15 @@ class PointPath:
             assert calib64.is_cuda and calib64.dtype == torch.float64 and calib64.is_contiguous() and calib64.shape == calib32.shape
             assert calib_f64 is not None and calib_f64.is_cuda and calib_f64.dtype == torch.int32 and calib_f64.numel() == calib32.shape[0]
             a.calib64, a.calib_f64 = calib64.data_ptr(), calib_f64.data_ptr()
+        self._launch(a, (off, points, calib32, point_calib, calib64, calib_f64), maps, map_hw, want_grid, train)
+        return (self.grid_out if want_grid else None), self.counts
+
+    def _launch(self, a, keep, maps: List[torch.Tensor], map_hw, want_grid: bool, train: bool):
+        """Fills the fields both entries share, runs the fused path (training variant with `train`) and records the forward."""
+        a.grid = self.grid
+        a.B, a.cap = self.B, self.cap
         for l in range(3):
-            assert maps[l].is_contiguous() and maps[l].shape[0] == B and maps[l].shape[1] == 256
+            assert maps[l].is_cuda and maps[l].is_contiguous() and maps[l].shape[0] == self.B and maps[l].shape[1] == 256
             a.maps[l] = maps[l].data_ptr()
             a.map_h[l], a.map_w[l] = map_hw[l]
         a.map_c = 256
@@ -194,15 +256,11 @@ class PointPath:
         a.counts = self.counts.data_ptr()
         a.workspace, a.workspace_bytes = self._ws.data_ptr(), self._ws.numel()
         a.stream = torch.cuda.current_stream().cuda_stream
-        self._fwd_call = getattr(self, '_fwd_call', 0) + 1
         if train:
             check(lib.mvx_pointpath_forward_train(ctypes.byref(a)), 'pointpath_forward_train')
-            self._train_args = (a, off, points, calib32, maps, point_calib, calib64, calib_f64)      # kept alive for backward()
         else:
             check(lib.mvx_pointpath_forward(ctypes.byref(a)), 'pointpath_forward')
-            self._train_args = None
-        self._last_args = (a, off, points, calib32, maps, point_calib, calib64, calib_f64)           # kept alive for cml_conv1()
-        return (self.grid_out if want_grid else None), self.counts
+        self._record = _Forward(a, keep, maps, train)
 
     # ---- the reference's own arguments: MVXNet.forward(voxels, imgs, idx, calibs, imsize) (MVXNet.py:21-27) ----------------
     def forward_voxels(self, voxels, idx, maps: List[torch.Tensor], want_grid: bool = True, train: bool = False,
@@ -237,36 +295,11 @@ class PointPath:
         if grid_out is not None:
             assert grid_out.is_contiguous() and grid_out.dtype == torch.float32
             self.grid_out = grid_out
-            if getattr(self, 'counts', None) is None or self.counts.shape[0] != B:
+            if self.counts is None or self.counts.shape[0] != B:
                 self.counts = torch.empty((B, 4), dtype=torch.int32, device=self.device)
-        self._subs_active = False
         a = _lib.PointPathArgs()
-        a.grid = self.grid
-        a.B, a.cap = B, cap
         a.voxels_dense, a.voxel_idx, a.vox_off_host = vcat.data_ptr(), icat.data_ptr(), voff_c
-        for l in range(3):
-            assert maps[l].is_cuda and maps[l].is_contiguous() and maps[l].shape[0] == B and maps[l].shape[1] == 256
-            a.maps[l] = maps[l].data_ptr()
-            a.map_h[l], a.map_w[l] = map_hw[l]
-        a.map_c = 256
-        a.imsize_h, a.imsize_w = self.imsize_hw
-        a.gather_eps, a.bn_eps = self.eps, self.eps
-        for l in range(8):
-            a.wt[l] = self.wt[l].data_ptr()
-            a.bias[l] = self.bias[l].data_ptr()
-        a.grid_out = self.grid_out.data_ptr() if want_grid else None
-        a.counts = self.counts.data_ptr()
-        a.workspace, a.workspace_bytes = self._ws.data_ptr(), self._ws.numel()
-        a.stream = torch.cuda.current_stream().cuda_stream
-        keep = (a, voff_c, vcat, icat, maps)
-        self._fwd_call = getattr(self, '_fwd_call', 0) + 1
-        if train:
-            check(lib.mvx_pointpath_forward_train(ctypes.byref(a)), 'pointpath_forward_train')
-            self._train_args = keep
-        else:
-            check(lib.mvx_pointpath_forward(ctypes.byref(a)), 'pointpath_forward')
-            self._train_args = None
-        self._last_args = keep
+        self._launch(a, (voff_c, vcat, icat), maps, map_hw, want_grid, train)
         if not single_inplace:                                 # the in-place side effect, for callers that handed in views / lists
             for f, v in enumerate(orig):
                 v.copy_(vcat[voff[f]:voff[f + 1]].reshape(v.shape))
@@ -278,22 +311,20 @@ class PointPath:
         forward, computed sparsely from the voxel features (the forward may have run with want_grid=False).
         weight (64,128,3,3,3), bias (64) as in the reference checkpoint (`backbone.cml.conv1.conv.*`).
         Returns (B, 64, (nz+1)//2, nx, ny) fp32 on the GPU, per-frame BatchNorm statistics like the batch-1 reference."""
-        if getattr(self, '_last_args', None) is None or getattr(self, '_subs_active', False):
+        rec = self._record
+        if rec is None or rec.subs is not None:
             raise RuntimeError('cml_conv1() needs a preceding forward (device entry) on this PointPath')
-        a = self._last_args[0]
+        a = rec.args
         w = weight.detach().to(self.device, torch.float32).contiguous()
         b = bias.detach().to(self.device, torch.float32).contiguous()
         assert tuple(w.shape) == (64, 128, 3, 3, 3) and tuple(b.shape) == (64,)
         nz, nx, ny = self.grid.shape[2], self.grid.shape[0], self.grid.shape[1]
-        nbytes = ctypes.c_size_t()
-        check(lib.mvx_cml_conv1_workspace_bytes(ctypes.byref(a), ctypes.byref(nbytes)), 'cml_conv1_workspace_bytes')
-        if getattr(self, '_cml_ws', None) is None or self._cml_ws.numel() < nbytes.value:
-            self._cml_ws = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+        self._cml_ws = self._scratch(self._cml_ws, lib.mvx_cml_conv1_workspace_bytes)
         out = torch.empty((self.B, 64, (nz + 2 - 3) // 2 + 1, nx, ny), dtype=torch.float32, device=self.device)
         a.stream = torch.cuda.current_stream().cuda_stream
         check(lib.mvx_cml_conv1_sparse(ctypes.byref(a), ptr(w), ptr(b), float(self.eps if eps is None else eps), ptr(out),
                                        ptr(self._cml_ws), self._cml_ws.numel()), 'cml_conv1_sparse')
-        self._cml_call = self._fwd_call      # the saved state in _cml_ws belongs to this forward
+        rec.cml_done = True
         return out
 
     def cml_conv1_backward(self, d_out: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, eps: float | None = None,
@@ -302,18 +333,15 @@ class PointPath:
         Returns (d_vfeat, d_w, d_b): d_vfeat (B, cap, 128) = dLoss/d voxel features for `backward(d_vfeat=...)` (rows past
         each frame's voxel count are zero), or None with want_d_vfeat=False; d_w (64,128,3,3,3) and d_b (64) summed over the
         frames. grads=(d_w, d_b): add into these tensors instead of returning new ones."""
-        if getattr(self, '_cml_call', None) is None or self._cml_call != getattr(self, '_fwd_call', None) or self._subs_active:
+        if self._record is None or not self._record.cml_done:
             raise RuntimeError('cml_conv1_backward() needs the cml_conv1() of the latest forward on this PointPath')
-        a = self._last_args[0]
+        a = self._record.args
         w = weight.detach().to(self.device, torch.float32).contiguous()
         b = bias.detach().to(self.device, torch.float32).contiguous()
         nz, nx, ny = self.grid.shape[2], self.grid.shape[0], self.grid.shape[1]
         assert tuple(d_out.shape) == (self.B, 64, (nz + 2 - 3) // 2 + 1, nx, ny) and d_out.dtype == torch.float32 and d_out.is_cuda
         d_out = d_out.contiguous()
-        nbytes = ctypes.c_size_t()
-        check(lib.mvx_cml_conv1_backward_workspace_bytes(ctypes.byref(a), ctypes.byref(nbytes)), 'cml_conv1_backward_workspace_bytes')
-        if getattr(self, '_cml_bws', None) is None or self._cml_bws.numel() < nbytes.value:
-            self._cml_bws = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+        self._cml_bws = self._scratch(self._cml_bws, lib.mvx_cml_conv1_backward_workspace_bytes)
         if grads is None:
             d_w = torch.empty((64, 128, 3, 3, 3), dtype=torch.float32, device=self.device)
             d_b = torch.empty(64, dtype=torch.float32, device=self.device)
@@ -342,7 +370,7 @@ class PointPath:
             off[name] = o
             o += (n + 255) // 256 * 256
         nbytes = ctypes.c_size_t()
-        check(lib.mvx_cml_conv1_workspace_bytes(ctypes.byref(self._last_args[0]), ctypes.byref(nbytes)), 'cml_conv1_workspace_bytes')
+        check(lib.mvx_cml_conv1_workspace_bytes(ctypes.byref(self._record.args), ctypes.byref(nbytes)), 'cml_conv1_workspace_bytes')
         assert o == nbytes.value, 'cml_saved() is out of step with sc_layout'
         view = lambda name, dtype, shape: self._cml_ws[off[name]:off[name] + int(np.prod(shape)) * 4].view(dtype).view(*shape)
         return dict(act_count=view('act_count', torch.int32, (B,)), act_idx=view('act_idx', torch.int32, (B, go)),
@@ -375,9 +403,10 @@ class PointPath:
         d_maps: three contiguous fp32 CUDA tensors shaped like the forward's FPN maps (B,256,H_l,W_l): they are overwritten
         with dLoss/d maps (the gradient an unfrozen image backbone receives; mvx_pointpath_backward_maps). None: no map
         gradient, and nothing beyond the parameter backward runs."""
-        if getattr(self, '_train_args', None) is None:
+        rec = self._record
+        if rec is None or not rec.train:
             raise RuntimeError('backward() needs a preceding forward_train() on this PointPath')
-        a = self._train_args[0]
+        a = rec.args
         n = int(lib.mvx_grad_floats())
         if grad_flat is None:
             grad_flat = torch.empty(n, dtype=torch.float32, device=self.device)
@@ -390,14 +419,10 @@ class PointPath:
         check(lib.mvx_pointpath_backward(ctypes.byref(a), ptr(d_vfeat), ptr(d_grid), grad_flat.data_ptr(), int(bool(accumulate)),
                                          self._bws.data_ptr(), self._bws.numel()), 'pointpath_backward')
         if d_maps is not None:
-            maps = self._train_args[4]
-            assert len(d_maps) == len(maps) == _lib.NUM_LEVELS
-            for t, m in zip(d_maps, maps):
+            assert len(d_maps) == len(rec.maps) == _lib.NUM_LEVELS
+            for t, m in zip(d_maps, rec.maps):
                 assert t.is_cuda and t.is_contiguous() and t.dtype == torch.float32 and t.shape == m.shape, (tuple(t.shape), tuple(m.shape))
-            nbytes = ctypes.c_size_t()
-            check(lib.mvx_pointpath_backward_maps_workspace_bytes(ctypes.byref(a), ctypes.byref(nbytes)), 'pointpath_backward_maps_workspace_bytes')
-            if getattr(self, '_map_bws', None) is None or self._map_bws.numel() < nbytes.value:
-                self._map_bws = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+            self._map_bws = self._scratch(self._map_bws, lib.mvx_pointpath_backward_maps_workspace_bytes)
             out = (ctypes.c_void_p * _lib.NUM_LEVELS)(*[t.data_ptr() for t in d_maps])
             check(lib.mvx_pointpath_backward_maps(ctypes.byref(a), self._bws.data_ptr(), self._bws.numel(), out, self._map_bws.data_ptr(),
                                                   self._map_bws.numel()), 'pointpath_backward_maps')
@@ -423,28 +448,23 @@ class PointPath:
         if n_split == 1:
             return self.forward_device(points, offsets, calib32, maps, want_grid)
         key = (B, n_split)
-        if getattr(self, '_split_key', None) != key:
+        if self._split_key != key:
             bounds = [round(i * B / n_split) for i in range(n_split + 1)]
-            self._split = []
-            for i in range(n_split):
-                c = self._child()
-                c.f0, c.f1 = bounds[i], bounds[i + 1]
-                c.stream = torch.cuda.Stream(device=self.device)
-                self._split.append(c)
+            self._split = [self._sub_context(bounds[i], bounds[i + 1], torch.cuda.Stream(device=self.device)) for i in range(n_split)]
             self._split_key = key
         self._alloc_outputs(B)
         self.B = B
         cur = torch.cuda.current_stream()
-        for c in self._split:
-            p0, p1 = int(offsets[c.f0]), int(offsets[c.f1])
-            c.stream.wait_stream(cur)
-            with torch.cuda.stream(c.stream):
-                c.forward_device(points[p0:p1], [int(o) - p0 for o in offsets[c.f0:c.f1 + 1]], calib32[c.f0:c.f1],
-                                 [m[c.f0:c.f1] for m in maps], want_grid,
-                                 grid_out=self.grid_out[c.f0:c.f1] if want_grid else None, counts=self.counts[c.f0:c.f1])
-        for c in self._split:
-            cur.wait_stream(c.stream)
-        self._subs, self._sub_chunk, self._subs_active = self._split, None, True
+        for s in self._split:
+            p0, p1 = int(offsets[s.f0]), int(offsets[s.f1])
+            s.stream.wait_stream(cur)
+            with torch.cuda.stream(s.stream):
+                s.path.forward_device(points[p0:p1], [int(o) - p0 for o in offsets[s.f0:s.f1 + 1]], calib32[s.f0:s.f1],
+                                      [m[s.f0:s.f1] for m in maps], want_grid,
+                                      grid_out=self.grid_out[s.f0:s.f1] if want_grid else None, counts=self.counts[s.f0:s.f1])
+        for s in self._split:
+            cur.wait_stream(s.stream)
+        self._record = _Forward(subs=self._split)
         return (self.grid_out if want_grid else None), self.counts
 
     def __call__(self, points_list: List, calibs: List[dict], fpn_maps: List, want_grid: bool = True,
@@ -486,15 +506,6 @@ class PointPath:
                                    calib64=c64, calib_f64=f64)
 
     # ---- host-buffer entry: H2D of this batch's inputs, the fused path, D2H of the counts ---------------
-    def _child(self):
-        c = object.__new__(PointPath)
-        c.device, c.grid_spec, c.grid, c.imsize_hw, c.eps = self.device, self.grid_spec, self.grid, self.imsize_hw, self.eps
-        c.wt, c.bias = self.wt, self.bias          # shared weights
-        c._ws = c._ws_key = c._args = c._subs = None
-        c._sub_chunk, c.host_chunk, c.host_taper = 0, 0, False
-        c.shuffle, c.shuffle_generator, c.last_perm = self.shuffle, self.shuffle_generator, None
-        return c
-
     def forward_host(self, points_host: torch.Tensor, offsets: Sequence[int], calib32_host: torch.Tensor,
                      maps_host: List[torch.Tensor], want_grid: bool = True, head_rows: int = 1024, sync: bool = True):
         """Inputs in (ideally pinned) HOST memory: points (sum P, 4) fp32, calib32 (B,32), maps 3 x (B,256,Hf,Wf). The maps may
@@ -530,20 +541,19 @@ class PointPath:
         maxp = max([int(offsets[i + 1]) - int(offsets[i]) for i in range(B)] + [1])
         cap = (maxp + 4095) // 4096 * 4096
         stride = int(points_host.shape[1])
-        n_slots = max(1, int(getattr(self, 'host_slots', 2)))
+        n_slots = max(1, int(self.host_slots))
         key = (B, cap, stride, tuple(tuple(m.shape[1:]) + (m.is_cuda,) for m in maps_host), tuple(sizes), int(head_rows), n_slots)
-        if getattr(self, '_in_key', None) != key:
+        if self._in_key != key:
             self._slots = []
             for _ in range(n_slots):
                 slot = _HostSlot()
                 for f0, f1 in zip(bounds[:-1], bounds[1:]):
-                    c = self._child()
-                    c.f0, c.f1 = f0, f1
-                    c.in_points = torch.empty(((f1 - f0) * cap, stride), dtype=torch.float32, device=dev)
-                    c.in_calib = torch.empty((f1 - f0, 32), dtype=torch.float32, device=dev)
-                    c.in_maps = [None if m.is_cuda else torch.empty((f1 - f0,) + tuple(m.shape[1:]), dtype=torch.float32, device=dev) for m in maps_host]
-                    c.ev = torch.cuda.Event()
-                    slot.subs.append(c)
+                    s = self._sub_context(f0, f1)
+                    s.in_points = torch.empty(((f1 - f0) * cap, stride), dtype=torch.float32, device=dev)
+                    s.in_calib = torch.empty((f1 - f0, 32), dtype=torch.float32, device=dev)
+                    s.in_maps = [None if m.is_cuda else torch.empty((f1 - f0,) + tuple(m.shape[1:]), dtype=torch.float32, device=dev) for m in maps_host]
+                    s.ev = torch.cuda.Event()
+                    slot.subs.append(s)
                 nz, nx, ny = self.grid.shape[2], self.grid.shape[0], self.grid.shape[1]
                 slot.grid_out = torch.empty((B, 128, nz, nx, ny), dtype=torch.float32, device=dev) if want_grid else None
                 slot.counts = torch.empty((B, 4), dtype=torch.int32, device=dev)
@@ -569,38 +579,38 @@ class PointPath:
         if slot.used:
             cs.wait_event(slot.done)             # the kernels of the call that last used this slot have read its inputs
         with torch.cuda.stream(cs):              # every copy is queued up front: the copy engine never waits for the CPU
-            for c in slot.subs:
-                p0, p1 = int(offsets[c.f0]), int(offsets[c.f1])
-                c.offsets = [int(o) - p0 for o in offsets[c.f0:c.f1 + 1]]
-                c.n_points = p1 - p0
+            for s in slot.subs:
+                p0, p1 = int(offsets[s.f0]), int(offsets[s.f1])
+                s.offsets = [int(o) - p0 for o in offsets[s.f0:s.f1 + 1]]
+                s.n_points = p1 - p0
                 if p1 > p0:
-                    c.in_points[:p1 - p0].copy_(points_host[p0:p1], non_blocking=True)
-                c.in_calib.copy_(calib32_host[c.f0:c.f1], non_blocking=True)
-                for d, h in zip(c.in_maps, maps_host):
+                    s.in_points[:p1 - p0].copy_(points_host[p0:p1], non_blocking=True)
+                s.in_calib.copy_(calib32_host[s.f0:s.f1], non_blocking=True)
+                for d, h in zip(s.in_maps, maps_host):
                     if d is not None:
-                        d.copy_(h[c.f0:c.f1], non_blocking=True)
-                c.ev.record(cs)
-        for j, c in enumerate(slot.subs):
+                        d.copy_(h[s.f0:s.f1], non_blocking=True)
+                s.ev.record(cs)
+        for j, s in enumerate(slot.subs):
             ks = self._compute_streams[j % ns]
             if j < ns:
                 ks.wait_stream(cur)              # work the caller queued before this call (weight updates ...) is ordered first
             with torch.cuda.stream(ks):
-                ks.wait_event(c.ev)
-                sub_maps = [d if d is not None else h[c.f0:c.f1] for d, h in zip(c.in_maps, maps_host)]   # device-resident maps: a view
-                c.forward_device(c.in_points[:c.n_points], c.offsets, c.in_calib, sub_maps, want_grid, cap=cap,
-                                 grid_out=slot.grid_out[c.f0:c.f1] if want_grid else None, counts=slot.counts[c.f0:c.f1])
+                ks.wait_event(s.ev)
+                sub_maps = [d if d is not None else h[s.f0:s.f1] for d, h in zip(s.in_maps, maps_host)]   # device-resident maps: a view
+                s.path.forward_device(s.in_points[:s.n_points], s.offsets, s.in_calib, sub_maps, want_grid, cap=cap,
+                                      grid_out=slot.grid_out[s.f0:s.f1] if want_grid else None, counts=slot.counts[s.f0:s.f1])
         k0 = self._compute_streams[0]
         for s_ in self._compute_streams[1:]:
             k0.wait_stream(s_)
         with torch.cuda.stream(k0):              # device -> host read of the step's result
             slot.out_counts.copy_(slot.counts, non_blocking=True)
-            c0 = slot.subs[0]
+            c0 = slot.subs[0].path
             n_head = slot.out_head.shape[0]
             slot.out_head.copy_(c0.region('vfeat', torch.float32, (c0.B, c0.cap, 128))[0, :n_head], non_blocking=True)
             slot.done.record(k0)
         slot.used = True
         cur.wait_event(slot.done)                # later work on the caller's stream sees this call's device outputs
-        self._subs, self._sub_chunk, self._subs_active = slot.subs, None, True
+        self._record = _Forward(subs=slot.subs)
         self._d2h_bytes = slot.out_counts.numel() * 4 + slot.out_head.numel() * 4
         step = HostStep(slot)
         return step.wait() if sync else step
@@ -618,9 +628,9 @@ class PointPath:
         """(N_f,128) fp32 features and (N_f,4) int64 idx [batch, ix, iy, iz] of frame f (after a forward)."""
         n = int(self.counts[f, 0].item())
         src, fl = self, f
-        if getattr(self, '_subs_active', False):   # the last forward ran in sub-batches: frame f lives in one of them
-            src = next(c for c in self._subs if c.f0 <= f < c.f1)
-            fl = f - src.f0
+        if self._record.subs is not None:          # the last forward ran in sub-batches: frame f lives in one of them
+            s = next(s for s in self._record.subs if s.f0 <= f < s.f1)
+            src, fl = s.path, f - s.f0
         vfeat = src.region('vfeat', torch.float32, (src.B, src.cap, 128))[fl, :n]
         coord = src.region('vox_coord', torch.int32, (src.B, src.cap, 4))[fl, :n, :3].to(torch.int64)
         idx = torch.cat([torch.full((n, 1), f, dtype=torch.int64, device=coord.device), coord], dim=1)

@@ -67,31 +67,27 @@ class FlatAdamW:
 class HotPathTrainer:
     def __init__(self, state_dict: Dict, grid: synth.GridSpec = synth.KITTI_GRID, lr: float = 1e-3, eps: float = 1e-6,
                  betas: Sequence[float] = (0.9, 0.999), weight_decay: float = 1e-2, device='cuda'):
-        from .pipeline import PointPath       # needs the CUDA library; FlatAdamW above does not
+        from ._lib import lib                 # needs the CUDA library; FlatAdamW above does not
+        from .pipeline import PointPath
         self.path = PointPath(state_dict, grid, device=device)
         dev = self.path.device
-        self.layout = PointPath.grad_layout()
-        n = self.layout[-1][1] + int(np.prod(self.layout[-1][2]))
+        n = int(lib.mvx_grad_floats())
         self.params = torch.empty(n, dtype=torch.float32, device=dev)
-        for name, o, shape in self.layout:
+        views = self.path.grads(self.params)
+        for name, v in views.items():
             t = torch.as_tensor(np.asarray(state_dict[name])) if not isinstance(state_dict[name], torch.Tensor) else state_dict[name]
-            self.params[o:o + t.numel()] = t.detach().reshape(-1).to(dev, torch.float32)
+            v.copy_(t.detach().reshape(v.shape))
+        self._param_views = list(views.values())      # checkpoint order: what PointPath.load_parameters takes
         self.bucket = torch.zeros(n + 1, dtype=torch.float32, device=dev)   # gradients + one slot for the frame count
         self.grad = self.bucket[:n]                                          # what the CUDA backward fills
         self.opt = FlatAdamW(self.params, lr, eps, betas, weight_decay)
-        self._push_weights()
 
     def state_dict(self) -> Dict[str, torch.Tensor]:
-        return {name: self.params[o:o + int(np.prod(shape))].view(*shape).clone() for name, o, shape in self.layout}
+        return {name: v.clone() for name, v in self.path.grads(self.params).items()}
 
     def _push_weights(self):
         """flat parameters -> the W^T (Cin_pad, Cout) / bias tensors the kernels read (in place: pointers stay valid)"""
-        for l, (name, cin, cout, _) in enumerate(synth.HOT_LAYERS):
-            _, ow, _ = self.layout[2 * l]
-            _, ob, _ = self.layout[2 * l + 1]
-            w = self.params[ow:ow + cout * cin].view(cout, cin)
-            self.path.wt[l][:cin].copy_(w.t())
-            self.path.bias[l].copy_(self.params[ob:ob + cout])
+        self.path.load_parameters(self._param_views)
 
     def step(self, points, offsets, calib32, maps, d_vfeat=None, d_grid=None, global_frames: int | None = None,
              want_grid: bool = True):

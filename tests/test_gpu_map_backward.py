@@ -56,7 +56,7 @@ def adjoint_on_saved(path, sd, f):
     proj = path.region('proj', torch.float32, (path.B, capA, 2))[f, :K].cpu()
     xyz = path.region('vox8', torch.float32, (path.B, capA, 8))[f, :K, :3].cpu()
     real = (xyz != 0).any(1)
-    hw = [tuple(m.shape[-2:]) for m in path._train_args[4]]
+    hw = [tuple(m.shape[-2:]) for m in path._record.maps]
     return MA.map_adjoint(dpre1, torch.from_numpy(np.asarray(sd[W1])), proj, real, hw, path.imsize_hw, path.eps)
 
 
@@ -64,7 +64,7 @@ def map_entry(path, d_maps):
     """mvx_pointpath_backward_maps alone, on the state the last PointPath.backward(d_maps=...) left"""
     import ctypes
     from mvxnet_makise_b200 import _lib
-    a = path._train_args[0]
+    a = path._record.args
     out = (ctypes.c_void_p * 3)(*[t.data_ptr() for t in d_maps])
     _lib.check(_lib.lib.mvx_pointpath_backward_maps(ctypes.byref(a), path._bws.data_ptr(), path._bws.numel(), out,
                                                     path._map_bws.data_ptr(), path._map_bws.numel()), 'backward_maps')

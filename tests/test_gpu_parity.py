@@ -829,6 +829,39 @@ def test_device_split_equals_single_call(mvx, n_split):
         assert torch.equal(g[f][:, i[:, 3], i[:, 1], i[:, 2]].T, vf)                          # placement: a copy of the features
 
 
+def test_load_state_dict_reaches_existing_sub_batch_contexts(mvx):
+    """load_state_dict after forward_host / forward_device_split have built their sub-batch contexts: the next calls of both
+    compute with the new weights, like a fresh PointPath of them."""
+    from mvxnet_makise_b200.modules import pack_calib
+    sd_a, sd_b = synth.make_weights(4), synth.make_weights(5)
+    calib = synth.kitti_calib()
+    frames = [synth.make_points(150 + f, P) for f, P in enumerate((700, 1100, 900, 500))]
+    B = len(frames)
+    offsets = np.concatenate([[0], np.cumsum([p.shape[0] for p in frames])]).tolist()
+    pts_h = torch.from_numpy(np.concatenate(frames, 0)).pin_memory()
+    c32_h = torch.stack([pack_calib(calib) for _ in range(B)]).pin_memory()
+    maps_h = [torch.from_numpy(m).pin_memory() for m in small_maps(16, B=B)]
+    pts, c32, maps = pts_h.cuda(), c32_h.cuda(), [m.cuda() for m in maps_h]
+    ref = mvx.P.PointPath(sd_b, G)
+    ref.forward_device(pts, offsets, c32, maps)
+    want = [tuple(t.clone() for t in ref.voxel_features(f)) for f in range(B)]
+    path = mvx.P.PointPath(sd_a, G)
+    path.host_chunk = 2
+    runs = {}
+    for sd in ('a', 'b'):
+        if sd == 'b':
+            path.load_state_dict(sd_b)
+        path.forward_host(pts_h, offsets, c32_h, maps_h)
+        runs['host', sd] = [tuple(t.clone() for t in path.voxel_features(f)) for f in range(B)]
+        path.forward_device_split(pts, offsets, c32, maps, True, n_split=2)
+        runs['split', sd] = [tuple(t.clone() for t in path.voxel_features(f)) for f in range(B)]
+    for entry in ('host', 'split'):
+        assert rel_err(runs[entry, 'a'][0][0], want[0][0]) > 1e-2       # weights A and B give different features
+        for f in range(B):
+            vf, idx = runs[entry, 'b'][f]
+            assert torch.equal(idx, want[f][1]) and rel_err(vf, want[f][0]) < 1e-5, (entry, f)
+
+
 def test_fused_path_full_size_properties(mvx):
     """BASELINE-size frame (P = 120 000, real FPN shapes): size-independent properties."""
     sd = synth.make_weights(0)

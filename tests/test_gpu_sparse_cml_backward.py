@@ -374,6 +374,25 @@ def test_dropin_full_cml_train_step_and_cml_only_finetuning():
     assert min(cos) > 0.999, cos
 
 
+@pytest.mark.parametrize('sparse,freeze_hot', [(False, False), (True, False), (True, True)])
+def test_dropin_backward_after_another_forward_raises(sparse, freeze_hot):
+    """HotPathFunction / SparseConv1Function (also with the hot path frozen: CML-only fine-tuning): another forward of the
+    model, training or inference, before the backward of the first overwrites what that backward reads, so it raises."""
+    from mvxnet_makise_b200.dropin import accelerate, hot_parameters
+    voxel, idx = _frame_inputs(34, 700)
+    m = accelerate(_standin(4), grid=SMALL, sparse_cml_conv1=sparse)
+    for p in hot_parameters(m):
+        p.requires_grad_(not freeze_hot)
+    for second in ('training', 'inference'):
+        score, _ = _run(m, voxel, idx)
+        with torch.set_grad_enabled(second == 'training'):
+            _run(m, voxel, idx)
+        with pytest.raises(RuntimeError, match='another forward'):
+            score.sum().backward()
+    score, _ = _run(m, voxel, idx)
+    score.sum().backward()                  # the latest forward's backward runs
+
+
 def test_dropin_rejects_non_stock_conv1():
     from mvxnet_makise_b200.dropin import accelerate
     m = _standin(3)

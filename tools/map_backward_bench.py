@@ -42,7 +42,7 @@ px = sum(h * w for h, w in synth.fpn_shapes())
 
 
 def entry():
-    a = path._train_args[0]
+    a = path._record.args
     out = (ctypes.c_void_p * 3)(*[t.data_ptr() for t in d_maps])
     _lib.check(_lib.lib.mvx_pointpath_backward_maps(ctypes.byref(a), path._bws.data_ptr(), path._bws.numel(), out,
                                                     path._map_bws.data_ptr(), path._map_bws.numel()), 'backward_maps')
