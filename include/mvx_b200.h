@@ -254,6 +254,9 @@ int mvx_dense_voxel_counts(const float *voxels_dense, const int32_t *vox_off_hos
 int mvx_pointpath_workspace_bytes(const mvx_pointpath_args_t *args, size_t *bytes);
 int mvx_pointpath_layout(const mvx_pointpath_args_t *args, int64_t *offsets /* [MVX_WS_REGIONS] */);
 const char *mvx_pointpath_layout_name(int32_t region);
+/* The workspace carries state from one call to the next in its "tiles" region: which row tiles of the per-pixel products Z are
+ * known to hold zeros. Zero that region when the workspace is new (or was used for anything else); then every row tile of Z that
+ * no point samples is zero after each call. No output depends on it: only inactive tiles of Z, which nothing reads. */
 int mvx_pointpath_forward(const mvx_pointpath_args_t *args);
 /* How gather + fcn1 (Pipe.py:62-82 + Pipe.py:94) are evaluated inside the fused path. The 4-corner sample is linear in
  * the map values, so fcn1 commutes with it:

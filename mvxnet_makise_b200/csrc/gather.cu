@@ -5,6 +5,7 @@
 
 #include <cuda_bf16.h>
 #include "project.cuh"
+#include "voxelize.cuh"
 
 #include <climits>
 #include <cuda_fp16.h>
@@ -90,11 +91,15 @@ __device__ __forceinline__ void pk_split(float x0, float x1, uint32_t &hi, uint3
 #endif
 constexpr int kPackUnroll = MVX_PACK_UNROLL;   // channel rows in flight per thread (A/B on the serialised stage: 4: 0.147-0.167 ms, 8: 0.181, 16: 0.133-0.147, 32: 0.167)
 __global__ void __launch_bounds__(256) pack_maps_f16_kernel(const float *__restrict__ in, int C, int HW, uint8_t *__restrict__ apack,
-                                                            float *__restrict__ rowinv) {
+                                                            float *__restrict__ rowinv, const unsigned *__restrict__ tile_bits) {
     __shared__ float tile[256][33];
     __shared__ float s_max[8][32];
     __shared__ float s_scale[32];
     const int f = blockIdx.y, p0 = blockIdx.x * 32, tid = threadIdx.x, tx = tid & 31, ty = tid >> 5;
+    if (tile_bits) {   // the pixel GEMM multiplies active row tiles only; 32 pixels span at most two tiles
+        const size_t t0 = ((size_t)f * HW + p0) / kPixTileRows, t1 = ((size_t)f * HW + min(p0 + 31, HW - 1)) / kPixTileRows;
+        if (!((tile_bits[t0 >> 5] >> (t0 & 31)) & 1u) && !((tile_bits[t1 >> 5] >> (t1 & 31)) & 1u)) return;
+    }
     const float *src = in + (size_t)f * C * HW;
     float mx = 0.f;
 #pragma unroll kPackUnroll
@@ -139,6 +144,145 @@ __global__ void __launch_bounds__(256) pack_maps_f16_kernel(const float *__restr
         *reinterpret_cast<uint4 *>(dst) = hi;
         *reinterpret_cast<uint4 *>(dst + 16384) = lo;
     }
+}
+
+// (row, col) image coordinates of point gp (global index) of frame f = lidar2Img(...)[:, [1, 0]] (train.py:33). Merged point sets
+// (GT-paste, train.py:36-41): every point is projected through the calibration it came with (point_calib); a float64 calibration
+// (calib_f64) projects in fp64 and rounds once (torch.Tensor(voxel), train.py:125). c32 = the frame's calib32 row (shared memory)
+// when there is no point_calib. rows_build_kernel and the pixel-tile mark both project through here.
+__device__ __forceinline__ float2 point_row_col(const float *calib32, const int *point_calib, const double *calib64, const int *calib_f64,
+                                                const float *c32, size_t gp, int f, float x, float y, float z) {
+    float u, vv;
+    const int cs = point_calib ? point_calib[gp] : f;
+    if (calib_f64 && calib_f64[cs]) {
+        double ud, vd, czd;
+        project_point_z_f64(calib64 + (size_t)cs * 32, x, y, z, ud, vd, czd);
+        u = (float)ud, vv = (float)vd;
+    } else {
+        project_point(point_calib ? calib32 + (size_t)cs * 32 : c32, x, y, z, u, vv);
+    }
+    return make_float2(vv, u);
+}
+
+// ---- active pixel tiles ------------------------------------------------------------------------------------------------
+// Invariant: the marked set is a SUPERSET of the Z rows any combine kernel reads. A combine row is a kept point; kept points are
+// in-grid points that are not at the exact origin (vox_cell_index, the origin test of rows_build_kernel), projected through the
+// same calibration choice (point_row_col), and the combine loads exactly the clamped corners of cell_of (corner_pos) at each
+// level. The mark takes every in-grid, non-origin point - kept or dropped by the T / cap limits - through the same functions.
+// One CTA = 256 points of one frame; the frame's tiles of a level are a contiguous range, so the CTA keeps their bits in shared
+// memory (word-aligned with the global bitmap) and ORs each non-zero word into the global bitmap once.
+__global__ void __launch_bounds__(256) tile_mark_kernel(TileMarkArgs m, PixelTiles pt) {
+    extern __shared__ unsigned s_bits[];
+    const int f = blockIdx.y;
+    __shared__ float c32[32];
+    __shared__ int s_w0[MVX_NUM_LEVELS + 1], s_g0[MVX_NUM_LEVELS];   // shared-word offset, first global word of each level
+    if (threadIdx.x == 0) {
+        int o = 0;
+        for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
+            const long long HW = (long long)m.h[l] * m.w[l];
+            const int g0 = (int)(((long long)f * HW / kPixTileRows) >> 5), g1 = (int)((((long long)(f + 1) * HW - 1) / kPixTileRows) >> 5);
+            s_w0[l] = o, s_g0[l] = g0;
+            o += g1 - g0 + 1;
+        }
+        s_w0[MVX_NUM_LEVELS] = o;
+    }
+    if (!m.point_calib && threadIdx.x < 32) c32[threadIdx.x] = m.calib32[f * 32 + threadIdx.x];
+    __syncthreads();
+    for (int i = threadIdx.x; i < s_w0[MVX_NUM_LEVELS]; i += blockDim.x) s_bits[i] = 0u;
+    __syncthreads();
+    const int P = m.off[f + 1] - m.off[f];
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < P) {
+        const size_t gp = (size_t)m.off[f] + i;
+        float x, y, z;
+        if (m.point_stride == 4) {
+            const float4 q = __ldg(reinterpret_cast<const float4 *>(m.points) + gp);
+            x = q.x, y = q.y, z = q.z;
+        } else {
+            const float *q = m.points + gp * m.point_stride;
+            x = q[0], y = q[1], z = q[2];
+        }
+        int ix, iy, iz;
+        if (vox_cell_index(m.lo, m.size, m.shape, x, y, z, ix, iy, iz) && !(x == 0.f && y == 0.f && z == 0.f)) {
+            const float2 pr = point_row_col(m.calib32, m.point_calib, m.calib64, m.calib_f64, c32, gp, f, x, y, z);
+#pragma unroll
+            for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
+                const int H = m.h[l], W = m.w[l];
+                const CornerPos cp = corner_pos(cell_of(pr.x, pr.y, m.rs_h[l], m.rs_w[l], m.eps), H, W);
+                const long long rb = (long long)f * H * W;
+                const long long t00 = (rb + (long long)cp.y0 * W + cp.x0) / kPixTileRows, t01 = (rb + (long long)cp.y0 * W + cp.x1) / kPixTileRows;
+                const long long t10 = (rb + (long long)cp.y1 * W + cp.x0) / kPixTileRows, t11 = (rb + (long long)cp.y1 * W + cp.x1) / kPixTileRows;
+                unsigned *sb = s_bits + s_w0[l];
+                const long long tt[4] = {t00, t01, t10, t11};
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    if (k > 0 && tt[k] == tt[k - 1]) continue;   // corners mostly share a tile
+                    const long long w = (tt[k] >> 5) - s_g0[l];
+                    const unsigned bit = 1u << (tt[k] & 31);
+                    if (!(sb[w] & bit)) atomicOr(sb + w, bit);
+                }
+            }
+        }
+    }
+    __syncthreads();
+    for (int l = 0; l < MVX_NUM_LEVELS; ++l)
+        for (int k = threadIdx.x; k < s_w0[l + 1] - s_w0[l]; k += blockDim.x) {
+            const unsigned v = s_bits[s_w0[l] + k];
+            if (v) atomicOr(pt.bits + pt.word0[l] + s_g0[l] + k, v);
+        }
+}
+
+// one CTA: entries (level << 24 | tile): active ones ascending from 0, then the inactive ones that need zeros (not known zero for
+// this element size of Z), then the remaining inactive ones; afterwards the zero state is that of the end of this call
+__global__ void __launch_bounds__(1024) tile_list_kernel(PixelTiles pt, int all, int z_esize) {
+    const int n = pt.tile0[MVX_NUM_LEVELS];
+    const bool known = pt.meta[5] == z_esize;   // the zero state refers to this layout of Z
+    auto level_of = [&](int g) {
+        int l = 0;
+        while (l + 1 < MVX_NUM_LEVELS && g >= pt.tile0[l + 1]) ++l;
+        return l;
+    };
+    auto bit = [&](const unsigned *b, int g) -> int {
+        const int l = level_of(g), t = g - pt.tile0[l];
+        return (int)((b[pt.word0[l] + (t >> 5)] >> (t & 31)) & 1u);
+    };
+    auto active = [&](int g) -> int { return all ? 1 : bit(pt.bits, g); };
+    auto needs_zero = [&](int g) -> int { return !active(g) && !(known && bit(pt.zbits, g)); };
+    __shared__ int s_count, s_nz;
+    {   // pass 1: number of active tiles and of tiles to zero
+        int c = 0, z = 0;
+        for (int g = threadIdx.x; g < n; g += blockDim.x) c += active(g), z += needs_zero(g);
+        int total, ztotal;
+        block_exclusive_scan(c, &total);
+        block_exclusive_scan(z, &ztotal);
+        if (threadIdx.x == 0) s_count = total, s_nz = ztotal;
+        __syncthreads();
+    }
+    const int count = s_count, nz = s_nz;
+    int carry = 0, zcarry = 0;
+    for (int g0 = 0; g0 < n; g0 += blockDim.x) {
+        const int g = g0 + threadIdx.x;
+        const int a = g < n ? active(g) : 0, z = g < n ? needs_zero(g) : 0;
+        int total, ztotal;
+        const int ex = carry + block_exclusive_scan(a, &total);
+        const int zx = zcarry + block_exclusive_scan(z, &ztotal);
+        if (g < n) {
+            const int l = level_of(g);
+            const int e = (l << 24) | (g - pt.tile0[l]);
+            pt.list[a ? ex : (z ? count + zx : count + nz + (g - ex - zx))] = e;
+            if (g == pt.tile0[l]) pt.meta[l] = ex;   // active entries before the first tile of level l
+        }
+        carry += total, zcarry += ztotal;
+    }
+    __syncthreads();   // every thread has read the old zero state
+    for (int w = threadIdx.x; w < pt.word0[MVX_NUM_LEVELS]; w += blockDim.x) {
+        int l = 0;
+        while (l + 1 < MVX_NUM_LEVELS && w >= pt.word0[l + 1]) ++l;
+        const int t0 = (w - pt.word0[l]) * 32, left = pt.ntiles[l] - t0;
+        const unsigned valid = left >= 32 ? 0xFFFFFFFFu : ((1u << left) - 1u);
+        pt.zbits[w] = all ? 0u : (~pt.bits[w] & valid);   // inactive tiles hold zeros once this call's pixel GEMM is done
+    }
+    if (threadIdx.x == 0) pt.meta[MVX_NUM_LEVELS] = count, pt.meta[4] = count + nz, pt.meta[5] = z_esize;
 }
 
 // ---- the 4-corner weighted gather of one row, one warp, all levels ------------------------------------
@@ -247,17 +391,7 @@ __global__ void __launch_bounds__(256) rows_build_kernel(RowsParams p) {
         if (!(x == 0.f && y == 0.f && z == 0.f)) {  // a real point at the exact origin is treated as a pad slot (Pipe.py:53-59)
             lo = make_float4(x, y, z, (float)((double)x - sx / (double)n));
             hi = make_float4((float)((double)y - sy / (double)n), (float)((double)z - sz / (double)n), refl, 0.f);
-            float u, vv;
-            // merged point sets (GT-paste, train.py:36-41): every point is projected through the calibration it came with
-            const int cs = p.point_calib ? p.point_calib[p.off[f] + pi] : f;
-            if (p.calib_f64 && p.calib_f64[cs]) {   // float64 calibration: fp64 projection, rounded once (torch.Tensor(voxel), train.py:125)
-                double ud, vd, czd;
-                project_point_z_f64(p.calib64 + (size_t)cs * 32, x, y, z, ud, vd, czd);
-                u = (float)ud, vv = (float)vd;
-            } else {
-                project_point(p.point_calib ? p.calib32 + (size_t)cs * 32 : c32, x, y, z, u, vv);
-            }
-            pr = make_float2(vv, u);  // (row, col) = lidar2Img(...)[:, [1, 0]]  (train.py:33)
+            pr = point_row_col(p.calib32, p.point_calib, p.calib64, p.calib_f64, c32, (size_t)p.off[f] + pi, f, x, y, z);
         }
     }
     float4 *dst = reinterpret_cast<float4 *>(p.vox8 + ro * 8);
@@ -404,9 +538,8 @@ __global__ void __launch_bounds__(kCombWarps * 32, MVX_COMB_MINB) combine_rows_k
             const float4 cw = corner_weights(c, H, W);
             CombRec rec;
             rec.w[0] = cw.x, rec.w[1] = cw.y, rec.w[2] = cw.z, rec.w[3] = cw.w;
-            const int y0 = min(max(c.i0, 0), H - 1), y1 = min(max(c.i0 + 1, 0), H - 1);
-            const int x0 = min(max(c.i1, 0), W - 1), x1 = min(max(c.i1 + 1, 0), W - 1);
-            rec.cell = x0 | (y0 << 12) | ((x1 - x0) << 24) | ((y1 - y0) << 25);
+            const CornerPos cp = corner_pos(c, H, W);
+            rec.cell = cp.x0 | (cp.y0 << 12) | ((cp.x1 - cp.x0) << 24) | ((cp.y1 - cp.y0) << 25);
             s_recw[i][l] = make_float4(rec.w[0], rec.w[1], rec.w[2], rec.w[3]);
             s_cell[i][l] = rec.cell;
         }
@@ -557,10 +690,9 @@ __global__ void __launch_bounds__(kCombWarps * 32, MVX_COMB_MINB) combine_runs_k
         for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
             const CellRef c = cell_of(pr.x, pr.y, a.rs_h[l], a.rs_w[l], a.eps);
             const int H = a.h[l], W = a.w[l];
-            const int y0 = min(max(c.i0, 0), H - 1), y1 = min(max(c.i0 + 1, 0), H - 1);
-            const int x0 = min(max(c.i1, 0), W - 1), x1 = min(max(c.i1 + 1, 0), W - 1);
+            const CornerPos cp = corner_pos(c, H, W);
             s_recw[i][l] = corner_weights(c, H, W);
-            s_cell[i][l] = none ? -1 : (x0 | (y0 << 12) | ((x1 - x0) << 24) | ((y1 - y0) << 25));
+            s_cell[i][l] = none ? -1 : (cp.x0 | (cp.y0 << 12) | ((cp.x1 - cp.x0) << 24) | ((cp.y1 - cp.y0) << 25));
         }
     }
     __syncthreads();
@@ -775,9 +907,47 @@ int launch_combine_rows(const CombineArgs &a, int B, cudaStream_t st) {
     return MVX_OK;
 }
 
-int launch_pack_maps_f16(const float *in, void *apack, float *rowinv, int B, int C, int HW, cudaStream_t st) {
+int launch_pack_maps_f16(const float *in, void *apack, float *rowinv, int B, int C, int HW, const unsigned *tile_bits, cudaStream_t st) {
     MVX_REQUIRE(C == 256, MVX_EINVAL, "pack_maps: C must be 256");
-    pack_maps_f16_kernel<<<dim3((HW + 31) / 32, B), 256, 0, st>>>(in, C, HW, static_cast<uint8_t *>(apack), rowinv);
+    pack_maps_f16_kernel<<<dim3((HW + 31) / 32, B), 256, 0, st>>>(in, C, HW, static_cast<uint8_t *>(apack), rowinv, tile_bits);
+    MVX_LAUNCH_CHECK();
+    return MVX_OK;
+}
+
+void pixel_tiles_init(PixelTiles &pt, int B, const int *map_h, const int *map_w, void *mem) {
+    pt.tile0[0] = 0, pt.word0[0] = 0;
+    for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
+        pt.ntiles[l] = (int)ceil_div((long long)B * map_h[l] * map_w[l], kPixTileRows);
+        pt.tile0[l + 1] = pt.tile0[l] + pt.ntiles[l];
+        pt.word0[l + 1] = pt.word0[l] + (pt.ntiles[l] + 31) / 32;
+    }
+    pt.bits = static_cast<unsigned *>(mem);
+    pt.zbits = pt.bits + pt.word0[MVX_NUM_LEVELS];
+    pt.list = reinterpret_cast<int *>(pt.zbits + pt.word0[MVX_NUM_LEVELS]);
+    pt.meta = pt.list + pt.tile0[MVX_NUM_LEVELS];
+}
+
+int launch_pixel_tiles(const TileMarkArgs &m, const PixelTiles &pt, int B, bool all, int z_esize, cudaStream_t st) {
+    MVX_REQUIRE(pt.tile0[MVX_NUM_LEVELS] < (1 << 24), MVX_EINVAL, "pixel tiles: more than 2^24 row tiles");
+    if (!all) {
+        MVX_CUDA_CHECK(cudaMemsetAsync(pt.bits, 0, (size_t)pt.word0[MVX_NUM_LEVELS] * 4, st));
+        int maxP = 0, words = 0;
+        for (int f = 0; f < B; ++f) {
+            maxP = max(maxP, m.off[f + 1] - m.off[f]);
+            int wf = 0;
+            for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
+                const long long HW = (long long)m.h[l] * m.w[l];
+                wf += (int)((((f + 1) * HW - 1) / kPixTileRows) >> 5) - (int)(((f * HW) / kPixTileRows) >> 5) + 1;
+            }
+            words = max(words, wf);
+        }
+        MVX_REQUIRE(words * 4 <= 48 * 1024, MVX_EINVAL, "pixel tiles: FPN maps too large for the shared tile bitmap");
+        if (maxP > 0) {
+            tile_mark_kernel<<<dim3((maxP + 255) / 256, B), 256, words * 4, st>>>(m, pt);
+            MVX_LAUNCH_CHECK();
+        }
+    }
+    tile_list_kernel<<<1, 1024, 0, st>>>(pt, all ? 1 : 0, z_esize);
     MVX_LAUNCH_CHECK();
     return MVX_OK;
 }

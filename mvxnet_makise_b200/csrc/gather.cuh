@@ -36,6 +36,18 @@ __device__ __forceinline__ float4 corner_weights(const CellRef &c, int H, int W)
     return make_float4((r0 && c0) ? c.wa * c.wb : 0.f, (r1 && c0) ? wa_ * c.wb : 0.f, (r0 && c1) ? c.wa * wb_ : 0.f,
                        (r1 && c1) ? wa_ * wb_ : 0.f);
 }
+// The pixels a combine kernel LOADS for a cell: the four corners clamped to [0,H-1] x [0,W-1]. A corner with weight 0 is still
+// loaded (its product is multiplied by 0), so a point projecting outside the map reads a border pixel. Both combine kernels
+// and the pixel-tile mark take their corner positions from here.
+struct CornerPos {
+    int y0, y1, x0, x1;
+};
+__device__ __forceinline__ CornerPos corner_pos(const CellRef &c, int H, int W) {
+    CornerPos p;
+    p.y0 = min(max(c.i0, 0), H - 1), p.y1 = min(max(c.i0 + 1, 0), H - 1);
+    p.x0 = min(max(c.i1, 0), W - 1), p.x1 = min(max(c.i1 + 1, 0), W - 1);
+    return p;
+}
 
 // NCHW (B,C,H,W) -> NHWC (B,H,W,C)
 // rowmax (optional): [B][HW] max |x| over the C channels of every pixel (float; zeroed and filled here)
@@ -44,7 +56,54 @@ int launch_nchw_to_nhwc(const float *in, float *out, int B, int C, int HW, float
 
 // NCHW (B,C,HW) fp32 -> pre-packed fp16 hi/lo A operand of the pixel GEMM (rows R = f*HW + p), rowinv[R] = 1 / row scale.
 // apack must hold round_up(B*HW, 256) * C * 4 bytes; rows beyond B*HW are never read back (their outputs are not stored).
-int launch_pack_maps_f16(const float *in, void *apack, float *rowinv, int B, int C, int HW, cudaStream_t st);
+// tile_bits (optional): the level's active row-tile bitmap (PixelTiles); rows of inactive tiles are neither packed nor scaled.
+int launch_pack_maps_f16(const float *in, void *apack, float *rowinv, int B, int C, int HW, const unsigned *tile_bits, cudaStream_t st);
+
+// ---- active pixel tiles of the pixel-first fcn1 ---------------------------------------------------------------------------
+// The per-pixel GEMM computes Z_l for 256-row tiles (rows R = f*HW_l + p) of every level, but the combine reads only the corner
+// pixels of the kept rows, and LiDAR points never project into the upper image. The mark kernel sets the bit of every row tile
+// that some point's clamped corners (corner_pos) fall in; the list kernel compacts the bitmap into entries (level << 24 | tile):
+// the active ones in ascending (level, tile) order, then the inactive tiles that may hold products of an earlier call, then the
+// inactive tiles already known to be zero (each group ascending). The pixel GEMM multiplies the active tiles and writes zeros into
+// the second group, so after every call an inactive tile of Z is zero. The zero state persists in the workspace (zbits, and the
+// element size of Z it refers to in meta[5]); a workspace whose `tiles` region is zeroed (PointPath does that when it allocates
+// one) starts with every tile unknown. Nothing the path computes reads an inactive tile, so the state only decides which zeros
+// must be rewritten: the sky band no point samples is zeroed once per workspace, not once per call.
+constexpr int kPixTileRows = 256;
+struct PixelTiles {
+    int ntiles[MVX_NUM_LEVELS];   // row tiles of level l: ceil(B * HW_l / 256)
+    int tile0[MVX_NUM_LEVELS + 1];// first list index of level l in the (level, tile) order of all tiles; tile0[3] = all tiles
+    int word0[MVX_NUM_LEVELS + 1];// first bitmap word of level l; word0[3] = bitmap words
+    unsigned *bits;               // [word0[3]] active tiles of this call
+    unsigned *zbits;              // [word0[3]] tiles of Z known to hold zeros (persists across calls)
+    int *list;                    // [tile0[3]] entries: active, then inactive to zero, then inactive and already zero
+    int *meta;                    // [8]: first active entry of each level (meta[0..2]), number of active entries (meta[3]), end of
+                                  // the entries to zero (meta[4]), element size of Z the zero state refers to (meta[5], 0: none)
+};
+inline size_t pixel_tiles_bytes(const int *ntiles) {
+    size_t t = 0, w = 0;
+    for (int l = 0; l < MVX_NUM_LEVELS; ++l) t += ntiles[l], w += (ntiles[l] + 31) / 32;
+    return (2 * w + t + 8) * 4;
+}
+void pixel_tiles_init(PixelTiles &pt, int B, const int *map_h, const int *map_w, void *mem);   // fills the extents and pointers
+struct TileMarkArgs {
+    const float *points;
+    int point_stride;
+    int off[33];            // frame point offsets (host)
+    // the calibration choice of rows_build_kernel (RowsParams)
+    const float *calib32;
+    const int *point_calib;
+    const double *calib64;
+    const int *calib_f64;
+    double lo[3], size[3];  // the voxel grid: only in-grid points become rows
+    int shape[3];
+    int h[MVX_NUM_LEVELS], w[MVX_NUM_LEVELS];
+    float rs_h[MVX_NUM_LEVELS], rs_w[MVX_NUM_LEVELS];
+    float eps;
+};
+// zero the bitmap, mark (raw points) or mark everything (all = true: the dense-voxel entry), then build the list; z_esize = bytes per
+// element of Z in this call (4: fp32, 2: bf16)
+int launch_pixel_tiles(const TileMarkArgs &m, const PixelTiles &pt, int B, bool all, int z_esize, cudaStream_t st);
 
 struct RowsParams {
     int B, cap, capA, T;

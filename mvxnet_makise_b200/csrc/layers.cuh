@@ -36,6 +36,10 @@ struct LayerArgs {
     // applied to row r).
     const void *a_pack;
     const float *a_rowinv;   // NULL: no per-row scale
+    // pre-packed A only (optional): grid row y is row tile tile_list[tile_bounds[0] + y] & 0xFFFFFF, CTAs past tile_bounds[1] exit
+    // (the active tiles of one level of the pixel GEMM, gather.cuh PixelTiles)
+    const int *tile_list;
+    const int *tile_bounds;
     // fused concat (16-bit tensor-core producer only): input columns [Cin - x2_cols, Cin) of row r come from
     // X2[f][v(r)][0:x2_cols] (float bits, e.g. the per-voxel max of the producer layer) instead of X, with
     // v(r) = r >= K_f ? r - K_f : cat_row_vox[f][r]; both parts are normalised with the same in_stats (in_C channels)
@@ -84,8 +88,22 @@ int launch_layer_tc(const LayerArgs &a, int F, float *wpack, cudaStream_t st);
 bool tc3_layer_eligible(const LayerArgs &a);
 int launch_layer_tc3(const LayerArgs &a, int F, float *wpack, cudaStream_t st);
 // persistent pre-packed-operand GEMM for the per-pixel half of fcn1 (tc3_layer.cu)
-bool pixel_gemm_persistent_eligible(const LayerArgs &a);
-int launch_pixel_gemm_persistent(const LayerArgs &a, float *wpack, cudaStream_t st);
+// Per-pixel products of fcn1 for all FPN levels, Z_l = F_l W1[:, l Cin : (l+1) Cin]^T, over the pixel-tile list (gather.cuh
+// PixelTiles): active row tiles are multiplied, inactive ones are written as zeros, so every element of Z is defined.
+struct PixelGemmArgs {
+    const void *a_pack[MVX_NUM_LEVELS];       // pre-packed A of each level (pack_maps_f16_kernel)
+    const float *a_rowinv[MVX_NUM_LEVELS];
+    void *Z[MVX_NUM_LEVELS];                  // (R_l, Cout) fp32, or bf16 with z_bf16
+    long long R[MVX_NUM_LEVELS];              // rows (pixels of all frames) of each level
+    const float *Wt;                          // W1^T (levels * Cin, Cout)
+    int Cin, Cout, z_bf16;
+    const int *list, *meta;                   // PixelTiles::list / ::meta
+    int n_entries;                            // all row tiles of all levels
+};
+// one persistent launch for the three levels (the weights of the three K blocks packed by one launch into wpack)
+int launch_pixel_gemm_levels(const PixelGemmArgs &a, float *wpack, cudaStream_t st);
+// mvx_set_gemm_mode(12): the one-tile kernel per level over the level's active tiles, then the zeros of the inactive tiles
+int launch_pixel_gemm_one_tile(const PixelGemmArgs &a, float *wpack, cudaStream_t st);
 void set_pixel_persistent(int on);
 bool pixel_persistent_enabled();
 void set_tc3(int on);

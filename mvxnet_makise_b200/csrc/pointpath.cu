@@ -19,7 +19,7 @@ namespace mvx {
 const char *kRegionNames[R_COUNT] = {
     "vox_ws", "vox_coord", "vox_cnt", "vox_row0", "row_point", "row_vox", "cell2vid", "nhwc0", "nhwc1", "nhwc2",
     "vox8", "proj", "rowA_w", "A1", "Y1", "Y2", "Y3", "Y4", "Y5", "X6", "Y6", "X7", "Y7", "rowB_w", "rowB_v", "X8",
-    "vfeat", "stats", "vmax6", "vmax7", "vmax8", "wpack", "occ", "vfeat_t", "Z", "bin_count", "bin_start", "perm", "rowmax", "chmax", "A1max", "Y8"};
+    "vfeat", "stats", "vmax6", "vmax7", "vmax8", "wpack", "occ", "vfeat_t", "Z", "bin_count", "bin_start", "perm", "rowmax", "chmax", "A1max", "tiles", "Y8"};
 
 // 1 (default): pixel-first fcn1 - one tensor-core GEMM per FPN level over the map pixels, then a 12-corner combine per
 // point row (gather.cuh CombineArgs); 0: materialise the gathered (K,768) matrix A1 and run fcn1 over the point rows
@@ -90,6 +90,9 @@ int make_layout(const mvx_pointpath_args_t *a, Layout &L) {
         take(R_ROWMAX, B * px * 4);
         take(R_CHMAX, B * 768 * 4);
         take(R_A1MAX, B * capA * 4);
+        int ntiles[MVX_NUM_LEVELS];
+        for (int l = 0; l < MVX_NUM_LEVELS; ++l) ntiles[l] = (int)ceil_div((long long)B * a->map_h[l] * a->map_w[l], kPixTileRows);
+        take(R_TILES, pixel_tiles_bytes(ntiles));   // active pixel tiles of the pixel GEMM: bitmap, list, counts
     }
     L.total = o;
     take(R_Y8, B * capB * 128 * 4);   // last region: only present in a training workspace
@@ -229,18 +232,37 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     auto z_at = [&](size_t elem_off) -> float * {   // element offset into Z, whatever its element size
         return bf16_mem ? reinterpret_cast<float *>(reinterpret_cast<uint16_t *>(ws + L.off[R_Z]) + elem_off) : F32(R_Z) + elem_off;
     };
+    PixelTiles pt{};
+    pixel_tiles_init(pt, B, a->map_h, a->map_w, ws + L.off[R_TILES]);
     auto map_branch = [&](MapSet &m) -> int {
         stamp.begin(S_NHWC, ms);
-        size_t rowmax_off = 0;
         for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
-            const int HW = a->map_h[l] * a->map_w[l];
             m.h[l] = a->map_h[l], m.w[l] = a->map_w[l];
             m.rs_h[l] = a->imsize_h / (float)a->map_h[l];
             m.rs_w[l] = a->imsize_w / (float)a->map_w[l];
             m.nhwc[l] = F32((Region)(R_NHWC0 + l));
-            m.frame_stride[l] = (size_t)HW * a->map_c;
+            m.frame_stride[l] = (size_t)a->map_h[l] * a->map_w[l] * a->map_c;
+        }
+        if (pixel_first) {   // which 256-row tiles of Z the combine can read: from the raw points and the calibration only
+            TileMarkArgs tm{};
+            if (!dense_in) {
+                tm.points = a->points, tm.point_stride = a->point_stride;
+                for (int f = 0; f <= B; ++f) tm.off[f] = a->pt_off_host[f];
+                tm.calib32 = a->calib32, tm.point_calib = a->point_calib;
+                tm.calib64 = a->calib64, tm.calib_f64 = a->calib64 ? a->calib_f64 : nullptr;   // as RowsParams below
+                for (int d = 0; d < 3; ++d) tm.lo[d] = a->grid.range_lo[d], tm.size[d] = a->grid.voxel_size[d], tm.shape[d] = a->grid.shape[d];
+                for (int l = 0; l < MVX_NUM_LEVELS; ++l) tm.h[l] = m.h[l], tm.w[l] = m.w[l], tm.rs_h[l] = m.rs_h[l], tm.rs_w[l] = m.rs_w[l];
+                tm.eps = a->gather_eps;
+            }
+            int r = launch_pixel_tiles(tm, pt, B, dense_in, bf16_mem ? 2 : 4, ms);   // dense-voxel entry: no raw points, every tile is active
+            if (r) return r;
+        }
+        size_t rowmax_off = 0;
+        for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
+            const int HW = a->map_h[l] * a->map_w[l];
             if (apack) {
-                int r = launch_pack_maps_f16(a->maps[l], ws + L.off[R_NHWC0 + l], F32(R_ROWMAX) + rowmax_off, B, a->map_c, HW, ms);
+                int r = launch_pack_maps_f16(a->maps[l], ws + L.off[R_NHWC0 + l], F32(R_ROWMAX) + rowmax_off, B, a->map_c, HW,
+                                             dense_in ? nullptr : pt.bits + pt.word0[l], ms);
                 if (r) return r;
                 rowmax_off += (size_t)B * HW;
                 continue;
@@ -252,22 +274,22 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
         }
         stamp.end(S_NHWC, ms);
         if (!pixel_first) return MVX_OK;
-        // Z_l = F_l W1[:, 256 l : 256 (l+1)]^T for every pixel of every frame (plain GEMM: no bias / ReLU / statistics)
+        // Z_l = F_l W1[:, 256 l : 256 (l+1)]^T for the active pixel tiles of every level, zeros elsewhere (plain GEMM: no bias /
+        // ReLU / statistics)
         stamp.begin(S_GATHER, ms);
+        MVX_REQUIRE(apack, MVX_EINVAL, "pixel-first fcn1 needs the pre-packed maps");
+        PixelGemmArgs pg{};
         size_t zoff = 0;
         for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
             const long long px = (long long)B * a->map_h[l] * a->map_w[l];
-            LayerArgs la{};
-            la.X = m.nhwc[l], la.ldx = a->map_c, la.Cin = a->map_c;
-            la.Wt = a->wt[0] + (size_t)l * a->map_c * 768, la.bias = nullptr, la.Cout = 768;
-            la.Y = z_at(zoff), la.ldy = 768, la.y_bf16 = bf16_mem;
-            la.rows_fixed = px, la.rows_mode = 0, la.rowcap = 0, la.T = 1, la.eps = a->bn_eps, la.plain = 1;
-            la.f16_ok = 1, la.row_max = F32(R_ROWMAX) + zoff / 768;   // raw FPN features: per-pixel power-of-two scaling
-            if (apack) la.a_pack = ws + L.off[R_NHWC0 + l], la.a_rowinv = F32(R_ROWMAX) + zoff / 768, la.row_max = nullptr;
-            int r = pixel_gemm_persistent_eligible(la) ? launch_pixel_gemm_persistent(la, F32(R_WPACK), ms) : launch_layer_auto(la, 1, F32(R_WPACK), ms);
-            if (r) return r;
+            pg.a_pack[l] = ws + L.off[R_NHWC0 + l], pg.a_rowinv[l] = F32(R_ROWMAX) + zoff / 768;
+            pg.Z[l] = z_at(zoff), pg.R[l] = px;
             zoff += (size_t)px * 768;
         }
+        pg.Wt = a->wt[0], pg.Cin = a->map_c, pg.Cout = 768, pg.z_bf16 = bf16_mem;
+        pg.list = pt.list, pg.meta = pt.meta, pg.n_entries = pt.tile0[MVX_NUM_LEVELS];
+        int r = pixel_persistent_enabled() ? launch_pixel_gemm_levels(pg, F32(R_WPACK), ms) : launch_pixel_gemm_one_tile(pg, F32(R_WPACK), ms);
+        if (r) return r;
         stamp.end(S_GATHER, ms);
         return MVX_OK;
     };

@@ -601,8 +601,11 @@ __global__ void __launch_bounds__(t3_threads(NCG, NEG), 1) tc3_layer_kernel(cons
 // The one-tile kernel it replaces (tc_layer_kernel<128, F16, -, TWO, APK>, two CTAs per SM) restarts its 2-stage ring for every
 // tile: ncu attributes 42 % of its samples to the epilogue warps idling through an ~6 us main loop that exposes one L2 round trip
 // per pair of chunks, then ~10 us of epilogue per CTA for 3.7 us of MMAs (profiles/r5v_pixel_gemm_stall_lines.txt).
-// Tile order: t = row tile x 6 + column block, striped over the CTAs, so the six tiles that share an A tile run at the same time
-// on neighbouring CTAs (one DRAM read of A, five L2 hits).
+// One launch covers the three FPN levels: it walks the pixel-tile list (gather.cuh PixelTiles). MMA tiles: t = active entry x 6 +
+// column block, striped over the CTAs, so the six tiles that share an A tile run at the same time on neighbouring CTAs (one DRAM
+// read of A, five L2 hits); the entries ascend, so the striping is that of one level after the other. Zero tiles (inactive entry
+// that may hold products of an earlier call x 6 + column block; gather.cuh PixelTiles) are epilogue-only: no loads, no MMAs, four tensor stores per warp from a zeroed shared block. Each CTA
+// spreads its zero tiles evenly between its MMA tiles, so these stores run while the tensor pipe works on the next accumulator.
 // =====================================================================================================================
 #ifndef MVX_PG_STAGES
 #define MVX_PG_STAGES 3
@@ -616,28 +619,32 @@ constexpr int PG_EPI_WARPS = 8, PG_THREADS = (2 + PG_EPI_WARPS) * 32;
 struct PgSmem {
     static constexpr int kRing = 0;
     static constexpr int kStg = kRing + PG_STAGES * PG_STAGE;        // [2 groups] 128 x 32 fp32 staging block
-    static constexpr int kBars = kStg + 2 * T3_STG_BYTES;            // full[], empty[], acc_full[2], acc_empty[2] (the column scales are read from global memory: L1 hits, and the fourth stage needs their 3 KB)
+    static constexpr int kZero = kStg + 2 * T3_STG_BYTES;            // 32 x 32 fp32 zeros: the source of the zero tiles' stores
+    static constexpr int kBars = kZero + 32 * 32 * 4;                // full[], empty[], acc_full[2], acc_empty[2] (the column scales are read from global memory: L1 hits, and the fourth stage needs their 3 KB)
     static constexpr int kTmemPtr = kBars + 8 * (2 * PG_STAGES + 4);
     static constexpr int kTotal = kTmemPtr + 16 + 1024;
 };
 static_assert(PgSmem::kTotal <= 232448, "pixel GEMM: shared memory");
 
-struct PgArgs {
-    const uint8_t *a_pack;     // [row tiles][nk][hi 16 KB | lo 16 KB]
-    const float *a_rowinv;     // [R] inverse power-of-two row scales (or NULL)
-    const uint8_t *wpack;      // [column blocks][nk][hi 8 KB | lo 8 KB], then Cout inverse column scales
-    long long R;               // rows (pixels of all frames of the level)
-    int Cin, Cout, row_tiles;
+struct PgArgs {   // per FPN level l:
+    const uint8_t *a_pack[MVX_NUM_LEVELS];     // [row tiles][nk][hi 16 KB | lo 16 KB]
+    const float *a_rowinv[MVX_NUM_LEVELS];     // [R] inverse power-of-two row scales (or NULL)
+    const uint8_t *wpack[MVX_NUM_LEVELS];      // [column blocks][nk][hi 8 KB | lo 8 KB], then Cout inverse column scales
+    long long R[MVX_NUM_LEVELS];               // rows (pixels of all frames of the level)
+    const int *list, *meta;                    // pixel-tile list: entries (level << 24 | row tile), active ones first; meta[3] = active, meta[4] = end of the ones to zero
+    int n_entries, Cin, Cout;
+};
+struct PgMaps {
+    CUtensorMap z[MVX_NUM_LEVELS];             // Z of each level: rows past R_l are clipped at the level's own end
 };
 
 // ZB: Z is written as bf16 (the bf16 mode stores its two largest intermediates, Z and Y1, as bf16; the products stay 3xFP16)
 template <bool ZB>
-__global__ void __launch_bounds__(PG_THREADS, 1) pixel_gemm_persistent_kernel(const __grid_constant__ PgArgs g, const __grid_constant__ CUtensorMap tmZ) {
+__global__ void __launch_bounds__(PG_THREADS, 1) pixel_gemm_persistent_kernel(const __grid_constant__ PgArgs g, const __grid_constant__ PgMaps tm) {
     using S = PgSmem;
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t *smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
     const uint32_t sbase = smem_u32(smem);
-    const float *colinv = reinterpret_cast<const float *>(g.wpack + (size_t)g.Cin * g.Cout * 4);
     const uint32_t bars = sbase + S::kBars;
     auto full_bar = [&](int s) { return bars + 8u * s; };
     auto empty_bar = [&](int s) { return bars + 8u * (PG_STAGES + s); };
@@ -646,7 +653,8 @@ __global__ void __launch_bounds__(PG_THREADS, 1) pixel_gemm_persistent_kernel(co
     volatile uint32_t *tmem_ptr = reinterpret_cast<volatile uint32_t *>(smem + S::kTmemPtr);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int nk = g.Cin / PG_KB, ncb = g.Cout / PG_BN;
-    const int total = g.row_tiles * ncb;
+    const int n_active = g.meta[3];
+    const int total = n_active * ncb, total_zero = (g.meta[4] - n_active) * ncb;   // MMA tiles, zero tiles
 
     if (tid == 0) {
         for (int s = 0; s < PG_STAGES; ++s) mbar_init(full_bar(s), 1), mbar_init(empty_bar(s), 1);
@@ -657,6 +665,8 @@ __global__ void __launch_bounds__(PG_THREADS, 1) pixel_gemm_persistent_kernel(co
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(sbase + S::kTmemPtr), "r"(512u) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
+    for (int i = tid; i < 32 * 32; i += PG_THREADS) reinterpret_cast<float *>(smem + S::kZero)[i] = 0.f;
+    fence_async_smem();   // the zeros are read by the tensor stores (async proxy)
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -667,9 +677,10 @@ __global__ void __launch_bounds__(PG_THREADS, 1) pixel_gemm_persistent_kernel(co
         if (lane == 0) {
             int gc = 0;
             for (int t = blockIdx.x; t < total; t += gridDim.x) {
-                const int rt = t / ncb, cb = t - rt * ncb;
-                const uint8_t *asrc = g.a_pack + (size_t)rt * nk * (2 * PG_A_HALF);
-                const uint8_t *bsrc = g.wpack + (size_t)cb * nk * (2 * PG_B_HALF);
+                const int e = t / ncb, cb = t - e * ncb;
+                const int ent = g.list[e], lv = ent >> 24, rt = ent & 0xFFFFFF;
+                const uint8_t *asrc = g.a_pack[lv] + (size_t)rt * nk * (2 * PG_A_HALF);
+                const uint8_t *bsrc = g.wpack[lv] + (size_t)cb * nk * (2 * PG_B_HALF);
                 for (int kc = 0; kc < nk; ++kc, ++gc) {
                     const int s = gc % PG_STAGES;
                     mbar_wait(empty_bar(s), ((gc / PG_STAGES) & 1) ^ 1);
@@ -716,14 +727,38 @@ __global__ void __launch_bounds__(PG_THREADS, 1) pixel_gemm_persistent_kernel(co
         const int q = warp & 3, eg = (warp - 2) >> 2;
         const int et = (tid - 64) & 127;
         uint8_t *stg = smem + S::kStg + eg * T3_STG_BYTES;
-        if (et == 0) prefetch_tmap(&tmZ);
+        if (et == 0) {
+#pragma unroll
+            for (int l = 0; l < MVX_NUM_LEVELS; ++l) prefetch_tmap(&tm.z[l]);
+        }
+        // this CTA's MMA tiles and zero tiles; before MMA tile `it` the warp has stored the zero tiles up to (it + 1) nz / (nm + 1)
+        const int nm = blockIdx.x < total ? (total - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
+        const int nz = blockIdx.x < total_zero ? (total_zero - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
+        int zdone = 0;
+        auto zero_upto = [&](int target) {   // this warp's 32 rows x 128 columns of each zero tile: four boxes of zeros
+            for (; zdone < target; ++zdone) {
+                const int z = (int)blockIdx.x + zdone * (int)gridDim.x;
+                const int e = z / ncb, cb = z - e * ncb;
+                const int ent = g.list[n_active + e], lv = ent >> 24, rt = ent & 0xFFFFFF;
+                const long long r = (long long)rt * PG_TM + eg * 128 + q * 32;
+                if (lane == 0 && r < g.R[lv]) {   // rows beyond R_l are clipped by the level's tensor map
+#pragma unroll
+                    for (int c32 = 0; c32 < 4; ++c32) tma_store_2d(&tm.z[lv], cb * PG_BN + c32 * 32, (int)r, sbase + S::kZero);
+                    tma_store_commit();
+                }
+            }
+        };
         int it = 0;
         for (int t = blockIdx.x; t < total; t += gridDim.x, ++it) {
-            const int rt = t / ncb, cb = t - rt * ncb;
+            const int e = t / ncb, cb = t - e * ncb;
+            const int ent = g.list[e], lv = ent >> 24, rt = ent & 0xFFFFFF;
             const int ab = it & 1;
             const long long row0 = (long long)rt * PG_TM + eg * 128;
             const int rloc = q * 32 + lane;
-            const float rinv = (g.a_rowinv && row0 + rloc < g.R) ? __ldg(g.a_rowinv + row0 + rloc) : 1.f;   // in flight during the wait below
+            const float *rowinv = g.a_rowinv[lv];
+            const float rinv = (rowinv && row0 + rloc < g.R[lv]) ? __ldg(rowinv + row0 + rloc) : 1.f;   // in flight during the wait below
+            const float *colinv = reinterpret_cast<const float *>(g.wpack[lv] + (size_t)g.Cin * g.Cout * 4);
+            zero_upto((int)((long long)(it + 1) * nz / (nm + 1)));
             mbar_wait(acc_full(ab), (it >> 1) & 1);
             tc_fence_after();
 #pragma unroll 1
@@ -764,11 +799,12 @@ __global__ void __launch_bounds__(PG_THREADS, 1) pixel_gemm_persistent_kernel(co
                 fence_async_smem();
                 __syncwarp();
                 if (lane == 0) {   // 32 rows x 32 columns: rows beyond R are clipped by the tensor map
-                    tma_store_2d(&tmZ, cb * PG_BN + c32 * 32, (int)(row0 + q * 32), smem_u32(stg + q * (ZB ? 2048 : 4096)));
+                    tma_store_2d(&tm.z[lv], cb * PG_BN + c32 * 32, (int)(row0 + q * 32), smem_u32(stg + q * (ZB ? 2048 : 4096)));
                     tma_store_commit();
                 }
             }
         }
+        zero_upto(nz);
         if (lane == 0) tma_store_wait_all();
     }
     __syncwarp();
@@ -879,31 +915,74 @@ static int g_pixel_persistent = 1;   // 0: the one-tile two-CTAs-per-SM kernel o
 void set_pixel_persistent(int on) { g_pixel_persistent = on; }
 bool pixel_persistent_enabled() { return g_pixel_persistent != 0; }
 
-bool pixel_gemm_persistent_eligible(const LayerArgs &a) {
-    return g_pixel_persistent && a.plain && a.a_pack && a.Y && !a.counts && a.rows_fixed > 0 && a.Cin % PG_KB == 0 && a.Cout % PG_BN == 0 &&
-           a.Cout <= 768 && a.ldy % 8 == 0;
-}
+// the weights of the three K blocks, one after the other in wpack (Cin x Cout fp16 hi/lo images, then Cout column scales)
+static size_t pixel_wpack_level_bytes(int Cin, int Cout) { return (size_t)round_up((int64_t)Cin * Cout * 4 + (int64_t)Cout * 4, 256); }
+int pack_weights_f16_128_levels(const float *Wt, int Cin, int Cout, int levels, void *wpack, size_t level_bytes, cudaStream_t st);
 
-int launch_pixel_gemm_persistent(const LayerArgs &a, float *wpack, cudaStream_t st) {
-    MVX_REQUIRE(pixel_gemm_persistent_eligible(a) && wpack, MVX_EINVAL, "layer not eligible for the persistent pixel GEMM");
-    int rc = pack_weights_f16_128(a.Wt, a.Cin, a.Cout, wpack, st, false);
+int launch_pixel_gemm_levels(const PixelGemmArgs &a, float *wpack, cudaStream_t st) {
+    MVX_REQUIRE(wpack && a.Wt && a.list && a.meta && a.n_entries > 0 && a.Cin % PG_KB == 0 && a.Cout % PG_BN == 0 && a.Cout <= 768, MVX_EINVAL,
+                "pixel GEMM: bad arguments");
+    const size_t lb = pixel_wpack_level_bytes(a.Cin, a.Cout);
+    int rc = pack_weights_f16_128_levels(a.Wt, a.Cin, a.Cout, MVX_NUM_LEVELS, wpack, lb, st);
     if (rc) return rc;
     PgArgs g{};
-    g.a_pack = static_cast<const uint8_t *>(a.a_pack), g.a_rowinv = a.a_rowinv, g.wpack = reinterpret_cast<const uint8_t *>(wpack);
-    g.R = a.rows_fixed, g.Cin = a.Cin, g.Cout = a.Cout, g.row_tiles = (int)ceil_div(a.rows_fixed, (long long)PG_TM);
-    CUtensorMap tmZ;
-    rc = make_tmap(&tmZ, a.Y, a.rows_fixed, a.Cout, a.ldy, a.y_bf16 != 0, 32);   // one 32-row box per epilogue warp
-    if (rc) return rc;
+    PgMaps tm;
+    for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
+        MVX_REQUIRE(a.a_pack[l] && a.Z[l] && a.R[l] > 0, MVX_EINVAL, "pixel GEMM: null level operand");
+        g.a_pack[l] = static_cast<const uint8_t *>(a.a_pack[l]), g.a_rowinv[l] = a.a_rowinv[l];
+        g.wpack[l] = reinterpret_cast<const uint8_t *>(wpack) + l * lb, g.R[l] = a.R[l];
+        rc = make_tmap(&tm.z[l], a.Z[l], a.R[l], a.Cout, a.Cout, a.z_bf16 != 0, 32);   // one 32-row box per epilogue warp
+        if (rc) return rc;
+    }
+    g.list = a.list, g.meta = a.meta, g.n_entries = a.n_entries, g.Cin = a.Cin, g.Cout = a.Cout;
     static bool attr_set = false;
     if (!attr_set) {
         MVX_CUDA_CHECK(cudaFuncSetAttribute(pixel_gemm_persistent_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PgSmem::kTotal));
         MVX_CUDA_CHECK(cudaFuncSetAttribute(pixel_gemm_persistent_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PgSmem::kTotal));
         attr_set = true;
     }
-    const long long tiles = (long long)g.row_tiles * (a.Cout / PG_BN);
+    const long long tiles = (long long)a.n_entries * (a.Cout / PG_BN);   // MMA + zero tiles: the active count is on the device
     const int grid = (int)(tiles < kSMs ? tiles : kSMs);
-    if (a.y_bf16) pixel_gemm_persistent_kernel<true><<<grid, PG_THREADS, PgSmem::kTotal, st>>>(g, tmZ);
-    else pixel_gemm_persistent_kernel<false><<<grid, PG_THREADS, PgSmem::kTotal, st>>>(g, tmZ);
+    if (a.z_bf16) pixel_gemm_persistent_kernel<true><<<grid, PG_THREADS, PgSmem::kTotal, st>>>(g, tm);
+    else pixel_gemm_persistent_kernel<false><<<grid, PG_THREADS, PgSmem::kTotal, st>>>(g, tm);
+    MVX_LAUNCH_CHECK();
+    return MVX_OK;
+}
+
+namespace {
+// zeros of the inactive entries that need them (one CTA per entry; CTAs past them exit): the one-tile kernel of gemm mode 12 writes
+// only its active tiles
+__global__ void __launch_bounds__(256) zero_inactive_tiles_kernel(PgArgs g, uint8_t *z0, uint8_t *z1, uint8_t *z2, int esize) {
+    const int n_active = g.meta[3], e = n_active + (int)blockIdx.x;
+    if (e >= g.meta[4]) return;
+    const int ent = g.list[e], lv = ent >> 24, rt = ent & 0xFFFFFF;
+    uint8_t *z = lv == 0 ? z0 : (lv == 1 ? z1 : z2);
+    const long long r0 = (long long)rt * PG_TM, r1 = min(r0 + PG_TM, g.R[lv]);
+    const size_t row_bytes = (size_t)g.Cout * esize;
+    uint4 *p = reinterpret_cast<uint4 *>(z + (size_t)r0 * row_bytes);
+    const size_t n = (size_t)(r1 - r0) * row_bytes / 16;
+    for (size_t i = threadIdx.x; i < n; i += blockDim.x) p[i] = make_uint4(0u, 0u, 0u, 0u);
+}
+}  // namespace
+
+int launch_pixel_gemm_one_tile(const PixelGemmArgs &a, float *wpack, cudaStream_t st) {
+    MVX_REQUIRE(wpack && a.Wt && a.list && a.meta && a.n_entries > 0 && !a.z_bf16, MVX_EINVAL, "pixel GEMM (one-tile kernel): bad arguments");
+    for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
+        LayerArgs la{};
+        la.X = nullptr, la.ldx = a.Cin, la.Cin = a.Cin;
+        la.Wt = a.Wt + (size_t)l * a.Cin * a.Cout, la.bias = nullptr, la.Cout = a.Cout;
+        la.Y = static_cast<float *>(a.Z[l]), la.ldy = a.Cout;
+        la.rows_fixed = a.R[l], la.rows_mode = 0, la.rowcap = 0, la.T = 1, la.plain = 1, la.f16_ok = 1;
+        la.a_pack = a.a_pack[l], la.a_rowinv = a.a_rowinv[l];
+        la.tile_list = a.list, la.tile_bounds = a.meta + l;
+        int rc = launch_layer_tc(la, 1, wpack, st);
+        if (rc) return rc;
+    }
+    PgArgs g{};
+    for (int l = 0; l < MVX_NUM_LEVELS; ++l) g.R[l] = a.R[l];
+    g.list = a.list, g.meta = a.meta, g.n_entries = a.n_entries, g.Cout = a.Cout;
+    zero_inactive_tiles_kernel<<<a.n_entries, 256, 0, st>>>(g, static_cast<uint8_t *>(a.Z[0]), static_cast<uint8_t *>(a.Z[1]),
+                                                           static_cast<uint8_t *>(a.Z[2]), 4);
     MVX_LAUNCH_CHECK();
     return MVX_OK;
 }

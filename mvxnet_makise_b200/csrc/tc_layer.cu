@@ -79,10 +79,14 @@ __global__ void __launch_bounds__(256) pack_weights_kernel(const float *__restri
 // W^T (Cin, Cout) -> per (column tile, 32-k chunk) the shared-memory image [hi | lo] in fp16, columns pre-scaled;
 // colinv[n] = 1 / scale_n. One CTA per output column.
 template <int BN, bool BF1>
+// blockIdx.y = K block: W^T rows [y Cin, (y+1) Cin) packed at out + y * level_bytes (the pixel GEMM's three FPN levels in one launch)
 __global__ void __launch_bounds__(256) pack_weights_f16_kernel(const float *__restrict__ Wt, int Cin, int Cout, uint8_t *__restrict__ out,
-                                                               float *__restrict__ colinv) {
+                                                               float *__restrict__ colinv, size_t level_bytes = 0) {
     __shared__ float s_max[256];
     const int n = blockIdx.x, tid = threadIdx.x;
+    Wt += (size_t)blockIdx.y * Cin * Cout;
+    out += blockIdx.y * level_bytes;
+    colinv = reinterpret_cast<float *>(reinterpret_cast<uint8_t *>(colinv) + blockIdx.y * level_bytes);
     float mx = 0.f;
     for (int k = tid; k < Cin; k += 256) mx = fmaxf(mx, fabsf(Wt[(size_t)k * Cout + n]));
     s_max[tid] = mx;
@@ -154,7 +158,15 @@ __global__ void __launch_bounds__(tc_producer_warps(F16, TWO) * 32 + 64, TWO ? 2
         n_rows = a.rows_mode == 1 ? Kf + 1 : (a.rows_mode == 2 ? Kf + N : (a.rows_mode == 3 ? N : a.rows_fixed));
         Rstat = (double)N * (double)a.T;
     }
-    const long long row0 = (long long)blockIdx.y * kTM;  // column tiles of one row tile are launch-adjacent: A hits L2
+    long long row_tile = blockIdx.y;
+    if constexpr (APK) {
+        if (a.tile_list) {   // pixel GEMM: blockIdx.y walks the level's active row tiles (gather.cuh PixelTiles)
+            const int e = a.tile_bounds[0] + (int)blockIdx.y;
+            if (e >= a.tile_bounds[1]) return;
+            row_tile = a.tile_list[e] & 0xFFFFFF;
+        }
+    }
+    const long long row0 = row_tile * kTM;  // column tiles of one row tile are launch-adjacent: A hits L2
     if (row0 >= n_rows) return;  // uniform for the CTA, before any barrier / TMEM allocation
     const int nk = a.Cin / KB;
     float *s_rowinv = reinterpret_cast<float *>(smem + S::kRowInv);   // F16: 1 / (power-of-two scale of each row)
@@ -376,7 +388,7 @@ __global__ void __launch_bounds__(tc_producer_warps(F16, TWO) * 32 + 64, TWO ? 2
                 mbar_wait(empty_bar(s), ph ^ 1);
                 if constexpr (APK) {
                     mbar_arrive_expect_tx(full_bar(s), 2 * S::kAHalf + 2 * S::kBHalf);
-                    const uint8_t *asrc = static_cast<const uint8_t *>(a.a_pack) + ((size_t)blockIdx.y * nk + kc) * (2 * S::kAHalf);
+                    const uint8_t *asrc = static_cast<const uint8_t *>(a.a_pack) + ((size_t)row_tile * nk + kc) * (2 * S::kAHalf);
                     bulk_g2s(sbase + s * S::kStage, asrc, 2 * S::kAHalf, full_bar(s));
                 } else {
                     mbar_arrive_expect_tx(full_bar(s), 2 * S::kBHalf);
@@ -602,6 +614,14 @@ int pack_weights_f16_128(const float *Wt, int Cin, int Cout, void *wpack, cudaSt
     if (bf16) pack_weights_f16_kernel<128, true><<<Cout, 256, 0, st>>>(Wt, Cin, Cout, blob, reinterpret_cast<float *>(blob + (size_t)Cin * Cout * 4));
     else
     pack_weights_f16_kernel<128, false><<<Cout, 256, 0, st>>>(Wt, Cin, Cout, blob, reinterpret_cast<float *>(blob + (size_t)Cin * Cout * 4));
+    MVX_LAUNCH_CHECK();
+    return MVX_OK;
+}
+
+int pack_weights_f16_128_levels(const float *Wt, int Cin, int Cout, int levels, void *wpack, size_t level_bytes, cudaStream_t st) {
+    uint8_t *blob = static_cast<uint8_t *>(wpack);
+    pack_weights_f16_kernel<128, false><<<dim3(Cout, levels), 256, 0, st>>>(Wt, Cin, Cout, blob, reinterpret_cast<float *>(blob + (size_t)Cin * Cout * 4),
+                                                                              level_bytes);
     MVX_LAUNCH_CHECK();
     return MVX_OK;
 }

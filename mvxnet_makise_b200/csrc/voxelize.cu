@@ -63,11 +63,7 @@ __global__ void __launch_bounds__(256) vox_insert_kernel(VoxParams p) {
                 const float *q = p.points + gp * p.point_stride;
                 x = q[0], y = q[1], z = q[2];
             }
-            // fp64 subtract and TRUE division, C truncation (Preprocessing.py:67-69; SURVEY.md trap 1)
-            ix = (int)(((double)x - p.lo[0]) / p.size[0]);
-            iy = (int)(((double)y - p.lo[1]) / p.size[1]);
-            iz = (int)(((double)z - p.lo[2]) / p.size[2]);
-            bad = ix < 0 || ix >= p.shape[0] || iy < 0 || iy >= p.shape[1] || iz < 0 || iz >= p.shape[2];
+            bad = !vox_cell_index(p.lo, p.size, p.shape, x, y, z, ix, iy, iz);
         }
         if (!bad) key = pack_key(ix, iy, iz);
     }

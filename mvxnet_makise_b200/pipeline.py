@@ -168,6 +168,8 @@ class PointPath:
             nbytes = fwd_b
             self._bws = torch.empty(bwd_b.value, dtype=torch.uint8, device=self.device)
         self._ws = torch.empty(nbytes.value, dtype=torch.uint8, device=self.device)
+        # the pixel GEMM keeps the zero state of Z's row tiles in the `tiles` region across calls: a new workspace starts unknown
+        self._ws[self.layout['tiles']:self.layout['Y8']].zero_()
         self._ws_key = key
         if own_outputs:
             self._alloc_outputs(B)
