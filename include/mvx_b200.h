@@ -266,7 +266,8 @@ int mvx_pointpath_forward(const mvx_pointpath_args_t *args);
  *               layout the training-mode backward uses).  Timing segments "gather"/"fcn1" then mean
  *               (pixel GEMMs, combine) in mode 1 and (gather, row GEMM) in mode 0.
  *   2           pixel-first like 1 but without running the map branch (channels-last copy + pixel GEMMs) on a side stream
- *               concurrently with the point branch (voxelization, row build, row sort) - for per-stage profiling. */
+ *               concurrently with the point branch (voxelization, row build, row sort) - for per-stage profiling.
+ * Any other value is rejected with MVX_EINVAL (mvx_last_error() names the accepted values). */
 int mvx_set_fusion_mode(int32_t mode);
 /* Pixel-first inference only. 0: the run-structured combine kernel (default);
  * 2: the first version of the combine kernel (row-by-row walk; kept for A/B measurements). Any other value is rejected with

@@ -529,11 +529,8 @@ __global__ void __launch_bounds__(256) dw_pad_row_kernel(DwArgs a) {
 template <int MH, int TK>
 int launch_dw_tc(const DwArgs &a_in, int B, cudaStream_t st) {
     using S = DwSmem<MH, TK>;
-    static bool attr_set = false;
-    if (!attr_set) {
-        MVX_CUDA_CHECK(cudaFuncSetAttribute(dw_tc_kernel<MH, TK>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
-        attr_set = true;
-    }
+    const int rc = set_smem_attributes<dw_tc_kernel<MH, TK>>(S::kTotal);
+    if (rc) return rc;
     DwArgs a = a_in;
     const int tiles = (a.Cout / (MH * 128)) * (a.Cin / TK);
     const long long per = (long long)tiles * B;
@@ -548,10 +545,8 @@ int launch_dw_tc(const DwArgs &a_in, int B, cudaStream_t st) {
     return MVX_OK;
 }
 
-static int g_dw_tc = 1;   // 1: tensor-core dW where eligible, 0: SIMT everywhere (mvx_set_gemm_mode(0) also selects SIMT)
-
 int launch_dw_auto(const DwArgs &a, int B, cudaStream_t st) {
-    if (g_dw_tc && gemm_mode() == 1 && a.dmax && a.Cout % 128 == 0 && a.Cin % 128 == 0) {
+    if (a.dmax && dw_uses_tc(a.Cout, a.Cin)) {
         if (a.Cout % 256 == 0 && a.Cin % 256 == 0) return launch_dw_tc<2, 256>(a, B, st);
         if (a.Cin % 256 == 0) return launch_dw_tc<1, 256>(a, B, st);
         return launch_dw_tc<1, 128>(a, B, st);
@@ -566,6 +561,8 @@ int launch_dw_auto(const DwArgs &a, int B, cudaStream_t st) {
 }
 
 }  // namespace
+
+bool dw_uses_tc(int Cout, int Cin) { return !simt_only() && Cout % 128 == 0 && Cin % 128 == 0; }
 
 int launch_dw_voxel_rows(const float *D, int Cout, const float *X, int Cin, const int *counts, int rowcap, const int *dmax, float *dW, int B,
                          cudaStream_t st, const int *xmax) {

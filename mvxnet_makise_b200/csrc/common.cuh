@@ -38,7 +38,35 @@ void count_launch(int n = 1);
         }                                                                                            \
     } while (0)
 
+// Kernel selection by the mode switches of the C ABI (defined in runtime.cu, where the modes are described)
+bool simt_only();               // gemm mode 0: the exact-fp32 SIMT kernels everywhere
+bool dense_f16();               // gemm mode 5: the dense layer API uses fp16 operands
+bool tc3_enabled();             // gemm mode 1, 6, 10 or 12: conv1 / fcn2 / last FCN on the TMA-fed kernel (tc3_layer.cu)
+bool bf16_mode();               // gemm mode 6
+bool pixel_gemm_persistent();   // gemm mode other than 12: the persistent pixel GEMM
+bool vfe_fused();               // gemm mode other than 10: inference builds the VFE inputs in the layer's loader
+bool combine_v1();              // fold mode 2: the first (row-by-row) combine kernel
+bool pixel_first(bool train);   // a forward runs fcn1 pixel-first: not training, fusion mode other than 0, gemm mode other than 0
+bool map_on_side_stream();      // fusion mode other than 2: the map branch of a pixel-first forward runs on a side stream
+
 constexpr int kSMs = 148;  // B200
+constexpr int kMaxDevices = 64;
+
+// Raises kernel K's dynamic shared-memory limit to `bytes` (and sets its shared-memory carveout when carveout >= 0) on the current
+// device, once per device: function attributes belong to a device's context, so every device a process launches K on needs its own
+// call.
+template <auto K>
+int set_smem_attributes(int bytes, int carveout = -1) {
+    static bool done[kMaxDevices] = {};
+    int dev = 0;
+    MVX_CUDA_CHECK(cudaGetDevice(&dev));
+    MVX_REQUIRE(dev >= 0 && dev < kMaxDevices, MVX_EINVAL, "device ordinal out of range");
+    if (done[dev]) return MVX_OK;
+    MVX_CUDA_CHECK(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    if (carveout >= 0) MVX_CUDA_CHECK(cudaFuncSetAttribute(K, cudaFuncAttributePreferredSharedMemoryCarveout, carveout));
+    done[dev] = true;
+    return MVX_OK;
+}
 
 static inline int64_t round_up(int64_t a, int64_t b) { return (a + b - 1) / b * b; }
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }

@@ -876,17 +876,11 @@ int launch_combine_sort(const CombineArgs &a, int B, cudaStream_t st) {
     return MVX_OK;
 }
 
-static int g_comb_v1 = 0;     // 1: the first combine kernel (row-by-row walk) instead of the run-structured one - kept for A/B runs
-void set_combine_v1(int on) { g_comb_v1 = on; }
-
 template <bool ZB, bool YB>
 static int launch_combine_runs_t(const CombineArgs &a, dim3 grid, cudaStream_t st) {
     using S = CombSmem<ZB>;
-    static bool attr_set = false;
-    if (!attr_set) {
-        MVX_CUDA_CHECK(cudaFuncSetAttribute(combine_runs_kernel<ZB, YB>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
-        attr_set = true;
-    }
+    const int rc = set_smem_attributes<combine_runs_kernel<ZB, YB>>(S::kTotal);
+    if (rc) return rc;
     combine_runs_kernel<ZB, YB><<<grid, kCombWarps * 32, S::kTotal, st>>>(a);
     MVX_LAUNCH_CHECK();
     return MVX_OK;
@@ -897,10 +891,10 @@ int launch_combine_rows(const CombineArgs &a, int B, cudaStream_t st) {
     MVX_REQUIRE(a.capA <= 0xFFFFFF, MVX_EINVAL, "combine: more than 2^24 rows per frame");
     if (a.z_bf16 || a.y1_bf16) {
         MVX_REQUIRE(a.z_bf16 && a.y1_bf16, MVX_EINVAL, "combine: the bf16 mode stores both Z and Y1 as bf16");
-        if (!g_comb_v1) return launch_combine_runs_t<true, true>(a, grid, st);
+        if (!combine_v1()) return launch_combine_runs_t<true, true>(a, grid, st);
         combine_rows_kernel<true, true><<<grid, kCombWarps * 32, 0, st>>>(a);
     } else {
-        if (!g_comb_v1) return launch_combine_runs_t<false, false>(a, grid, st);
+        if (!combine_v1()) return launch_combine_runs_t<false, false>(a, grid, st);
         combine_rows_kernel<><<<grid, kCombWarps * 32, 0, st>>>(a);
     }
     MVX_LAUNCH_CHECK();

@@ -157,7 +157,6 @@ struct CombineArgs {
 inline int combine_bins(int h0, int w0) { return ((h0 + 3) / 4) * ((w0 + 3) / 4) * 16; }
 int launch_combine_sort(const CombineArgs &a, int B, cudaStream_t st);   // counting sort of the rows (needs vox8 / proj only)
 int launch_combine_rows(const CombineArgs &a, int B, cudaStream_t st);   // the combine itself (needs Z and the sort)
-void set_combine_v1(int on);   // 1: the first (row-by-row) combine kernel instead of the run-structured one (A/B runs)
 
 // dense-voxel entry (dense_entry.cu): compact rows from the reference's (N,T,9) voxel tensor + (N,4) index list
 int dense_rows_run(const mvx_pointpath_args_t *a, int capA, long long G, int *vox_coord, int *vox_cnt, int *vox_row0, int *row_point,

@@ -527,10 +527,6 @@ int launch_layer(const LayerArgs &a, int F, cudaStream_t st) {
     return MVX_OK;
 }
 
-static int g_vfe_fused = 1;   // 0: prep_vfe1 / prep_vfe2 + plain layers also in inference (mvx_set_gemm_mode(10), A/B timing)
-bool vfe_fused_enabled() { return g_vfe_fused != 0; }
-void set_vfe_fused(int on) { g_vfe_fused = on; }
-
 int launch_vfe1_fused(const LayerArgs &a, const RowFuseArgs &z, int F, cudaStream_t st) {
     MVX_REQUIRE(a.Cin == 32 && a.Cout == 16 && a.rows_mode == 1 && a.counts && z.vox8 && z.Y && z.in_stats, MVX_EINVAL, "vfe1 fused: bad arguments");
     const unsigned tiles = (unsigned)ceil_div(ceil_div((long long)a.rowcap, kBM), kTilesPerCta);
@@ -547,13 +543,8 @@ int launch_vfe2_fused(const LayerArgs &a, const RowFuseArgs &z, int F, cudaStrea
     return MVX_OK;
 }
 
-static int g_gemm_mode = 1;
-int gemm_mode() { return g_gemm_mode; }
-
-static int g_dense_f16 = 0;
-
 int launch_layer_auto(const LayerArgs &a, int F, float *wpack, cudaStream_t st) {
-    if (g_gemm_mode == 1 && wpack) {
+    if (!simt_only() && wpack) {
         if (tc_layer_eligible(a)) return launch_layer_tc(a, F, wpack, st);
     }
     return launch_layer(a, F, st);
@@ -594,34 +585,11 @@ static int dense_layer(const float *x, int64_t R, int32_t T, int32_t Cin, const 
     a.X = x, a.ldx = Cin, a.Cin = Cin, a.Wt = wt, a.bias = bias, a.Cout = Cout, a.Y = y, a.ldy = ldy;
     a.out_stats = stats, a.vmax = vmax, a.rows_mode = 0, a.rows_fixed = R, a.rowcap = 0, a.vcap = 0, a.T = T > 0 ? T : 1;
     a.eps = eps;
-    a.f16_ok = g_dense_f16;   // arbitrary caller data: 3xTF32 unless mode 5 promises O(1) inputs
+    a.f16_ok = dense_f16();   // arbitrary caller data: 3xTF32 unless mode 5 promises O(1) inputs
     return launch_layer_auto(a, 1, wpack, st);
 }
 
 }  // namespace mvx
-
-// 0 = the exact-fp32 SIMT kernel everywhere
-// 1 = tensor cores where eligible (default): 3xFP16 for the fused path's BatchNorm-ed layers, 3xTF32 for the dense layer API;
-//     conv1 / fcn2 / last FCN through the TMA-fed A-from-TMEM persistent kernel (tc3_layer.cu)
-// 5 = like 1 with tc_layer.cu's one-tile kernel for those layers, and the dense layer API (mvx_fcn_forward ...) also uses fp16
-//     operands: the caller promises inputs of O(1) magnitude (tests)
-// 6 = bf16 mode: single-pass bf16 operands for the same layers mode 1 runs in 3xFP16
-// 9 = like 1 with the one-tile kernel of tc_layer.cu for conv1 / fcn2 / last FCN
-// 10 = like 1 with prep_vfe1 / prep_vfe2 materialising the VFE inputs also in inference (the earlier default, kept for A/B timing and
-//      for inspecting X6 / X7)
-// 12 = like 1 with the one-tile two-CTAs-per-SM kernel (tc_layer.cu) for the pixel GEMM instead of the persistent one (A/B timing)
-// 2, 3, 4, 7, 8 and 11 selected variants that have been removed (DESIGN.md §5) and are rejected; the modes above keep their numbers.
-extern "C" int mvx_set_gemm_mode(int32_t mode) {
-    constexpr unsigned kModes = 1u << 0 | 1u << 1 | 1u << 5 | 1u << 6 | 1u << 9 | 1u << 10 | 1u << 12;
-    MVX_REQUIRE(mode >= 0 && mode <= 12 && (kModes >> mode & 1u), MVX_EINVAL, "gemm mode must be 0, 1, 5, 6, 9, 10 or 12");
-    mvx::set_tc_bf16(mode == 6);
-    mvx::g_dense_f16 = mode == 5;
-    mvx::g_gemm_mode = mode == 0 ? 0 : 1;
-    mvx::set_tc3(mode == 1 || mode == 6 || mode == 10 || mode == 12);
-    mvx::set_pixel_persistent(mode != 12);
-    mvx::set_vfe_fused(mode != 10);
-    return MVX_OK;
-}
 
 extern "C" int mvx_layer_workspace_bytes(int32_t Cin, int32_t Cout, size_t *bytes) {
     if (!bytes || Cin <= 0 || Cout <= 0) return MVX_EINVAL;

@@ -77,8 +77,6 @@ struct RowFuseArgs {
 };
 int launch_vfe1_fused(const LayerArgs &a, const RowFuseArgs &z, int F, cudaStream_t st);   // a.X unused: input = [vox7 | norm5(Y5) | 0]
 int launch_vfe2_fused(const LayerArgs &a, const RowFuseArgs &z, int F, cudaStream_t st);   // a.X unused: input = [norm6(Y6) | norm6(max6[v])]; writes rowB_w / rowB_v
-bool vfe_fused_enabled();
-void set_vfe_fused(int on);
 
 // tensor-core (tcgen05, 3xTF32) implementation of the same layer; wpack = tc_wpack_bytes() of scratch
 bool tc_layer_eligible(const LayerArgs &a);
@@ -104,13 +102,7 @@ struct PixelGemmArgs {
 int launch_pixel_gemm_levels(const PixelGemmArgs &a, float *wpack, cudaStream_t st);
 // mvx_set_gemm_mode(12): the one-tile kernel per level over the level's active tiles, then the zeros of the inactive tiles
 int launch_pixel_gemm_one_tile(const PixelGemmArgs &a, float *wpack, cudaStream_t st);
-void set_pixel_persistent(int on);
-bool pixel_persistent_enabled();
-void set_tc3(int on);
-bool tc_bf16_enabled();
-void set_tc_bf16(int on);  // 1: single-pass bf16 operands where LayerArgs::f16_ok (reduced precision, tolerance stated in the tests)
-// dispatch by mvx_set_gemm_mode(): 0 = SIMT everywhere, 1 = tensor cores where eligible (default)
-int gemm_mode();
+// dispatch by mvx_set_gemm_mode(): the SIMT kernel in gemm mode 0, tensor cores where eligible otherwise
 int launch_layer_auto(const LayerArgs &a, int F, float *wpack, cudaStream_t st);
 
 // dW (Cout, Cin) += sum over the frames and their N_f voxel rows r of D[f][r]^T X[f][r] (backward.cu): rows of weight 1, X used
@@ -119,6 +111,8 @@ int launch_layer_auto(const LayerArgs &a, int F, float *wpack, cudaStream_t st);
 // (scale 1)
 int launch_dw_voxel_rows(const float *D, int Cout, const float *X, int Cin, const int *counts, int rowcap, const int *dmax, float *dW, int B,
                          cudaStream_t st, const int *xmax = nullptr);
+// true when launch_dw_voxel_rows (given dmax) runs a (Cout, Cin) dW on the tensor-core kernel, the only dW kernel that reads xmax
+bool dw_uses_tc(int Cout, int Cin);
 // batch-statistic BatchNorm + ReLU backward of ONE frame of N_f = counts[0] rows of multiplicity row_w (backward.cu, T = 1): G (rowcap,
 // C) holds dz on entry and dpre on exit; dbias (C) += column sums of dpre (fp32 atomics); bstats (C, 2) must be zeroed; dmax (C) as in
 // launch_dw_voxel_rows (zeroed by the caller) or NULL. C: 768 or a multiple of 4 up to 512 with C / 4 dividing 256.

@@ -150,7 +150,7 @@ int layer_backward(LayerKind kind, const float *x, long long R, int T, int Cin, 
     rc = launch_bn_back_voxel_rows(G, y_raw, Cout, static_cast<const double *>(stats_ws), bstats, db, eps, counts, Ri, ones, dmax, st);
     if (rc) return rc;
     // dW = dpre^T x: the tensor-core kernel scales the raw x per column
-    const bool tc_dw = gemm_mode() == 1 && Cout % 128 == 0 && Cin % 128 == 0;
+    const bool tc_dw = dw_uses_tc(Cout, Cin);
     if (tc_dw) {
         col_absmax_kernel<<<(unsigned)ceil_div(R, kColRows), 256, 0, st>>>(x, Ri, Cin, xmax);
         MVX_LAUNCH_CHECK();

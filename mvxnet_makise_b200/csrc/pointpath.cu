@@ -21,13 +21,6 @@ const char *kRegionNames[R_COUNT] = {
     "vox8", "proj", "rowA_w", "A1", "Y1", "Y2", "Y3", "Y4", "Y5", "X6", "Y6", "X7", "Y7", "rowB_w", "rowB_v", "X8",
     "vfeat", "stats", "vmax6", "vmax7", "vmax8", "wpack", "occ", "vfeat_t", "Z", "bin_count", "bin_start", "perm", "rowmax", "chmax", "A1max", "tiles", "Y8"};
 
-// 1 (default): pixel-first fcn1 - one tensor-core GEMM per FPN level over the map pixels, then a 12-corner combine per
-// point row (gather.cuh CombineArgs); 0: materialise the gathered (K,768) matrix A1 and run fcn1 over the point rows
-// (the layout the training-mode backward needs: dW1 = dpre1^T A1).
-static int g_fusion_mode = 1;
-int fusion_mode() { return g_fusion_mode; }
-static int g_overlap = 1;   // 1: run the map branch of the pixel-first path on a side stream (mvx_set_fusion_mode(2) = pixel-first, serial)
-
 int make_layout(const mvx_pointpath_args_t *a, Layout &L) {
     MVX_REQUIRE(a, MVX_EINVAL, "null args");
     MVX_REQUIRE(a->B >= 1 && a->B <= kMaxFrames, MVX_EINVAL, "B must be in [1,32]");
@@ -151,10 +144,10 @@ struct SideStream {
     int device = -1;
 };
 static int side_stream(SideStream **out) {
-    static SideStream per_device[64];
+    static SideStream per_device[kMaxDevices];
     int dev = 0;
     MVX_CUDA_CHECK(cudaGetDevice(&dev));
-    MVX_REQUIRE(dev >= 0 && dev < 64, MVX_EINVAL, "device ordinal out of range");
+    MVX_REQUIRE(dev >= 0 && dev < kMaxDevices, MVX_EINVAL, "device ordinal out of range");
     SideStream &s = per_device[dev];
     if (!s.stream) {
         MVX_CUDA_CHECK(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
@@ -204,7 +197,7 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     const Stamp stamp(st);
     if (train) MVX_CUDA_CHECK(cudaMemsetAsync(I32(R_CHMAX), 0, (size_t)B * 768 * 4, st));
     // training keeps the gathered matrix A1 (dW1 = dpre1^T A1), so it always runs row-first
-    const bool pixel_first = !train && g_fusion_mode == 1 && gemm_mode() == 1;
+    const bool pixel_first = mvx::pixel_first(train);
     double *stats = reinterpret_cast<double *>(ws + L.off[R_STATS]);
     auto stat_of = [&](int layer) { return stats + (size_t)layer * B * kStatStride; };
     // NOTE: stats are stored [F][Cout][2] with the layer's own Cout as the frame stride
@@ -214,21 +207,16 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     // under it; joined before the first kernel that needs both
     cudaStream_t ms = st;
     SideStream *side = nullptr;
-    if (pixel_first && g_overlap) {
+    if (pixel_first && map_on_side_stream()) {
         rc = side_stream(&side);
         if (rc) return rc;
         ms = side->stream;
         MVX_CUDA_CHECK(cudaEventRecord(side->fork, st));
         MVX_CUDA_CHECK(cudaStreamWaitEvent(ms, side->fork, 0));
     }
-    // pixel-first with 3xFP16: the maps are written directly as the pre-packed A operand of the pixel GEMM (no NHWC copy)
-    // bf16 mode too: its per-pixel GEMM keeps the 3xFP16 products of the pre-packed operands (the persistent kernel is bound by its
-    // loads and stores, not by the MMAs) and only writes Z as bf16; without the persistent kernel (gemm mode 12) the bf16 mode keeps its
-    // channels-last copy + one-product kernel
-    const bool apack = pixel_first && (!tc_bf16_enabled() || pixel_persistent_enabled());
     // bf16 mode (mvx_set_gemm_mode(6)): the two largest intermediates - the per-pixel products Z and the raw fcn1 rows Y1 - are
     // stored as bf16 (half the bytes written and read back); every sum in between stays fp32
-    const bool bf16_mem = pixel_first && tc_bf16_enabled();
+    const bool bf16_mem = pixel_first && bf16_mode();
     auto z_at = [&](size_t elem_off) -> float * {   // element offset into Z, whatever its element size
         return bf16_mem ? reinterpret_cast<float *>(reinterpret_cast<uint16_t *>(ws + L.off[R_Z]) + elem_off) : F32(R_Z) + elem_off;
     };
@@ -260,15 +248,12 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
         size_t rowmax_off = 0;
         for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
             const int HW = a->map_h[l] * a->map_w[l];
-            if (apack) {
-                int r = launch_pack_maps_f16(a->maps[l], ws + L.off[R_NHWC0 + l], F32(R_ROWMAX) + rowmax_off, B, a->map_c, HW,
-                                             dense_in ? nullptr : pt.bits + pt.word0[l], ms);
-                if (r) return r;
-                rowmax_off += (size_t)B * HW;
-                continue;
-            }
-            int r = launch_nchw_to_nhwc(a->maps[l], F32((Region)(R_NHWC0 + l)), B, a->map_c, HW, F32(R_ROWMAX) + rowmax_off,
-                                        train ? I32(R_CHMAX) + l * a->map_c : nullptr, MVX_NUM_LEVELS * a->map_c, ms);
+            // pixel-first: the maps are written directly as the pre-packed 3xFP16 A operand of the pixel GEMM (no NHWC copy), in the
+            // bf16 mode too (the persistent kernel is bound by its loads and stores, not by the MMAs; only Z is written as bf16)
+            const int r = pixel_first ? launch_pack_maps_f16(a->maps[l], ws + L.off[R_NHWC0 + l], F32(R_ROWMAX) + rowmax_off, B, a->map_c, HW,
+                                                             dense_in ? nullptr : pt.bits + pt.word0[l], ms)
+                                      : launch_nchw_to_nhwc(a->maps[l], F32((Region)(R_NHWC0 + l)), B, a->map_c, HW, F32(R_ROWMAX) + rowmax_off,
+                                                            train ? I32(R_CHMAX) + l * a->map_c : nullptr, MVX_NUM_LEVELS * a->map_c, ms);
             if (r) return r;
             rowmax_off += (size_t)B * HW;
         }
@@ -277,7 +262,6 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
         // Z_l = F_l W1[:, 256 l : 256 (l+1)]^T for the active pixel tiles of every level, zeros elsewhere (plain GEMM: no bias /
         // ReLU / statistics)
         stamp.begin(S_GATHER, ms);
-        MVX_REQUIRE(apack, MVX_EINVAL, "pixel-first fcn1 needs the pre-packed maps");
         PixelGemmArgs pg{};
         size_t zoff = 0;
         for (int l = 0; l < MVX_NUM_LEVELS; ++l) {
@@ -288,7 +272,7 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
         }
         pg.Wt = a->wt[0], pg.Cin = a->map_c, pg.Cout = 768, pg.z_bf16 = bf16_mem;
         pg.list = pt.list, pg.meta = pt.meta, pg.n_entries = pt.tile0[MVX_NUM_LEVELS];
-        int r = pixel_persistent_enabled() ? launch_pixel_gemm_levels(pg, F32(R_WPACK), ms) : launch_pixel_gemm_one_tile(pg, F32(R_WPACK), ms);
+        int r = pixel_gemm_persistent() ? launch_pixel_gemm_levels(pg, F32(R_WPACK), ms) : launch_pixel_gemm_one_tile(pg, F32(R_WPACK), ms);
         if (r) return r;
         stamp.end(S_GATHER, ms);
         return MVX_OK;
@@ -393,7 +377,7 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
 
     // inference: VFE1 / VFE2 build their input rows on the fly (fused loaders of the SIMT kernel) instead of reading the X6 / X7 matrices that
     // prep_vfe1 / prep_vfe2 materialise; training keeps X6 / X7 (dW = dpre^T X)
-    const bool fuse_vfe = !train && vfe_fused_enabled();
+    const bool fuse_vfe = !train && vfe_fused();
     stamp.mark(S_PREP1);
     if (!fuse_vfe) {
         rc = launch_prep_vfe1(vp, st);
@@ -440,7 +424,7 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
     stamp.mark(S_PREP3);
     // inference: the concat [norm7(Y7) | norm7(max7)] that prep_fcn materialises as X8 is built by the FCN's own
     // A-producer instead (16-bit tensor-core kernel); training keeps X8 (dW8 = dpre8^T X8)
-    const bool fuse_cat = !train && gemm_mode() == 1;
+    const bool fuse_cat = !train && !simt_only();
     if (!fuse_cat) {
         rc = launch_prep_fcn(vp, st);
         if (rc) return rc;
@@ -513,7 +497,7 @@ extern "C" int mvx_timing_read(int32_t call, float *ms) {
 
 extern "C" const char *mvx_timing_segment_name(int32_t segment) {
     if (segment < 0 || segment >= mvx::S_COUNT) return nullptr;
-    if (mvx::g_fusion_mode == 1 && mvx::gemm_mode() == 1) {  // pixel-first fcn1: the two segments change meaning
+    if (mvx::pixel_first(false)) {  // the timing leg times inference; pixel-first fcn1: the two segments change meaning
         if (segment == mvx::S_GATHER) return "pixel_gemm";
         if (segment == mvx::S_FCN1) return "fcn1_combine";
     }
@@ -543,17 +527,3 @@ extern "C" const char *mvx_pointpath_layout_name(int32_t region) {
 }
 
 extern "C" int mvx_pointpath_forward(const mvx_pointpath_args_t *args) { return mvx::pointpath_forward(args, false); }
-
-extern "C" int mvx_set_fold_mode(int32_t mode) {
-    // 1 (conv1 with fcn1's BatchNorm folded into per-frame weights) was removed: measured slower
-    MVX_REQUIRE(mode == 0 || mode == 2, MVX_EINVAL, "fold mode must be 0 or 2");
-    mvx::set_combine_v1(mode == 2);
-    return MVX_OK;
-}
-
-extern "C" int mvx_set_fusion_mode(int32_t mode) {
-    if (mode < 0 || mode > 2) return MVX_EINVAL;   // 2 = pixel-first without the side stream (serial, for per-stage profiling)
-    mvx::g_fusion_mode = mode == 0 ? 0 : 1;
-    mvx::g_overlap = mode != 2;
-    return MVX_OK;
-}

@@ -18,8 +18,6 @@ constexpr int kCin[MVX_NUM_LAYERS] = {768, 768, 128, 128, 16, 32, 32, 128};   //
 constexpr int kCout[MVX_NUM_LAYERS] = {768, 128, 128, 16, 16, 16, 64, 128};
 constexpr int kStatStride = 768 * 2;  // doubles per (layer, frame)
 
-int fusion_mode();
-
 struct Layout {
     size_t off[R_COUNT];
     size_t total;        // inference workspace (everything but Y8)

@@ -848,11 +848,8 @@ static int make_tmap(CUtensorMap *m, const void *base, long long rows, int cols,
 template <bool RESIDENT, bool CAT, int PREC>
 int launch_tc3_t(const T3Args &g, const CUtensorMap &tmX, const CUtensorMap &tmY, const CUtensorMap &tmX2, int grid, cudaStream_t st) {
     using S = T3Smem<RESIDENT>;
-    static bool attr_set = false;
-    if (!attr_set) {
-        MVX_CUDA_CHECK(cudaFuncSetAttribute(tc3_layer_kernel<RESIDENT, CAT, PREC>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
-        attr_set = true;
-    }
+    const int rc = set_smem_attributes<tc3_layer_kernel<RESIDENT, CAT, PREC>>(S::kTotal);
+    if (rc) return rc;
     tc3_layer_kernel<RESIDENT, CAT, PREC><<<grid, t3_threads(RESIDENT ? 2 : 3, RESIDENT ? 2 : 1), S::kTotal, st>>>(g, tmX, tmY, tmX2);
     MVX_LAUNCH_CHECK();
     return MVX_OK;
@@ -875,7 +872,7 @@ int pack_weights_f16_128(const float *Wt, int Cin, int Cout, void *wpack, cudaSt
 
 int launch_layer_tc3(const LayerArgs &a, int F, float *wpack, cudaStream_t st) {
     MVX_REQUIRE(tc3_layer_eligible(a) && wpack, MVX_EINVAL, "layer not eligible for the TMA-fed tensor-core kernel");
-    const bool bf = tc_bf16_enabled();
+    const bool bf = bf16_mode();
     MVX_REQUIRE(bf || !a.x_bf16, MVX_EINVAL, "bf16 rows need the bf16 mode");
     int rc = pack_weights_f16_128(a.Wt, a.Cin, a.Cout, wpack, st, bf);
     if (rc) return rc;
@@ -910,11 +907,6 @@ int launch_layer_tc3(const LayerArgs &a, int F, float *wpack, cudaStream_t st) {
     return launch_tc3_t<false, false, 0>(g, tmX, tmY, tmX2, grid, st);
 }
 
-// defined in tc_layer.cu
-static int g_pixel_persistent = 1;   // 0: the one-tile two-CTAs-per-SM kernel of tc_layer.cu for the pixel GEMM (mvx_set_gemm_mode(12), A/B timing)
-void set_pixel_persistent(int on) { g_pixel_persistent = on; }
-bool pixel_persistent_enabled() { return g_pixel_persistent != 0; }
-
 // the weights of the three K blocks, one after the other in wpack (Cin x Cout fp16 hi/lo images, then Cout column scales)
 static size_t pixel_wpack_level_bytes(int Cin, int Cout) { return (size_t)round_up((int64_t)Cin * Cout * 4 + (int64_t)Cout * 4, 256); }
 int pack_weights_f16_128_levels(const float *Wt, int Cin, int Cout, int levels, void *wpack, size_t level_bytes, cudaStream_t st);
@@ -935,12 +927,9 @@ int launch_pixel_gemm_levels(const PixelGemmArgs &a, float *wpack, cudaStream_t 
         if (rc) return rc;
     }
     g.list = a.list, g.meta = a.meta, g.n_entries = a.n_entries, g.Cin = a.Cin, g.Cout = a.Cout;
-    static bool attr_set = false;
-    if (!attr_set) {
-        MVX_CUDA_CHECK(cudaFuncSetAttribute(pixel_gemm_persistent_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PgSmem::kTotal));
-        MVX_CUDA_CHECK(cudaFuncSetAttribute(pixel_gemm_persistent_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PgSmem::kTotal));
-        attr_set = true;
-    }
+    rc = a.z_bf16 ? set_smem_attributes<pixel_gemm_persistent_kernel<true>>(PgSmem::kTotal)
+                  : set_smem_attributes<pixel_gemm_persistent_kernel<false>>(PgSmem::kTotal);
+    if (rc) return rc;
     const long long tiles = (long long)a.n_entries * (a.Cout / PG_BN);   // MMA + zero tiles: the active count is on the device
     const int grid = (int)(tiles < kSMs ? tiles : kSMs);
     if (a.z_bf16) pixel_gemm_persistent_kernel<true><<<grid, PG_THREADS, PgSmem::kTotal, st>>>(g, tm);

@@ -585,12 +585,8 @@ __global__ void __launch_bounds__(tc_producer_warps(F16, TWO) * 32 + 64, TWO ? 2
 template <int BN, bool F16, bool BF1 = false, bool TWO = false, bool APK = false>
 int launch_tc(const LayerArgs &a, int F, float *wpack, cudaStream_t st) {
     using S = Smem<BN, TWO ? 2 : kStages, TWO>;
-    static bool attr_set = false;
-    if (!attr_set) {
-        MVX_CUDA_CHECK(cudaFuncSetAttribute(tc_layer_kernel<BN, F16, BF1, TWO, APK>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
-        if (TWO) MVX_CUDA_CHECK(cudaFuncSetAttribute(tc_layer_kernel<BN, F16, BF1, TWO, APK>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        attr_set = true;
-    }
+    const int rc = set_smem_attributes<tc_layer_kernel<BN, F16, BF1, TWO, APK>>(S::kTotal, TWO ? 100 : -1);
+    if (rc) return rc;
     const int total = a.Cin * a.Cout;
     if (F16) {   // [fp16 hi|lo images: Cin*Cout*4 bytes][inverse column scales: Cout floats]
         uint8_t *blob = reinterpret_cast<uint8_t *>(wpack);
@@ -626,13 +622,6 @@ int pack_weights_f16_128_levels(const float *Wt, int Cin, int Cout, int levels, 
     return MVX_OK;
 }
 
-static int g_tc3 = 1;           // conv1 / fcn2 / last FCN through the TMA-fed, A-from-TMEM persistent kernel (tc3_layer.cu): default since r4
-                                // (conv1 0.79 -> 0.68 ms, fcn2 0.32 -> 0.21, FCN 0.47 -> 0.39); mvx_set_gemm_mode(9) = mode 1 with the one-tile kernel
-void set_tc3(int on) { g_tc3 = on; }
-static int g_tc_bf16 = 0;
-void set_tc_bf16(int on) { g_tc_bf16 = on; }
-bool tc_bf16_enabled() { return g_tc_bf16 != 0; }
-
 bool tc_layer_eligible(const LayerArgs &a) {
     // the 768 bound sizes the shared BatchNorm tables of the input: a plain product without them may be deeper
     return a.Cin % kBK == 0 && (a.Cin <= 768 || (a.plain && !a.in_stats)) && a.Cout % 128 == 0 && a.ldx % 4 == 0 &&
@@ -656,8 +645,8 @@ int launch_layer_tc(const LayerArgs &a_in, int F, float *wpack, cudaStream_t st)
     }
     MVX_REQUIRE(!a.X2 || (a.f16_ok && a.Cin % 32 == 0 && a.x2_cols % 32 == 0 && a.counts), MVX_EINVAL,
                 "fused concat input needs the 16-bit tensor-core producer");
-    if (g_tc3 && g_tc_bf16 && tc3_layer_eligible(a)) return launch_layer_tc3(a, F, wpack, st);   // bf16 mode of the TMA-fed kernel
-    if (a.f16_ok && g_tc_bf16 && a.Cin % 32 == 0) {          // reduced precision: one bf16 product per K-step
+    if (bf16_mode() && tc3_layer_eligible(a)) return launch_layer_tc3(a, F, wpack, st);   // bf16 mode of the TMA-fed kernel
+    if (a.f16_ok && bf16_mode() && a.Cin % 32 == 0) {   // reduced precision: one bf16 product per K-step
         if (a.Cout % 256 == 0) return launch_tc<256, true, true>(a, F, wpack, st);
         return launch_tc<128, true, true>(a, F, wpack, st);
     }
@@ -669,7 +658,9 @@ int launch_layer_tc(const LayerArgs &a_in, int F, float *wpack, cudaStream_t st)
         // GEMM against 0.593 ms with one 256-column CTA per SM)
         return launch_tc<128, true, false, true, true>(a, F, wpack, st);
     }
-    if (g_tc3 && tc3_layer_eligible(a)) return launch_layer_tc3(a, F, wpack, st);
+    // conv1 / fcn2 / last FCN on the TMA-fed, A-from-TMEM persistent kernel (conv1 0.79 -> 0.68 ms, fcn2 0.32 -> 0.21, FCN 0.47 -> 0.39
+    // against the one-tile kernel, which gemm modes 5 and 9 keep)
+    if (tc3_enabled() && tc3_layer_eligible(a)) return launch_layer_tc3(a, F, wpack, st);
     if (a.f16_ok && a.Cin % 32 == 0) {   // 3xFP16: half the tensor cycles and operand bytes of 3xTF32
         if (a.Cout % 256 == 0) return launch_tc<256, true>(a, F, wpack, st);
         return launch_tc<128, true>(a, F, wpack, st);

@@ -75,9 +75,15 @@ def test_mode_switches_accept_only_the_modes_that_exist():
         assert _lib.lib.mvx_set_fold_mode(1) == einval
         assert b'fold mode must be' in _lib.lib.mvx_last_error()
         assert _lib.lib.mvx_set_fold_mode(2) == 0
+        for m in (-1, 3):
+            assert _lib.lib.mvx_set_fusion_mode(m) == einval, m
+            assert b'fusion mode must be' in _lib.lib.mvx_last_error()
+        for m in (0, 1, 2):
+            assert _lib.lib.mvx_set_fusion_mode(m) == 0, m
     finally:
         assert _lib.lib.mvx_set_gemm_mode(1) == 0
         assert _lib.lib.mvx_set_fold_mode(0) == 0
+        assert _lib.lib.mvx_set_fusion_mode(1) == 0
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason='CPU-only behaviour')

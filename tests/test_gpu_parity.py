@@ -405,6 +405,26 @@ def test_fused_path_matches_reference_golden(mvx, golden_dir, tag, fusion_mode):
     assert rel_err(gcpu, ref64['grid'][0]) < TOL
 
 
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs two visible devices')
+def test_fused_path_on_a_second_device_in_the_same_process(mvx, golden_dir):
+    """Kernel attributes such as the dynamic shared-memory limit of the tensor-core kernels belong to one device's context: after
+    a forward on cuda:0, a forward on cuda:1 in the same process must run and compute what cuda:0 computed."""
+    g = np.load(os.path.join(golden_dir, 'path_a.npz'))
+    maps = [torch.from_numpy(m) for m in small_maps(int(g['map_seed']))]
+    sd = synth.make_weights(int(g['weight_seed']))
+    calib = synth.kitti_calib()
+    out = []
+    for dev in ('cuda:0', 'cuda:1'):
+        with torch.cuda.device(dev):
+            path = mvx.P.PointPath(sd, G, device=dev)
+            _, counts = path([g['pcd4']], [calib], maps, want_grid=False)
+            vfeat, idx = path.voxel_features(0)
+            out.append((counts.cpu(), idx.cpu(), vfeat.cpu()))
+    assert torch.equal(out[0][0], out[1][0])
+    assert torch.equal(out[0][1], out[1][1])
+    assert rel_err(out[1][2], out[0][2]) < 1e-5      # run-to-run: fp64 atomics of the statistics are unordered
+
+
 def test_grid_fill_rewrites_every_cell(mvx):
     """The plane-sequential fill of the fused path writes every cell of the grid, zeros included: a second run into a
     NaN-filled grid gives the grid of the first run (voxels sharing a sector, sectors at frame / plane borders, an empty
