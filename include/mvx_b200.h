@@ -183,15 +183,28 @@ int mvx_fcn_max_backward(const float *x, int64_t R, int32_t T, int32_t Cin, cons
                          const void *stats_ws, double eps, const float *dy, float *dx, float *dW, float *db, int32_t accumulate,
                          void *ws, size_t ws_bytes, void *stream);
 
+/* Element types of a dense grid (the `*_typed` scatter entries, mvx_pointpath_args_t.grid_dtype). A 16-bit grid holds every fp32
+ * feature rounded once to nearest-even (what `grid_fp32.to(torch.float16 / torch.bfloat16)` gives); a 16-bit grid gradient is
+ * widened to fp32 exactly. Any other value is rejected with MVX_EINVAL (mvx_last_error() names the accepted values). */
+#define MVX_DTYPE_F32 0
+#define MVX_DTYPE_F16 1
+#define MVX_DTYPE_BF16 2
+
 /* ------------------------------------------------------------------------------------------------
  * Stage 4 — scatter into the dense middle-layer grid.  Replaces modules/voxelnet/VoxelNet.py:16-22
- * (`reindex`): out (1,C,nz,nx,ny) fp32 fully written (zeros + features) in ONE streaming pass.
+ * (`reindex`): out (1,C,nz,nx,ny) fully written (zeros + features) in ONE streaming pass, fp32 or, with the typed entry,
+ * out_dtype (MVX_DTYPE_*; `out` is then read as that element type).
  * idx (N,4) int64 [batch, ix, iy, iz] (train.py:119,126).  map_ws: (G + G/32 + 1) int32 of scratch, G = nz*nx*ny.
  * ------------------------------------------------------------------------------------------------ */
+int mvx_scatter_dense_typed(const float *feat, const int64_t *idx, int64_t N, int32_t C, int32_t nx, int32_t ny,
+                            int32_t nz, void *out, int32_t out_dtype, int32_t *map_ws, void *stream);
 int mvx_scatter_dense(const float *feat, const int64_t *idx, int64_t N, int32_t C, int32_t nx, int32_t ny,
-                      int32_t nz, float *out, int32_t *map_ws, void *stream);
+                      int32_t nz, float *out, int32_t *map_ws, void *stream);   /* = the typed entry with MVX_DTYPE_F32 */
 /* Backward of `reindex` for the values (torch's index_put_ backward): d_feat (N,C)[n][c] = d_grid (1,C,nz,nx,ny)[0][c][iz][ix][iy], a
- * gather, so voxels sharing a cell each receive that cell's gradient; rows whose cell lies outside the grid receive 0. */
+ * gather, so voxels sharing a cell each receive that cell's gradient; rows whose cell lies outside the grid receive 0.
+ * d_feat is fp32; d_grid has element type `dtype` (MVX_DTYPE_*) in the typed entry, fp32 in the other. */
+int mvx_scatter_dense_backward_typed(const void *d_grid, int32_t dtype, const int64_t *idx, int64_t N, int32_t C, int32_t nx,
+                                     int32_t ny, int32_t nz, float *d_feat, void *stream);
 int mvx_scatter_dense_backward(const float *d_grid, const int64_t *idx, int64_t N, int32_t C, int32_t nx, int32_t ny, int32_t nz,
                                float *d_feat, void *stream);
 
@@ -217,7 +230,8 @@ typedef struct {
     double bn_eps;             /* cfg.eps (Blocks.py:10) */
     const float *wt[MVX_NUM_LAYERS];   /* device W^T (Cin_pad, Cout) fp32; Cin_pad: 768,768,128,128,16,32,32,128 */
     const float *bias[MVX_NUM_LAYERS]; /* device (Cout) */
-    float *grid_out;           /* device (B, 128, nz, nx, ny) fp32, fully overwritten; may be NULL (skip stage 4) */
+    float *grid_out;           /* device (B, 128, nz, nx, ny), fully overwritten; may be NULL (skip stage 4). Elements of type
+                                  grid_dtype: with MVX_DTYPE_F16 / MVX_DTYPE_BF16 the pointer is reinterpreted as a 16-bit grid */
     int32_t *counts;           /* device [B][4]: N_f, K_f, #invalid points, max points per voxel */
     void *workspace;
     size_t workspace_bytes;
@@ -242,6 +256,10 @@ typedef struct {
     float *voxels_dense;
     const int64_t *voxel_idx;
     const int32_t *vox_off_host;
+    /* Element type of grid_out (forward, forward_train) and of d_grid (mvx_pointpath_backward): MVX_DTYPE_F32 (0, what a
+     * zero-initialised struct holds), MVX_DTYPE_F16 or MVX_DTYPE_BF16; any other value is rejected with MVX_EINVAL before any
+     * CUDA call. Nothing else of the path depends on it. */
+    int32_t grid_dtype;
 } mvx_pointpath_args_t;
 
 /* counts[f] = (N_f, K_f = slots of frame f with (x,y,z) != 0, 0, max real slots per voxel) for a dense voxel tensor: what a
@@ -282,7 +300,8 @@ int mvx_set_fold_mode(int32_t mode);
  *     gathered matrix A1) and also keeps the raw output of the last FCN; args->workspace must hold `forward_bytes`.
  *   mvx_pointpath_backward: call after forward_train with the SAME args (same workspace, weights, counts).
  *     Upstream gradient: exactly one of d_vfeat (B, cap, 128: dLoss/d voxel features, reference voxel order, rows
- *     >= N_f ignored) or d_grid (B,128,nz,nx,ny: dLoss/d dense grid; reindex's backward is an index select).
+ *     >= N_f ignored) or d_grid (B,128,nz,nx,ny: dLoss/d dense grid; reindex's backward is an index select), whose
+ *     elements are of type args->grid_dtype (the d_grid pointer is reinterpreted as a 16-bit grid for F16 / BF16).
  *     grad_flat: mvx_grad_floats() = 726 880 fp32, per layer [weight (Cout,Cin) | bias (Cout)] in checkpoint order
  *     (fcn1 conv1 fcn2 conv2 fcn3 vfe1 vfe2 fcn) - the one flat bucket the NCCL all-reduce sums; gradients of all B
  *     frames are summed into it (accumulate != 0: added to its current contents).

@@ -20,6 +20,7 @@ NUM_LAYERS = 8
 NUM_LEVELS = 3
 WS_REGIONS = 64
 NUM_SEGMENTS = 20
+DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2     # MVX_DTYPE_*: element types of a dense grid
 
 # every symbol include/mvx_b200.h declares (tests check that the .so exports all of them)
 EXPORTS = [
@@ -28,6 +29,7 @@ EXPORTS = [
     'mvx_crop_workspace_bytes', 'mvx_crop_points', 'mvx_crop_points_f64',
     'mvx_lidar2img', 'mvx_lidar2img_f64', 'mvx_dense_voxel_counts', 'mvx_maps_nhwc_bytes', 'mvx_feature_mapping',
     'mvx_set_gemm_mode', 'mvx_layer_workspace_bytes', 'mvx_fcn_forward', 'mvx_vfe_forward', 'mvx_fcn_max_forward', 'mvx_scatter_dense',
+    'mvx_scatter_dense_typed', 'mvx_scatter_dense_backward_typed',
     'mvx_feature_mapping_backward_workspace_bytes', 'mvx_feature_mapping_backward', 'mvx_fcn_forward_train', 'mvx_vfe_forward_train',
     'mvx_fcn_max_forward_train', 'mvx_fcn_backward_workspace_bytes', 'mvx_vfe_backward_workspace_bytes',
     'mvx_fcn_max_backward_workspace_bytes', 'mvx_fcn_backward', 'mvx_vfe_backward', 'mvx_fcn_max_backward', 'mvx_scatter_dense_backward',
@@ -57,7 +59,7 @@ class PointPathArgs(ctypes.Structure):
                 ('wt', c_void_p * NUM_LAYERS), ('bias', c_void_p * NUM_LAYERS), ('grid_out', c_void_p),
                 ('counts', c_void_p), ('workspace', c_void_p), ('workspace_bytes', c_size_t), ('stream', c_void_p),
                 ('point_calib', c_void_p), ('calib64', c_void_p), ('calib_f64', c_void_p),
-                ('voxels_dense', c_void_p), ('voxel_idx', c_void_p), ('vox_off_host', POINTER(c_int32))]
+                ('voxels_dense', c_void_p), ('voxel_idx', c_void_p), ('vox_off_host', POINTER(c_int32)), ('grid_dtype', c_int32)]
 
 
 def make_grid(velorange, voxelsize, voxelshape, T) -> Grid:
@@ -99,6 +101,7 @@ def _load():
     lib.mvx_vfe_forward.argtypes = [vp, i64, i32, i32, vp, vp, i32, c_double, vp, vp, vp, vp]
     lib.mvx_fcn_max_forward.argtypes = [vp, i64, i32, i32, vp, vp, i32, c_double, vp, vp, vp, vp]
     lib.mvx_scatter_dense.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp, vp, vp]
+    lib.mvx_scatter_dense_typed.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp, i32, vp, vp]
     lib.mvx_feature_mapping_backward_workspace_bytes.argtypes = [i64, POINTER(i32), POINTER(i32), POINTER(c_size_t)]
     lib.mvx_feature_mapping_backward.argtypes = [vp, i64, vp, POINTER(i32), POINTER(i32), i32, c_float, c_float, c_float, POINTER(vp),
                                                  vp, c_size_t, vp]
@@ -112,6 +115,7 @@ def _load():
     lib.mvx_vfe_backward.argtypes = [vp, i64, i32, i32, vp, i32, vp, vp, c_double, vp, vp, vp, vp, i32, vp, c_size_t, vp]
     lib.mvx_fcn_max_backward.argtypes = [vp, i64, i32, i32, vp, i32, vp, vp, c_double, vp, vp, vp, vp, i32, vp, c_size_t, vp]
     lib.mvx_scatter_dense_backward.argtypes = [vp, vp, i64, i32, i32, i32, i32, vp, vp]
+    lib.mvx_scatter_dense_backward_typed.argtypes = [vp, i32, vp, i64, i32, i32, i32, i32, vp, vp]
     lib.mvx_pointpath_workspace_bytes.argtypes = [POINTER(PointPathArgs), POINTER(c_size_t)]
     lib.mvx_pointpath_layout.argtypes = [POINTER(PointPathArgs), POINTER(i64)]
     lib.mvx_pointpath_layout_name.argtypes = [i32]
@@ -152,6 +156,15 @@ def check(rc: int, what: str = ''):
     if rc != 0:
         msg = lib.mvx_last_error().decode('utf-8', 'replace')
         raise RuntimeError(f'mvx_b200 {what} failed: {ERRORS.get(rc, rc)}: {msg}')
+
+
+def grid_dtype_code(dtype) -> int:
+    """MVX_DTYPE_* of a dense grid's torch dtype: torch.float32, torch.float16 or torch.bfloat16; ValueError otherwise."""
+    import torch
+    codes = {torch.float32: DTYPE_F32, torch.float16: DTYPE_F16, torch.bfloat16: DTYPE_BF16}
+    if not isinstance(dtype, torch.dtype) or dtype not in codes:
+        raise ValueError(f'grid dtype must be torch.float32, torch.float16 or torch.bfloat16, not {dtype!r}')
+    return codes[dtype]
 
 
 def require_cuda():

@@ -13,6 +13,7 @@
 // tools/compact_backward_proto.py validates these formulas against autograd through the dense oracle chain.
 #include "layers.cuh"
 #include "pointpath.cuh"
+#include "scatter.cuh"
 #include "tc_common.cuh"
 
 #include <algorithm>
@@ -670,14 +671,16 @@ __global__ void __launch_bounds__(256) slice_im16_kernel(const float *__restrict
     G5[((size_t)f * capA + r) * 16 + c] = dX6[((size_t)f * capA + r) * 32 + 7 + c];
 }
 
-// d vfeat[f][v][c] = d grid[f][c][cell(v)]   (backward of VoxelNet.reindex, VoxelNet.py:16-22: an index select)
-__global__ void __launch_bounds__(256) grid_grad_gather_kernel(const float *__restrict__ dgrid, const int *__restrict__ vox_coord,
+// d vfeat[f][v][c] = d grid[f][c][cell(v)]   (backward of VoxelNet.reindex, VoxelNet.py:16-22: an index select); a 16-bit
+// d grid widens to fp32 exactly
+template <typename T>
+__global__ void __launch_bounds__(256) grid_grad_gather_kernel(const T *__restrict__ dgrid, const int *__restrict__ vox_coord,
                                                                const int *counts, int cap, long long G, float *__restrict__ dv) {
     const int f = blockIdx.y, N = counts[f * 4 + 0];
     const int e = blockIdx.x * blockDim.x + threadIdx.x, v = e >> 7, c = e & 127;
     if (v >= N) return;
     const int cell = vox_coord[((size_t)f * cap + v) * 4 + 3];
-    dv[((size_t)f * cap + v) * 128 + c] = dgrid[((size_t)f * 128 + c) * G + cell];
+    dv[((size_t)f * cap + v) * 128 + c] = grid_f32(dgrid[((size_t)f * 128 + c) * G + cell]);
 }
 
 enum BRegion { BR_G1 = 0, BR_G2, BR_G3, BR_G4, BR_G5, BR_DX6, BR_G6, BR_DX7, BR_G7, BR_DX8, BR_G8, BR_BSTATS, BR_WT, BR_DVFEAT, BR_DMAX, BR_COUNT };
@@ -780,10 +783,15 @@ int pointpath_backward(const mvx_pointpath_args_t *a, const float *d_vfeat, cons
         transpose_w_kernel<<<(n + 255) / 256, 256, 0, st>>>(a->wt[l], wT + BL.wt_off[l], kCin[l], kCout[l]);
         MVX_LAUNCH_CHECK();
     }
-    if (d_grid) {
-        grid_grad_gather_kernel<<<dim3((unsigned)ceil_div((long long)cap * 128, 256), B), 256, 0, st>>>(d_grid, I32(R_VOX_COORD), a->counts, cap,
-                                                                                                         L.G, BF(BR_DVFEAT));
-        MVX_LAUNCH_CHECK();
+    if (d_grid) {   // d_grid holds elements of the forward's grid dtype
+        rc = with_grid_dtype(a->grid_dtype, [&](auto t) {
+            using T = decltype(t);
+            grid_grad_gather_kernel<T><<<dim3((unsigned)ceil_div((long long)cap * 128, 256), B), 256, 0, st>>>(
+                reinterpret_cast<const T *>(d_grid), I32(R_VOX_COORD), a->counts, cap, L.G, BF(BR_DVFEAT));
+            MVX_LAUNCH_CHECK();
+            return MVX_OK;
+        });
+        if (rc) return rc;
         d_vfeat = BF(BR_DVFEAT);
     }
     const RowSet rsA{a->counts, 1, L.capA, F32(R_ROWA_W), T}, rsB{a->counts, 2, L.capB, F32(R_ROWB_W), T};

@@ -76,6 +76,13 @@ __device__ __forceinline__ void st_cs_f4(float4 *p, float4 v) {
     asm volatile("st.global.cs.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
                  : "memory");
 }
+// the same for 16 and 8 bytes of packed 16-bit elements
+__device__ __forceinline__ void st_cs_u4(uint4 *p, uint4 v) {
+    asm volatile("st.global.cs.v4.b32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
+__device__ __forceinline__ void st_cs_u2(uint2 *p, uint2 v) {
+    asm volatile("st.global.cs.v2.b32 [%0], {%1, %2};" ::"l"(p), "r"(v.x), "r"(v.y) : "memory");
+}
 __device__ __forceinline__ float4 ld_nc_f4(const float4 *p) {
     float4 r;
     asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];"

@@ -13,6 +13,7 @@
 // (torch.max's argmax on the dense tensor); for VFE that half of dy is first summed over the T rows it was tiled onto.
 #include "layers.cuh"
 #include "pointpath.cuh"
+#include "scatter.cuh"
 
 namespace mvx {
 
@@ -64,8 +65,9 @@ __global__ void __launch_bounds__(256) col_absmax_kernel(const float *__restrict
 }
 
 // d_feat[n][c] = d_grid[0][c][iz][ix][iy] (the adjoint of reindex's index_put_ for the values: a gather, also with duplicate cells);
-// rows whose cell lies outside the grid (the forward skips them, the reference would raise) get 0
-__global__ void __launch_bounds__(256) scatter_back_kernel(const float *__restrict__ d_grid, const long long *__restrict__ idx, long long N,
+// rows whose cell lies outside the grid (the forward skips them, the reference would raise) get 0; a 16-bit d_grid widens exactly
+template <typename T>
+__global__ void __launch_bounds__(256) scatter_back_kernel(const T *__restrict__ d_grid, const long long *__restrict__ idx, long long N,
                                                            int C, int nx, int ny, int nz, float *__restrict__ d_feat) {
     const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= N * C) return;
@@ -74,7 +76,7 @@ __global__ void __launch_bounds__(256) scatter_back_kernel(const float *__restri
     const long long ix = idx[n * 4 + 1], iy = idx[n * 4 + 2], iz = idx[n * 4 + 3];
     float g = 0.f;
     if (ix >= 0 && ix < nx && iy >= 0 && iy < ny && iz >= 0 && iz < nz)
-        g = d_grid[(size_t)c * nx * ny * nz + ((size_t)iz * nx + ix) * ny + iy];   // grid is (nz, nx, ny) (VoxelNet.py:19-21)
+        g = grid_f32(d_grid[(size_t)c * nx * ny * nz + ((size_t)iz * nx + ix) * ny + iy]);   // grid is (nz, nx, ny) (VoxelNet.py:19-21)
     d_feat[e] = g;
 }
 
@@ -212,13 +214,22 @@ extern "C" int mvx_fcn_max_backward(const float *x, int64_t R, int32_t T, int32_
                                static_cast<cudaStream_t>(stream));
 }
 
-extern "C" int mvx_scatter_dense_backward(const float *d_grid, const int64_t *idx, int64_t N, int32_t C, int32_t nx, int32_t ny, int32_t nz,
-                                          float *d_feat, void *stream) {
+extern "C" int mvx_scatter_dense_backward_typed(const void *d_grid, int32_t dtype, const int64_t *idx, int64_t N, int32_t C, int32_t nx,
+                                                int32_t ny, int32_t nz, float *d_feat, void *stream) {
+    MVX_REQUIRE(mvx::grid_dtype_ok(dtype), MVX_EINVAL, MVX_GRID_DTYPE_MSG);
     MVX_REQUIRE(N >= 0 && C > 0 && nx > 0 && ny > 0 && nz > 0, MVX_EINVAL, "bad scatter backward argument");
     if (N == 0) return MVX_OK;
     MVX_REQUIRE(d_grid && idx && d_feat, MVX_EINVAL, "null d_grid / idx / d_feat");
-    mvx::scatter_back_kernel<<<(unsigned)mvx::ceil_div(N * C, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        d_grid, reinterpret_cast<const long long *>(idx), N, C, nx, ny, nz, d_feat);
-    MVX_LAUNCH_CHECK();
-    return MVX_OK;
+    return mvx::with_grid_dtype(dtype, [&](auto t) {
+        using T = decltype(t);
+        mvx::scatter_back_kernel<T><<<(unsigned)mvx::ceil_div(N * C, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+            static_cast<const T *>(d_grid), reinterpret_cast<const long long *>(idx), N, C, nx, ny, nz, d_feat);
+        MVX_LAUNCH_CHECK();
+        return MVX_OK;
+    });
+}
+
+extern "C" int mvx_scatter_dense_backward(const float *d_grid, const int64_t *idx, int64_t N, int32_t C, int32_t nx, int32_t ny, int32_t nz,
+                                          float *d_feat, void *stream) {
+    return mvx_scatter_dense_backward_typed(d_grid, MVX_DTYPE_F32, idx, N, C, nx, ny, nz, d_feat, stream);
 }

@@ -26,6 +26,7 @@ int make_layout(const mvx_pointpath_args_t *a, Layout &L) {
     MVX_REQUIRE(a->B >= 1 && a->B <= kMaxFrames, MVX_EINVAL, "B must be in [1,32]");
     MVX_REQUIRE(a->cap >= 128 && a->cap % 128 == 0, MVX_EINVAL, "cap must be a positive multiple of 128");
     MVX_REQUIRE(a->map_c == 256, MVX_EINVAL, "map_c must be 256 (3 x 256 = the 768 inputs of fcn1)");
+    MVX_REQUIRE(grid_dtype_ok(a->grid_dtype), MVX_EINVAL, MVX_GRID_DTYPE_MSG);   // element type of grid_out / d_grid
     const size_t B = a->B, cap = a->cap;
     L.capA = a->cap + 128;
     L.capB = 2 * a->cap;
@@ -456,9 +457,10 @@ int pointpath_forward(const mvx_pointpath_args_t *a, bool train) {
             unsigned *occ = reinterpret_cast<unsigned *>(ws + L.off[R_OCC]);
             rc = launch_occ_from_map(vo.cell2vid, occ, B, L.G, st);
             if (rc) return rc;
-            rc = launch_grid_fill_planes(occ, vo.cell2vid, F32(R_VFEAT_T), (long long)cap * 128, 1, cap, a->grid_out, B, L.G, 128, st);
+            rc = launch_grid_fill_planes(occ, vo.cell2vid, F32(R_VFEAT_T), (long long)cap * 128, 1, cap, a->grid_out, a->grid_dtype, B, L.G, 128,
+                                         st);
         } else {
-            rc = launch_grid_fill(vo.cell2vid, F32(R_VFEAT), a->grid_out, B, L.G, 128, cap, st);
+            rc = launch_grid_fill(vo.cell2vid, F32(R_VFEAT), a->grid_out, a->grid_dtype, B, L.G, 128, cap, st);
         }
         if (rc) return rc;
     }

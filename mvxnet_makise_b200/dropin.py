@@ -25,7 +25,7 @@ from typing import List, Sequence
 
 import torch
 
-from . import synth
+from . import _lib, synth
 from .modules import _records
 from .pipeline import PointPath
 
@@ -86,14 +86,14 @@ class HotPathFunction(torch.autograd.Function):
         maps = _path_inputs(path, params, (m0, m1, m2))
         nz, nx, ny = path.grid.shape[2], path.grid.shape[0], path.grid.shape[1]
         B = len(voxels) if isinstance(voxels, (list, tuple)) else 1
-        grid = torch.empty((B, 128, nz, nx, ny), dtype=torch.float32, device=path.device)   # a fresh tensor: the CML saves it for ITS backward
+        grid = torch.empty((B, 128, nz, nx, ny), dtype=path.grid_dtype, device=path.device)   # a fresh tensor: the CML saves it for ITS backward
         path.forward_voxels(voxels, idx, maps, want_grid=True, train=True, grid_out=grid)
         ctx.path, ctx.record = path, path._record
         ctx.map_dtypes = [m.dtype for m in (m0, m1, m2)]
         return grid
 
     @staticmethod
-    def backward(ctx, d_grid):
+    def backward(ctx, d_grid):          # in the grid's dtype, which the path backward reads as it is
         _check_record(ctx)
         grads, map_grads = _path_backward(ctx, ctx.needs_input_grad[3:6], ctx.needs_input_grad[6:], d_grid=d_grid.contiguous())
         return (None, None, None, *map_grads, *grads)
@@ -183,6 +183,10 @@ def _forward(self, voxels, imgs, idx, calibs, imsize):
                           self._mvx_conv1_eps)
         outs = [self.backbone.rpn(cml.conv3(cml.conv2(y1[b:b + 1])).reshape((1, -1, nx, ny))) for b in range(y1.shape[0])]
         return outs[0] if len(outs) == 1 else outs
+    gd = self._mvx_grid_dtype
+    if gd == 'autocast':                             # the dtype the CML's conv1 would cast the grid to at this call
+        gd = torch.get_autocast_dtype('cuda') if torch.is_autocast_enabled('cuda') else torch.float32
+    path.grid_dtype = gd
     grid = hot_path(path, voxels, idx.to(torch.int64), feats, hot_parameters(self))
     outs = []
     for b in range(grid.shape[0]):                   # CML / RPN are batch-1 in the reference (VoxelNet.py:35-37)
@@ -192,14 +196,24 @@ def _forward(self, voxels, imgs, idx, calibs, imsize):
 
 
 def accelerate(model, grid: synth.GridSpec = synth.KITTI_GRID, imsize_hw: Sequence[int] = synth.KITTI_IMSIZE_HW, eps: float = 1e-6,
-               sparse_cml_conv1: bool = False):
+               sparse_cml_conv1: bool = False, grid_dtype=torch.float32):
     """Swap the hot path of a reference `MVXNet` instance (already on its CUDA device) for the fused sm_100a path, in place.
     `grid` / `eps` mirror config.yml (velorange, voxelshape, samplenum; eps 1e-6 with half: False). Returns the model.
 
     sparse_cml_conv1=True also computes `backbone.cml.conv1` sparsely from the voxel features, forward and backward, so the
     dense (B,128,nz,nx,ny) grid is never written; conv2 / conv3 and the RPN remain the model's own modules. Opt-in because a
     caller can tell the difference: `backbone.cml` and `cml.conv1` are not called as modules (their hooks do not fire) and
-    no grid tensor exists. conv1 must be the stock block (ValueError otherwise)."""
+    no grid tensor exists. conv1 must be the stock block (ValueError otherwise).
+
+    grid_dtype: element type of the dense grid handed to `backbone.cml` - torch.float32 (default), torch.float16,
+    torch.bfloat16, or 'autocast': at each call, `torch.get_autocast_dtype('cuda')` when `torch.is_autocast_enabled('cuda')`,
+    fp32 otherwise (the reference's `half: True` loop: eps 1e-3, fp16 autocast, GradScaler). A 16-bit grid holds each fp32
+    feature rounded once to nearest-even, which is what the CML's fp16 conv1 would cast it to; its gradient comes back in the
+    same dtype. ValueError for any other value. The sparse conv1 route writes no grid and ignores it."""
+    if not (isinstance(grid_dtype, str) and grid_dtype == 'autocast'):
+        if isinstance(grid_dtype, str):
+            raise ValueError(f"grid_dtype must be torch.float32, torch.float16, torch.bfloat16 or 'autocast', not {grid_dtype!r}")
+        _lib.grid_dtype_code(grid_dtype)
     params = hot_parameters(model)                   # raises AttributeError if this is not the reference's module tree
     conv1_eps = _stock_conv1_eps(model.backbone.cml) if sparse_cml_conv1 else None
     dev = params[0].device
@@ -209,6 +223,7 @@ def accelerate(model, grid: synth.GridSpec = synth.KITTI_GRID, imsize_hw: Sequen
     model._mvx_path = PointPath(sd, grid, imsize_hw, eps, device=dev)
     model._mvx_imsize = {}
     model._mvx_sparse_conv1, model._mvx_conv1_eps = bool(sparse_cml_conv1), conv1_eps
+    model._mvx_grid_dtype = grid_dtype
     model.forward = types.MethodType(_forward, model)
     return model
 

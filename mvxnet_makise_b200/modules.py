@@ -329,44 +329,49 @@ class SVFE(nn.Module):
         return self.vfe2(self.vfe1(x))
 
 
-def _reindex_call(x: torch.Tensor, idx: torch.Tensor, voxelshape: Sequence[int]) -> torch.Tensor:
+def _reindex_call(x: torch.Tensor, idx: torch.Tensor, voxelshape: Sequence[int], dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    code = _lib.grid_dtype_code(dtype)
     _lib.require_cuda()
     nx, ny, nz = (int(s) for s in voxelshape)
     x = x.detach().to(torch.float32).contiguous()
     N, C = x.shape
-    out = torch.empty((1, C, nz, nx, ny), dtype=torch.float32, device=x.device)
+    out = torch.empty((1, C, nz, nx, ny), dtype=dtype, device=x.device)
     G = nx * ny * nz
     mapws = torch.empty(G + G // 32 + 1, dtype=torch.int32, device=x.device)
-    check(lib.mvx_scatter_dense(ptr(x), ptr(idx), N, C, nx, ny, nz, ptr(out), ptr(mapws), stream_ptr()), 'scatter_dense')
+    check(lib.mvx_scatter_dense_typed(ptr(x), ptr(idx), N, C, nx, ny, nz, ptr(out), code, ptr(mapws), stream_ptr()), 'scatter_dense_typed')
     return out
 
 
 class _ReindexFunction(torch.autograd.Function):
-    """reindex with x as input; backward = mvx_scatter_dense_backward (a gather of the grid gradient at every voxel's cell)."""
+    """reindex with x as input; backward = mvx_scatter_dense_backward_typed (a gather of the grid gradient at every voxel's cell,
+    read in the grid's own dtype)."""
 
     @staticmethod
-    def forward(ctx, x, idx, voxelshape):
+    def forward(ctx, x, idx, voxelshape, dtype):
         ctx.save_for_backward(idx)
         ctx.voxelshape, ctx.x_dtype = voxelshape, x.dtype
-        return _reindex_call(x, idx, voxelshape)
+        return _reindex_call(x, idx, voxelshape, dtype)
 
     @staticmethod
     def backward(ctx, d_grid):
         idx, = ctx.saved_tensors
         nx, ny, nz = (int(s) for s in ctx.voxelshape)
-        d_grid = d_grid.to(torch.float32).contiguous()
+        d_grid = d_grid.contiguous()
         N, C = idx.shape[0], d_grid.shape[1]
         dx = torch.empty((N, C), dtype=torch.float32, device=d_grid.device)
-        check(lib.mvx_scatter_dense_backward(ptr(d_grid), ptr(idx), N, C, nx, ny, nz, ptr(dx), stream_ptr()), 'scatter_dense_backward')
-        return dx.to(ctx.x_dtype), None, None
+        check(lib.mvx_scatter_dense_backward_typed(ptr(d_grid), _lib.grid_dtype_code(d_grid.dtype), ptr(idx), N, C, nx, ny, nz, ptr(dx),
+                                                   stream_ptr()), 'scatter_dense_backward_typed')
+        return dx.to(ctx.x_dtype), None, None, None
 
 
-def reindex(x: torch.Tensor, idx: torch.Tensor, voxelshape: Sequence[int] = VOXELSHAPE) -> torch.Tensor:
-    """Drop-in for ``VoxelNet.reindex`` (VoxelNet.py:16-22): (N,C) + idx (N,4) int64 -> (1,C,nz,nx,ny)."""
+def reindex(x: torch.Tensor, idx: torch.Tensor, voxelshape: Sequence[int] = VOXELSHAPE, dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    """Drop-in for ``VoxelNet.reindex`` (VoxelNet.py:16-22): (N,C) + idx (N,4) int64 -> (1,C,nz,nx,ny) of `dtype` (torch.float32,
+    torch.float16 or torch.bfloat16: the reference allocates its zeros in cfg.dtype, fp16 with `half: True`); a 16-bit grid
+    holds each fp32 value rounded once to nearest-even."""
     idx = idx.to(torch.int64).contiguous()
     if _records(x):
-        return _ReindexFunction.apply(x, idx, tuple(voxelshape))
-    return _reindex_call(x, idx, voxelshape)
+        return _ReindexFunction.apply(x, idx, tuple(voxelshape), dtype)
+    return _reindex_call(x, idx, voxelshape, dtype)
 
 
 class VoxelNetHead(nn.Module):

@@ -5,6 +5,9 @@ train.py:26-49 (projection + voxelization) moved onto the GPU.
     path = PointPath(state_dict)                      # reference parameter names (SURVEY.md §8b)
     grid, counts = path(points_list, calibs, fpn_maps)   # (B,128,nz,nx,ny) fp32 on the GPU, counts (B,4) int32
 
+`PointPath(..., grid_dtype=torch.float16)` (or bfloat16; also a settable attribute) writes the grid in that dtype instead:
+every element is the fp32 feature rounded once to nearest-even, what a half-precision CML would cast it to.
+
 Frames are independent (per-frame BatchNorm statistics, as in the batch-1 reference), so multi-GPU use is pure
 frame sharding: see ``mvxnet_makise_b200.dist``.
 """
@@ -27,8 +30,9 @@ class _Forward:
     """The record of one forward: everything a later call on its results (backward, cml_conv1, voxel_features, the drop-in's
     autograd nodes) reads. Every forward makes a new one, so a stale holder can tell by identity."""
 
-    def __init__(self, args=None, keep=(), maps=None, train=False, subs=None):
+    def __init__(self, args=None, keep=(), maps=None, train=False, subs=None, grid_dtype=torch.float32):
         self.args = args            # the PointPathArgs of the launch (workspace pointers, B, cap)
+        self.grid_dtype = grid_dtype   # dtype of the grid it wrote: backward(d_grid=...) takes exactly this one
         self.keep = keep            # host arrays and tensors the pointers in `args` refer to, kept alive with it
         self.maps = maps            # the fp32 FPN maps it read (the shapes of dLoss/d maps)
         self.train = train          # forward_train: the workspace holds the activations backward() needs
@@ -69,7 +73,9 @@ class HostStep:
 
 class PointPath:
     def __init__(self, state_dict: Dict[str, torch.Tensor], grid: synth.GridSpec = synth.KITTI_GRID,
-                 imsize_hw: Sequence[int] = synth.KITTI_IMSIZE_HW, eps: float = 1e-6, device='cuda'):
+                 imsize_hw: Sequence[int] = synth.KITTI_IMSIZE_HW, eps: float = 1e-6, device='cuda',
+                 grid_dtype: torch.dtype = torch.float32):
+        _lib.grid_dtype_code(grid_dtype)
         _lib.require_cuda()
         dev = torch.device(device)
         # the parameter format the kernels read: W^T (Cin_pad16, Cout) with zero pad rows, and the bias, per layer; allocated
@@ -77,7 +83,19 @@ class PointPath:
         wt = [torch.zeros((cin + (-cin) % 16, cout), dtype=torch.float32, device=dev) for _, cin, cout, _ in synth.HOT_LAYERS]
         bias = [torch.empty(cout, dtype=torch.float32, device=dev) for _, _, cout, _ in synth.HOT_LAYERS]
         self._init(dev, grid, (float(imsize_hw[0]), float(imsize_hw[1])), float(eps), wt, bias)
+        self.grid_dtype = grid_dtype
         self.load_state_dict(state_dict)
+
+    @property
+    def grid_dtype(self) -> torch.dtype:
+        """Element type of the dense grid every forward writes (and of `backward`'s d_grid): torch.float32 (default),
+        torch.float16 or torch.bfloat16. A 16-bit grid holds each fp32 feature rounded once to nearest-even."""
+        return self._grid_dtype
+
+    @grid_dtype.setter
+    def grid_dtype(self, dtype):
+        _lib.grid_dtype_code(dtype)      # ValueError for anything else
+        self._grid_dtype = dtype
 
     def _init(self, device, grid_spec: synth.GridSpec, imsize_hw, eps: float, wt, bias):
         """Declares every attribute; `__init__` and `_sub_context` call it."""
@@ -100,6 +118,7 @@ class PointPath:
         self.last_perm = None
         self.B = self.cap = 0
         self.grid_out = self.counts = None
+        self._grid_dtype = torch.float32
         self.layout = {}           # workspace region name -> byte offset (region())
         self._ws = self._bws = None                # forward workspace; backward scratch of a training forward
         self._ws_key = None
@@ -117,6 +136,7 @@ class PointPath:
         c = PointPath.__new__(PointPath)
         c._init(self.device, self.grid_spec, self.imsize_hw, self.eps, self.wt, self.bias)
         c.shuffle, c.shuffle_generator = self.shuffle, self.shuffle_generator
+        c.grid_dtype = self.grid_dtype
         return _Sub(c, f0, f1, stream)
 
     def load_state_dict(self, sd):
@@ -144,6 +164,8 @@ class PointPath:
         key = (B, cap, tuple(map_hw), own_outputs, train)
         self.cap, self.B = cap, B
         if self._ws_key == key:
+            if own_outputs:
+                self._alloc_outputs(B)      # re-allocates the grid when grid_dtype changed
             return
         a = _lib.PointPathArgs()
         a.grid = self.grid
@@ -176,8 +198,8 @@ class PointPath:
 
     def _alloc_outputs(self, B: int):
         nz, nx, ny = self.grid.shape[2], self.grid.shape[0], self.grid.shape[1]
-        if self.grid_out is None or self.grid_out.shape[0] != B:
-            self.grid_out = torch.empty((B, 128, nz, nx, ny), dtype=torch.float32, device=self.device)
+        if self.grid_out is None or self.grid_out.shape[0] != B or self.grid_out.dtype != self.grid_dtype:
+            self.grid_out = torch.empty((B, 128, nz, nx, ny), dtype=self.grid_dtype, device=self.device)
             self.counts = torch.empty((B, 4), dtype=torch.int32, device=self.device)
 
     def region(self, name: str, dtype, shape):
@@ -193,7 +215,7 @@ class PointPath:
                        point_calib: torch.Tensor | None = None, shuffle: bool | None = None,
                        calib64: torch.Tensor | None = None, calib_f64: torch.Tensor | None = None):
         """points (sum P, stride>=4) fp32 CUDA, offsets host [B+1], calib32 (B,32) CUDA, maps 3 x (B,256,Hf,Wf) CUDA.
-        grid_out / counts: optional caller-owned outputs ((B,128,nz,nx,ny) fp32, (B,4) int32, contiguous).
+        grid_out / counts: optional caller-owned outputs ((B,128,nz,nx,ny) of dtype `self.grid_dtype`, (B,4) int32, contiguous).
         train=True keeps every activation for `backward` (row-first fcn1; mvx_pointpath_forward_train).
         point_calib: optional (sum P) int32 CUDA — merged point sets (GT-paste, train.py:29-42): calibration set of every
         point; calib32 is then the (n_sets, 32) table it indexes.
@@ -221,6 +243,7 @@ class PointPath:
         self._prepare(B, cap, map_hw, own_outputs=counts is None, train=train)
         if counts is not None:
             assert counts.is_contiguous() and counts.shape == (B, 4) and (grid_out is None or grid_out.is_contiguous())
+            assert grid_out is None or grid_out.dtype == self.grid_dtype, (grid_out.dtype, self.grid_dtype)
             self.grid_out, self.counts = grid_out, counts
         a = _lib.PointPathArgs()
         if points.shape[0] == 0:     # all-empty batch: the kernels read no point, but the ABI wants a valid pointer
@@ -255,6 +278,7 @@ class PointPath:
             a.wt[l] = self.wt[l].data_ptr()
             a.bias[l] = self.bias[l].data_ptr()
         a.grid_out = self.grid_out.data_ptr() if want_grid else None
+        a.grid_dtype = _lib.grid_dtype_code(self.grid_dtype)
         a.counts = self.counts.data_ptr()
         a.workspace, a.workspace_bytes = self._ws.data_ptr(), self._ws.numel()
         a.stream = torch.cuda.current_stream().cuda_stream
@@ -262,7 +286,7 @@ class PointPath:
             check(lib.mvx_pointpath_forward_train(ctypes.byref(a)), 'pointpath_forward_train')
         else:
             check(lib.mvx_pointpath_forward(ctypes.byref(a)), 'pointpath_forward')
-        self._record = _Forward(a, keep, maps, train)
+        self._record = _Forward(a, keep, maps, train, grid_dtype=self.grid_dtype)
 
     # ---- the reference's own arguments: MVXNet.forward(voxels, imgs, idx, calibs, imsize) (MVXNet.py:21-27) ----------------
     def forward_voxels(self, voxels, idx, maps: List[torch.Tensor], want_grid: bool = True, train: bool = False,
@@ -295,7 +319,7 @@ class PointPath:
         map_hw = [(int(m.shape[-2]), int(m.shape[-1])) for m in maps]
         self._prepare(B, cap, map_hw, own_outputs=grid_out is None, train=train)
         if grid_out is not None:
-            assert grid_out.is_contiguous() and grid_out.dtype == torch.float32
+            assert grid_out.is_contiguous() and grid_out.dtype == self.grid_dtype, (grid_out.dtype, self.grid_dtype)
             self.grid_out = grid_out
             if self.counts is None or self.counts.shape[0] != B:
                 self.counts = torch.empty((B, 4), dtype=torch.int32, device=self.device)
@@ -401,7 +425,7 @@ class PointPath:
                  d_maps: Sequence[torch.Tensor] | None = None) -> torch.Tensor:
         """Gradients of the 8 hot-path layers for the last forward_train call, summed over its frames, as ONE flat fp32
         bucket (the message of the NCCL all-reduce; `grad_layout()` names its slices). Give dLoss/d voxel features
-        (B, cap, 128) or dLoss/d dense grid (B,128,nz,nx,ny).
+        (B, cap, 128) fp32 or dLoss/d dense grid (B,128,nz,nx,ny) in the grid dtype of that forward (ValueError otherwise).
         d_maps: three contiguous fp32 CUDA tensors shaped like the forward's FPN maps (B,256,H_l,W_l): they are overwritten
         with dLoss/d maps (the gradient an unfrozen image backbone receives; mvx_pointpath_backward_maps). None: no map
         gradient, and nothing beyond the parameter backward runs."""
@@ -414,9 +438,12 @@ class PointPath:
             grad_flat = torch.empty(n, dtype=torch.float32, device=self.device)
             accumulate = False
         assert grad_flat.is_contiguous() and grad_flat.numel() == n and grad_flat.dtype == torch.float32
-        for t, shape in ((d_vfeat, (self.B, self.cap, 128)), (d_grid, tuple(self.grid_out.shape) if self.grid_out is not None else None)):
+        if d_grid is not None and d_grid.dtype != rec.grid_dtype:
+            raise ValueError(f'd_grid must have the dtype of the grid the forward wrote ({rec.grid_dtype}), not {d_grid.dtype}')
+        for t, shape, dt in ((d_vfeat, (self.B, self.cap, 128), torch.float32),
+                             (d_grid, tuple(self.grid_out.shape) if self.grid_out is not None else None, rec.grid_dtype)):
             if t is not None:
-                assert t.is_cuda and t.is_contiguous() and t.dtype == torch.float32 and tuple(t.shape) == shape, (tuple(t.shape), shape)
+                assert t.is_cuda and t.is_contiguous() and t.dtype == dt and tuple(t.shape) == shape, (tuple(t.shape), shape)
         a.stream = torch.cuda.current_stream().cuda_stream
         check(lib.mvx_pointpath_backward(ctypes.byref(a), ptr(d_vfeat), ptr(d_grid), grad_flat.data_ptr(), int(bool(accumulate)),
                                          self._bws.data_ptr(), self._bws.numel()), 'pointpath_backward')
@@ -458,6 +485,7 @@ class PointPath:
         self.B = B
         cur = torch.cuda.current_stream()
         for s in self._split:
+            s.path.grid_dtype = self.grid_dtype
             p0, p1 = int(offsets[s.f0]), int(offsets[s.f1])
             s.stream.wait_stream(cur)
             with torch.cuda.stream(s.stream):
@@ -466,7 +494,7 @@ class PointPath:
                                       grid_out=self.grid_out[s.f0:s.f1] if want_grid else None, counts=self.counts[s.f0:s.f1])
         for s in self._split:
             cur.wait_stream(s.stream)
-        self._record = _Forward(subs=self._split)
+        self._record = _Forward(subs=self._split, grid_dtype=self.grid_dtype)
         return (self.grid_out if want_grid else None), self.counts
 
     def __call__(self, points_list: List, calibs: List[dict], fpn_maps: List, want_grid: bool = True,
@@ -557,7 +585,7 @@ class PointPath:
                     s.ev = torch.cuda.Event()
                     slot.subs.append(s)
                 nz, nx, ny = self.grid.shape[2], self.grid.shape[0], self.grid.shape[1]
-                slot.grid_out = torch.empty((B, 128, nz, nx, ny), dtype=torch.float32, device=dev) if want_grid else None
+                slot.grid_out = torch.empty((B, 128, nz, nx, ny), dtype=self.grid_dtype, device=dev) if want_grid else None
                 slot.counts = torch.empty((B, 4), dtype=torch.int32, device=dev)
                 slot.out_counts = torch.empty((B, 4), dtype=torch.int32).pin_memory()
                 slot.out_head = torch.empty((min(int(head_rows), cap), 128), dtype=torch.float32).pin_memory()
@@ -570,9 +598,9 @@ class PointPath:
             self._in_key = key
         slot = self._slots[self._host_calls % len(self._slots)]
         self._host_calls += 1
-        if want_grid and slot.grid_out is None:
+        if want_grid and (slot.grid_out is None or slot.grid_out.dtype != self.grid_dtype):
             nz, nx, ny = self.grid.shape[2], self.grid.shape[0], self.grid.shape[1]
-            slot.grid_out = torch.empty((B, 128, nz, nx, ny), dtype=torch.float32, device=dev)
+            slot.grid_out = torch.empty((B, 128, nz, nx, ny), dtype=self.grid_dtype, device=dev)
         self._h2d_bytes = (points_host.numel() + calib32_host.numel() + sum(m.numel() for m in maps_host if not m.is_cuda)) * 4
         self.B, self.grid_out, self.counts = B, slot.grid_out, slot.counts
         cur = torch.cuda.current_stream()
@@ -596,6 +624,7 @@ class PointPath:
             ks = self._compute_streams[j % ns]
             if j < ns:
                 ks.wait_stream(cur)              # work the caller queued before this call (weight updates ...) is ordered first
+            s.path.grid_dtype = self.grid_dtype
             with torch.cuda.stream(ks):
                 ks.wait_event(s.ev)
                 sub_maps = [d if d is not None else h[s.f0:s.f1] for d, h in zip(s.in_maps, maps_host)]   # device-resident maps: a view
@@ -612,7 +641,7 @@ class PointPath:
             slot.done.record(k0)
         slot.used = True
         cur.wait_event(slot.done)                # later work on the caller's stream sees this call's device outputs
-        self._record = _Forward(subs=slot.subs)
+        self._record = _Forward(subs=slot.subs, grid_dtype=self.grid_dtype)
         self._d2h_bytes = slot.out_counts.numel() * 4 + slot.out_head.numel() * 4
         step = HostStep(slot)
         return step.wait() if sync else step
